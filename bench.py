@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the img_completion hot path (BASELINE.json metric: frames/s at 1216x352).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload lidar_only|guided|stereo]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload lidar_only|guided|stereo] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A step is one pass of the hot path over one batch of synthetic frames (default: BASELINE configs[1],
@@ -63,7 +63,15 @@ def parse_args():
     ap.add_argument("--host-multi", action="store_true", help="single process: also time dcmt_img_completion_u16_host_multi over all visible GPUs")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ref-frames-per-core", type=int, default=16, help="reference arm: frames per host core per step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="--impl ours: after the timed steps, write the output of the last one as DIR/<name>.npy (float32, at most "
+                         "64 MB: a fixed, seeded sample of frames when the batch is larger)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":  # the reference arm's workers hand back one pixel per frame, not the frames
+        ap.error("--dump-outputs needs --impl ours: the reference arm keeps only out[0, 0] of each frame it times")
+    return args
 
 
 # --------------------------------------------------------------------------- reference (CPU) arm
@@ -354,6 +362,34 @@ def ncu_traffic(workload):
         return None
 
 
+DUMP_BYTES = 60 * 10**6  # payload of --dump-outputs: below 64 MB with the .npy header
+DUMP_SEED = 0
+
+
+def dump_outputs(directory, name, out):
+    """Write `out` (frames first) as directory/name.npy in float32.  When the whole batch is over DUMP_BYTES, a seeded
+    sample of whole frames in frame order (of single elements when one frame is already over it): the same arguments pick
+    the same sample, so that two builds of the project can be compared output for output."""
+    import numpy as np
+    import torch
+
+    os.makedirs(directory, exist_ok=True)
+    n, frame_elems = out.shape[0], out[0].numel()
+    keep = DUMP_BYTES // (4 * frame_elems)
+    rng = np.random.default_rng(DUMP_SEED)
+    if keep >= n:
+        sample, what = out, f"all {n} frames"
+    elif keep >= 1:
+        idx = np.sort(rng.choice(n, keep, replace=False))
+        sample, what = out[torch.from_numpy(idx).to(out.device)], f"frames {idx.tolist()} of {n}"
+    else:
+        idx = np.sort(rng.choice(out.numel(), DUMP_BYTES // 4, replace=False))
+        sample, what = out.reshape(-1)[torch.from_numpy(idx).to(out.device)], f"{idx.size} seeded elements of {out.numel()}"
+    path = os.path.join(directory, name + ".npy")
+    np.save(path, sample.to(torch.float32).cpu().numpy())
+    print(f"--dump-outputs: {path} = {what}", file=sys.stderr)
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -485,6 +521,8 @@ def run_ours(args):
 
     # ---- validation payload: checksums of the unique outputs (+ digests vs the committed golden file)
     out_t = d_out if args.workload == "lidar_only" else holder["out"]
+    if args.dump_outputs and rank == 0:  # every rank computes the same frames
+        dump_outputs(args.dump_outputs, "depth", out_t)
     sums = sharding.frame_checksums(out_t[: min(n, UNIQUE)])
     replicas_equal = all(bool(torch.equal(out_t[UNIQUE * k_:UNIQUE * (k_ + 1)], out_t[:UNIQUE][: max(0, min(UNIQUE, n - UNIQUE * k_))]))
                          for k_ in range(1, reps) if n - UNIQUE * k_ > 0)

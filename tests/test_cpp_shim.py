@@ -11,6 +11,7 @@ import pytest
 
 from depth_completion_mt_b200 import build, synth
 from oracle import c_oracle as co
+from oracle import ref_oracle as ro
 from tests.conftest import ROOT, assert_bit_equal
 
 
@@ -77,7 +78,7 @@ def test_shim_with_product_library_on_gpu(tmp_path, gpu_lib):
 # way the reference writes them.  Checked against the C restatement and -- where the prebuilt oracle/_ref travelled --
 # against the reference's own compiled sources.
 REFSHIM = os.path.join(ROOT, "oracle", "refshim")
-REF_SLIC_DIR = "/root/reference/src/DC_lidar_camera"
+REF_SLIC_DIR = os.path.join(ro._REF, "src", "DC_lidar_camera")  # the reference checkout ref_oracle builds from (DCMT_REFERENCE_DIR)
 
 
 def compile_cv_shim(tmp_path, lib_path, reference_slic_h=False):
