@@ -80,6 +80,8 @@ _SIGNATURES = {
     "dcmt_slic_center_count": (C.c_int, [C.c_int, C.c_int, C.c_int]),
     "dcmt_slic_u8c3": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P]),
     "dcmt_slic_u8c3_host": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
+    "dcmt_slic_bgr_u8c3": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P]),
+    "dcmt_slic_bgr_u8c3_host": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
     "dcmt_img_completion_f32_host_multi": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int]),
     "dcmt_img_completion_u16_host_multi": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int]),
     "dcmt_interpolate_with_superpixels_f32_host_multi": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int]),
@@ -87,6 +89,8 @@ _SIGNATURES = {
     "dcmt_debug_host_copy_u16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, C.c_int]),
     "dcmt_bgr2gray_u8": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, _P]),
     "dcmt_bgr2gray_u8_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int]),
+    "dcmt_bgr2lab_u8": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, _P]),
+    "dcmt_bgr2lab_u8_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int]),
     "dcmt_entries_measurement_derivatives": (C.c_int, [_P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, _P]),
     "dcmt_entries_measurement_derivatives_host": (C.c_int, [_P, C.c_int, C.c_int, C.c_size_t, C.c_size_t]),
     "dcmt_entries_optimize_ig": (C.c_int, [_P, C.c_size_t, _P, C.c_size_t, C.c_size_t, _P, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, _P]),

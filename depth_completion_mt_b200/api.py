@@ -440,6 +440,27 @@ def bgr2gray(bgr, *, stream=None, lib: _lib.Library | None = None):
     return out[0] if squeeze else out
 
 
+def bgr2lab(bgr, *, stream=None, lib: _lib.Library | None = None):
+    """cv::cvtColor(img, lab, COLOR_BGR2Lab) (main_lc.cpp:182-183, main_sl.cpp:438): (rows, cols, 3) or (n, rows, cols, 3)
+    uint8 BGR -> uint8 Lab of the same shape, bit-equal to OpenCV's 8-bit conversion."""
+    lib = lib or _lib.load()
+    is_t = _is_torch(bgr)
+    x = _prep_torch(bgr, torch.uint8, "bgr") if is_t else _prep_numpy(bgr, np.uint8, "bgr")
+    if x.ndim not in (3, 4) or x.shape[-1] != 3:
+        raise ValueError("bgr must be (rows, cols, 3) or (n, rows, cols, 3)")
+    squeeze = x.ndim == 3
+    x4 = x[None] if squeeze else x
+    n, rows, cols = int(x4.shape[0]), int(x4.shape[1]), int(x4.shape[2])
+    if is_t:
+        out = torch.empty((n, rows, cols, 3), dtype=torch.uint8, device=x.device)
+        with torch.cuda.device(x.device):
+            lib.check(lib.dcmt_bgr2lab_u8(x4.data_ptr(), out.data_ptr(), rows, cols, 0, 0, n, _stream_ptr(stream)))
+    else:
+        out = np.empty((n, rows, cols, 3), np.uint8)
+        lib.check(lib.dcmt_bgr2lab_u8_host(_np_ptr(x4), _np_ptr(out), rows, cols, 0, 0, n))
+    return out[0] if squeeze else out
+
+
 def lidar_project_batch(points, counts, T, P, rows: int, cols: int, norm=(0.0, 80.0), *, stream=None, lib: _lib.Library | None = None):
     """main_sl.cpp:478-523 for a batch of clouds in four launches.  ``points``: CUDA tensor (n_clouds, max_points, 4) float32;
     ``counts``: CUDA int32 (n_clouds,) points per cloud, or None (max_points each).  Returns (projected, normalized, n_projected):
@@ -471,26 +492,41 @@ def generate_superpixels(lab_image, step, nc: int, *, iterations: int = 10, retu
     like the reference's int parameter (main_lc.cpp:197-201 passes a double).  Returns the label map ``Slic::clusters`` as
     int32 [row][col] (-1 = never assigned) and, optionally, ``Slic::centers`` (K, 5) float64 (with a leading batch
     dimension for a batch).  ``K = len(centers)`` is the ``n_clusters`` argument of interpolate_with_superpixels."""
+    return _superpixels("dcmt_slic_u8c3", lab_image, "lab_image", step, nc, iterations, return_centers, stream, lib)
+
+
+def generate_superpixels_bgr(bgr_image, step, nc: int, *, iterations: int = 10, return_centers: bool = False, stream=None,
+                             lib: _lib.Library | None = None):
+    """cv::cvtColor(img, lab, COLOR_BGR2Lab) followed by Slic::generate_superpixels(lab, step, nc) (main_lc.cpp:182-201,
+    main_sl.cpp:438-450) in one call: ``bgr_image`` is the uint8 colour image as read, (rows, cols, 3) or
+    (n, rows, cols, 3).  The Lab image stays on the device.  Returns what generate_superpixels returns for
+    ``bgr2lab(bgr_image)``."""
+    return _superpixels("dcmt_slic_bgr_u8c3", bgr_image, "bgr_image", step, nc, iterations, return_centers, stream, lib)
+
+
+def _superpixels(entry: str, image, what: str, step, nc, iterations, return_centers, stream, lib):
+    """SLIC through the C entry point ``entry`` (device) / ``entry + '_host'`` on a CV_8UC3 image or batch."""
     lib = lib or _lib.load()
     step = int(step)
-    is_t = _is_torch(lab_image)
-    lab = _prep_torch(lab_image, torch.uint8, "lab_image") if is_t else _prep_numpy(lab_image, np.uint8, "lab_image")
-    if lab.ndim not in (3, 4) or lab.shape[-1] != 3:
-        raise ValueError("lab_image must be (rows, cols, 3) or (n, rows, cols, 3)")
-    squeeze = lab.ndim == 3
-    n = 1 if squeeze else int(lab.shape[0])
-    rows, cols = int(lab.shape[-3]), int(lab.shape[-2])
+    is_t = _is_torch(image)
+    img = _prep_torch(image, torch.uint8, what) if is_t else _prep_numpy(image, np.uint8, what)
+    if img.ndim not in (3, 4) or img.shape[-1] != 3:
+        raise ValueError(f"{what} must be (rows, cols, 3) or (n, rows, cols, 3)")
+    squeeze = img.ndim == 3
+    n = 1 if squeeze else int(img.shape[0])
+    rows, cols = int(img.shape[-3]), int(img.shape[-2])
     k = lib.dcmt_slic_center_count(rows, cols, step)
     if is_t:
-        labels = torch.empty((n, rows, cols), dtype=torch.int32, device=lab.device)
-        centers = torch.empty((n, max(k, 1), 5), dtype=torch.float64, device=lab.device)
-        with torch.cuda.device(lab.device):
-            lib.check(lib.dcmt_slic_u8c3(lab.data_ptr(), rows, cols, n, step, int(nc), int(iterations), labels.data_ptr(),
-                                         centers.data_ptr(), _stream_ptr(stream)))
+        labels = torch.empty((n, rows, cols), dtype=torch.int32, device=img.device)
+        centers = torch.empty((n, max(k, 1), 5), dtype=torch.float64, device=img.device)
+        with torch.cuda.device(img.device):
+            lib.check(getattr(lib, entry)(img.data_ptr(), rows, cols, n, step, int(nc), int(iterations), labels.data_ptr(),
+                                          centers.data_ptr(), _stream_ptr(stream)))
     else:
         labels = np.empty((n, rows, cols), np.int32)
         centers = np.empty((n, max(k, 1), 5), np.float64)
-        lib.check(lib.dcmt_slic_u8c3_host(_np_ptr(lab), rows, cols, n, step, int(nc), int(iterations), _np_ptr(labels), _np_ptr(centers)))
+        lib.check(getattr(lib, entry + "_host")(_np_ptr(img), rows, cols, n, step, int(nc), int(iterations), _np_ptr(labels),
+                                                _np_ptr(centers)))
     centers = centers[:, :k]
     if squeeze:
         labels, centers = labels[0], centers[0]

@@ -17,6 +17,7 @@
 #include "generic.cuh"
 #include "project.cuh"
 #include "rank_f32.cuh"
+#include "color.cuh"
 #include "slic.cuh"
 #include "stereo.cuh"
 
@@ -1108,9 +1109,11 @@ int dcmt_slic_center_count(int rows, int cols, int step) {
     return dcmt::slic_center_count(rows, cols, step);
 }
 
-int dcmt_slic_u8c3(const uint8_t* lab, int rows, int cols, int n_frames, int step, int nc, int iterations, int32_t* labels,
-                   double* centers, void* cuda_stream) {
-    if (!lab || !labels) return fail(DCMT_E_BADARG, "null pointer");
+// Slic::generate_superpixels on the Lab image `img`, or, with from_bgr, on the cvtColor(COLOR_BGR2Lab) of the BGR image
+// `img`: the Lab frames then live in the SLIC workspace of (device, stream) and never leave the device
+static int slic_device(const uint8_t* img, bool from_bgr, int rows, int cols, int n_frames, int step, int nc, int iterations,
+                       int32_t* labels, double* centers, void* cuda_stream) {
+    if (!img || !labels) return fail(DCMT_E_BADARG, "null pointer");
     int rc = check_planes(rows, cols, n_frames);
     if (rc) return rc;
     if (nc == 0 || iterations < 0) return fail(DCMT_E_BADARG, "nc %d, iterations %d", nc, iterations);
@@ -1127,7 +1130,8 @@ int dcmt_slic_u8c3(const uint8_t* lab, int rows, int cols, int n_frames, int ste
     const size_t kk = (k > 0 ? (size_t)k : 1) * n_frames, nb = nbins * n_frames;
     Arena* ar = nullptr;
     if ((rc = arena_acquire(st, 2 * carve_bytes(kk * 5, sizeof(double)) + carve_bytes(kk * 6, sizeof(unsigned long long)) +
-                                    carve_bytes(nb + n_frames, sizeof(int)) + carve_bytes(nb, sizeof(int)) + carve_bytes(kk, sizeof(int)),
+                                    carve_bytes(nb + n_frames, sizeof(int)) + carve_bytes(nb, sizeof(int)) + carve_bytes(kk, sizeof(int)) +
+                                    (from_bgr ? carve_bytes((size_t)rows * cols * 3 * n_frames, 1) : 0),
                             &ar)))
         return rc;
     w.centers = carve<double>(ar, kk * 5);
@@ -1136,16 +1140,31 @@ int dcmt_slic_u8c3(const uint8_t* lab, int rows, int cols, int n_frames, int ste
     w.bin_fill = carve<int>(ar, nb);
     w.bin_items = carve<int>(ar, kk);
     w.sorted = carve<double>(ar, kk * 5);
+    uint8_t* lab = from_bgr ? carve<uint8_t>(ar, (size_t)rows * cols * 3 * n_frames) : nullptr;
     if ((rc = arena_ok(ar))) return rc;
-    API_CUDA(dcmt::slic_run(lab, rows, cols, n_frames, step, nc, iterations, labels, k, w, st), "SLIC launch");
+    if (from_bgr) {
+        const size_t pitch = (size_t)cols * 3;
+        API_CUDA(dcmt::color_bgr2lab(img, pitch, pitch * rows, lab, pitch, pitch * rows, rows, cols, n_frames, st), "BGR2Lab launch");
+    }
+    API_CUDA(dcmt::slic_run(from_bgr ? lab : img, rows, cols, n_frames, step, nc, iterations, labels, k, w, st), "SLIC launch");
     if (centers && k > 0)
         API_CUDA(cudaMemcpyAsync(centers, w.centers, (size_t)k * n_frames * 5 * sizeof(double), cudaMemcpyDeviceToDevice, st), "centre copy");
     return DCMT_OK;
 }
 
-int dcmt_slic_u8c3_host(const uint8_t* lab, int rows, int cols, int n_frames, int step, int nc, int iterations, int32_t* labels,
-                        double* centers) {
-    if (!lab || !labels) return fail(DCMT_E_BADARG, "null pointer");
+int dcmt_slic_u8c3(const uint8_t* lab, int rows, int cols, int n_frames, int step, int nc, int iterations, int32_t* labels,
+                   double* centers, void* cuda_stream) {
+    return slic_device(lab, false, rows, cols, n_frames, step, nc, iterations, labels, centers, cuda_stream);
+}
+
+int dcmt_slic_bgr_u8c3(const uint8_t* bgr, int rows, int cols, int n_frames, int step, int nc, int iterations, int32_t* labels,
+                       double* centers, void* cuda_stream) {
+    return slic_device(bgr, true, rows, cols, n_frames, step, nc, iterations, labels, centers, cuda_stream);
+}
+
+static int slic_host(const uint8_t* img, bool from_bgr, int rows, int cols, int n_frames, int step, int nc, int iterations,
+                     int32_t* labels, double* centers) {
+    if (!img || !labels) return fail(DCMT_E_BADARG, "null pointer");
     int rc = check_planes(rows, cols, n_frames);
     if (rc) return rc;
     if (n_frames == 0) return DCMT_OK;
@@ -1161,16 +1180,26 @@ int dcmt_slic_u8c3_host(const uint8_t* lab, int rows, int cols, int n_frames, in
         cudaStream_t st2 = call.lanes[0].hs->s[1];
         if ((rc = arena_acquire(st2, carve_bytes(n * 3, 1) + carve_bytes(n, 4) + carve_bytes((k > 0 ? k : 1) * 5, sizeof(double)), &stage))) return rc;
     }
-    uint8_t* d_lab = carve<uint8_t>(stage, n * 3);
+    uint8_t* d_img = carve<uint8_t>(stage, n * 3);
     int32_t* d_labels = carve<int32_t>(stage, n);
     double* d_centers = carve<double>(stage, (k > 0 ? k : 1) * 5);
     if ((rc = arena_ok(stage))) return rc;
     call.use(call.lanes[0]);
-    API_CUDA(cudaMemcpyAsync(d_lab, lab, n * 3, cudaMemcpyHostToDevice, st), "host to device copy");
-    if ((rc = dcmt_slic_u8c3(d_lab, rows, cols, n_frames, step, nc, iterations, d_labels, centers ? d_centers : nullptr, st))) return rc;
+    API_CUDA(cudaMemcpyAsync(d_img, img, n * 3, cudaMemcpyHostToDevice, st), "host to device copy");
+    if ((rc = slic_device(d_img, from_bgr, rows, cols, n_frames, step, nc, iterations, d_labels, centers ? d_centers : nullptr, st))) return rc;
     API_CUDA(cudaMemcpyAsync(labels, d_labels, n * 4, cudaMemcpyDeviceToHost, st), "device to host copy");
     if (centers && k > 0) API_CUDA(cudaMemcpyAsync(centers, d_centers, k * 5 * sizeof(double), cudaMemcpyDeviceToHost, st), "device to host copy");
     return call.finish();
+}
+
+int dcmt_slic_u8c3_host(const uint8_t* lab, int rows, int cols, int n_frames, int step, int nc, int iterations, int32_t* labels,
+                        double* centers) {
+    return slic_host(lab, false, rows, cols, n_frames, step, nc, iterations, labels, centers);
+}
+
+int dcmt_slic_bgr_u8c3_host(const uint8_t* bgr, int rows, int cols, int n_frames, int step, int nc, int iterations, int32_t* labels,
+                            double* centers) {
+    return slic_host(bgr, true, rows, cols, n_frames, step, nc, iterations, labels, centers);
 }
 
 int dcmt_lidar_project_f32(const float* points, int n_points, const float* T_host, const float* P_host, int rows, int cols,
@@ -1466,6 +1495,57 @@ int dcmt_bgr2gray_u8_host(const uint8_t* bgr, uint8_t* gray, int rows, int cols,
     API_CUDA(cudaMemcpy2DAsync(d_in, in_row, bgr, bgr_pitch_bytes, in_row, frames_rows, cudaMemcpyHostToDevice, st), "host to device copy");
     if ((rc = dcmt_bgr2gray_u8(d_in, d_out, rows, cols, 0, 0, n_frames, st))) return rc;
     API_CUDA(cudaMemcpy2DAsync(gray, gray_pitch_bytes, d_out, cols, cols, frames_rows, cudaMemcpyDeviceToHost, st), "device to host copy");
+    return call.finish();
+}
+
+// ---- cv::cvtColor(COLOR_BGR2Lab) in front of Slic::generate_superpixels (main_lc.cpp:182-184, main_sl.cpp:438) ----
+static int check_lab(const uint8_t* bgr, const uint8_t* lab, int rows, int cols, size_t* bgr_pitch, size_t* lab_pitch, int n_frames) {
+    if (!bgr || !lab) return fail(DCMT_E_BADARG, "null pointer");
+    int rc = check_planes(rows, cols, n_frames);
+    if (rc) return rc;
+    if (n_frames > 65535) return fail(DCMT_E_UNSUPPORTED, "at most 65535 frames");
+    if ((size_t)rows * (size_t)cols >= (size_t)1 << 31) return fail(DCMT_E_UNSUPPORTED, "frame of 2^31 pixels or more");
+    const size_t row = (size_t)cols * 3;
+    if (*bgr_pitch == 0) *bgr_pitch = row;
+    if (*lab_pitch == 0) *lab_pitch = row;
+    if (*bgr_pitch < row || *lab_pitch < row) return fail(DCMT_E_BADARG, "pitch too small");
+    if (n_frames == 0) return DCMT_OK;
+    // the byte ranges the call reads and writes must not overlap (no aliasing, dcmt.h)
+    const size_t last = (size_t)rows * n_frames - 1;
+    const uintptr_t in = reinterpret_cast<uintptr_t>(bgr), out = reinterpret_cast<uintptr_t>(lab);
+    if (in < out + *lab_pitch * last + row && out < in + *bgr_pitch * last + row) return fail(DCMT_E_BADARG, "input and output overlap");
+    return DCMT_OK;
+}
+
+int dcmt_bgr2lab_u8(const uint8_t* bgr, uint8_t* lab, int rows, int cols, size_t bgr_pitch_bytes, size_t lab_pitch_bytes, int n_frames,
+                    void* cuda_stream) {
+    int rc = check_lab(bgr, lab, rows, cols, &bgr_pitch_bytes, &lab_pitch_bytes, n_frames);
+    if (rc) return rc;
+    if (n_frames == 0) return DCMT_OK;
+    if ((rc = check_device())) return rc;
+    API_CUDA(dcmt::color_bgr2lab(bgr, bgr_pitch_bytes, bgr_pitch_bytes * rows, lab, lab_pitch_bytes, lab_pitch_bytes * rows, rows, cols,
+                                 n_frames, static_cast<cudaStream_t>(cuda_stream)),
+             "BGR2Lab launch");
+    return DCMT_OK;
+}
+
+int dcmt_bgr2lab_u8_host(const uint8_t* bgr, uint8_t* lab, int rows, int cols, size_t bgr_pitch_bytes, size_t lab_pitch_bytes, int n_frames) {
+    int rc = check_lab(bgr, lab, rows, cols, &bgr_pitch_bytes, &lab_pitch_bytes, n_frames);
+    if (rc) return rc;
+    if (n_frames == 0) return DCMT_OK;
+    HostCall call;
+    if ((rc = call.open(nullptr, 0, false))) return rc;
+    cudaStream_t st = call.lanes[0].hs->s[0];
+    const size_t row = (size_t)cols * 3, frames_rows = (size_t)rows * n_frames;
+    Arena* ar = nullptr;
+    if ((rc = arena_acquire(st, 2 * carve_bytes(row * frames_rows, 1), &ar))) return rc;
+    uint8_t* d_in = carve<uint8_t>(ar, row * frames_rows);
+    uint8_t* d_out = carve<uint8_t>(ar, row * frames_rows);
+    if ((rc = arena_ok(ar))) return rc;
+    call.use(call.lanes[0]);
+    API_CUDA(cudaMemcpy2DAsync(d_in, row, bgr, bgr_pitch_bytes, row, frames_rows, cudaMemcpyHostToDevice, st), "host to device copy");
+    if ((rc = dcmt_bgr2lab_u8(d_in, d_out, rows, cols, 0, 0, n_frames, st))) return rc;
+    API_CUDA(cudaMemcpy2DAsync(lab, lab_pitch_bytes, d_out, row, row, frames_rows, cudaMemcpyDeviceToHost, st), "device to host copy");
     return call.finish();
 }
 

@@ -126,3 +126,20 @@ def lab_image(frame: int, rows: int = KITTI_ROWS, cols: int = KITTI_COLS) -> np.
         base = 128 + 60 * np.sin(f[0] * xx + ph[0]) * np.cos(f[1] * yy + ph[1]) + 30 * np.sign(np.sin(f[2] * xx + f[3] * yy + ph[2]))
         img[:, :, c] = base + rng.normal(0, 4, (rows, cols))
     return np.clip(np.rint(img), 0, 255).astype(np.uint8)
+
+
+def bgr_image(frame: int, rows: int = KITTI_ROWS, cols: int = KITTI_COLS) -> np.ndarray:
+    """Synthetic CV_8UC3 BGR camera frame (what cv::imread hands to cv::cvtColor(COLOR_BGR2Lab), main_lc.cpp:182-184):
+    a few smooth colour regions split by straight edges, with a shading gradient and sensor noise."""
+    rng = np.random.default_rng(BASE_SEED + 700001 + frame)
+    yy, xx = np.mgrid[0:rows, 0:cols].astype(np.float64)
+    img = np.zeros((rows, cols, 3), np.float64)
+    region = np.zeros((rows, cols), np.int64)
+    for bit in range(3):  # three random half-planes: up to 8 regions with straight edges
+        t = rng.uniform(0, np.pi)
+        region |= ((np.cos(t) * (xx - rng.uniform(0, cols)) + np.sin(t) * (yy - rng.uniform(0, rows))) > 0).astype(np.int64) << bit
+    colours = rng.uniform(20, 235, (8, 3))
+    img[:] = colours[region]
+    shade = 0.75 + 0.25 * np.sin(rng.uniform(0.002, 0.01) * xx + rng.uniform(0, 6.28)) * np.cos(rng.uniform(0.002, 0.01) * yy)
+    img = img * shade[:, :, None] + rng.normal(0, 3, (rows, cols, 3))
+    return np.clip(np.rint(img), 0, 255).astype(np.uint8)

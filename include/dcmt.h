@@ -244,6 +244,16 @@ DCMT_API int dcmt_bgr2gray_u8(const uint8_t *bgr, uint8_t *gray, int rows, int c
 DCMT_API int dcmt_bgr2gray_u8_host(const uint8_t *bgr, uint8_t *gray, int rows, int cols, size_t bgr_pitch_bytes,
                                    size_t gray_pitch_bytes, int n_frames);
 
+/* cv::cvtColor(img, lab, COLOR_BGR2Lab) on CV_8UC3 images, the conversion in front of Slic::generate_superpixels
+ * (main_lc.cpp:182-183; main_sl.cpp:438 in withSuperPixels): OpenCV's 8-bit path -- sRGB gamma and the Lab cube root by
+ * table, XYZ and L, a, b in fixed point -- bit-equal to OpenCV 4.13 for all 2^24 colours.  CV_8UC3 Lab out (L * 255 / 100,
+ * a + 128, b + 128).  n_frames images follow each other at rows * pitch; pitches in bytes (0 = dense: cols * 3).
+ * Input and output byte ranges that overlap are DCMT_E_BADARG. */
+DCMT_API int dcmt_bgr2lab_u8(const uint8_t *bgr, uint8_t *lab, int rows, int cols, size_t bgr_pitch_bytes,
+                             size_t lab_pitch_bytes, int n_frames, void *cuda_stream);
+DCMT_API int dcmt_bgr2lab_u8_host(const uint8_t *bgr, uint8_t *lab, int rows, int cols, size_t bgr_pitch_bytes,
+                                  size_t lab_pitch_bytes, int n_frames);
+
 /* (a3) the same four functions on the reference's OWN containers, so that its call sites (main_sl.cpp:1192-1246) need no
  * change of data layout:
  *   - EntryType matrices (main_sl.cpp:23-26: struct { float value; Eigen::Vector2f derivative; }, 12 bytes) as
@@ -346,6 +356,15 @@ DCMT_API int dcmt_slic_u8c3(const uint8_t *lab, int rows, int cols, int n_frames
                             int32_t *labels, double *centers_or_null, void *cuda_stream);
 DCMT_API int dcmt_slic_u8c3_host(const uint8_t *lab, int rows, int cols, int n_frames, int step, int nc, int iterations,
                                  int32_t *labels, double *centers_or_null);
+/* the pair cv::cvtColor(img, lab, COLOR_BGR2Lab) + slic.generate_superpixels(lab, step, nc) in one call, from the
+ * CV_8UC3 BGR image as read (main_lc.cpp:182-201; main_sl.cpp:438-450 with 100 superpixels and nc = 40): the Lab
+ * frames are made by dcmt_bgr2lab_u8 inside the workspace of (device, stream) and segmented as by dcmt_slic_u8c3, so
+ * labels and centres equal dcmt_slic_u8c3 on OpenCV's Lab.  Arguments as for dcmt_slic_u8c3 with `bgr` (contiguous,
+ * n_frames x rows x cols x 3) in place of `lab`; a host caller moves 3 bytes per pixel in and the labels out. */
+DCMT_API int dcmt_slic_bgr_u8c3(const uint8_t *bgr, int rows, int cols, int n_frames, int step, int nc, int iterations,
+                                int32_t *labels, double *centers_or_null, void *cuda_stream);
+DCMT_API int dcmt_slic_bgr_u8c3_host(const uint8_t *bgr, int rows, int cols, int n_frames, int step, int nc, int iterations,
+                                     int32_t *labels, double *centers_or_null);
 
 /* debugging aid: runs the generic pipeline on ONE frame and snapshots intermediate images
  * (device memory, n_stages * rows * cols floats, stage order of oracle/dcmt_oracle.c; stages the

@@ -209,6 +209,13 @@ inline void bgr2gray(const MatView& bgr, MatView& gray) {
     check(dcmt_bgr2gray_u8_host(static_cast<const uint8_t*>(bgr.data), static_cast<uint8_t*>(gray.data), bgr.rows, bgr.cols, bgr.step, gray.step, 1));
 }
 
+// cv::cvtColor(img, lab, cv::COLOR_BGR2Lab) (main_lc.cpp:182-183, main_sl.cpp:438) on CV_8UC3 views: OpenCV's 8-bit
+// conversion, the input of Slic::generate_superpixels (dcmt_slic_bgr_u8c3_host does both in one call)
+inline void bgr2lab(const MatView& bgr, MatView& lab) {
+    if (bgr.rows != lab.rows || bgr.cols != lab.cols || !bgr.data || !lab.data) throw std::invalid_argument("dcmt: bgr2lab needs same-shaped Mats");
+    check(dcmt_bgr2lab_u8_host(static_cast<const uint8_t*>(bgr.data), static_cast<uint8_t*>(lab.data), bgr.rows, bgr.cols, bgr.step, lab.step, 1));
+}
+
 // main_sl.cpp:1165-1253 in one call: gray images (CV_8UC1 views) + initial dense depth -> refined depth
 inline void stereo_refine(const MatView& depth_ig, const MatView& left_gray, const MatView& right_gray, MatView& depth_out,
                           const dcmt_stereo_params* params = nullptr) {

@@ -1,6 +1,7 @@
 #!/usr/bin/env python
-"""Throughput of the SURVEY.md 8(f) rows (SLIC, LiDAR projection, evaluation) at 352x1216 on one GPU, next to the C
-oracle (the literal CPU loops, one core) on the same inputs.  One JSON line per row.
+"""Throughput of the SURVEY.md 8(f) rows (SLIC, LiDAR projection, evaluation) and of cvtColor(BGR2Lab) at 352x1216 on
+one GPU, next to the C oracle (the literal CPU loops, one core) or single-threaded cv2 on the same inputs.  One JSON line
+per row; the first line names the GPU and its power limit.
 
     python tools/bench_rows.py [--reps 20]
 """
@@ -9,6 +10,7 @@ from __future__ import annotations
 import argparse
 import json
 import os
+import subprocess
 import sys
 import time
 
@@ -49,8 +51,31 @@ def main():
     a = ap.parse_args()
     lib = _lib.load()
     rows, cols = 352, 1216
-    peak = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))["hbm_gbs"]
-    out = []
+    peaks = os.path.join(ROOT, "MEASURED_PEAKS.json")
+    peak = json.load(open(peaks))["hbm_gbs"] if os.path.exists(peaks) else 6558.7  # measured B200 HBM peak (SURVEY.md)
+    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader", "-i",
+                          str(torch.cuda.current_device())], capture_output=True, text=True)
+    out = [{"gpu": torch.cuda.get_device_name(), "nvidia_smi": smi.stdout.strip() or smi.stderr.strip(), "hbm_peak_GBps": peak}]
+    # ---- cvtColor(COLOR_BGR2Lab): 1024 device-resident frames (1.3 GB in, 1.3 GB out: well above the 126 MB L2), 6 B/px
+    nl = 1024
+    bgr = torch.from_numpy(np.stack([synth.bgr_image(f, rows, cols) for f in range(8)])).cuda().repeat(nl // 8, 1, 1, 1).contiguous()
+    labo = torch.empty_like(bgr)
+
+    def convert(src, dst, n):
+        lib.check(lib.dcmt_bgr2lab_u8(src.data_ptr(), dst.data_ptr(), rows, cols, 0, 0, n, torch.cuda.current_stream().cuda_stream))
+    ms = gpu_time(lambda: convert(bgr, labo, nl), a.reps)
+    ms1 = gpu_time(lambda: convert(bgr, labo, 1), 10 * a.reps)
+    import cv2
+
+    cv2.setNumThreads(1)
+    b0 = bgr[0].cpu().numpy()
+    cms = cpu_time(lambda: cv2.cvtColor(b0, cv2.COLOR_BGR2Lab), reps=20)
+    byt = 6 * rows * cols * nl
+    out.append({"row": "cvtColor(BGR2Lab) (main_lc.cpp:182-183), batch of 1024 frames (dcmt_bgr2lab_u8)", "frames": nl, "ms": ms,
+                "frames_per_s": nl / ms * 1e3, "ms_per_frame": ms / nl, "achieved_GBps": byt / ms / 1e6, "frac_of_hbm_peak": byt / ms / 1e6 / peak,
+                "single_frame_call_ms": ms1, "cv2_1thread_ms_per_frame": cms, "cv2_version": cv2.__version__,
+                "note": "6 algorithmic B/px (3 in, 3 out); single_frame_call_ms: one frame per call, L2-resident"})
+    del labo
     # ---- evaluation: batch of 256 frames, 8 B/px
     n = 256
     gt = torch.from_numpy(np.stack([synth.sparse_depth(f, rows, cols, 0.3) for f in range(8)])).cuda().repeat(n // 8, 1, 1).contiguous()
@@ -108,6 +133,27 @@ def main():
         return api.evaluate(sparse64, d, "lidar_camera", lib=lib)
     ms = gpu_time(chain64, 3)
     out.append({"row": "DC_lidar_camera chain, batch of 64 frames", "ms": ms, "frames_per_s": 64e3 / ms})
+    # ---- the same front from the BGR frame as read: cvtColor(BGR2Lab) -> SLIC -> guided completion -> evaluation
+    # (main_lc.cpp:182-225), the conversion inside dcmt_slic_bgr_u8c3; next to the Lab-in chain on the same batches
+    for nf in (64, 256):
+        bgrs = bgr[:nf].contiguous()
+        labs_n = api.bgr2lab(bgrs, lib=lib)
+        sp = sparse64.repeat(nf // 64, 1, 1).contiguous()
+
+        def chain_bgr():
+            labels = api.generate_superpixels_bgr(bgrs, 18, 50, lib=lib)
+            d = api.interpolate_with_superpixels(labels, sp, "gaussian", 1, n_clusters=k, lib=lib)
+            return api.evaluate(sp, d, "lidar_camera", lib=lib)
+
+        def chain_lab():
+            labels = api.generate_superpixels(labs_n, 18, 50, lib=lib)
+            d = api.interpolate_with_superpixels(labels, sp, "gaussian", 1, n_clusters=k, lib=lib)
+            return api.evaluate(sp, d, "lidar_camera", lib=lib)
+        ms_lab = gpu_time(chain_lab, 3)
+        ms_bgr = gpu_time(chain_bgr, 3)
+        out.append({"row": f"DC_lidar_camera chain from BGR: BGR2Lab -> SLIC -> interpolate_with_superpixels -> evaluate, batch of {nf} frames",
+                    "ms": ms_bgr, "frames_per_s": nf * 1e3 / ms_bgr, "lab_in_chain_ms": ms_lab, "lab_in_chain_frames_per_s": nf * 1e3 / ms_lab,
+                    "added_by_conversion": ms_bgr / ms_lab - 1})
     for o in out:
         print(json.dumps(o), flush=True)
 
