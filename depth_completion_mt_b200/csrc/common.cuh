@@ -6,6 +6,7 @@
 #ifdef DCMT_EMU
 // CPU emulation of the CUDA execution model, tests only (tests/emu/cuda_emu.h); never defined for libdcmt.so
 #include "cuda_emu.h"
+#include <cstring>
 #else
 #include <cuda.h>  // CUtensorMap and its enums only; the encoder is fetched with cudaGetDriverEntryPoint (no -lcuda)
 #include <cuda_runtime.h>
@@ -25,37 +26,52 @@ namespace dcmt { void note_launch(); }  // launch counter behind dcmt_launch_cou
 
 namespace dcmt {
 
-// ---- TMA (cp.async.bulk.tensor) tile load of a uint16 plane: one thread issues one 3-D box copy (columns, rows,
-// frame) global -> shared; elements of the box outside the tensor are ZERO-filled by the hardware, the copy signals an
-// mbarrier with its byte count.  The emulator build replaces the map by a plain description and copies in place.
+// ---- TMA (cp.async.bulk.tensor) tile load of a uint16 or float32 plane: one thread issues one 3-D box copy (columns,
+// rows, frame) global -> shared; elements of the box outside the tensor are ZERO-filled by the hardware, the copy signals
+// an mbarrier with its byte count.  A map cannot be encoded (an error is returned) unless the base, the row pitch and
+// the frame stride are multiples of 16 bytes.  The emulator build replaces the map by a plain description, refuses
+// the same layouts and copies in place.
 #ifdef DCMT_EMU
 struct TensorMap3D {
-    const uint16_t* base;
+    const void* base;
+    int elem;           // bytes per element
     int dim[3];         // elements: columns, rows, frames
     size_t stride[2];   // bytes between rows, between frames
     int box[2];         // columns, rows of the box (one frame)
 };
+inline cudaError_t tma_encode_3d(TensorMap3D* m, const void* base, int elem, int cols, int rows, int frames, size_t row_bytes,
+                                 size_t frame_bytes, int box_cols, int box_rows) {
+    if (box_cols > 256 || box_rows > 256 || (row_bytes & 15) || (frame_bytes & 15) || (reinterpret_cast<uintptr_t>(base) & 15))
+        return cudaErrorInvalidValue;
+    *m = TensorMap3D{base, elem, {cols, rows, frames}, {row_bytes, frame_bytes}, {box_cols, box_rows}};
+    return cudaSuccess;
+}
 inline cudaError_t tma_encode_u16_3d(TensorMap3D* m, const uint16_t* base, int cols, int rows, int frames, size_t row_bytes,
                                      size_t frame_bytes, int box_cols, int box_rows) {
-    *m = TensorMap3D{base, {cols, rows, frames}, {row_bytes, frame_bytes}, {box_cols, box_rows}};
-    return cudaSuccess;
+    return tma_encode_3d(m, base, 2, cols, rows, frames, row_bytes, frame_bytes, box_cols, box_rows);
+}
+inline cudaError_t tma_encode_f32_3d(TensorMap3D* m, const float* base, int cols, int rows, int frames, size_t row_bytes,
+                                     size_t frame_bytes, int box_cols, int box_rows) {
+    return tma_encode_3d(m, base, 4, cols, rows, frames, row_bytes, frame_bytes, box_cols, box_rows);
 }
 inline void tma_bar_init(uint64_t*) {}
 inline void tma_load_3d(void* smem_dst, const TensorMap3D* m, int c0, int c1, int c2, uint64_t*, uint32_t) {
-    uint16_t* d = static_cast<uint16_t*>(smem_dst);
+    char* d = static_cast<char*>(smem_dst);
     for (int r = 0; r < m->box[1]; ++r)
         for (int c = 0; c < m->box[0]; ++c) {
             const int x = c0 + c, y = c1 + r;
             const bool in = x >= 0 && x < m->dim[0] && y >= 0 && y < m->dim[1] && c2 >= 0 && c2 < m->dim[2];
-            d[(size_t)r * m->box[0] + c] =
-                in ? *reinterpret_cast<const uint16_t*>(reinterpret_cast<const char*>(m->base) + (size_t)c2 * m->stride[1] + (size_t)y * m->stride[0] + (size_t)x * 2)
-                   : (uint16_t)0;
+            char* o = d + ((size_t)r * m->box[0] + c) * m->elem;
+            if (in) std::memcpy(o, static_cast<const char*>(m->base) + (size_t)c2 * m->stride[1] + (size_t)y * m->stride[0] + (size_t)x * m->elem, m->elem);
+            else std::memset(o, 0, m->elem);
         }
 }
 inline void tma_bar_wait(uint64_t*, uint32_t) {}
 #else
 typedef CUtensorMap TensorMap3D;
 cudaError_t tma_encode_u16_3d(TensorMap3D* m, const uint16_t* base, int cols, int rows, int frames, size_t row_bytes,
+                              size_t frame_bytes, int box_cols, int box_rows);  // fused_q8.cu
+cudaError_t tma_encode_f32_3d(TensorMap3D* m, const float* base, int cols, int rows, int frames, size_t row_bytes,
                               size_t frame_bytes, int box_cols, int box_rows);  // fused_q8.cu
 __device__ __forceinline__ void tma_bar_init(uint64_t* bar) {  // one thread; follow with __syncthreads()
     const unsigned b = (unsigned)__cvta_generic_to_shared(bar);

@@ -151,6 +151,7 @@ struct FrontArgs {
     ItemsDesc i_half;               // half-quad columns of the computed quads: 2 (RQ - 1) per row of items
     long long* prof;              // optional: 16 clock64() stamps per CTA (debugging aid)
     int codes;                    // in16 holds CODES (the dictionary encoding of rank_f32.cu: already e), not KITTI uint16
+    int use_tma;                  // k_q8_front: region loaded by one TMA box copy (else front_load's per-thread loads)
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -538,9 +539,56 @@ __device__ __forceinline__ void front_load(const FrontArgs& a, const void* in0v,
     }
 }
 
+// pass 0 from a region staged in shared memory by one TMA box copy: RH rows x RQ * 8 pixels at S (row r of the box at
+// word r * RQ * 8 for float input, r * RQ * 4 for uint16), zero wherever the box leaves the image.  The staged floats
+// fill planes A and B, so every thread first decodes its quads into registers -- at most kStagedSweeps per thread, the
+// host uses front_load beyond that -- and writes A only after the barrier.  Cells outside the image are decided by
+// position, as in front_load, and zeroed in both planes: the zero fill itself would encode as a hole, not as absent.
+constexpr int kStagedSweeps = 6;
+template <bool kIn16, bool kValidate, bool kCodes = false>
+__device__ __forceinline__ void front_decode_staged(const FrontArgs& a, const uint32_t* S, uint32_t* A, uint32_t* B, const Tile& t,
+                                                    float& bad) {
+    const ColMap& m = a.m_load;
+    const int r0 = fast_div((int)threadIdx.x, m.magic), q = (int)threadIdx.x - r0 * m.nq;
+    const bool q_in = r0 < m.nrt && q >= t.qlo && q < t.qhi;
+    const int sstep = m.nrt * (kIn16 ? t.pitchw : 2 * t.pitchw);
+    const uint32_t* p = S + r0 * (kIn16 ? t.pitchw : 2 * t.pitchw) + q * (kIn16 ? 4 : 8);
+    uint4 o[kStagedSweeps];
+#pragma unroll
+    for (int u = 0; u < kStagedSweeps; ++u, p += sstep) {
+        const int r = r0 + u * m.nrt;
+        o[u] = splat4(0u);
+        if (!q_in || r < t.rlo || r >= t.rhi) continue;
+        if (kCodes) {
+            o[u] = lds4(p);
+        } else if (kIn16) {
+            const uint4 h = lds4(p);
+            o[u] = make_uint4(encode_u16_pair(h.x), encode_u16_pair(h.y), encode_u16_pair(h.z), encode_u16_pair(h.w));
+        } else {
+            const uint4 f0 = lds4(p), f1 = lds4(p + 4);
+            o[u] = make_uint4(encode_pair<kValidate>(__uint_as_float(f0.x), __uint_as_float(f0.y), bad),
+                              encode_pair<kValidate>(__uint_as_float(f0.z), __uint_as_float(f0.w), bad),
+                              encode_pair<kValidate>(__uint_as_float(f1.x), __uint_as_float(f1.y), bad),
+                              encode_pair<kValidate>(__uint_as_float(f1.z), __uint_as_float(f1.w), bad));
+        }
+        if (q == t.qs) o[u] = and4(o[u], t.smask);  // lanes right of the image: absent
+    }
+    __syncthreads();  // every staged value is in registers: A and B may be overwritten
+    if (r0 >= m.nrt) return;
+    int off = (r0 * t.RQ + q) * 4;
+#pragma unroll
+    for (int u = 0; u < kStagedSweeps; ++u, off += m.nrt * t.pitchw) {
+        const int r = r0 + u * m.nrt;
+        if (r >= t.RH) break;
+        sts4(A + off, o[u]);
+        if (!q_in || r < t.rlo || r >= t.rhi) sts4(B + off, splat4(0u));
+    }
+}
+
 template <bool kStraddle>
-__global__ void __launch_bounds__(QT, DCMT_FRONT_CTAS) k_q8_front(FrontArgs a) {
+__global__ void __launch_bounds__(QT, DCMT_FRONT_CTAS) k_q8_front(FrontArgs a, const __grid_constant__ TensorMap3D tmap) {
     DCMT_DYN_SMEM(uint32_t, smem);
+    __shared__ __align__(8) uint64_t s_bar;  // mbarrier the TMA tile load signals
     const int th = a.th, tw = a.tw, rows = a.rows, cols = a.cols;
     Tile t;
     t.RH = th + FU + FD;
@@ -562,7 +610,20 @@ __global__ void __launch_bounds__(QT, DCMT_FRONT_CTAS) k_q8_front(FrontArgs a) {
 
     DCMT_STAMP(a, 0);
     float bad = 0.0f;
-    if (a.in16 && a.codes) front_load<true, false, true>(a, a.in16 + origin, A, B, t, gx0, bad);  // dictionary codes (rank_f32.cu)
+    if (a.use_tma) {
+        // ONE box copy of the region (zero outside the image) to the start of the dynamic shared memory, which is 128-byte
+        // aligned: RH x RQ * 8 floats fill A and B exactly (A starts one quad in, B ends one quad short of the allocation)
+        if (threadIdx.x == 0) {
+            tma_bar_init(&s_bar);
+            tma_load_3d(smem, &tmap, gx0, gy0, frame, &s_bar, (uint32_t)(t.RH * t.pitchw * (a.in16 ? 4 : 8)));
+        }
+        __syncthreads();  // the mbarrier is initialised before anyone waits on it
+        tma_bar_wait(&s_bar, 0);
+        if (a.in16 && a.codes) front_decode_staged<true, false, true>(a, smem, A, B, t, bad);
+        else if (a.in16) front_decode_staged<true, false>(a, smem, A, B, t, bad);
+        else if (a.validate) front_decode_staged<false, true>(a, smem, A, B, t, bad);
+        else front_decode_staged<false, false>(a, smem, A, B, t, bad);
+    } else if (a.in16 && a.codes) front_load<true, false, true>(a, a.in16 + origin, A, B, t, gx0, bad);  // dictionary codes (rank_f32.cu)
     else if (a.in16) front_load<true, false>(a, a.in16 + origin, A, B, t, gx0, bad);  // uint16 input is q8 by construction
     else if (a.validate) front_load<false, true>(a, a.in + origin, A, B, t, gx0, bad);
     else front_load<false, false>(a, a.in + origin, A, B, t, gx0, bad);
@@ -1770,8 +1831,8 @@ __global__ void k_q8_write_stats(const FrameCounters* __restrict__ c, int32_t* _
 }  // namespace
 
 #ifndef DCMT_EMU
-cudaError_t tma_encode_u16_3d(TensorMap3D* m, const uint16_t* base, int cols, int rows, int frames, size_t row_bytes,
-                              size_t frame_bytes, int box_cols, int box_rows) {
+static cudaError_t tma_encode_3d(TensorMap3D* m, CUtensorMapDataType type, const void* base, int cols, int rows, int frames,
+                                 size_t row_bytes, size_t frame_bytes, int box_cols, int box_rows) {
     typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -1787,12 +1848,26 @@ cudaError_t tma_encode_u16_3d(TensorMap3D* m, const uint16_t* base, int cols, in
     const cuuint64_t strides[2] = {(cuuint64_t)row_bytes, (cuuint64_t)frame_bytes};
     const cuuint32_t box[3] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows, 1u};
     const cuuint32_t estr[3] = {1u, 1u, 1u};
-    const CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_UINT16, 3, const_cast<uint16_t*>(base), dims, strides, box, estr,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    const CUresult r = fn(m, type, 3, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                          CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     return r == CUDA_SUCCESS ? cudaSuccess : cudaErrorInvalidValue;
 }
+cudaError_t tma_encode_u16_3d(TensorMap3D* m, const uint16_t* base, int cols, int rows, int frames, size_t row_bytes,
+                              size_t frame_bytes, int box_cols, int box_rows) {
+    return tma_encode_3d(m, CU_TENSOR_MAP_DATA_TYPE_UINT16, base, cols, rows, frames, row_bytes, frame_bytes, box_cols, box_rows);
+}
+cudaError_t tma_encode_f32_3d(TensorMap3D* m, const float* base, int cols, int rows, int frames, size_t row_bytes,
+                              size_t frame_bytes, int box_cols, int box_rows) {
+    return tma_encode_3d(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, base, cols, rows, frames, row_bytes, frame_bytes, box_cols, box_rows);
+}
 #endif
+
+// DCMT_NO_TMA=1: the front and the tail load their tiles with per-thread copies (the path for inputs a tensor map cannot
+// describe), e.g. to test that path on any input
+static bool tma_disabled() {
+    static const bool no_tma = [] { const char* e = getenv("DCMT_NO_TMA"); return e && e[0] == '1'; }();
+    return no_tma;
+}
 
 size_t q8_front_smem(int th, int tw) {
     // two region planes, the core-sized D plane, one quad of padding in front of / behind the region planes
@@ -1888,9 +1963,18 @@ cudaError_t q8_run_front(const Q8Plan& plan, const float* in, const uint16_t* in
                 make_colmap(p.tw / 8 + FLQ + FRQ, QT), make_colmap(p.tw / 8 + FLQ + FRQ - 1, QT), make_colmap(p.tw / 8, QT),
                 make_items(2 * (p.tw / 8 + FLQ + FRQ - 1), QT), p.prof_front};
     a.codes = p.codes_in;
+    // region load by TMA: a 3-D map (columns, rows, frames) of this chunk's input with the region as its box, unless the
+    // input's layout cannot be mapped or a thread would hold more than kStagedSweeps quads of the staged region
+    TensorMap3D tmap{};
+    const int RH = p.th + FU + FD, RQ = p.tw / 8 + FLQ + FRQ;
+    if (!tma_disabled() && RH <= kStagedSweeps * (QT / RQ)) {
+        const cudaError_t e = in16 ? tma_encode_u16_3d(&tmap, in16, p.cols, p.rows, n_frames, in_pitch * 2, in_fstride * 2, RQ * 8, RH)
+                                   : tma_encode_f32_3d(&tmap, in, p.cols, p.rows, n_frames, in_pitch * 4, in_fstride * 4, RQ * 8, RH);
+        a.use_tma = e == cudaSuccess;
+    }
     const dim3 grid((p.cols + p.tw - 1) / p.tw, (p.rows + p.th - 1) / p.th, n_frames);
-    if (p.cols % 8 != 0) DCMT_LAUNCH(k_q8_front<true>, grid, dim3(QT), q8_front_smem(p.th, p.tw), st, a);
-    else DCMT_LAUNCH(k_q8_front<false>, grid, dim3(QT), q8_front_smem(p.th, p.tw), st, a);
+    if (p.cols % 8 != 0) DCMT_LAUNCH(k_q8_front<true>, grid, dim3(QT), q8_front_smem(p.th, p.tw), st, a, tmap);
+    else DCMT_LAUNCH(k_q8_front<false>, grid, dim3(QT), q8_front_smem(p.th, p.tw), st, a, tmap);
     return cudaGetLastError();
 }
 
@@ -1969,8 +2053,7 @@ cudaError_t q8_run_tail(const Q8Plan& p, float* out, size_t out_pitch, size_t ou
     // tile load by TMA: a 3-D map (columns, rows, slots) of the intermediate plane whose column extent is the true
     // image width, so that the padding columns of the plane read as absent like everything else outside the image
     TensorMap3D tmap{};
-    static const bool no_tma = [] { const char* e = getenv("DCMT_NO_TMA"); return e && e[0] == '1'; }();
-    const int use_tma = !no_tma && tma_encode_u16_3d(&tmap, p.mid, p.cols, p.rows, p.max_frames, (size_t)p.mid_pitch * 2,
+    const int use_tma = !tma_disabled() && tma_encode_u16_3d(&tmap, p.mid, p.cols, p.rows, p.max_frames, (size_t)p.mid_pitch * 2,
                                                      (size_t)p.mid_pitch * p.rows * 2, RQ * 8, RH) == cudaSuccess;
     TailArgs a{p.mid, (size_t)p.mid_pitch, (size_t)p.mid_pitch * p.rows, p.col_first, p.col_last, p.ctr, out, out_pitch,
                out_fstride, p.rows, p.cols, p.th, p.tw, blur, vec2, 1, use_tma,
