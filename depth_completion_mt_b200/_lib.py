@@ -87,6 +87,17 @@ _SIGNATURES = {
     "dcmt_interpolate_with_superpixels_f32_host_multi": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int]),
     "dcmt_debug_host_copy_f32": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, C.c_int]),
     "dcmt_debug_host_copy_u16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, C.c_int]),
+    "dcmt_debug_host_copy_u16_u16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, C.c_int]),
+    "dcmt_img_completion_u16_u16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P, _P]),
+    "dcmt_img_completion_u16_u16_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P]),
+    "dcmt_img_completion_u16_u16_host_multi": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int]),
+    "dcmt_interpolate_with_superpixels_u16": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P, _P]),
+    "dcmt_interpolate_with_superpixels_u16_host": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P]),
+    "dcmt_interpolate_with_superpixels_u16_host_multi": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int]),
+    "dcmt_interpolate_with_superpixels_u16_u16": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P, _P]),
+    "dcmt_interpolate_with_superpixels_u16_u16_host": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P]),
+    "dcmt_interpolate_with_superpixels_u16_u16_host_multi": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int]),
+    "dcmt_depth_to_u16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, _P]),
     "dcmt_bgr2gray_u8": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, _P]),
     "dcmt_bgr2gray_u8_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int]),
     "dcmt_bgr2lab_u8": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, _P]),

@@ -83,8 +83,44 @@ def _device_list(devices):
     return arr, arr, len(devices)
 
 
+def _u16_output(out_dtype, u16_in: bool) -> bool:
+    """out_dtype None / float32 -> float32 metres; uint16 (numpy or torch) -> KITTI uint16 = metres * 256, which the library
+    produces from uint16 input only (float32 results go through depth_to_u16)."""
+    if out_dtype is None:
+        return False
+    if torch is not None and isinstance(out_dtype, torch.dtype):
+        name = {torch.float32: "float32", torch.uint16: "uint16"}.get(out_dtype)
+    else:
+        try:
+            name = np.dtype(out_dtype).name
+        except TypeError:
+            name = None
+    if name not in ("float32", "uint16"):
+        raise ValueError(f"out_dtype must be float32 or uint16, got {out_dtype!r}")
+    if name == "uint16" and not u16_in:
+        raise ValueError("uint16 output needs uint16 (KITTI) input; convert a float32 result with depth_to_u16")
+    return name == "uint16"
+
+
+def _out_torch(out, like, dtype):
+    """the output tensor of a call whose (n, rows, cols) input is `like`: a new one, or the caller's `out` checked"""
+    if out is None:
+        return torch.empty(like.shape, dtype=dtype, device=like.device)
+    if not (_is_torch(out) and out.is_cuda and out.dtype == dtype and out.is_contiguous() and out.numel() == like.numel()):
+        raise ValueError(f"out must be a contiguous {str(dtype).replace('torch.', '')} CUDA tensor of the input's size")
+    return out.view(like.shape)
+
+
+def _out_numpy(out, like, dtype):
+    if out is None:
+        return np.empty(like.shape, dtype)
+    if not (isinstance(out, np.ndarray) and out.dtype == dtype and out.flags.c_contiguous and out.size == like.size):
+        raise ValueError(f"out must be a C-contiguous {np.dtype(dtype).name} array of the input's size")
+    return out.reshape(like.shape)
+
+
 def img_completion(sparse, extr: bool = False, blur_type="gaussian", *, path: str = "auto", return_stats: bool = False,
-                   out=None, stream=None, devices=None, lib: _lib.Library | None = None):
+                   out=None, stream=None, devices=None, out_dtype=None, lib: _lib.Library | None = None):
     """img_completion(sparse_r_img, dense_r_img, extr, blur_type) -- img_completion.cpp:17-204.
 
     ``extr`` is accepted and ignored exactly like the reference (:103 ``int densify = true``).
@@ -93,7 +129,10 @@ def img_completion(sparse, extr: bool = False, blur_type="gaussian", *, path: st
     Returns ``dense`` (and an int32 (n, 4) stats array when ``return_stats``).  ``out`` optionally supplies the
     output buffer (same type/shape as ``sparse``, contiguous) so that steady-state callers allocate nothing.
     ``devices`` (host arrays only): "all" or a list of CUDA device ordinals -- the frames of the batch are partitioned
-    over those GPUs inside the one call (``dcmt_img_completion_*_host_multi``)."""
+    over those GPUs inside the one call (``dcmt_img_completion_*_host_multi``).
+    ``out_dtype`` uint16 (``np.uint16`` / ``torch.uint16``, uint16 input only) returns the result in the KITTI format as
+    well -- uint16 = metres * 256 by ``convertTo(CV_16U, 256)``'s rule (``dcmt_img_completion_u16_u16``); ``out`` must then
+    be uint16."""
     del extr
     lib = lib or _lib.load()
     blur = _blur_code(blur_type)
@@ -101,19 +140,18 @@ def img_completion(sparse, extr: bool = False, blur_type="gaussian", *, path: st
         if devices is not None:
             raise ValueError("devices= applies to host (numpy) input; a CUDA tensor already lives on one device")
         u16 = sparse.dtype == torch.uint16
+        u16_out = _u16_output(out_dtype, u16)
         s = _prep_torch(sparse, torch.uint16 if u16 else torch.float32, "sparse")
         s3, squeeze = _batch3(s, "sparse")
         n, rows, cols = s3.shape
-        if out is None:
-            out = torch.empty(s3.shape, dtype=torch.float32, device=s.device)
-        else:
-            if not (_is_torch(out) and out.is_cuda and out.dtype == torch.float32 and out.is_contiguous() and out.numel() == s3.numel()):
-                raise ValueError("out must be a contiguous float32 CUDA tensor of the input's size")
-            out = out.view(s3.shape)
+        out = _out_torch(out, s3, torch.uint16 if u16_out else torch.float32)
         stats = torch.zeros((n, STATS_STRIDE), dtype=torch.int32, device=s.device) if return_stats else None
         st_ptr = stats.data_ptr() if return_stats else None
         with torch.cuda.device(s.device):
-            if u16:
+            if u16_out:
+                lib.check(lib.dcmt_img_completion_u16_u16(s3.data_ptr(), out.data_ptr(), rows, cols, 0, 0, 0, 0, n, blur, PATH[path],
+                                                          st_ptr, _stream_ptr(stream)))
+            elif u16:
                 lib.check(lib.dcmt_img_completion_u16(s3.data_ptr(), out.data_ptr(), rows, cols, 0, 0, 0, 0, n, blur, PATH[path],
                                                       st_ptr, _stream_ptr(stream)))
             else:
@@ -121,19 +159,20 @@ def img_completion(sparse, extr: bool = False, blur_type="gaussian", *, path: st
                                                       st_ptr, _stream_ptr(stream)))
     else:
         u16 = isinstance(sparse, np.ndarray) and sparse.dtype == np.uint16
+        u16_out = _u16_output(out_dtype, u16)
         s = _prep_numpy(sparse, np.uint16 if u16 else np.float32, "sparse")
         s3, squeeze = _batch3(s, "sparse")
         n, rows, cols = s3.shape
-        if out is None:
-            out = np.empty(s3.shape, np.float32)
-        else:
-            if not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.flags.c_contiguous and out.size == s3.size):
-                raise ValueError("out must be a C-contiguous float32 array of the input's size")
-            out = out.reshape(s3.shape)
+        out = _out_numpy(out, s3, np.uint16 if u16_out else np.float32)
         stats = np.zeros((n, STATS_STRIDE), np.int32) if return_stats else None
         st_ptr = _np_ptr(stats) if return_stats else None
         keep, dev_ptr, n_dev = _device_list(devices)
-        if devices is not None and u16:
+        if devices is not None and u16_out:
+            lib.check(lib.dcmt_img_completion_u16_u16_host_multi(_np_ptr(s3), _np_ptr(out), rows, cols, 0, 0, 0, 0, n, blur, PATH[path],
+                                                                 st_ptr, dev_ptr, n_dev))
+        elif u16_out:
+            lib.check(lib.dcmt_img_completion_u16_u16_host(_np_ptr(s3), _np_ptr(out), rows, cols, 0, 0, 0, 0, n, blur, PATH[path], st_ptr))
+        elif devices is not None and u16:
             lib.check(lib.dcmt_img_completion_u16_host_multi(_np_ptr(s3), _np_ptr(out), rows, cols, 0, 0, 0, 0, n, blur, PATH[path], st_ptr,
                                                              dev_ptr, n_dev))
         elif devices is not None:
@@ -149,17 +188,21 @@ def img_completion(sparse, extr: bool = False, blur_type="gaussian", *, path: st
 
 
 def interpolate_with_superpixels(labels, sparse, blur_type="gaussian", use_superpixel: int = 1, *, n_clusters=None,
-                                 path: str = "auto", return_stats: bool = False, out=None, stream=None,
+                                 path: str = "auto", return_stats: bool = False, out=None, stream=None, out_dtype=None,
                                  lib: _lib.Library | None = None):
     """interpolate_with_superpixels(slic, sparse, dense, blur_type, use_superpixel) -- img_completion_lc.cpp:34-203.
 
     ``labels`` stands for ``slic.clusters`` as an int32 [row][col] map (the reference indexes [col][row], :83);
     ``n_clusters`` for ``slic.centers.size()`` (default: max label + 1).  ``blur_type`` is ignored, as in the
-    reference (:183-192 blurs unconditionally)."""
+    reference (:183-192 blurs unconditionally).  ``sparse`` is float32 metres or KITTI uint16 (metres * 256: the PNG
+    payload main_lc.cpp reads, ``dcmt_interpolate_with_superpixels_u16``); with uint16 input, ``out_dtype`` uint16
+    returns KITTI uint16 as for ``img_completion``."""
     del blur_type
     lib = lib or _lib.load()
     if _is_torch(sparse):
-        s = _prep_torch(sparse, torch.float32, "sparse")
+        u16 = sparse.dtype == torch.uint16
+        u16_out = _u16_output(out_dtype, u16)
+        s = _prep_torch(sparse, torch.uint16 if u16 else torch.float32, "sparse")
         s3, squeeze = _batch3(s, "sparse")
         n, rows, cols = s3.shape
         lab_ptr = None
@@ -171,19 +214,22 @@ def interpolate_with_superpixels(labels, sparse, blur_type="gaussian", use_super
             if n_clusters is None:
                 n_clusters = int(lab3.max().item()) + 1
             lab_ptr = lab3.data_ptr()
-        if out is None:
-            out = torch.empty_like(s3)
-        else:
-            if not (_is_torch(out) and out.is_cuda and out.dtype == torch.float32 and out.is_contiguous() and out.numel() == s3.numel()):
-                raise ValueError("out must be a contiguous float32 CUDA tensor of the input's size")
-            out = out.view(s3.shape)
+        out = _out_torch(out, s3, torch.uint16 if u16_out else torch.float32)
         stats = torch.zeros((n, STATS_STRIDE), dtype=torch.int32, device=s.device) if return_stats else None
+        st_ptr = stats.data_ptr() if return_stats else None
         with torch.cuda.device(s.device):
-            lib.check(lib.dcmt_interpolate_with_superpixels_ex_f32(
-                s3.data_ptr(), lab_ptr, int(n_clusters or 0), out.data_ptr(), rows, cols, 0, 0, n, int(use_superpixel), PATH[path],
-                stats.data_ptr() if return_stats else None, _stream_ptr(stream)))
+            if u16:
+                fn = lib.dcmt_interpolate_with_superpixels_u16_u16 if u16_out else lib.dcmt_interpolate_with_superpixels_u16
+                lib.check(fn(s3.data_ptr(), lab_ptr, int(n_clusters or 0), out.data_ptr(), rows, cols, 0, 0, 0, 0, n, int(use_superpixel),
+                             PATH[path], st_ptr, _stream_ptr(stream)))
+            else:
+                lib.check(lib.dcmt_interpolate_with_superpixels_ex_f32(
+                    s3.data_ptr(), lab_ptr, int(n_clusters or 0), out.data_ptr(), rows, cols, 0, 0, n, int(use_superpixel), PATH[path],
+                    st_ptr, _stream_ptr(stream)))
     else:
-        s = _prep_numpy(sparse, np.float32, "sparse")
+        u16 = isinstance(sparse, np.ndarray) and sparse.dtype == np.uint16
+        u16_out = _u16_output(out_dtype, u16)
+        s = _prep_numpy(sparse, np.uint16 if u16 else np.float32, "sparse")
         s3, squeeze = _batch3(s, "sparse")
         n, rows, cols = s3.shape
         lab_ptr = None
@@ -194,18 +240,32 @@ def interpolate_with_superpixels(labels, sparse, blur_type="gaussian", use_super
             if n_clusters is None:
                 n_clusters = int(lab3.max()) + 1
             lab_ptr = _np_ptr(lab3)
-        if out is None:
-            out = np.empty_like(s3)
-        else:
-            if not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.flags.c_contiguous and out.size == s3.size):
-                raise ValueError("out must be a C-contiguous float32 array of the input's size")
-            out = out.reshape(s3.shape)
+        out = _out_numpy(out, s3, np.uint16 if u16_out else np.float32)
         stats = np.zeros((n, STATS_STRIDE), np.int32) if return_stats else None
-        lib.check(lib.dcmt_interpolate_with_superpixels_ex_f32_host(
-            _np_ptr(s3), lab_ptr, int(n_clusters or 0), _np_ptr(out), rows, cols, 0, 0, n, int(use_superpixel), PATH[path],
-            _np_ptr(stats) if return_stats else None))
+        st_ptr = _np_ptr(stats) if return_stats else None
+        if u16:
+            fn = lib.dcmt_interpolate_with_superpixels_u16_u16_host if u16_out else lib.dcmt_interpolate_with_superpixels_u16_host
+            lib.check(fn(_np_ptr(s3), lab_ptr, int(n_clusters or 0), _np_ptr(out), rows, cols, 0, 0, 0, 0, n, int(use_superpixel), PATH[path],
+                         st_ptr))
+        else:
+            lib.check(lib.dcmt_interpolate_with_superpixels_ex_f32_host(
+                _np_ptr(s3), lab_ptr, int(n_clusters or 0), _np_ptr(out), rows, cols, 0, 0, n, int(use_superpixel), PATH[path], st_ptr))
     out = out[0] if squeeze else out
     return (out, stats) if return_stats else out
+
+
+def depth_to_u16(depth, *, out=None, stream=None, lib: _lib.Library | None = None):
+    """``depth.convertTo(png, CV_16U, 256)`` on the device (``dcmt_depth_to_u16``): float32 metres (CUDA tensor, (rows, cols)
+    or (n, rows, cols)) -> KITTI uint16 = metres * 256, rounded half to even, clamped to [0, 65535], NaN -> 0."""
+    lib = lib or _lib.load()
+    if not _is_torch(depth):
+        raise TypeError("depth_to_u16 takes a float32 CUDA tensor")
+    d3, squeeze = _batch3(_prep_torch(depth, torch.float32, "depth"), "depth")
+    n, rows, cols = d3.shape
+    out = _out_torch(out, d3, torch.uint16)
+    with torch.cuda.device(d3.device):
+        lib.check(lib.dcmt_depth_to_u16(d3.data_ptr(), out.data_ptr(), rows, cols, 0, 0, 0, 0, n, _stream_ptr(stream)))
+    return out[0] if squeeze else out
 
 
 def stereo_params(official: bool = False, num_iterations: int | None = None, lib: _lib.Library | None = None,

@@ -214,7 +214,8 @@ bool fused_applies(const CompletionCall& cc) {
            (!cc.guided || dcmt::q8_guided_smem(th, tw) <= 200 * 1024);
 }
 
-size_t completion_ws_bytes(int rows, int cols, int n_frames, bool bilateral, bool fused, bool u16_in = false, bool rank = false) {
+size_t completion_ws_bytes(int rows, int cols, int n_frames, bool bilateral, bool fused, bool u16_in = false, bool rank = false,
+                           bool u16_out = false) {
     const int chunk = fused ? fused_chunk_frames(rows, cols, n_frames) : generic_chunk_frames(rows, cols, n_frames);
     size_t b = generic_ws_bytes(rows, cols, chunk, bilateral);
     if (fused && rank) {  // dictionary, its sizes, the code plane (rank_f32.cu)
@@ -223,6 +224,7 @@ size_t completion_ws_bytes(int rows, int cols, int n_frames, bool bilateral, boo
              carve_bytes((size_t)rows * code_pitch * chunk, sizeof(uint16_t));
     }
     if (u16_in && !fused) b += carve_bytes((size_t)rows * cols * chunk, sizeof(float));
+    if (u16_out && !fused) b += carve_bytes((size_t)rows * cols * chunk, sizeof(float));  // float plane in front of depth_to_u16
     if (fused) {
         const size_t mid_pitch = ((size_t)cols + 7) / 8 * 8;
         b += carve_bytes((size_t)rows * mid_pitch * chunk, sizeof(uint16_t)) + 2 * carve_bytes(mid_pitch * chunk, sizeof(uint32_t));
@@ -236,7 +238,7 @@ size_t completion_ws_bytes(int rows, int cols, int n_frames, bool bilateral, boo
 // frames that turned out not to be strict q8: their output is NOT valid and the caller must redo them with
 // DCMT_PATH_GENERIC.  *used_fused tells the caller which path ran.
 //
-// Input is either float32 metres (`sparse`, sharing pitch / fstride with the output) or -- `in16.p` non-null -- KITTI
+// Input is either float32 metres (`sparse`, `pitch` / `fstride` in elements) or -- `in16.p` non-null -- KITTI
 // uint16 (metres * 256, main.cpp:75-82) with its own pitch / frame stride in elements.  uint16 input is strict q8 by
 // construction: the fused kernels read it directly and nothing is validated or redone; shapes the fused kernels do
 // not serve get a convertTo(CV_32F, 1/256) (main.cpp:79) into a workspace plane in front of the generic pipeline.
@@ -245,7 +247,22 @@ struct U16Input {
     size_t pitch = 0, fstride = 0;  // elements
 };
 
-int enqueue_completion(const CompletionCall& cc, const float* sparse, const int32_t* labels, float* dense, size_t pitch,
+// Output is float32 metres or -- `out.u` non-null, uint16 input only -- KITTI uint16 (metres * 256, the rule of
+// dcmt_depth_to_u16): the fused tail stores it directly; the generic pipeline writes a float workspace plane that
+// depth_to_u16 converts.
+struct OutDesc {
+    float* f = nullptr;
+    uint16_t* u = nullptr;
+    size_t pitch = 0, fstride = 0;  // elements of the output type
+    OutDesc frames_from(size_t f0) const {
+        OutDesc o = *this;
+        if (u) o.u += f0 * fstride;
+        else o.f += f0 * fstride;
+        return o;
+    }
+};
+
+int enqueue_completion(const CompletionCall& cc, const float* sparse, const int32_t* labels, const OutDesc& out, size_t pitch,
                        size_t fstride, int n_frames, int32_t* stats, int32_t* redo_flags, float* stages,
                        uint32_t* stage_mask, Arena* ar, cudaStream_t st, bool* used_fused, U16Input in16 = U16Input{}) {
     const int rows = cc.rows, cols = cc.cols;
@@ -301,7 +318,11 @@ int enqueue_completion(const CompletionCall& cc, const float* sparse, const int3
                 else
                     API_CUDA(dcmt::q8_run_front(p, nullptr, codes, (size_t)p.mid_pitch, (size_t)p.mid_pitch * rows, nf, 0, st),
                              "fused front launch");
-            } else if (cc.guided)
+            } else if (cc.guided && in16.p)
+                API_CUDA(dcmt::q8_run_guided_front(p, nullptr, in16.p + (size_t)f0 * in16.fstride, in16.pitch, in16.fstride,
+                                                   labels + (size_t)f0 * fpix, cc.n_clusters, nf, 0, tile_flags, st),
+                         "fused guided front launch");
+            else if (cc.guided)
                 API_CUDA(dcmt::q8_run_guided_front(p, sparse + (size_t)f0 * fstride, nullptr, pitch, fstride, labels + (size_t)f0 * fpix,
                                                    cc.n_clusters, nf, cc.flags != DCMT_PATH_FUSED, tile_flags, st),
                          "fused guided front launch");
@@ -313,7 +334,8 @@ int enqueue_completion(const CompletionCall& cc, const float* sparse, const int3
                                             cc.flags != DCMT_PATH_FUSED, st),
                          "fused front launch");
             API_CUDA(prof_mark(st, 1, &pe), "profiling event");
-            API_CUDA(dcmt::q8_run_tail(p, dense + (size_t)f0 * fstride, pitch, fstride, nf, cc.blur, st), "fused tail launch");
+            const OutDesc o = out.frames_from((size_t)f0);
+            API_CUDA(dcmt::q8_run_tail(p, o.f, o.u, o.pitch, o.fstride, nf, cc.blur, st), "fused tail launch");
             API_CUDA(prof_mark(st, 2, &pe), "profiling event");
             if (g_prof_on) {
                 std::lock_guard<std::mutex> lk(g_mu);
@@ -327,6 +349,7 @@ int enqueue_completion(const CompletionCall& cc, const float* sparse, const int3
         return DCMT_OK;
     }
     float* conv = in16.p ? carve<float>(ar, fpix * chunk) : nullptr;
+    float* staged = out.u ? carve<float>(ar, fpix * chunk) : nullptr;
     if (int rc = arena_ok(ar)) return rc;
     for (int f0 = 0; f0 < n_frames; f0 += chunk) {
         const int nf = n_frames - f0 < chunk ? n_frames - f0 : chunk;
@@ -345,9 +368,10 @@ int enqueue_completion(const CompletionCall& cc, const float* sparse, const int3
         c.labels = cc.guided ? labels + (size_t)f0 * fpix : nullptr;
         c.n_clusters = cc.n_clusters;
         c.guided = cc.guided;
-        c.out = dense + (size_t)f0 * fstride;
-        c.out_pitch = pitch;
-        c.out_fstride = fstride;
+        const OutDesc o = out.frames_from((size_t)f0);
+        c.out = staged ? staged : o.f;
+        c.out_pitch = staged ? (size_t)cols : o.pitch;
+        c.out_fstride = staged ? fpix : o.fstride;
         c.rows = rows;
         c.cols = cols;
         c.n_frames = nf;
@@ -362,6 +386,8 @@ int enqueue_completion(const CompletionCall& cc, const float* sparse, const int3
         c.stage_mask = stage_mask;
         c.skip_front = false;
         API_CUDA(dcmt::generic_run_chunk(c, st), "generic pipeline launch");
+        if (staged)
+            API_CUDA(dcmt::depth_to_u16(staged, (size_t)cols, fpix, o.u, o.pitch, o.fstride, rows, cols, nf, st), "uint16 conversion launch");
     }
     return DCMT_OK;
 }
@@ -431,8 +457,8 @@ int run_completion(const float* sparse, const int32_t* labels, int n_clusters, b
         return rc;
     int32_t* d_flags = fused ? carve<int32_t>(ar, (size_t)n_frames) : nullptr;
     bool used = false;
-    if ((rc = enqueue_completion(cc, sparse, labels, dense, g.pitch, g.fstride, n_frames, stats, d_flags, stages, stage_mask, ar,
-                                 st, &used)))
+    if ((rc = enqueue_completion(cc, sparse, labels, OutDesc{dense, nullptr, g.pitch, g.fstride}, g.pitch, g.fstride, n_frames, stats,
+                                 d_flags, stages, stage_mask, ar, st, &used)))
         return rc;
     if (!used || flags == DCMT_PATH_FUSED || flags == DCMT_PATH_GENERIC) return DCMT_OK;  // DCMT_PATH_FUSED: fully asynchronous, stats[3] = -1 marks bad frames
     // DCMT_PATH_AUTO / DCMT_PATH_RANK: read the per-frame "not served" flags back (one synchronisation per pass) and redo
@@ -455,7 +481,7 @@ int run_completion(const float* sparse, const int32_t* labels, int n_clusters, b
             if ((rc = arena_acquire(st, completion_ws_bytes(rows, cols, e - f, bilateral, want_flags, false, want_flags) + fb, &ar))) return rc;
             int32_t* run_flags = want_flags ? carve<int32_t>(ar, (size_t)(e - f)) : nullptr;
             if ((rc = enqueue_completion(cc, sparse + (size_t)f * g.fstride, guided ? labels + (size_t)f * rows * cols : nullptr,
-                                         dense + (size_t)f * g.fstride, g.pitch, g.fstride, e - f,
+                                         OutDesc{dense + (size_t)f * g.fstride, nullptr, g.pitch, g.fstride}, g.pitch, g.fstride, e - f,
                                          stats ? stats + (size_t)f * DCMT_STATS_STRIDE : nullptr, run_flags, nullptr, nullptr, ar, st, nullptr)))
                 return rc;
             if (want_flags) {
@@ -641,15 +667,18 @@ int copy_frames_h2d(void* d, size_t d_pitch_bytes, const void* h, size_t h_pitch
     return DCMT_OK;
 }
 
-int copy_frames_d2h(void* h, size_t h_pitch_bytes, size_t h_fstride_bytes, const void* d, size_t row_bytes, int rows, int nf, cudaStream_t st) {
-    if (h_pitch_bytes == row_bytes && h_fstride_bytes == row_bytes * rows) {
+// device frames are back to back with rows of d_pitch_bytes (0 = row_bytes)
+int copy_frames_d2h(void* h, size_t h_pitch_bytes, size_t h_fstride_bytes, const void* d, size_t row_bytes, int rows, int nf, cudaStream_t st,
+                    size_t d_pitch_bytes = 0) {
+    if (d_pitch_bytes == 0) d_pitch_bytes = row_bytes;
+    if (d_pitch_bytes == row_bytes && h_pitch_bytes == row_bytes && h_fstride_bytes == row_bytes * rows) {
         API_CUDA(cudaMemcpyAsync(h, d, row_bytes * rows * nf, cudaMemcpyDeviceToHost, st), "device to host copy");
     } else if (h_fstride_bytes == h_pitch_bytes * (size_t)rows) {
-        API_CUDA(cudaMemcpy2DAsync(h, h_pitch_bytes, d, row_bytes, row_bytes, (size_t)rows * nf, cudaMemcpyDeviceToHost, st), "device to host copy");
+        API_CUDA(cudaMemcpy2DAsync(h, h_pitch_bytes, d, d_pitch_bytes, row_bytes, (size_t)rows * nf, cudaMemcpyDeviceToHost, st), "device to host copy");
     } else {
         for (int f = 0; f < nf; ++f)
             API_CUDA(cudaMemcpy2DAsync(static_cast<char*>(h) + (size_t)f * h_fstride_bytes, h_pitch_bytes,
-                                       static_cast<const char*>(d) + (size_t)f * rows * row_bytes, row_bytes, row_bytes, rows,
+                                       static_cast<const char*>(d) + (size_t)f * rows * d_pitch_bytes, d_pitch_bytes, row_bytes, rows,
                                        cudaMemcpyDeviceToHost, st),
                      "device to host copy");
     }
@@ -708,7 +737,8 @@ int run_completion_host(const float* sparse, const int32_t* labels, int n_cluste
                      "host to device copy");
         if (copy_only) {
             d_out = d_in;
-        } else if ((rc2 = enqueue_completion(c2, d_in, d_lab, d_out, cols, fpix, nf, stats ? d_stats : nullptr, fused2 ? d_flags : nullptr,
+        } else if ((rc2 = enqueue_completion(c2, d_in, d_lab, OutDesc{d_out, nullptr, (size_t)cols, fpix}, cols, fpix, nf,
+                                             stats ? d_stats : nullptr, fused2 ? d_flags : nullptr,
                                              nullptr, nullptr, ar, st, nullptr))) {
             return rc2;
         }
@@ -775,47 +805,58 @@ int run_completion_host(const float* sparse, const int32_t* labels, int n_cluste
     return DCMT_OK;
 }
 
-// ---- KITTI uint16 input (main.cpp:75-82: imread(IMREAD_ANYDEPTH) + convertTo(CV_32F, 1/256) + img_completion) ----
-int validate_completion_u16(const uint16_t* sparse, float* dense, int rows, int cols, size_t in_pitch_bytes,
-                            size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames,
-                            int blur_type, int flags, Geometry* gi, Geometry* go) {
+// ---- KITTI uint16 input (main.cpp:75-82: imread(IMREAD_ANYDEPTH) + convertTo(CV_32F, 1/256) + img_completion, or
+// main_lc.cpp:159-180 + interpolate_with_superpixels), float32 or KITTI uint16 output (convertTo(CV_16U, 256) in front of
+// cv::imwrite).  `dense` is a float* or -- u16_out -- a uint16_t*.
+int validate_completion_u16(const uint16_t* sparse, const int32_t* labels, bool guided, const void* dense, bool u16_out, int rows,
+                            int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                            size_t out_frame_stride_bytes, int n_frames, int blur_type, int flags, Geometry* gi, Geometry* go) {
     if (!sparse || !dense) return fail(DCMT_E_BADARG, "null image pointer");
+    if (guided && !labels) return fail(DCMT_E_BADARG, "null label pointer");
     if (blur_type < DCMT_BLUR_NONE || blur_type > DCMT_BLUR_BILATERAL) return fail(DCMT_E_BADARG, "blur_type %d", blur_type);
     if (flags < DCMT_PATH_AUTO || flags > DCMT_PATH_RANK) return fail(DCMT_E_BADARG, "flags %d", flags);
     int rc = check_geometry(rows, cols, in_pitch_bytes, in_frame_stride_bytes, n_frames, gi, sizeof(uint16_t));
     if (rc) return rc;
-    if ((rc = check_geometry(rows, cols, out_pitch_bytes, out_frame_stride_bytes, n_frames, go, sizeof(float)))) return rc;
+    if ((rc = check_geometry(rows, cols, out_pitch_bytes, out_frame_stride_bytes, n_frames, go, u16_out ? sizeof(uint16_t) : sizeof(float))))
+        return rc;
     if (n_frames && overlaps(sparse, gi->span_bytes, dense, go->span_bytes)) return fail(DCMT_E_BADARG, "input and output overlap");
     return DCMT_OK;
 }
 
-int run_completion_u16(const uint16_t* sparse, float* dense, int rows, int cols, size_t in_pitch_bytes,
-                       size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames,
-                       int blur_type, int flags, int32_t* stats, cudaStream_t st) {
+OutDesc out_desc(void* dense, bool u16_out, const Geometry& go) {
+    return u16_out ? OutDesc{nullptr, static_cast<uint16_t*>(dense), go.pitch, go.fstride}
+                   : OutDesc{static_cast<float*>(dense), nullptr, go.pitch, go.fstride};
+}
+
+int run_completion_u16(const uint16_t* sparse, const int32_t* labels, int n_clusters, bool guided, void* dense, bool u16_out, int rows,
+                       int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                       size_t out_frame_stride_bytes, int n_frames, int blur_type, int flags, int32_t* stats, cudaStream_t st) {
     Geometry gi, go;
-    int rc = validate_completion_u16(sparse, dense, rows, cols, in_pitch_bytes, in_frame_stride_bytes, out_pitch_bytes,
-                                     out_frame_stride_bytes, n_frames, blur_type, flags, &gi, &go);
+    int rc = validate_completion_u16(sparse, labels, guided, dense, u16_out, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
+                                     out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, &gi, &go);
     if (rc) return rc;
     if (n_frames == 0) return DCMT_OK;
     if ((rc = check_device())) return rc;
     API_CUDA(dcmt::generic_configure(), "kernel attribute setup");
     API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
     // uint16 input needs no validation: AUTO and FUSED are the same thing here
-    CompletionCall cc{nullptr, 0, false, rows, cols, blur_type, flags == DCMT_PATH_GENERIC ? DCMT_PATH_GENERIC : DCMT_PATH_FUSED};
+    CompletionCall cc{labels, n_clusters, guided, rows, cols, blur_type, flags == DCMT_PATH_GENERIC ? DCMT_PATH_GENERIC : DCMT_PATH_FUSED};
     const bool fused = fused_applies(cc);
     Arena* ar = nullptr;
-    if ((rc = arena_acquire(st, completion_ws_bytes(rows, cols, n_frames, blur_type == DCMT_BLUR_BILATERAL, fused, true), &ar))) return rc;
-    return enqueue_completion(cc, nullptr, nullptr, dense, go.pitch, go.fstride, n_frames, stats, nullptr, nullptr, nullptr, ar, st,
-                              nullptr, U16Input{sparse, gi.pitch, gi.fstride});
+    if ((rc = arena_acquire(st, completion_ws_bytes(rows, cols, n_frames, blur_type == DCMT_BLUR_BILATERAL, fused, true, false, u16_out), &ar)))
+        return rc;
+    return enqueue_completion(cc, nullptr, labels, out_desc(dense, u16_out, go), 0, 0, n_frames, stats, nullptr, nullptr, nullptr, ar,
+                              st, nullptr, U16Input{sparse, gi.pitch, gi.fstride});
 }
 
-int run_completion_u16_host(const uint16_t* sparse, float* dense, int rows, int cols, size_t in_pitch_bytes,
-                            size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames,
-                            int blur_type, int flags, int32_t* stats, const int* devices = nullptr, int n_devices = 0, bool multi = false,
-                            bool copy_only = false) {
+// copy_only: the kernels left out; uint16 output echoes the input, float32 output is zeroed (dcmt_debug_host_copy_u16*)
+int run_completion_u16_host(const uint16_t* sparse, const int32_t* labels, int n_clusters, bool guided, void* dense, bool u16_out,
+                            int rows, int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                            size_t out_frame_stride_bytes, int n_frames, int blur_type, int flags, int32_t* stats,
+                            const int* devices = nullptr, int n_devices = 0, bool multi = false, bool copy_only = false) {
     Geometry gi, go;
-    int rc = validate_completion_u16(sparse, dense, rows, cols, in_pitch_bytes, in_frame_stride_bytes, out_pitch_bytes,
-                                     out_frame_stride_bytes, n_frames, blur_type, flags, &gi, &go);
+    int rc = validate_completion_u16(sparse, labels, guided, dense, u16_out, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
+                                     out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, &gi, &go);
     if (rc) return rc;
     if (n_frames == 0) return DCMT_OK;
     HostCall call;
@@ -823,14 +864,15 @@ int run_completion_u16_host(const uint16_t* sparse, float* dense, int rows, int 
     call.split(n_frames);
     const size_t fpix = (size_t)rows * cols;
     const size_t in_pitch = ((size_t)cols + 7) / 8 * 8;  // device rows 16-byte aligned: vector loads in k_q8_front
+    const size_t out_elem = u16_out ? sizeof(uint16_t) : sizeof(float);
     int longest = 0;
     for (Lane& l : call.lanes) longest = std::max(longest, l.f_end - l.f_begin);
     const int hc = host_chunk_frames(rows, cols, longest);
-    CompletionCall cc{nullptr, 0, false, rows, cols, blur_type, flags == DCMT_PATH_GENERIC ? DCMT_PATH_GENERIC : DCMT_PATH_FUSED};
+    CompletionCall cc{labels, n_clusters, guided, rows, cols, blur_type, flags == DCMT_PATH_GENERIC ? DCMT_PATH_GENERIC : DCMT_PATH_FUSED};
     const bool fused = fused_applies(cc);
-    const size_t bytes = carve_bytes((size_t)rows * in_pitch * hc, sizeof(uint16_t)) + carve_bytes(fpix * hc, sizeof(float)) +
-                         carve_bytes((size_t)hc * DCMT_STATS_STRIDE, sizeof(int32_t)) +
-                         completion_ws_bytes(rows, cols, hc, blur_type == DCMT_BLUR_BILATERAL, fused, true);
+    const size_t bytes = carve_bytes((size_t)rows * in_pitch * hc, sizeof(uint16_t)) + carve_bytes(fpix * hc, out_elem) +
+                         (guided ? carve_bytes(fpix * hc, sizeof(int32_t)) : 0) + carve_bytes((size_t)hc * DCMT_STATS_STRIDE, sizeof(int32_t)) +
+                         completion_ws_bytes(rows, cols, hc, blur_type == DCMT_BLUR_BILATERAL, fused, true, false, u16_out);
     for (Lane& l : call.lanes) {
         if (l.f_end == l.f_begin) continue;
         if ((rc = call.use(l))) return rc;
@@ -850,20 +892,29 @@ int run_completion_u16_host(const uint16_t* sparse, float* dense, int rows, int 
             Arena* ar = nullptr;
             if ((rc = arena_acquire(st, bytes, &ar))) return rc;
             uint16_t* d_in = carve<uint16_t>(ar, (size_t)rows * in_pitch * hc);
-            float* d_out = carve<float>(ar, fpix * hc);
+            void* d_out = u16_out ? static_cast<void*>(carve<uint16_t>(ar, fpix * hc)) : static_cast<void*>(carve<float>(ar, fpix * hc));
+            int32_t* d_lab = guided ? carve<int32_t>(ar, fpix * hc) : nullptr;
             int32_t* d_stats = carve<int32_t>(ar, (size_t)hc * DCMT_STATS_STRIDE);
             if ((rc = arena_ok(ar))) return rc;
             if ((rc = copy_frames_h2d(d_in, in_pitch * sizeof(uint16_t), sparse + (size_t)f0 * gi.fstride, gi.pitch * sizeof(uint16_t),
                                       gi.fstride * sizeof(uint16_t), (size_t)cols * sizeof(uint16_t), rows, nf, st)))
                 return rc;
-            if (copy_only) {
+            if (guided)
+                API_CUDA(cudaMemcpyAsync(d_lab, labels + (size_t)f0 * fpix, fpix * nf * sizeof(int32_t), cudaMemcpyHostToDevice, st),
+                         "host to device copy");
+            size_t d_pitch_bytes = (size_t)cols * out_elem;
+            if (copy_only && u16_out) {
+                d_out = d_in;
+                d_pitch_bytes = in_pitch * sizeof(uint16_t);
+            } else if (copy_only) {
                 API_CUDA(cudaMemsetAsync(d_out, 0, fpix * nf * sizeof(float), st), "memset");
-            } else if ((rc = enqueue_completion(cc, nullptr, nullptr, d_out, cols, fpix, nf, stats ? d_stats : nullptr, nullptr, nullptr,
-                                                nullptr, ar, st, nullptr, U16Input{d_in, in_pitch, (size_t)rows * in_pitch}))) {
+            } else if ((rc = enqueue_completion(cc, nullptr, d_lab, out_desc(d_out, u16_out, Geometry{(size_t)cols, fpix, 0}), 0, 0, nf,
+                                                stats ? d_stats : nullptr, nullptr, nullptr, nullptr, ar, st, nullptr,
+                                                U16Input{d_in, in_pitch, (size_t)rows * in_pitch}))) {
                 return rc;
             }
-            if ((rc = copy_frames_d2h(dense + (size_t)f0 * go.fstride, go.pitch * sizeof(float), go.fstride * sizeof(float), d_out,
-                                      (size_t)cols * sizeof(float), rows, nf, st)))
+            if ((rc = copy_frames_d2h(static_cast<char*>(dense) + (size_t)f0 * go.fstride * out_elem, go.pitch * out_elem,
+                                      go.fstride * out_elem, d_out, (size_t)cols * out_elem, rows, nf, st, d_pitch_bytes)))
                 return rc;
             if (stats && !copy_only)
                 API_CUDA(cudaMemcpyAsync(stats + (size_t)f0 * DCMT_STATS_STRIDE, d_stats, (size_t)nf * DCMT_STATS_STRIDE * sizeof(int32_t),
@@ -986,15 +1037,16 @@ int dcmt_img_completion_f32_host(const float* sparse, float* dense, int rows, in
 int dcmt_img_completion_u16(const uint16_t* sparse_u16, float* dense, int rows, int cols, size_t in_pitch_bytes,
                             size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames,
                             int blur_type, int flags, int32_t* stats, void* cuda_stream) {
-    return run_completion_u16(sparse_u16, dense, rows, cols, in_pitch_bytes, in_frame_stride_bytes, out_pitch_bytes,
-                              out_frame_stride_bytes, n_frames, blur_type, flags, stats, static_cast<cudaStream_t>(cuda_stream));
+    return run_completion_u16(sparse_u16, nullptr, 0, false, dense, false, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
+                              out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, stats,
+                              static_cast<cudaStream_t>(cuda_stream));
 }
 
 int dcmt_img_completion_u16_host(const uint16_t* sparse_u16, float* dense, int rows, int cols, size_t in_pitch_bytes,
                                  size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
                                  int n_frames, int blur_type, int flags, int32_t* stats) {
-    return run_completion_u16_host(sparse_u16, dense, rows, cols, in_pitch_bytes, in_frame_stride_bytes, out_pitch_bytes,
-                                   out_frame_stride_bytes, n_frames, blur_type, flags, stats);
+    return run_completion_u16_host(sparse_u16, nullptr, 0, false, dense, false, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
+                                   out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, stats);
 }
 
 int dcmt_img_completion_f32_host_multi(const float* sparse, float* dense, int rows, int cols, size_t pitch_bytes,
@@ -1007,8 +1059,102 @@ int dcmt_img_completion_f32_host_multi(const float* sparse, float* dense, int ro
 int dcmt_img_completion_u16_host_multi(const uint16_t* sparse_u16, float* dense, int rows, int cols, size_t in_pitch_bytes,
                                        size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
                                        int n_frames, int blur_type, int flags, int32_t* stats, const int* devices, int n_devices) {
-    return run_completion_u16_host(sparse_u16, dense, rows, cols, in_pitch_bytes, in_frame_stride_bytes, out_pitch_bytes,
-                                   out_frame_stride_bytes, n_frames, blur_type, flags, stats, devices, n_devices, true);
+    return run_completion_u16_host(sparse_u16, nullptr, 0, false, dense, false, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
+                                   out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, stats, devices, n_devices, true);
+}
+
+int dcmt_img_completion_u16_u16(const uint16_t* sparse_u16, uint16_t* dense_u16, int rows, int cols, size_t in_pitch_bytes,
+                                size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames,
+                                int blur_type, int flags, int32_t* stats, void* cuda_stream) {
+    return run_completion_u16(sparse_u16, nullptr, 0, false, dense_u16, true, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
+                              out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, stats,
+                              static_cast<cudaStream_t>(cuda_stream));
+}
+
+int dcmt_img_completion_u16_u16_host(const uint16_t* sparse_u16, uint16_t* dense_u16, int rows, int cols, size_t in_pitch_bytes,
+                                     size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
+                                     int n_frames, int blur_type, int flags, int32_t* stats) {
+    return run_completion_u16_host(sparse_u16, nullptr, 0, false, dense_u16, true, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
+                                   out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, stats);
+}
+
+int dcmt_img_completion_u16_u16_host_multi(const uint16_t* sparse_u16, uint16_t* dense_u16, int rows, int cols, size_t in_pitch_bytes,
+                                           size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
+                                           int n_frames, int blur_type, int flags, int32_t* stats, const int* devices, int n_devices) {
+    return run_completion_u16_host(sparse_u16, nullptr, 0, false, dense_u16, true, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
+                                   out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, stats, devices, n_devices, true);
+}
+
+// (a2) on KITTI uint16 input; the blur is unconditionally Gaussian in the reference (img_completion_lc.cpp:183-192)
+int dcmt_interpolate_with_superpixels_u16(const uint16_t* sparse_u16, const int32_t* labels, int n_clusters, float* dense, int rows,
+                                          int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                          size_t out_frame_stride_bytes, int n_frames, int use_superpixel, int flags, int32_t* stats,
+                                          void* cuda_stream) {
+    return run_completion_u16(sparse_u16, labels, n_clusters, use_superpixel != 0, dense, false, rows, cols, in_pitch_bytes,
+                              in_frame_stride_bytes, out_pitch_bytes, out_frame_stride_bytes, n_frames, DCMT_BLUR_GAUSSIAN, flags, stats,
+                              static_cast<cudaStream_t>(cuda_stream));
+}
+
+int dcmt_interpolate_with_superpixels_u16_host(const uint16_t* sparse_u16, const int32_t* labels, int n_clusters, float* dense, int rows,
+                                               int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                               size_t out_frame_stride_bytes, int n_frames, int use_superpixel, int flags,
+                                               int32_t* stats) {
+    return run_completion_u16_host(sparse_u16, labels, n_clusters, use_superpixel != 0, dense, false, rows, cols, in_pitch_bytes,
+                                   in_frame_stride_bytes, out_pitch_bytes, out_frame_stride_bytes, n_frames, DCMT_BLUR_GAUSSIAN, flags,
+                                   stats);
+}
+
+int dcmt_interpolate_with_superpixels_u16_host_multi(const uint16_t* sparse_u16, const int32_t* labels, int n_clusters, float* dense,
+                                                     int rows, int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes,
+                                                     size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames,
+                                                     int use_superpixel, int flags, int32_t* stats, const int* devices, int n_devices) {
+    return run_completion_u16_host(sparse_u16, labels, n_clusters, use_superpixel != 0, dense, false, rows, cols, in_pitch_bytes,
+                                   in_frame_stride_bytes, out_pitch_bytes, out_frame_stride_bytes, n_frames, DCMT_BLUR_GAUSSIAN, flags,
+                                   stats, devices, n_devices, true);
+}
+
+int dcmt_interpolate_with_superpixels_u16_u16(const uint16_t* sparse_u16, const int32_t* labels, int n_clusters, uint16_t* dense_u16,
+                                              int rows, int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes,
+                                              size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames, int use_superpixel,
+                                              int flags, int32_t* stats, void* cuda_stream) {
+    return run_completion_u16(sparse_u16, labels, n_clusters, use_superpixel != 0, dense_u16, true, rows, cols, in_pitch_bytes,
+                              in_frame_stride_bytes, out_pitch_bytes, out_frame_stride_bytes, n_frames, DCMT_BLUR_GAUSSIAN, flags, stats,
+                              static_cast<cudaStream_t>(cuda_stream));
+}
+
+int dcmt_interpolate_with_superpixels_u16_u16_host(const uint16_t* sparse_u16, const int32_t* labels, int n_clusters,
+                                                   uint16_t* dense_u16, int rows, int cols, size_t in_pitch_bytes,
+                                                   size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
+                                                   int n_frames, int use_superpixel, int flags, int32_t* stats) {
+    return run_completion_u16_host(sparse_u16, labels, n_clusters, use_superpixel != 0, dense_u16, true, rows, cols, in_pitch_bytes,
+                                   in_frame_stride_bytes, out_pitch_bytes, out_frame_stride_bytes, n_frames, DCMT_BLUR_GAUSSIAN, flags,
+                                   stats);
+}
+
+int dcmt_interpolate_with_superpixels_u16_u16_host_multi(const uint16_t* sparse_u16, const int32_t* labels, int n_clusters,
+                                                         uint16_t* dense_u16, int rows, int cols, size_t in_pitch_bytes,
+                                                         size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                                         size_t out_frame_stride_bytes, int n_frames, int use_superpixel, int flags,
+                                                         int32_t* stats, const int* devices, int n_devices) {
+    return run_completion_u16_host(sparse_u16, labels, n_clusters, use_superpixel != 0, dense_u16, true, rows, cols, in_pitch_bytes,
+                                   in_frame_stride_bytes, out_pitch_bytes, out_frame_stride_bytes, n_frames, DCMT_BLUR_GAUSSIAN, flags,
+                                   stats, devices, n_devices, true);
+}
+
+int dcmt_depth_to_u16(const float* depth, uint16_t* out, int rows, int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes,
+                      size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames, void* cuda_stream) {
+    if (!depth || !out) return fail(DCMT_E_BADARG, "null image pointer");
+    Geometry gi, go;
+    int rc = check_geometry(rows, cols, in_pitch_bytes, in_frame_stride_bytes, n_frames, &gi, sizeof(float));
+    if (rc) return rc;
+    if ((rc = check_geometry(rows, cols, out_pitch_bytes, out_frame_stride_bytes, n_frames, &go, sizeof(uint16_t)))) return rc;
+    if (n_frames && overlaps(depth, gi.span_bytes, out, go.span_bytes)) return fail(DCMT_E_BADARG, "input and output overlap");
+    if (n_frames == 0) return DCMT_OK;
+    if ((rc = check_device())) return rc;
+    API_CUDA(dcmt::depth_to_u16(depth, gi.pitch, gi.fstride, out, go.pitch, go.fstride, rows, cols, n_frames,
+                                static_cast<cudaStream_t>(cuda_stream)),
+             "uint16 conversion launch");
+    return DCMT_OK;
 }
 
 int dcmt_interpolate_with_superpixels_f32_host_multi(const float* sparse, const int32_t* labels, int n_clusters, float* dense, int rows,
@@ -1024,8 +1170,13 @@ int dcmt_debug_host_copy_f32(const float* in, float* out, int rows, int cols, in
 }
 
 int dcmt_debug_host_copy_u16(const uint16_t* in, float* out, int rows, int cols, int n_frames, const int* devices, int n_devices) {
-    return run_completion_u16_host(in, out, rows, cols, 0, 0, 0, 0, n_frames, DCMT_BLUR_NONE, DCMT_PATH_AUTO, nullptr, devices, n_devices,
-                                   devices != nullptr || n_devices != 0, true);
+    return run_completion_u16_host(in, nullptr, 0, false, out, false, rows, cols, 0, 0, 0, 0, n_frames, DCMT_BLUR_NONE, DCMT_PATH_AUTO,
+                                   nullptr, devices, n_devices, devices != nullptr || n_devices != 0, true);
+}
+
+int dcmt_debug_host_copy_u16_u16(const uint16_t* in, uint16_t* out, int rows, int cols, int n_frames, const int* devices, int n_devices) {
+    return run_completion_u16_host(in, nullptr, 0, false, out, true, rows, cols, 0, 0, 0, 0, n_frames, DCMT_BLUR_NONE, DCMT_PATH_AUTO,
+                                   nullptr, devices, n_devices, devices != nullptr || n_devices != 0, true);
 }
 
 int dcmt_interpolate_with_superpixels_ex_f32(const float* sparse, const int32_t* labels, int n_clusters, float* dense, int rows,
@@ -1100,7 +1251,7 @@ int dcmt_debug_q8_phase_cycles(const float* sparse, float* dense, int rows, int 
     p.prof_tail = tail_stamps;
     if (tiles_per_frame) *tiles_per_frame = ((cols + p.tw - 1) / p.tw) * ((rows + p.th - 1) / p.th);
     API_CUDA(dcmt::q8_run_front(p, sparse, nullptr, cols, fpix, n_frames, 1, st), "fused front launch");
-    API_CUDA(dcmt::q8_run_tail(p, dense, cols, fpix, n_frames, DCMT_BLUR_GAUSSIAN, st), "fused tail launch");
+    API_CUDA(dcmt::q8_run_tail(p, dense, nullptr, cols, fpix, n_frames, DCMT_BLUR_GAUSSIAN, st), "fused tail launch");
     return DCMT_OK;
 }
 

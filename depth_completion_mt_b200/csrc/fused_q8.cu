@@ -1155,8 +1155,8 @@ struct TailArgs {
     const uint32_t* col_first;
     const uint32_t* col_last;
     FrameCounters* ctr;
-    float* out;
-    size_t out_pitch, out_fstride;
+    void* out;                      // float32, or KITTI uint16 for k_q8_tail<false, true>
+    size_t out_pitch, out_fstride;  // elements of the output type
     int rows, cols, th, tw, blur, vec_ok;
     int one;          // the constant 1, opaque to the compiler (see other_of_pair)
     int use_tma;      // tile load by one TMA box copy (else 16-byte cp.async per thread)
@@ -1221,6 +1221,10 @@ __device__ __forceinline__ float finish_px(uint32_t o) {
     return fmaf(__uint_as_float(0x4b000000u + o), 1.0f / 65536.0f, -128.0f);
 }
 
+// q16 output value -> KITTI uint16 (metres * 256): o / 256 rounded half to even, i.e. cvRound(finish_px(o) * 256) (< 2^15,
+// no saturation needed).  With blur none o = 6553600 - 256 (e - 1), so u = 25600 - (e - 1) and u / 256 == finish_px(o).
+__device__ __forceinline__ uint32_t finish_u16(uint32_t o) { return (o + 127u + ((o >> 8) & 1u)) >> 8; }
+
 // 31-wide horizontal max of the vertical maxima for word w of row r (B holds 16-row maxima: rows r-15..r and r..r+15)
 __device__ __forceinline__ uint32_t hmax31(const uint32_t* __restrict__ B, int pitchw, int r, int w) {
     const uint32_t* b0 = B + (r - 15) * pitchw + w;
@@ -1267,8 +1271,10 @@ __device__ __forceinline__ void median_step(MedianRun& m, const PackedOps& ops, 
     if (two) o[pitchw] = rank5_of_6_5(ops, qq, m.E);
 }
 
-template <bool kRank>
+// kU16 (strict q8 only): a.out receives KITTI uint16 instead of float32
+template <bool kRank, bool kU16 = false>
 __global__ void __launch_bounds__(QTT, DCMT_TAIL_CTAS) k_q8_tail(TailArgs a, const __grid_constant__ TensorMap3D tmap) {
+    static_assert(!(kRank && kU16), "uint16 output is served on strict-q8 frames only");
     DCMT_DYN_SMEM(uint32_t, smem);
     const int th = a.th, tw = a.tw, rows = a.rows, cols = a.cols;
     const int RH = th + 2 * TV, RQ = tw / 8 + 2 * TQ, pitchw = RQ * 4;
@@ -1642,7 +1648,6 @@ __global__ void __launch_bounds__(QTT, DCMT_TAIL_CTAS) k_q8_tail(TailArgs a, con
 #endif
     __syncthreads();
     DCMT_STAMP(a, 7);
-    float* out = a.out + (size_t)slot * a.out_fstride;
     // ---- BORDER_REFLECT_101 for the Gaussian (:179): mirror the median image into the 2 cells beyond each edge.
     //      Columns beyond the edge (rows inside) and whole rows beyond the edge; both read in-image cells only (row and
     //      column mirrored at once), so no barrier is needed between the two loops.
@@ -1675,6 +1680,7 @@ __global__ void __launch_bounds__(QTT, DCMT_TAIL_CTAS) k_q8_tail(TailArgs a, con
         //      [.0625 .25 .375 .25 .0625], rows then columns (:176-179) -- masked copy (:181-188: every pixel is valid here),
         //      final inversion (:191-202).  Every pixel is decoded ONCE (a gather from the LUT in global memory) into a float
         //      plane that takes the place of plane A, dead since the median; it holds half the tile's rows at a time.
+        float* out = static_cast<float*>(a.out) + (size_t)slot * a.out_fstride;
         const float* lut = a.lut + (size_t)slot * kRankMaxValid;
         const uint32_t eh = a.e_hundred;
         // (cells of the tile that lie outside the image hold 0 / stale codes and only feed outputs that are never stored: the
@@ -1752,14 +1758,17 @@ __global__ void __launch_bounds__(QTT, DCMT_TAIL_CTAS) k_q8_tail(TailArgs a, con
     //      come straight from the packed words with 16-bit x 8-bit dot products (IDP.2A), the vertical combination
     //      runs on those 32-bit sums in registers.  Every pixel is valid here (a frame with holes left is redone by
     //      k_q8_fixup), so the masked copy (:181-188) always takes the blurred value and the inversion always
-    //      applies:  out16 = 6553600 - (g - 256)  with e = q + 1 and weights summing to 256.
+    //      applies:  out16 = 6553600 - (g - 256)  with e = q + 1 and weights summing to 256.  kU16: the same value as
+    //      KITTI uint16 (finish_u16), 8-byte stores.
     {
+        float* out = static_cast<float*>(a.out) + (size_t)slot * a.out_fstride;
+        uint16_t* out16 = static_cast<uint16_t*>(a.out) + (size_t)slot * a.out_fstride;
         const int NGR = (th + 3) / 4;  // items: tw / 4 per row of items (a.i_gauss)
         for (Items i(a.i_gauss); i.r < NGR; i.next()) {
             const int cy0 = i.r * 4, gx = x0 + i.q * 4;
             if (y0 + cy0 >= rows || gx >= cols) continue;
             const uint32_t* p = B + (TV + cy0) * pitchw + TQ * 4 + 2 * i.q;  // row cy0, first word of the pair
-            float* o = out + (size_t)(y0 + cy0) * a.out_pitch + gx;
+            const size_t o_off = (size_t)(y0 + cy0) * a.out_pitch + gx;
             uint32_t f[4][4];
             if (a.blur == 1) {
                 uint32_t h[8][4];
@@ -1790,13 +1799,25 @@ __global__ void __launch_bounds__(QTT, DCMT_TAIL_CTAS) k_q8_tail(TailArgs a, con
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
                 if (cy0 + j >= th || y0 + cy0 + j >= rows) break;  // rows past the core belong to the next tile
-                float* oj = o + (size_t)j * a.out_pitch;
-                if (gx + 4 <= cols && a.vec_ok) {
-                    *reinterpret_cast<float4*>(oj) = make_float4(finish_px(f[j][0]), finish_px(f[j][1]), finish_px(f[j][2]), finish_px(f[j][3]));
-                } else {
+                if (kU16) {
+                    uint16_t* oj = out16 + o_off + (size_t)j * a.out_pitch;
+                    if (gx + 4 <= cols && a.vec_ok) {
+                        *reinterpret_cast<uint2*>(oj) = make_uint2(finish_u16(f[j][0]) | finish_u16(f[j][1]) << 16,
+                                                                   finish_u16(f[j][2]) | finish_u16(f[j][3]) << 16);
+                    } else {
 #pragma unroll
-                    for (int c = 0; c < 4; ++c)
-                        if (gx + c < cols) oj[c] = finish_px(f[j][c]);
+                        for (int c = 0; c < 4; ++c)
+                            if (gx + c < cols) oj[c] = (uint16_t)finish_u16(f[j][c]);
+                    }
+                } else {
+                    float* oj = out + o_off + (size_t)j * a.out_pitch;
+                    if (gx + 4 <= cols && a.vec_ok) {
+                        *reinterpret_cast<float4*>(oj) = make_float4(finish_px(f[j][0]), finish_px(f[j][1]), finish_px(f[j][2]), finish_px(f[j][3]));
+                    } else {
+#pragma unroll
+                        for (int c = 0; c < 4; ++c)
+                            if (gx + c < cols) oj[c] = finish_px(f[j][c]);
+                    }
                 }
             }
         }
@@ -1809,6 +1830,33 @@ __global__ void __launch_bounds__(QTT, DCMT_TAIL_CTAS) k_q8_tail(TailArgs a, con
 __global__ void k_u16_to_f32(const uint16_t* __restrict__ in, size_t in_pitch, size_t in_fstride, float* __restrict__ out, int rows, int cols) {
     const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y, f = blockIdx.z;
     if (x < cols) out[((size_t)f * rows + y) * cols + x] = (float)in[(size_t)f * in_fstride + (size_t)y * in_pitch + x] * (1.0f / 256.0f);
+}
+
+// cv::Mat::convertTo(CV_16U, 256.0) of a CV_32FC1 depth map -- what a caller does in front of cv::imwrite of a KITTI depth
+// PNG: u = saturate_cast<uint16_t>(cvRound(v * 256)).  The product is exact (a power-of-two scaling), rounding is half to
+// even, the result is clamped to [0, 65535] and NaN gives 0.
+__device__ __forceinline__ uint32_t depth_u16(float v) {
+    const float s = v * 256.0f;
+    if (!(s > 0.0f)) return 0u;  // NaN, zeros, negatives
+    return s >= 65535.0f ? 65535u : (uint32_t)rintf(s);
+}
+
+// pitched, batched float32 -> uint16 by the rule above; a thread converts 4 pixels of a row (one 16-byte load and one
+// 8-byte store when `vec`: both layouts aligned), pixel by pixel at the ragged end.  Rows beyond the grid are strided.
+__global__ void k_depth_to_u16(const float* __restrict__ in, size_t in_pitch, size_t in_fstride, uint16_t* __restrict__ out,
+                               size_t out_pitch, size_t out_fstride, int rows, int cols, int vec) {
+    const int x = (blockIdx.x * blockDim.x + threadIdx.x) * 4, f = blockIdx.z;
+    if (x >= cols) return;
+    for (int y = blockIdx.y; y < rows; y += gridDim.y) {
+        const float* i = in + (size_t)f * in_fstride + (size_t)y * in_pitch + x;
+        uint16_t* o = out + (size_t)f * out_fstride + (size_t)y * out_pitch + x;
+        if (vec && x + 4 <= cols) {
+            const float4 v = *reinterpret_cast<const float4*>(i);
+            *reinterpret_cast<uint2*>(o) = make_uint2(depth_u16(v.x) | depth_u16(v.y) << 16, depth_u16(v.z) | depth_u16(v.w) << 16);
+        } else {
+            for (int c = 0; c < 4 && x + c < cols; ++c) o[c] = (uint16_t)depth_u16(i[c]);
+        }
+    }
 }
 
 __global__ void k_q8_zero_counters(FrameCounters* c, int n) {
@@ -1911,6 +1959,8 @@ cudaError_t q8_configure() {
     e = cudaFuncSetAttribute(k_q8_guided_front<false, GTW>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     if (e != cudaSuccess) return e;
     e = cudaFuncSetAttribute(k_q8_tail<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(k_q8_tail<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     if (e != cudaSuccess) return e;
     return cudaFuncSetAttribute(k_q8_tail<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
 }
@@ -2032,8 +2082,11 @@ cudaError_t q8_run_guided_front(const Q8Plan& plan, const float* in, const uint1
     return cudaGetLastError();
 }
 
-cudaError_t q8_run_tail(const Q8Plan& p, float* out, size_t out_pitch, size_t out_fstride, int n_frames, int blur, cudaStream_t st) {
-    const int vec2 = out_pitch % 4 == 0 && out_fstride % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0;
+cudaError_t q8_run_tail(const Q8Plan& p, float* out, uint16_t* out16, size_t out_pitch, size_t out_fstride, int n_frames, int blur,
+                        cudaStream_t st) {
+    // 4-pixel stores (16 bytes of float32 / 8 bytes of uint16) need every row start aligned to their size
+    const int vec2 = out_pitch % 4 == 0 && out_fstride % 4 == 0 &&
+                     (out16 ? (reinterpret_cast<uintptr_t>(out16) & 7) : (reinterpret_cast<uintptr_t>(out) & 15)) == 0;
     const int RQ = p.tw / 8 + 2 * TQ, RH = p.th + 2 * TV, SQ = p.tw / 8 + 2, MI = (p.tw / 2 + 2 + 3) / 4, NP = p.tw / 4;
     // shared-work median: word columns x runs of an even number of rows.  A run starts with four extra row sorts and a pair
     // merge, so longer runs execute fewer instructions while shorter ones keep more threads busy; measured on the B200 at the
@@ -2055,12 +2108,14 @@ cudaError_t q8_run_tail(const Q8Plan& p, float* out, size_t out_pitch, size_t ou
     TensorMap3D tmap{};
     const int use_tma = !tma_disabled() && tma_encode_u16_3d(&tmap, p.mid, p.cols, p.rows, p.max_frames, (size_t)p.mid_pitch * 2,
                                                      (size_t)p.mid_pitch * p.rows * 2, RQ * 8, RH) == cudaSuccess;
-    TailArgs a{p.mid, (size_t)p.mid_pitch, (size_t)p.mid_pitch * p.rows, p.col_first, p.col_last, p.ctr, out, out_pitch,
+    TailArgs a{p.mid, (size_t)p.mid_pitch, (size_t)p.mid_pitch * p.rows, p.col_first, p.col_last, p.ctr,
+               out16 ? static_cast<void*>(out16) : static_cast<void*>(out), out_pitch,
                out_fstride, p.rows, p.cols, p.th, p.tw, blur, vec2, 1, use_tma,
                make_items(RQ, QTT), make_items(RQ * 4, QTT), make_items(SQ, QTT), make_items(SQ * 4, QTT), make_items(MI, QTT),
                make_items(NP, QTT), make_items(RQ * 2, QTT), make_items(NW, QTT), med_len, med_segs, p.lut ? kRankHundred : E_HUNDRED, p.lut, p.prof_tail};
     const dim3 grid((p.cols + p.tw - 1) / p.tw, (p.rows + p.th - 1) / p.th, n_frames);
     if (p.lut) DCMT_LAUNCH(k_q8_tail<true>, grid, dim3(QTT), q8_tail_smem(p.th, p.tw), st, a, tmap);
+    else if (out16) DCMT_LAUNCH((k_q8_tail<false, true>), grid, dim3(QTT), q8_tail_smem(p.th, p.tw), st, a, tmap);
     else DCMT_LAUNCH(k_q8_tail<false>, grid, dim3(QTT), q8_tail_smem(p.th, p.tw), st, a, tmap);
     return cudaGetLastError();
 }
@@ -2079,6 +2134,21 @@ cudaError_t q8_convert_u16(const uint16_t* in, size_t in_pitch, size_t in_fstrid
                            cudaStream_t st) {
     DCMT_LAUNCH(k_u16_to_f32, dim3((cols + 255) / 256, rows, n_frames), dim3(256), 0, st, in, in_pitch, in_fstride, out, rows, cols);
     return cudaGetLastError();
+}
+
+cudaError_t depth_to_u16(const float* in, size_t in_pitch, size_t in_fstride, uint16_t* out, size_t out_pitch, size_t out_fstride,
+                         int rows, int cols, int n_frames, cudaStream_t st) {
+    const int vec = in_pitch % 4 == 0 && in_fstride % 4 == 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0 && out_pitch % 4 == 0 &&
+                    out_fstride % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 7) == 0;
+    const unsigned gx = (unsigned)((cols + 1023) / 1024), gy = (unsigned)(rows < 65535 ? rows : 65535);
+    for (int f0 = 0; f0 < n_frames; f0 += 65535) {  // grid z limit
+        const int nf = n_frames - f0 < 65535 ? n_frames - f0 : 65535;
+        DCMT_LAUNCH(k_depth_to_u16, dim3(gx, gy, nf), dim3(256), 0, st, in + (size_t)f0 * in_fstride, in_pitch, in_fstride,
+                    out + (size_t)f0 * out_fstride, out_pitch, out_fstride, rows, cols, vec);
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
 }
 
 cudaError_t q8_decode_plane(const uint16_t* mid, size_t mid_pitch, float* out, int rows, int cols, cudaStream_t st) {

@@ -49,9 +49,14 @@ size_t q8_guided_tile_flags(int rows, int cols, int th, int tw, int n_frames);
 // uint16 -> float32 metres (main.cpp:79) into a contiguous buffer, for frames served by the generic pipeline
 cudaError_t q8_convert_u16(const uint16_t* in, size_t in_pitch, size_t in_fstride, float* out, int rows, int cols, int n_frames,
                            cudaStream_t st);
-// A5..A10: plan.mid -> out (float32), blur in {none, gaussian}; then the fix-up kernel
-cudaError_t q8_run_tail(const Q8Plan& p, float* out, size_t out_pitch, size_t out_fstride, int n_frames, int blur,
+// A5..A10: plan.mid -> out (float32) or -- out16 non-null, strict q8 only (plan.lut null) -- out16 (KITTI uint16, the rule of
+// depth_to_u16); blur in {none, gaussian}.  Pitches in elements of the output type.
+cudaError_t q8_run_tail(const Q8Plan& p, float* out, uint16_t* out16, size_t out_pitch, size_t out_fstride, int n_frames, int blur,
                         cudaStream_t st);
+// float32 metres -> KITTI uint16 (cv::Mat::convertTo(CV_16U, 256.0): round half to even, clamp to [0, 65535], NaN -> 0),
+// pitched and batched; pitches in elements
+cudaError_t depth_to_u16(const float* in, size_t in_pitch, size_t in_fstride, uint16_t* out, size_t out_pitch, size_t out_fstride,
+                         int rows, int cols, int n_frames, cudaStream_t st);
 // zero the per-frame counters (what q8_run_front does itself unless plan.counters_ready)
 cudaError_t q8_zero_counters(const Q8Plan& p, int n_frames, cudaStream_t st);
 // counters -> stats[4*n] (optional) and flags[n] (1 = frame must be redone by the generic pipeline)

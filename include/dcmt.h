@@ -141,6 +141,31 @@ DCMT_API int dcmt_img_completion_u16_host(const uint16_t *sparse_u16, float *den
                                           size_t out_frame_stride_bytes, int n_frames, int blur_type, int flags,
                                           int32_t *stats_or_null);
 
+/* (a1, KITTI on-disk format in and out) the same with the output in KITTI's format as well: uint16 = metres * 256, 0 = empty
+ * -- what a caller that stores the completed map gets from convertTo(CV_16U, 256) in front of cv::imwrite, i.e. the rule of
+ * dcmt_depth_to_u16 applied to the float32 output of dcmt_img_completion_u16.  On the fused kernels the tail stores the
+ * uint16 values directly (the float32 output is an integer multiple of 2^-16 m there); with blur none the result is
+ * lossless (u / 256 equals the float32 output).  Frames the fused kernels do not serve (bilateral, frames under 32x32,
+ * DCMT_PATH_GENERIC) are completed in float32 and converted.  Pitches / frame strides in bytes (0 = dense), flags, stats
+ * and the never-synchronising behaviour as for dcmt_img_completion_u16; the host-to-device and device-to-host copies
+ * of the *_host variants both move 2 bytes per pixel. */
+DCMT_API int dcmt_img_completion_u16_u16(const uint16_t *sparse_u16, uint16_t *dense_u16, int rows, int cols, size_t in_pitch_bytes,
+                                         size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
+                                         int n_frames, int blur_type, int flags, int32_t *stats_or_null, void *cuda_stream);
+DCMT_API int dcmt_img_completion_u16_u16_host(const uint16_t *sparse_u16, uint16_t *dense_u16, int rows, int cols,
+                                              size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                              size_t out_frame_stride_bytes, int n_frames, int blur_type, int flags,
+                                              int32_t *stats_or_null);
+
+/* cv::Mat::convertTo(CV_16U, 256.0) of float32 depth maps (device pointers): u = saturate_cast<uint16_t>(cvRound(v * 256)) --
+ * the product is exact, rounding is half to even, the result is clamped to [0, 65535] and NaN gives 0.  (OpenCV's x86
+ * build gives 0 instead of 65535 where v * 256 is +inf or at least 2^31, because its cvRound overflows there; depth
+ * maps never get near that.)  For float-output callers -- the dictionary path, the stereo chain -- that store KITTI
+ * PNGs.  Pitches / frame strides in bytes (0 = dense); overlapping input and output ranges are DCMT_E_BADARG. */
+DCMT_API int dcmt_depth_to_u16(const float *depth, uint16_t *out, int rows, int cols, size_t in_pitch_bytes,
+                               size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames,
+                               void *cuda_stream);
+
 /* (e) the host-pointer entry points over several GPUs of one box: north_star's "batches are partitioned frame-wise
  * across the 8 B200s" for a C++ caller of the library (one process, one thread).  The frames of the call are split into
  * one contiguous block per device; chunks of the blocks flow H2D -> kernels -> D2H on three streams per device, all
@@ -155,6 +180,10 @@ DCMT_API int dcmt_img_completion_u16_host_multi(const uint16_t *sparse_u16, floa
                                                 size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
                                                 size_t out_frame_stride_bytes, int n_frames, int blur_type, int flags,
                                                 int32_t *stats_or_null, const int *devices_or_null, int n_devices);
+DCMT_API int dcmt_img_completion_u16_u16_host_multi(const uint16_t *sparse_u16, uint16_t *dense_u16, int rows, int cols,
+                                                    size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                                    size_t out_frame_stride_bytes, int n_frames, int blur_type, int flags,
+                                                    int32_t *stats_or_null, const int *devices_or_null, int n_devices);
 DCMT_API int dcmt_interpolate_with_superpixels_f32_host_multi(const float *sparse, const int32_t *labels, int n_clusters,
                                                               float *dense, int rows, int cols, size_t pitch_bytes,
                                                               size_t frame_stride_bytes, int n_frames, int use_superpixel,
@@ -168,6 +197,9 @@ DCMT_API int dcmt_debug_host_copy_f32(const float *in, float *out, int rows, int
                                       const int *devices_or_null, int n_devices);
 DCMT_API int dcmt_debug_host_copy_u16(const uint16_t *in, float *out, int rows, int cols, int n_frames,
                                       const int *devices_or_null, int n_devices);
+/* the uint16-in, uint16-out pipeline (dcmt_img_completion_u16_u16_host); echoes the input to the output */
+DCMT_API int dcmt_debug_host_copy_u16_u16(const uint16_t *in, uint16_t *out, int rows, int cols, int n_frames,
+                                          const int *devices_or_null, int n_devices);
 
 /* (a2) replaces interpolate_with_superpixels(Slic&, const cv::Mat&, cv::Mat&, const std::string&, int)
  * -- src/DC_lidar_camera/img_completion_lc.cpp:34-203.  `labels` is the Slic::clusters label map as
@@ -194,6 +226,44 @@ DCMT_API int dcmt_interpolate_with_superpixels_ex_f32_host(const float *sparse, 
                                                            float *dense, int rows, int cols, size_t pitch_bytes,
                                                            size_t frame_stride_bytes, int n_frames, int use_superpixel,
                                                            int flags, int32_t *stats_or_null);
+
+/* (a2, KITTI on-disk format) main_lc.cpp:159-180 + :220 in one call: the uint16 payload of the KITTI depth PNG, its
+ * convertTo(CV_32F, 1/256) and interpolate_with_superpixels.  Labels, n_clusters and use_superpixel as for
+ * dcmt_interpolate_with_superpixels_f32; pitches / frame strides in bytes (0 = dense); flags and stats as for
+ * dcmt_img_completion_u16 (uint16 input is strict q8: the fused guided front reads it directly unless n_clusters > 65535 or
+ * DCMT_PATH_GENERIC, and the call never synchronises).  The output equals dcmt_interpolate_with_superpixels_ex_f32 on
+ * sparse_u16 / 256; the _u16_u16 variants store it as KITTI uint16 by the rule of dcmt_depth_to_u16. */
+DCMT_API int dcmt_interpolate_with_superpixels_u16(const uint16_t *sparse_u16, const int32_t *labels, int n_clusters, float *dense,
+                                                   int rows, int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes,
+                                                   size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames,
+                                                   int use_superpixel, int flags, int32_t *stats_or_null, void *cuda_stream);
+DCMT_API int dcmt_interpolate_with_superpixels_u16_host(const uint16_t *sparse_u16, const int32_t *labels, int n_clusters,
+                                                        float *dense, int rows, int cols, size_t in_pitch_bytes,
+                                                        size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                                        size_t out_frame_stride_bytes, int n_frames, int use_superpixel, int flags,
+                                                        int32_t *stats_or_null);
+DCMT_API int dcmt_interpolate_with_superpixels_u16_host_multi(const uint16_t *sparse_u16, const int32_t *labels, int n_clusters,
+                                                              float *dense, int rows, int cols, size_t in_pitch_bytes,
+                                                              size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                                              size_t out_frame_stride_bytes, int n_frames, int use_superpixel,
+                                                              int flags, int32_t *stats_or_null, const int *devices_or_null,
+                                                              int n_devices);
+DCMT_API int dcmt_interpolate_with_superpixels_u16_u16(const uint16_t *sparse_u16, const int32_t *labels, int n_clusters,
+                                                       uint16_t *dense_u16, int rows, int cols, size_t in_pitch_bytes,
+                                                       size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                                       size_t out_frame_stride_bytes, int n_frames, int use_superpixel, int flags,
+                                                       int32_t *stats_or_null, void *cuda_stream);
+DCMT_API int dcmt_interpolate_with_superpixels_u16_u16_host(const uint16_t *sparse_u16, const int32_t *labels, int n_clusters,
+                                                            uint16_t *dense_u16, int rows, int cols, size_t in_pitch_bytes,
+                                                            size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                                            size_t out_frame_stride_bytes, int n_frames, int use_superpixel,
+                                                            int flags, int32_t *stats_or_null);
+DCMT_API int dcmt_interpolate_with_superpixels_u16_u16_host_multi(const uint16_t *sparse_u16, const int32_t *labels, int n_clusters,
+                                                                  uint16_t *dense_u16, int rows, int cols, size_t in_pitch_bytes,
+                                                                  size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                                                  size_t out_frame_stride_bytes, int n_frames, int use_superpixel,
+                                                                  int flags, int32_t *stats_or_null, const int *devices_or_null,
+                                                                  int n_devices);
 
 /* parameters of the stereo refinement; dcmt_stereo_params_default() fills the values hard-coded in
  * main_sl.cpp, dcmt_stereo_params_official() those of main_sl_OFFICIAL.cpp:832-918. */

@@ -86,6 +86,15 @@ inline void img_completion_u16(const MatView& sparse_u16, MatView& dense, const 
                                        sparse_u16.cols, sparse_u16.step, 0, dense.step, 0, 1, blur_code(blur_type), path, nullptr));
 }
 
+// main.cpp:75-93 followed by the caller's convertTo(png, CV_16U, 256) in front of cv::imwrite: KITTI uint16 in, KITTI uint16
+// out (metres * 256, rounded half to even; dcmt_img_completion_u16_u16).  Input and output have their own steps.
+inline void img_completion_u16_u16(const MatView& sparse_u16, MatView& dense_u16, const std::string& blur_type, int path = DCMT_PATH_AUTO) {
+    if (dense_u16.rows != sparse_u16.rows || dense_u16.cols != sparse_u16.cols || !dense_u16.data) throw std::invalid_argument("dcmt: dense view not allocated");
+    check(dcmt_img_completion_u16_u16_host(static_cast<const uint16_t*>(sparse_u16.data), static_cast<uint16_t*>(dense_u16.data),
+                                           sparse_u16.rows, sparse_u16.cols, sparse_u16.step, 0, dense_u16.step, 0, 1, blur_code(blur_type),
+                                           path, nullptr));
+}
+
 // The evaluation loops of the three programs (SURVEY.md 8f #3); GT and result must share one step.
 inline dcmt_eval_result evaluate(const MatView& GT_img, const MatView& r_img, float tolerance, int mode) {
     if (GT_img.rows != r_img.rows || GT_img.cols != r_img.cols || GT_img.step != r_img.step) throw std::invalid_argument("dcmt: evaluate needs same-shaped Mats");
@@ -127,22 +136,50 @@ inline int project_lidar(const float* points, int n_points, const float* T_row_m
 
 // img_completion_lc.cpp:34-203.  `clusters_col_major` is Slic::clusters, indexed [col][row] (:83); it is transposed
 // into the row-major int32 label map of the ABI here.  `n_centers` is slic.centers.size().
+inline std::vector<int32_t> row_major_labels(const std::vector<std::vector<int>>& clusters_col_major, int rows, int cols) {
+    if (clusters_col_major.size() < (size_t)cols) throw std::invalid_argument("dcmt: Slic::clusters has fewer columns than the image");
+    std::vector<int32_t> labels((size_t)rows * cols);
+    for (int j = 0; j < cols; ++j) {
+        if (clusters_col_major[j].size() < (size_t)rows) throw std::invalid_argument("dcmt: Slic::clusters has fewer rows than the image");
+        for (int i = 0; i < rows; ++i) labels[(size_t)i * cols + j] = clusters_col_major[j][i];
+    }
+    return labels;
+}
+
 inline void interpolate_with_superpixels(const std::vector<std::vector<int>>& clusters_col_major, size_t n_centers,
                                          const MatView& sparse, MatView& dense, const std::string& /*blur_type*/,
                                          int use_superpixel) {
     need_same_layout(sparse, dense, "interpolate_with_superpixels");
     std::vector<int32_t> labels;
-    if (use_superpixel) {
-        if (clusters_col_major.size() < (size_t)sparse.cols) throw std::invalid_argument("dcmt: Slic::clusters has fewer columns than the image");
-        labels.resize((size_t)sparse.rows * sparse.cols);
-        for (int j = 0; j < sparse.cols; ++j) {
-            if (clusters_col_major[j].size() < (size_t)sparse.rows) throw std::invalid_argument("dcmt: Slic::clusters has fewer rows than the image");
-            for (int i = 0; i < sparse.rows; ++i) labels[(size_t)i * sparse.cols + j] = clusters_col_major[j][i];
-        }
-    }
+    if (use_superpixel) labels = row_major_labels(clusters_col_major, sparse.rows, sparse.cols);
     check(dcmt_interpolate_with_superpixels_f32_host(static_cast<const float*>(sparse.data), use_superpixel ? labels.data() : nullptr,
                                                      (int)n_centers, static_cast<float*>(dense.data), sparse.rows, sparse.cols,
                                                      sparse.step, 0, 1, use_superpixel, nullptr));
+}
+
+// main_lc.cpp:159-180 + :220 in one call: the uint16 payload of the KITTI depth PNG (CV_16UC1 view, metres * 256) -> dense
+// float32 metres (interpolate_with_superpixels_u16) or KITTI uint16 (..._u16_u16, the convertTo(CV_16U, 256) of a caller that
+// writes the PNG).  Input and output have their own steps.
+inline void interpolate_with_superpixels_u16(const std::vector<std::vector<int>>& clusters_col_major, size_t n_centers,
+                                             const MatView& sparse_u16, MatView& dense, int use_superpixel, int path = DCMT_PATH_AUTO) {
+    if (dense.rows != sparse_u16.rows || dense.cols != sparse_u16.cols || !dense.data) throw std::invalid_argument("dcmt: dense view not allocated");
+    std::vector<int32_t> labels;
+    if (use_superpixel) labels = row_major_labels(clusters_col_major, sparse_u16.rows, sparse_u16.cols);
+    check(dcmt_interpolate_with_superpixels_u16_host(static_cast<const uint16_t*>(sparse_u16.data), use_superpixel ? labels.data() : nullptr,
+                                                     (int)n_centers, static_cast<float*>(dense.data), sparse_u16.rows, sparse_u16.cols,
+                                                     sparse_u16.step, 0, dense.step, 0, 1, use_superpixel, path, nullptr));
+}
+
+inline void interpolate_with_superpixels_u16_u16(const std::vector<std::vector<int>>& clusters_col_major, size_t n_centers,
+                                                 const MatView& sparse_u16, MatView& dense_u16, int use_superpixel,
+                                                 int path = DCMT_PATH_AUTO) {
+    if (dense_u16.rows != sparse_u16.rows || dense_u16.cols != sparse_u16.cols || !dense_u16.data) throw std::invalid_argument("dcmt: dense view not allocated");
+    std::vector<int32_t> labels;
+    if (use_superpixel) labels = row_major_labels(clusters_col_major, sparse_u16.rows, sparse_u16.cols);
+    check(dcmt_interpolate_with_superpixels_u16_u16_host(static_cast<const uint16_t*>(sparse_u16.data),
+                                                         use_superpixel ? labels.data() : nullptr, (int)n_centers,
+                                                         static_cast<uint16_t*>(dense_u16.data), sparse_u16.rows, sparse_u16.cols,
+                                                         sparse_u16.step, 0, dense_u16.step, 0, 1, use_superpixel, path, nullptr));
 }
 
 // ---- the stereo functions on EntryType matrices (views whose rows hold `cols` entries of kEntryBytes at the start) ----
@@ -260,16 +297,44 @@ inline void img_completion(const cv::Mat& sparse_r_img, cv::Mat& dense_r_img, co
 }
 
 // img_completion_lc.cpp:34-38.  Slic is the reference's class (slic.h:30-71): public `clusters` ([col][row]) and `centers`.
+// A CV_16UC1 input (the KITTI PNG as main_lc.cpp reads it) stands for its convertTo(CV_32F, 1.0 / 256.0) as well.
 template <class SlicT>
 inline void interpolate_with_superpixels(SlicT& slic, const cv::Mat& sparse_r_img, cv::Mat& dense_r_img, const std::string& blur_type,
                                          int use_superpixel) {
-    CV_Assert(sparse_r_img.type() == CV_32FC1);
-    const cv::Mat in = dcmt::continuous(sparse_r_img);
-    cv::Mat out(in.rows, in.cols, CV_32FC1);
+    cv::Mat out(sparse_r_img.rows, sparse_r_img.cols, CV_32FC1);
     dcmt::MatView d = dcmt::view_of(out);
-    dcmt::interpolate_with_superpixels(slic.clusters, slic.centers.size(), dcmt::view_of(in), d, blur_type, use_superpixel);
+    if (sparse_r_img.type() == CV_16UC1) {
+        dcmt::interpolate_with_superpixels_u16(slic.clusters, slic.centers.size(), dcmt::view_of(sparse_r_img), d, use_superpixel);
+    } else {
+        CV_Assert(sparse_r_img.type() == CV_32FC1);
+        const cv::Mat in = dcmt::continuous(sparse_r_img);
+        dcmt::interpolate_with_superpixels(slic.clusters, slic.centers.size(), dcmt::view_of(in), d, blur_type, use_superpixel);
+    }
     dense_r_img = out;
 }
+
+namespace dcmt {
+// KITTI PNG in, KITTI PNG payload out: img_completion on a CV_16UC1 matrix (metres * 256) whose result comes back as a fresh
+// continuous CV_16UC1 matrix -- what dense.convertTo(png, CV_16U, 256) in front of cv::imwrite gives, with half the
+// device-to-host copy.
+inline void img_completion_to_u16(const cv::Mat& sparse_u16, cv::Mat& dense_u16, const std::string& blur_type) {
+    CV_Assert(sparse_u16.type() == CV_16UC1);
+    cv::Mat out(sparse_u16.rows, sparse_u16.cols, CV_16UC1);
+    MatView d = view_of(out);
+    img_completion_u16_u16(view_of(sparse_u16), d, blur_type);
+    dense_u16 = out;
+}
+
+// the same for interpolate_with_superpixels (main_lc.cpp:159-220)
+template <class SlicT>
+inline void interpolate_with_superpixels_to_u16(SlicT& slic, const cv::Mat& sparse_u16, cv::Mat& dense_u16, int use_superpixel) {
+    CV_Assert(sparse_u16.type() == CV_16UC1);
+    cv::Mat out(sparse_u16.rows, sparse_u16.cols, CV_16UC1);
+    MatView d = view_of(out);
+    interpolate_with_superpixels_u16_u16(slic.clusters, slic.centers.size(), view_of(sparse_u16), d, use_superpixel);
+    dense_u16 = out;
+}
+}  // namespace dcmt
 
 // main_sl.cpp:715.  `img` is an EntryType matrix: cv::Mat(rows, cols, CV_32FC(sizeof(EntryType))) (:1165, :1169)
 inline void calculateMeasuementDerivatives(cv::Mat& img) {
