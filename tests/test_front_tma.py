@@ -61,11 +61,8 @@ def check_layout(lib, on_gpu, frames, pitch, offset, want_paths, what):
     for blur, name in ((GAUSSIAN, "gaussian"), (NONE, "none")):
         out, paths = run_device_entry(lib, on_gpu, frames, pitch, offset, blur)
         assert list(paths) == want_paths, f"{what}: paths {list(paths)}"
-        for f in range(len(frames)):
-            if paths[f] == 2 and name == "gaussian":  # not strict q8: redone by the generic pipeline, float32 Gaussian
-                assert np.abs(out[f] - co.img_completion(ref_in[f], name)).max() <= 1e-4, f"{what} frame {f}"
-            else:
-                assert_bit_equal(out[f], co.img_completion(ref_in[f], name), f"{what} frame {f} blur={name}")
+        for f in range(len(frames)):  # frames that are not strict q8 take the dictionary path: bit-exact as well
+            assert_bit_equal(out[f], co.img_completion(ref_in[f], name), f"{what} frame {f} blur={name}")
 
 
 def body_layouts(lib, on_gpu):

@@ -42,13 +42,13 @@ def body(lib, to_backend, sizes):
     behind[:, 0] = -np.abs(behind[:, 0]) - 1.0
     proj, nrm, cnt = api.lidar_project(to_backend(behind), T, P, 40, 60, return_count=True, lib=lib)
     assert cnt == co.lidar_project(behind, T, P, 40, 60)[2] == 0
-    # the projected image feeds the completion like main_sl.cpp:523 (float, not q8: generic pipeline)
+    # the projected image feeds the completion like main_sl.cpp:523 (float, not q8: the float32 dictionary path)
     pts = synth.velodyne_cloud(7, 40000)
     _, nrm = api.lidar_project(to_backend(pts), T, P, 96, 320, lib=lib)
     dense = api.img_completion(nrm, False, "gaussian", lib=lib)
     dn = dense if isinstance(dense, np.ndarray) else dense.cpu().numpy()
     ref = co.img_completion(co.lidar_project(pts, T, P, 96, 320)[1], "gaussian")
-    assert np.abs(dn - ref).max() <= 1e-4
+    assert_bit_equal(dn, ref, "completion of the normalised projection")
 
 
 def test_emu_project(emu_lib):
