@@ -102,32 +102,23 @@ int arena_ok(const Arena* a) {
 }
 size_t carve_bytes(size_t count, size_t elem) { return (count * elem + 255) & ~size_t(255); }
 
-// frames per generic chunk: a 2^27-pixel budget split evenly (313 KITTI frames, 1 GB of float scratch).  Larger grids
-// beat L2 residency of the two float planes here as well (20-frame chunks were 10 % slower).
-int generic_chunk_frames(int rows, int cols, int n_frames) {
-    static const long env = [] {
-        const char* s = getenv("DCMT_GENERIC_CHUNK");
-        return s ? atol(s) : 0L;
-    }();
-    long cap = env > 0 ? env : (long)(((size_t)1 << 27) / ((size_t)rows * cols));
-    if (cap < 1) cap = 1;
-    if (cap > 65535) cap = 65535;
-    const long nchunks = (n_frames + cap - 1) / cap;
-    long c = nchunks > 0 ? (n_frames + nchunks - 1) / nchunks : 1;
-    if (c < 1) c = 1;
-    return (int)c;
+long env_long(const char* name) {
+    const char* s = getenv(name);
+    return s ? atol(s) : 0L;
 }
 
-// frames per fused chunk: as many as a 2^28-pixel budget allows (627 KITTI frames; about 0.5 GB of uint16 intermediate
-// plus 2 GB of fix-up scratch), split evenly.  Large grids matter more than L2 residency of the intermediate plane:
-// the kernels are issue-bound (DRAM a few per cent busy), while every launch ends in a partially filled wave
-// (79-frame chunks: 8.5 waves per launch, 11 % slower end to end than 512-frame chunks on the B200).
-int fused_chunk_frames(int rows, int cols, int n_frames) {
-    static const long env = [] {
-        const char* s = getenv("DCMT_FUSED_CHUNK");
-        return s ? atol(s) : 0L;
-    }();
-    long cap = env > 0 ? env : (long)(((size_t)1 << 28) / ((size_t)rows * cols));
+// Frames per chunk: as many as a pixel budget allows (DCMT_FUSED_CHUNK / DCMT_GENERIC_CHUNK override it with a frame
+// count), split evenly.
+// - fused path, 2^28 pixels (627 KITTI frames; about 0.5 GB of uint16 intermediate plus 2 GB of fix-up scratch).  Large
+//   grids matter more than L2 residency of the intermediate plane: the kernels are issue-bound (DRAM a few per cent
+//   busy), while every launch ends in a partially filled wave (79-frame chunks: 8.5 waves per launch, 11 % slower end to
+//   end than 512-frame chunks on the B200).
+// - generic pipeline, 2^27 pixels (313 KITTI frames, 1 GB of float scratch).  Larger grids beat L2 residency of the two
+//   float planes here as well (20-frame chunks were 10 % slower).
+int chunk_frames(int rows, int cols, int n_frames, bool fused) {
+    static const long fused_env = env_long("DCMT_FUSED_CHUNK"), generic_env = env_long("DCMT_GENERIC_CHUNK");
+    const long env = fused ? fused_env : generic_env;
+    long cap = env > 0 ? env : (long)(((size_t)1 << (fused ? 28 : 27)) / ((size_t)rows * cols));
     if (cap < 1) cap = 1;
     if (cap > 65535) cap = 65535;
     const long nchunks = (n_frames + cap - 1) / cap;
@@ -195,7 +186,7 @@ cudaError_t prof_mark(cudaStream_t st, int which, ProfEvents* pe) {
     return cudaEventRecord(pe->e[which], st);
 }
 
-// validated description of one completion call
+// one completion call as its entry point describes it (checked by validate_completion)
 struct CompletionCall {
     const int32_t* labels;
     int n_clusters;
@@ -214,46 +205,29 @@ bool fused_applies(const CompletionCall& cc) {
            (!cc.guided || dcmt::q8_guided_smem(th, tw) <= 200 * 1024);
 }
 
-size_t completion_ws_bytes(int rows, int cols, int n_frames, bool bilateral, bool fused, bool u16_in = false, bool rank = false,
-                           bool u16_out = false) {
-    const int chunk = fused ? fused_chunk_frames(rows, cols, n_frames) : generic_chunk_frames(rows, cols, n_frames);
-    size_t b = generic_ws_bytes(rows, cols, chunk, bilateral);
-    if (fused && rank) {  // dictionary, its sizes, the code plane (rank_f32.cu)
-        const size_t code_pitch = ((size_t)cols + 7) / 8 * 8;
-        b += carve_bytes((size_t)dcmt::kRankMaxValid * chunk, sizeof(float)) + carve_bytes((size_t)chunk, sizeof(int)) +
-             carve_bytes((size_t)rows * code_pitch * chunk, sizeof(uint16_t));
+// One side of a completion call: float32 metres (`f`) or KITTI uint16, metres * 256 (`u`; main.cpp:75-82 on the way in,
+// the rule of dcmt_depth_to_u16 on the way out).  Pitch and frame stride are in elements; the entry points fill in the
+// ABI's bytes (0 = packed), which validate_completion checks and converts.
+struct InDesc {
+    const float* f = nullptr;
+    const uint16_t* u = nullptr;
+    size_t pitch = 0, fstride = 0;
+    size_t elem() const { return u ? sizeof(uint16_t) : sizeof(float); }
+    const void* ptr() const { return u ? static_cast<const void*>(u) : f; }
+    InDesc frames_from(size_t f0) const {
+        InDesc o = *this;
+        if (u) o.u += f0 * fstride;
+        else o.f += f0 * fstride;
+        return o;
     }
-    if (u16_in && !fused) b += carve_bytes((size_t)rows * cols * chunk, sizeof(float));
-    if (u16_out && !fused) b += carve_bytes((size_t)rows * cols * chunk, sizeof(float));  // float plane in front of depth_to_u16
-    if (fused) {
-        const size_t mid_pitch = ((size_t)cols + 7) / 8 * 8;
-        b += carve_bytes((size_t)rows * mid_pitch * chunk, sizeof(uint16_t)) + 2 * carve_bytes(mid_pitch * chunk, sizeof(uint32_t));
-        b += carve_bytes(((size_t)rows / 8 + 1) * ((size_t)cols / 8 + 1) * chunk, sizeof(int));  // tile flags of the guided front (upper bound)
-    }
-    return b;
-}
-
-// Enqueue n_frames through the pipeline; every pointer is a device pointer, the workspace is carved from `ar`.
-// Never synchronises.  On the fused path `redo_flags` (device, one int32 per frame, optional) receives 1 for
-// frames that turned out not to be strict q8: their output is NOT valid and the caller must redo them with
-// DCMT_PATH_GENERIC.  *used_fused tells the caller which path ran.
-//
-// Input is either float32 metres (`sparse`, `pitch` / `fstride` in elements) or -- `in16.p` non-null -- KITTI
-// uint16 (metres * 256, main.cpp:75-82) with its own pitch / frame stride in elements.  uint16 input is strict q8 by
-// construction: the fused kernels read it directly and nothing is validated or redone; shapes the fused kernels do
-// not serve get a convertTo(CV_32F, 1/256) (main.cpp:79) into a workspace plane in front of the generic pipeline.
-struct U16Input {
-    const uint16_t* p = nullptr;
-    size_t pitch = 0, fstride = 0;  // elements
 };
 
-// Output is float32 metres or -- `out.u` non-null, uint16 input only -- KITTI uint16 (metres * 256, the rule of
-// dcmt_depth_to_u16): the fused tail stores it directly; the generic pipeline writes a float workspace plane that
-// depth_to_u16 converts.
 struct OutDesc {
     float* f = nullptr;
     uint16_t* u = nullptr;
-    size_t pitch = 0, fstride = 0;  // elements of the output type
+    size_t pitch = 0, fstride = 0;
+    size_t elem() const { return u ? sizeof(uint16_t) : sizeof(float); }
+    void* ptr() const { return u ? static_cast<void*>(u) : f; }
     OutDesc frames_from(size_t f0) const {
         OutDesc o = *this;
         if (u) o.u += f0 * fstride;
@@ -262,14 +236,82 @@ struct OutDesc {
     }
 };
 
-int enqueue_completion(const CompletionCall& cc, const float* sparse, const int32_t* labels, const OutDesc& out, size_t pitch,
-                       size_t fstride, int n_frames, int32_t* stats, int32_t* redo_flags, float* stages,
-                       uint32_t* stage_mask, Arena* ar, cudaStream_t st, bool* used_fused, U16Input in16 = U16Input{}) {
+// The fused path's buffers for chunks of `chunk` frames, next to the generic pipeline's scratch (fix-up planes and
+// counters, shared): the uint16 intermediate plane and its column keys, the tile flags of the guided front and -- on
+// DCMT_PATH_RANK -- the per-frame dictionary, its sizes and the code plane (rank_f32.cu).  fused_ws_bytes() sizes what
+// carve_fused() takes, the tile flags for 8 x 8 tiles: a bound for every tile choice.
+struct FusedWork {
+    dcmt::Q8Plan p{};
+    int* tile_flags = nullptr;
+    float* lut = nullptr;
+    int* lut_count = nullptr;
+    uint16_t* codes = nullptr;
+};
+
+size_t pad8(int cols) { return ((size_t)cols + 7) / 8 * 8; }
+
+size_t fused_ws_bytes(int rows, int cols, int chunk, bool guided, bool rank) {
+    const size_t mp = pad8(cols);
+    size_t b = carve_bytes((size_t)rows * mp * chunk, sizeof(uint16_t)) + 2 * carve_bytes(mp * chunk, sizeof(uint32_t));
+    if (guided) b += carve_bytes(((size_t)rows / 8 + 1) * ((size_t)cols / 8 + 1) * chunk, sizeof(int));
+    if (rank)
+        b += carve_bytes((size_t)dcmt::kRankMaxValid * chunk, sizeof(float)) + carve_bytes((size_t)chunk, sizeof(int)) +
+             carve_bytes((size_t)rows * mp * chunk, sizeof(uint16_t));
+    return b;
+}
+
+FusedWork carve_fused(Arena* ar, int rows, int cols, int chunk, bool guided, bool rank, float* w1, float* w2, dcmt::FrameCounters* ctr) {
+    FusedWork w;
+    dcmt::Q8Plan& p = w.p;
+    p.rows = rows;
+    p.cols = cols;
+    dcmt::q8_choose_tile(rows, cols, &p.th, &p.tw);
+    p.mid_pitch = (int)pad8(cols);
+    p.max_frames = chunk;
+    p.mid = carve<uint16_t>(ar, (size_t)rows * p.mid_pitch * chunk);
+    p.col_first = carve<uint32_t>(ar, (size_t)p.mid_pitch * chunk);
+    p.col_last = carve<uint32_t>(ar, (size_t)p.mid_pitch * chunk);
+    p.ctr = ctr;
+    p.w1 = w1;
+    p.w2 = w2;
+    if (guided) w.tile_flags = carve<int>(ar, dcmt::q8_guided_tile_flags(rows, cols, p.th, p.tw, chunk));
+    if (rank) {
+        w.lut = carve<float>(ar, (size_t)dcmt::kRankMaxValid * chunk);
+        w.lut_count = carve<int>(ar, (size_t)chunk);
+        w.codes = carve<uint16_t>(ar, (size_t)rows * p.mid_pitch * chunk);
+        p.codes_in = 1;
+        p.counters_ready = 1;
+        p.lut = w.lut;
+    }
+    return w;
+}
+
+// device workspace of a completion call of n_frames frames (element sizes of its input and output)
+size_t completion_ws_bytes(const CompletionCall& cc, int n_frames, size_t in_elem, size_t out_elem) {
+    const bool fused = fused_applies(cc);
+    const int chunk = chunk_frames(cc.rows, cc.cols, n_frames, fused);
+    const size_t b = generic_ws_bytes(cc.rows, cc.cols, chunk, cc.blur == DCMT_BLUR_BILATERAL);
+    if (fused) return b + fused_ws_bytes(cc.rows, cc.cols, chunk, cc.guided, cc.flags == DCMT_PATH_RANK);
+    // the generic pipeline reads and writes float32: a plane in front of it for uint16 input, one behind it for uint16 output
+    const size_t plane = carve_bytes((size_t)cc.rows * cc.cols * chunk, sizeof(float));
+    return b + (in_elem == sizeof(uint16_t) ? plane : 0) + (out_elem == sizeof(uint16_t) ? plane : 0);
+}
+
+// Enqueue n_frames through the pipeline; every pointer is a device pointer, the workspace is carved from `ar`.
+// Never synchronises.  On the fused path `redo_flags` (device, one int32 per frame, optional) receives 1 for
+// frames that turned out not to be strict q8: their output is NOT valid and the caller must redo them with
+// DCMT_PATH_GENERIC.
+//
+// uint16 input is strict q8 by construction (the drivers map every path but DCMT_PATH_GENERIC to DCMT_PATH_FUSED): the
+// fused kernels read it directly and nothing is validated or redone; shapes the fused kernels do not serve get a
+// convertTo(CV_32F, 1/256) (main.cpp:79) into a workspace plane in front of the generic pipeline.  uint16 output: the
+// fused tail stores it directly; the generic pipeline writes a float workspace plane that depth_to_u16 converts.
+int enqueue_completion(const CompletionCall& cc, const InDesc& in, const int32_t* labels, const OutDesc& out, int n_frames,
+                       int32_t* stats, int32_t* redo_flags, float* stages, uint32_t* stage_mask, Arena* ar, cudaStream_t st) {
     const int rows = cc.rows, cols = cc.cols;
     const bool bilateral = cc.blur == DCMT_BLUR_BILATERAL;
     const bool fused = fused_applies(cc) && !stages;
-    const int chunk = fused ? fused_chunk_frames(rows, cols, n_frames) : generic_chunk_frames(rows, cols, n_frames);
-    if (used_fused) *used_fused = fused;
+    const int chunk = chunk_frames(rows, cols, n_frames, fused);
     const size_t fpix = (size_t)rows * cols;
     float* w1 = carve<float>(ar, fpix * chunk);
     float* w2 = carve<float>(ar, fpix * chunk);
@@ -277,62 +319,32 @@ int enqueue_completion(const CompletionCall& cc, const float* sparse, const int3
     unsigned* mm = bilateral ? carve<unsigned>(ar, 2 * (size_t)chunk) : nullptr;
     float* lut = bilateral ? carve<float>(ar, dcmt::generic_lut_floats() * chunk) : nullptr;
     if (fused) {
-        dcmt::Q8Plan p{};
-        p.rows = rows;
-        p.cols = cols;
-        dcmt::q8_choose_tile(rows, cols, &p.th, &p.tw);
-        p.mid_pitch = (cols + 7) / 8 * 8;
-        p.max_frames = chunk;
-        p.mid = carve<uint16_t>(ar, (size_t)rows * p.mid_pitch * chunk);
-        p.col_first = carve<uint32_t>(ar, (size_t)p.mid_pitch * chunk);
-        p.col_last = carve<uint32_t>(ar, (size_t)p.mid_pitch * chunk);
-        p.ctr = ctr;
-        p.w1 = w1;
-        p.w2 = w2;
-        int* tile_flags = cc.guided ? carve<int>(ar, dcmt::q8_guided_tile_flags(rows, cols, p.th, p.tw, chunk)) : nullptr;
         // DCMT_PATH_RANK: float32 frames through the per-frame dictionary (rank_f32.cu) in front of the same kernels
-        const bool rank = cc.flags == DCMT_PATH_RANK && !in16.p;
-        float* lut = rank ? carve<float>(ar, (size_t)dcmt::kRankMaxValid * chunk) : nullptr;
-        int* lut_count = rank ? carve<int>(ar, (size_t)chunk) : nullptr;
-        uint16_t* codes = rank ? carve<uint16_t>(ar, (size_t)rows * p.mid_pitch * chunk) : nullptr;
+        const bool rank = cc.flags == DCMT_PATH_RANK;
+        const FusedWork w = carve_fused(ar, rows, cols, chunk, cc.guided, rank, w1, w2, ctr);
+        const dcmt::Q8Plan& p = w.p;
         if (int rc = arena_ok(ar)) return rc;
-        if (rank) {
-            API_CUDA(dcmt::rank_configure(), "kernel attribute setup");
-            p.codes_in = 1;
-            p.counters_ready = 1;
-            p.lut = lut;
-        }
+        if (rank) API_CUDA(dcmt::rank_configure(), "kernel attribute setup");
         for (int f0 = 0; f0 < n_frames; f0 += chunk) {
             const int nf = n_frames - f0 < chunk ? n_frames - f0 : chunk;
             ProfEvents pe{};
             API_CUDA(prof_mark(st, 0, &pe), "profiling event");
+            // the front reads the dictionary codes, the uint16 input, or the float32 input (validated unless DCMT_PATH_FUSED)
+            InDesc fin = in.frames_from((size_t)f0);
             if (rank) {
                 API_CUDA(dcmt::q8_zero_counters(p, nf, st), "counter setup launch");
-                API_CUDA(dcmt::rank_build(sparse + (size_t)f0 * fstride, pitch, fstride, rows, cols, nf, lut, lut_count, codes,
-                                          (size_t)p.mid_pitch, ctr, st),
+                API_CUDA(dcmt::rank_build(fin.f, fin.pitch, fin.fstride, rows, cols, nf, w.lut, w.lut_count, w.codes, (size_t)p.mid_pitch,
+                                          ctr, st),
                          "dictionary launch");
-                if (cc.guided)
-                    API_CUDA(dcmt::q8_run_guided_front(p, nullptr, codes, (size_t)p.mid_pitch, (size_t)p.mid_pitch * rows,
-                                                       labels + (size_t)f0 * fpix, cc.n_clusters, nf, 0, tile_flags, st),
-                             "fused guided front launch");
-                else
-                    API_CUDA(dcmt::q8_run_front(p, nullptr, codes, (size_t)p.mid_pitch, (size_t)p.mid_pitch * rows, nf, 0, st),
-                             "fused front launch");
-            } else if (cc.guided && in16.p)
-                API_CUDA(dcmt::q8_run_guided_front(p, nullptr, in16.p + (size_t)f0 * in16.fstride, in16.pitch, in16.fstride,
-                                                   labels + (size_t)f0 * fpix, cc.n_clusters, nf, 0, tile_flags, st),
+                fin = InDesc{nullptr, w.codes, (size_t)p.mid_pitch, (size_t)p.mid_pitch * rows};
+            }
+            const int validate = fin.f && cc.flags != DCMT_PATH_FUSED;
+            if (cc.guided)
+                API_CUDA(dcmt::q8_run_guided_front(p, fin.f, fin.u, fin.pitch, fin.fstride, labels + (size_t)f0 * fpix, cc.n_clusters, nf,
+                                                   validate, w.tile_flags, st),
                          "fused guided front launch");
-            else if (cc.guided)
-                API_CUDA(dcmt::q8_run_guided_front(p, sparse + (size_t)f0 * fstride, nullptr, pitch, fstride, labels + (size_t)f0 * fpix,
-                                                   cc.n_clusters, nf, cc.flags != DCMT_PATH_FUSED, tile_flags, st),
-                         "fused guided front launch");
-            else if (in16.p)
-                API_CUDA(dcmt::q8_run_front(p, nullptr, in16.p + (size_t)f0 * in16.fstride, in16.pitch, in16.fstride, nf, 0, st),
-                         "fused front launch");
             else
-                API_CUDA(dcmt::q8_run_front(p, sparse + (size_t)f0 * fstride, nullptr, pitch, fstride, nf,
-                                            cc.flags != DCMT_PATH_FUSED, st),
-                         "fused front launch");
+                API_CUDA(dcmt::q8_run_front(p, fin.f, fin.u, fin.pitch, fin.fstride, nf, validate, st), "fused front launch");
             API_CUDA(prof_mark(st, 1, &pe), "profiling event");
             const OutDesc o = out.frames_from((size_t)f0);
             API_CUDA(dcmt::q8_run_tail(p, o.f, o.u, o.pitch, o.fstride, nf, cc.blur, st), "fused tail launch");
@@ -348,22 +360,22 @@ int enqueue_completion(const CompletionCall& cc, const float* sparse, const int3
         }
         return DCMT_OK;
     }
-    float* conv = in16.p ? carve<float>(ar, fpix * chunk) : nullptr;
+    float* conv = in.u ? carve<float>(ar, fpix * chunk) : nullptr;
     float* staged = out.u ? carve<float>(ar, fpix * chunk) : nullptr;
     if (int rc = arena_ok(ar)) return rc;
     for (int f0 = 0; f0 < n_frames; f0 += chunk) {
         const int nf = n_frames - f0 < chunk ? n_frames - f0 : chunk;
+        const InDesc i = in.frames_from((size_t)f0);
         dcmt::GenericChunk c{};
-        if (in16.p) {
-            API_CUDA(dcmt::q8_convert_u16(in16.p + (size_t)f0 * in16.fstride, in16.pitch, in16.fstride, conv, rows, cols, nf, st),
-                     "uint16 conversion launch");
+        if (conv) {
+            API_CUDA(dcmt::q8_convert_u16(i.u, i.pitch, i.fstride, conv, rows, cols, nf, st), "uint16 conversion launch");
             c.in = conv;
             c.in_pitch = (size_t)cols;
             c.in_fstride = fpix;
         } else {
-            c.in = sparse + (size_t)f0 * fstride;
-            c.in_pitch = pitch;
-            c.in_fstride = fstride;
+            c.in = i.f;
+            c.in_pitch = i.pitch;
+            c.in_fstride = i.fstride;
         }
         c.labels = cc.guided ? labels + (size_t)f0 * fpix : nullptr;
         c.n_clusters = cc.n_clusters;
@@ -424,50 +436,53 @@ int pinned_flags(cudaStream_t key, size_t n, int32_t** out) {
     return DCMT_OK;
 }
 
-int validate_completion(const float* sparse, const int32_t* labels, bool guided, float* dense, int rows, int cols,
-                        size_t pitch_bytes, size_t frame_stride_bytes, int n_frames, int blur_type, int flags, Geometry* g) {
-    if (!sparse || !dense) return fail(DCMT_E_BADARG, "null image pointer");
-    if (guided && !labels) return fail(DCMT_E_BADARG, "null label pointer");
-    if (blur_type < DCMT_BLUR_NONE || blur_type > DCMT_BLUR_BILATERAL) return fail(DCMT_E_BADARG, "blur_type %d", blur_type);
-    if (flags < DCMT_PATH_AUTO || flags > DCMT_PATH_RANK) return fail(DCMT_E_BADARG, "flags %d", flags);
-    int rc = check_geometry(rows, cols, pitch_bytes, frame_stride_bytes, n_frames, g);
+// Checks a completion call -- pointers, labels, blur, flags, input geometry, output geometry, overlap, in this order --
+// and converts the pitches and frame strides of `in` and `out` from the ABI's bytes into elements.
+int validate_completion(const CompletionCall& cc, InDesc* in, OutDesc* out, int n_frames) {
+    if (!in->ptr() || !out->ptr()) return fail(DCMT_E_BADARG, "null image pointer");
+    if (cc.guided && !cc.labels) return fail(DCMT_E_BADARG, "null label pointer");
+    if (cc.blur < DCMT_BLUR_NONE || cc.blur > DCMT_BLUR_BILATERAL) return fail(DCMT_E_BADARG, "blur_type %d", cc.blur);
+    if (cc.flags < DCMT_PATH_AUTO || cc.flags > DCMT_PATH_RANK) return fail(DCMT_E_BADARG, "flags %d", cc.flags);
+    Geometry gi, go;
+    int rc = check_geometry(cc.rows, cc.cols, in->pitch, in->fstride, n_frames, &gi, in->elem());
     if (rc) return rc;
-    if (n_frames && overlaps(sparse, g->span_bytes, dense, g->span_bytes)) return fail(DCMT_E_BADARG, "input and output overlap");
+    if ((rc = check_geometry(cc.rows, cc.cols, out->pitch, out->fstride, n_frames, &go, out->elem()))) return rc;
+    if (n_frames && overlaps(in->ptr(), gi.span_bytes, out->ptr(), go.span_bytes)) return fail(DCMT_E_BADARG, "input and output overlap");
+    in->pitch = gi.pitch;
+    in->fstride = gi.fstride;
+    out->pitch = go.pitch;
+    out->fstride = go.fstride;
     return DCMT_OK;
 }
 
-// device-pointer driver of (a1) and (a2)
-int run_completion(const float* sparse, const int32_t* labels, int n_clusters, bool guided, float* dense, int rows,
-                   int cols, size_t pitch_bytes, size_t frame_stride_bytes, int n_frames, int blur_type, int flags,
-                   int32_t* stats, float* stages, uint32_t* stage_mask, cudaStream_t st) {
-    Geometry g;
-    int rc = validate_completion(sparse, labels, guided, dense, rows, cols, pitch_bytes, frame_stride_bytes, n_frames,
-                                 blur_type, flags, &g);
+// uint16 input needs no validation: AUTO, RANK and FUSED are the same thing there
+int input_path(const InDesc& in, int flags) { return in.u && flags != DCMT_PATH_GENERIC ? DCMT_PATH_FUSED : flags; }
+
+// device-pointer driver of every completion entry point
+int run_completion(CompletionCall cc, InDesc in, OutDesc out, int n_frames, int32_t* stats, cudaStream_t st, float* stages = nullptr,
+                   uint32_t* stage_mask = nullptr) {
+    int rc = validate_completion(cc, &in, &out, n_frames);
     if (rc) return rc;
     if (n_frames == 0) return DCMT_OK;
     if ((rc = check_device())) return rc;
     API_CUDA(dcmt::generic_configure(), "kernel attribute setup");
     API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
-    CompletionCall cc{labels, n_clusters, guided, rows, cols, blur_type, flags};
+    cc.flags = input_path(in, cc.flags);
     const bool fused = fused_applies(cc) && !stages;
-    const bool bilateral = blur_type == DCMT_BLUR_BILATERAL;
+    const bool flagged = fused && in.f;  // float32 input on the fused path: frames the pass did not serve are flagged
     Arena* ar = nullptr;
-    const size_t flag_bytes = fused ? carve_bytes((size_t)n_frames, sizeof(int32_t)) : 0;
-    if ((rc = arena_acquire(st, completion_ws_bytes(rows, cols, n_frames, bilateral, fused, false, flags == DCMT_PATH_RANK) + flag_bytes, &ar)))
-        return rc;
-    int32_t* d_flags = fused ? carve<int32_t>(ar, (size_t)n_frames) : nullptr;
-    bool used = false;
-    if ((rc = enqueue_completion(cc, sparse, labels, OutDesc{dense, nullptr, g.pitch, g.fstride}, g.pitch, g.fstride, n_frames, stats,
-                                 d_flags, stages, stage_mask, ar, st, &used)))
-        return rc;
-    if (!used || flags == DCMT_PATH_FUSED || flags == DCMT_PATH_GENERIC) return DCMT_OK;  // DCMT_PATH_FUSED: fully asynchronous, stats[3] = -1 marks bad frames
+    const size_t flag_bytes = flagged ? carve_bytes((size_t)n_frames, sizeof(int32_t)) : 0;
+    if ((rc = arena_acquire(st, completion_ws_bytes(cc, n_frames, in.elem(), out.elem()) + flag_bytes, &ar))) return rc;
+    int32_t* d_flags = flagged ? carve<int32_t>(ar, (size_t)n_frames) : nullptr;
+    if ((rc = enqueue_completion(cc, in, cc.labels, out, n_frames, stats, d_flags, stages, stage_mask, ar, st))) return rc;
+    if (!fused || cc.flags == DCMT_PATH_FUSED || cc.flags == DCMT_PATH_GENERIC) return DCMT_OK;  // DCMT_PATH_FUSED: fully asynchronous, stats[3] = -1 marks bad frames
     // DCMT_PATH_AUTO / DCMT_PATH_RANK: read the per-frame "not served" flags back (one synchronisation per pass) and redo
     // those frames one level down: strict-q8 kernels -> dictionary (rank_f32.cu) -> generic pipeline
     int32_t* h_flags = nullptr;
     if ((rc = pinned_flags(st, (size_t)n_frames, &h_flags))) return rc;
     API_CUDA(cudaMemcpyAsync(h_flags, d_flags, (size_t)n_frames * sizeof(int32_t), cudaMemcpyDeviceToHost, st), "flag readback");
     API_CUDA(cudaStreamSynchronize(st), "kernel execution");
-    for (int level = flags == DCMT_PATH_AUTO ? DCMT_PATH_RANK : DCMT_PATH_GENERIC;; level = DCMT_PATH_GENERIC) {
+    for (int level = cc.flags == DCMT_PATH_AUTO ? DCMT_PATH_RANK : DCMT_PATH_GENERIC;; level = DCMT_PATH_GENERIC) {
         cc.flags = level;
         const bool want_flags = level == DCMT_PATH_RANK;
         bool any = false;
@@ -478,11 +493,11 @@ int run_completion(const float* sparse, const int32_t* labels, int n_clusters, b
             // the previous pass has completed (stream synchronised): the arena is free again, but it was sized for that
             // pass -- this one may need more (the generic pipeline: two float planes per frame of its chunk)
             const size_t fb = want_flags ? carve_bytes((size_t)(e - f), sizeof(int32_t)) : 0;
-            if ((rc = arena_acquire(st, completion_ws_bytes(rows, cols, e - f, bilateral, want_flags, false, want_flags) + fb, &ar))) return rc;
+            if ((rc = arena_acquire(st, completion_ws_bytes(cc, e - f, in.elem(), out.elem()) + fb, &ar))) return rc;
             int32_t* run_flags = want_flags ? carve<int32_t>(ar, (size_t)(e - f)) : nullptr;
-            if ((rc = enqueue_completion(cc, sparse + (size_t)f * g.fstride, guided ? labels + (size_t)f * rows * cols : nullptr,
-                                         OutDesc{dense + (size_t)f * g.fstride, nullptr, g.pitch, g.fstride}, g.pitch, g.fstride, e - f,
-                                         stats ? stats + (size_t)f * DCMT_STATS_STRIDE : nullptr, run_flags, nullptr, nullptr, ar, st, nullptr)))
+            if ((rc = enqueue_completion(cc, in.frames_from((size_t)f), cc.guided ? cc.labels + (size_t)f * cc.rows * cc.cols : nullptr,
+                                         out.frames_from((size_t)f), e - f, stats ? stats + (size_t)f * DCMT_STATS_STRIDE : nullptr,
+                                         run_flags, nullptr, nullptr, ar, st)))
                 return rc;
             if (want_flags) {
                 // arenas are reused by the next run of this pass in stream order; the flags leave through the pinned buffer first
@@ -667,10 +682,9 @@ int copy_frames_h2d(void* d, size_t d_pitch_bytes, const void* h, size_t h_pitch
     return DCMT_OK;
 }
 
-// device frames are back to back with rows of d_pitch_bytes (0 = row_bytes)
-int copy_frames_d2h(void* h, size_t h_pitch_bytes, size_t h_fstride_bytes, const void* d, size_t row_bytes, int rows, int nf, cudaStream_t st,
-                    size_t d_pitch_bytes = 0) {
-    if (d_pitch_bytes == 0) d_pitch_bytes = row_bytes;
+// device frames are back to back with rows of d_pitch_bytes
+int copy_frames_d2h(void* h, size_t h_pitch_bytes, size_t h_fstride_bytes, const void* d, size_t d_pitch_bytes, size_t row_bytes, int rows,
+                    int nf, cudaStream_t st) {
     if (d_pitch_bytes == row_bytes && h_pitch_bytes == row_bytes && h_fstride_bytes == row_bytes * rows) {
         API_CUDA(cudaMemcpyAsync(h, d, row_bytes * rows * nf, cudaMemcpyDeviceToHost, st), "device to host copy");
     } else if (h_fstride_bytes == h_pitch_bytes * (size_t)rows) {
@@ -685,68 +699,82 @@ int copy_frames_d2h(void* h, size_t h_pitch_bytes, size_t h_fstride_bytes, const
     return DCMT_OK;
 }
 
-// copy_only: the same buffers, chunking and streams with the kernels left out (the input is echoed to the output) --
-// the ceiling the host <-> device links put on the end-to-end rate (dcmt_debug_host_copy_*).
-int run_completion_host(const float* sparse, const int32_t* labels, int n_clusters, bool guided, float* dense, int rows,
-                        int cols, size_t pitch_bytes, size_t frame_stride_bytes, int n_frames, int blur_type, int flags,
-                        int32_t* stats, const int* devices = nullptr, int n_devices = 0, bool multi = false, bool copy_only = false) {
-    Geometry g;
-    int rc = validate_completion(sparse, labels, guided, dense, rows, cols, pitch_bytes, frame_stride_bytes, n_frames,
-                                 blur_type, flags, &g);
+// Host-pointer driver of every completion entry point.  Device staging rows are packed for float32 input and padded to
+// 16 bytes for uint16 input (vector loads in k_q8_front).
+// copy_only: the same buffers, chunking and streams with the kernels left out -- the ceiling the host <-> device links put
+// on the end-to-end rate (dcmt_debug_host_copy_*).  An output of the input's type echoes the input; a float32 output of
+// uint16 input is zeroed.
+int run_completion_host(CompletionCall cc, InDesc in, OutDesc out, int n_frames, int32_t* stats, const int* devices = nullptr,
+                        int n_devices = 0, bool multi = false, bool copy_only = false) {
+    int rc = validate_completion(cc, &in, &out, n_frames);
     if (rc) return rc;
     if (n_frames == 0) return DCMT_OK;
     HostCall call;
     if ((rc = call.open(devices, n_devices, multi))) return rc;
     call.split(n_frames);
+    const int rows = cc.rows, cols = cc.cols;
     const size_t fpix = (size_t)rows * cols;
-    const bool bilateral = blur_type == DCMT_BLUR_BILATERAL;
-    const size_t row_bytes = (size_t)cols * sizeof(float);
-    const CompletionCall cc{labels, n_clusters, guided, rows, cols, blur_type, flags};
+    const size_t in_elem = in.elem(), out_elem = out.elem();
+    const size_t d_pitch = in.u ? pad8(cols) : (size_t)cols;  // elements of a device staging row of the input
+    cc.flags = input_path(in, cc.flags);
     const bool fused = fused_applies(cc) && !copy_only;
+    const bool flagged = fused && in.f;  // float32 input on the fused path: per-frame flags, read back for the redo passes
     int longest = 0;
     for (Lane& l : call.lanes) longest = std::max(longest, l.f_end - l.f_begin);
     const int hc = host_chunk_frames(rows, cols, longest);
-    const size_t bytes = 2 * carve_bytes(fpix * hc, sizeof(float)) + (guided ? carve_bytes(fpix * hc, sizeof(int32_t)) : 0) +
-                         carve_bytes((size_t)hc * DCMT_STATS_STRIDE, sizeof(int32_t)) + carve_bytes((size_t)hc, sizeof(int32_t)) +
-                         completion_ws_bytes(rows, cols, hc, bilateral, fused, false, flags == DCMT_PATH_RANK);
     for (Lane& l : call.lanes) {
         if (l.f_end == l.f_begin) continue;
         if ((rc = call.use(l))) return rc;
         API_CUDA(dcmt::generic_configure(), "kernel attribute setup");
         API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
-        if (fused && (rc = pinned_flags(nullptr, (size_t)(l.f_end - l.f_begin), &l.h_flags))) return rc;
+        if (flagged && (rc = pinned_flags(nullptr, (size_t)(l.f_end - l.f_begin), &l.h_flags))) return rc;
     }
-    // one chunk [f0, f0 + nf) of lane l on its next stream: H2D, kernels, D2H
-    auto do_chunk = [&](Lane& l, int f0, int nf, const CompletionCall& c2, bool fused2, int hc2, size_t bytes2) -> int {
+    // one chunk [f0, f0 + nf) of lane l on its next stream: H2D, kernels, D2H; its arena is sized for chunks of hc2 frames
+    // of the pass: staging of input, output, labels, stats and flags, then the workspace
+    auto do_chunk = [&](Lane& l, int f0, int nf, const CompletionCall& c2, int hc2) -> int {
         int rc2;
         cudaStream_t st = l.hs->s[l.slot];
         l.slot = (l.slot + 1) % kHostStreams;
+        const bool flags2 = flagged && fused_applies(c2);  // the generic redo pass reports no flags
+        const size_t bytes = carve_bytes((size_t)rows * d_pitch * hc2, in_elem) + carve_bytes(fpix * hc2, out_elem) +
+                             (cc.guided ? carve_bytes(fpix * hc2, sizeof(int32_t)) : 0) +
+                             carve_bytes((size_t)hc2 * DCMT_STATS_STRIDE, sizeof(int32_t)) + (flagged ? carve_bytes((size_t)hc2, sizeof(int32_t)) : 0) +
+                             (copy_only ? 0 : completion_ws_bytes(c2, hc2, in_elem, out_elem));
         Arena* ar = nullptr;
-        if ((rc2 = arena_acquire(st, bytes2, &ar))) return rc2;  // stream order protects reuse by the chunk 3 steps later
-        float* d_in = carve<float>(ar, fpix * hc2);
-        float* d_out = carve<float>(ar, fpix * hc2);
-        int32_t* d_lab = guided ? carve<int32_t>(ar, fpix * hc2) : nullptr;
+        if ((rc2 = arena_acquire(st, bytes, &ar))) return rc2;  // stream order protects reuse by the chunk 3 steps later
+        char* d_in = carve<char>(ar, (size_t)rows * d_pitch * hc2 * in_elem);
+        char* d_out = carve<char>(ar, fpix * hc2 * out_elem);
+        int32_t* d_lab = cc.guided ? carve<int32_t>(ar, fpix * hc2) : nullptr;
         int32_t* d_stats = carve<int32_t>(ar, (size_t)hc2 * DCMT_STATS_STRIDE);
-        int32_t* d_flags = carve<int32_t>(ar, (size_t)hc2);
+        int32_t* d_flags = flagged ? carve<int32_t>(ar, (size_t)hc2) : nullptr;
         if ((rc2 = arena_ok(ar))) return rc2;
-        if ((rc2 = copy_frames_h2d(d_in, row_bytes, sparse + (size_t)f0 * g.fstride, g.pitch * sizeof(float), g.fstride * sizeof(float),
-                                   row_bytes, rows, nf, st)))
+        const InDesc hi = in.frames_from((size_t)f0);
+        if ((rc2 = copy_frames_h2d(d_in, d_pitch * in_elem, hi.ptr(), in.pitch * in_elem, in.fstride * in_elem, cols * in_elem, rows, nf, st)))
             return rc2;
-        if (guided)
-            API_CUDA(cudaMemcpyAsync(d_lab, labels + (size_t)f0 * fpix, fpix * nf * sizeof(int32_t), cudaMemcpyHostToDevice, st),
+        if (cc.guided)
+            API_CUDA(cudaMemcpyAsync(d_lab, cc.labels + (size_t)f0 * fpix, fpix * nf * sizeof(int32_t), cudaMemcpyHostToDevice, st),
                      "host to device copy");
-        if (copy_only) {
+        size_t d_out_pitch = cols;  // elements
+        if (copy_only && in_elem == out_elem) {
             d_out = d_in;
-        } else if ((rc2 = enqueue_completion(c2, d_in, d_lab, OutDesc{d_out, nullptr, (size_t)cols, fpix}, cols, fpix, nf,
-                                             stats ? d_stats : nullptr, fused2 ? d_flags : nullptr,
-                                             nullptr, nullptr, ar, st, nullptr))) {
-            return rc2;
+            d_out_pitch = d_pitch;
+        } else if (copy_only) {
+            API_CUDA(cudaMemsetAsync(d_out, 0, fpix * nf * out_elem, st), "memset");
+        } else {
+            const InDesc di = in.u ? InDesc{nullptr, reinterpret_cast<uint16_t*>(d_in), d_pitch, rows * d_pitch}
+                                   : InDesc{reinterpret_cast<float*>(d_in), nullptr, d_pitch, rows * d_pitch};
+            const OutDesc dout = out.u ? OutDesc{nullptr, reinterpret_cast<uint16_t*>(d_out), (size_t)cols, fpix}
+                                       : OutDesc{reinterpret_cast<float*>(d_out), nullptr, (size_t)cols, fpix};
+            if ((rc2 = enqueue_completion(c2, di, d_lab, dout, nf, stats ? d_stats : nullptr, flags2 ? d_flags : nullptr, nullptr, nullptr,
+                                          ar, st)))
+                return rc2;
         }
-        if (fused2)
+        if (flags2)
             API_CUDA(cudaMemcpyAsync(l.h_flags + (f0 - l.f_begin), d_flags, (size_t)nf * sizeof(int32_t), cudaMemcpyDeviceToHost, st),
                      "flag readback");
-        if ((rc2 = copy_frames_d2h(dense + (size_t)f0 * g.fstride, g.pitch * sizeof(float), g.fstride * sizeof(float), d_out, row_bytes, rows,
-                                   nf, st)))
+        const OutDesc ho = out.frames_from((size_t)f0);
+        if ((rc2 = copy_frames_d2h(ho.ptr(), out.pitch * out_elem, out.fstride * out_elem, d_out, d_out_pitch * out_elem, cols * out_elem,
+                                   rows, nf, st)))
             return rc2;
         if (stats && !copy_only)
             API_CUDA(cudaMemcpyAsync(stats + (size_t)f0 * DCMT_STATS_STRIDE, d_stats, (size_t)nf * DCMT_STATS_STRIDE * sizeof(int32_t),
@@ -762,18 +790,17 @@ int run_completion_host(const float* sparse, const int32_t* labels, int n_cluste
             if ((rc = call.use(l))) return rc;
             const int f0 = l.next, nf = std::min(hc, l.f_end - f0);
             l.next += nf;
-            if ((rc = do_chunk(l, f0, nf, cc, fused, hc, bytes))) return rc;
+            if ((rc = do_chunk(l, f0, nf, cc, hc))) return rc;
         }
     }
     if ((rc = call.finish())) return rc;
-    if (fused && (flags == DCMT_PATH_AUTO || flags == DCMT_PATH_RANK)) {
+    if (flagged && (cc.flags == DCMT_PATH_AUTO || cc.flags == DCMT_PATH_RANK)) {
         // frames the pass did not serve (not strict q8; dictionary too small) are redone one level down -- strict-q8
         // kernels -> dictionary (rank_f32.cu) -> generic pipeline -- in runs of consecutive frames, on the device that
         // served them, through the same chunk pipeline
-        for (int level = flags == DCMT_PATH_AUTO ? DCMT_PATH_RANK : DCMT_PATH_GENERIC;; level = DCMT_PATH_GENERIC) {
+        for (int level = cc.flags == DCMT_PATH_AUTO ? DCMT_PATH_RANK : DCMT_PATH_GENERIC;; level = DCMT_PATH_GENERIC) {
             CompletionCall cg = cc;
             cg.flags = level;
-            const bool lf = level == DCMT_PATH_RANK;
             bool any = false;
             // the runs are fixed before anything is enqueued: the rank pass overwrites the flags it reads
             struct Run { Lane* l; int f, e; };
@@ -791,11 +818,8 @@ int run_completion_host(const float* sparse, const int32_t* labels, int n_cluste
             for (const Run& r : runs) {
                 if ((rc = call.use(*r.l))) return rc;
                 const int hc2 = host_chunk_frames(rows, cols, r.e - r.f);
-                const size_t bytes2 = 2 * carve_bytes(fpix * hc2, sizeof(float)) + (guided ? carve_bytes(fpix * hc2, sizeof(int32_t)) : 0) +
-                                      carve_bytes((size_t)hc2 * DCMT_STATS_STRIDE, sizeof(int32_t)) + carve_bytes((size_t)hc2, sizeof(int32_t)) +
-                                      completion_ws_bytes(rows, cols, hc2, bilateral, lf, false, lf);
                 for (int f = r.f; f < r.e; f += hc2)
-                    if ((rc = do_chunk(*r.l, f, std::min(hc2, r.e - f), cg, lf, hc2, bytes2))) return rc;
+                    if ((rc = do_chunk(*r.l, f, std::min(hc2, r.e - f), cg, hc2))) return rc;
                 any = true;
             }
             if (any && (rc = call.finish())) return rc;
@@ -803,126 +827,6 @@ int run_completion_host(const float* sparse, const int32_t* labels, int n_cluste
         }
     }
     return DCMT_OK;
-}
-
-// ---- KITTI uint16 input (main.cpp:75-82: imread(IMREAD_ANYDEPTH) + convertTo(CV_32F, 1/256) + img_completion, or
-// main_lc.cpp:159-180 + interpolate_with_superpixels), float32 or KITTI uint16 output (convertTo(CV_16U, 256) in front of
-// cv::imwrite).  `dense` is a float* or -- u16_out -- a uint16_t*.
-int validate_completion_u16(const uint16_t* sparse, const int32_t* labels, bool guided, const void* dense, bool u16_out, int rows,
-                            int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
-                            size_t out_frame_stride_bytes, int n_frames, int blur_type, int flags, Geometry* gi, Geometry* go) {
-    if (!sparse || !dense) return fail(DCMT_E_BADARG, "null image pointer");
-    if (guided && !labels) return fail(DCMT_E_BADARG, "null label pointer");
-    if (blur_type < DCMT_BLUR_NONE || blur_type > DCMT_BLUR_BILATERAL) return fail(DCMT_E_BADARG, "blur_type %d", blur_type);
-    if (flags < DCMT_PATH_AUTO || flags > DCMT_PATH_RANK) return fail(DCMT_E_BADARG, "flags %d", flags);
-    int rc = check_geometry(rows, cols, in_pitch_bytes, in_frame_stride_bytes, n_frames, gi, sizeof(uint16_t));
-    if (rc) return rc;
-    if ((rc = check_geometry(rows, cols, out_pitch_bytes, out_frame_stride_bytes, n_frames, go, u16_out ? sizeof(uint16_t) : sizeof(float))))
-        return rc;
-    if (n_frames && overlaps(sparse, gi->span_bytes, dense, go->span_bytes)) return fail(DCMT_E_BADARG, "input and output overlap");
-    return DCMT_OK;
-}
-
-OutDesc out_desc(void* dense, bool u16_out, const Geometry& go) {
-    return u16_out ? OutDesc{nullptr, static_cast<uint16_t*>(dense), go.pitch, go.fstride}
-                   : OutDesc{static_cast<float*>(dense), nullptr, go.pitch, go.fstride};
-}
-
-int run_completion_u16(const uint16_t* sparse, const int32_t* labels, int n_clusters, bool guided, void* dense, bool u16_out, int rows,
-                       int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
-                       size_t out_frame_stride_bytes, int n_frames, int blur_type, int flags, int32_t* stats, cudaStream_t st) {
-    Geometry gi, go;
-    int rc = validate_completion_u16(sparse, labels, guided, dense, u16_out, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
-                                     out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, &gi, &go);
-    if (rc) return rc;
-    if (n_frames == 0) return DCMT_OK;
-    if ((rc = check_device())) return rc;
-    API_CUDA(dcmt::generic_configure(), "kernel attribute setup");
-    API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
-    // uint16 input needs no validation: AUTO and FUSED are the same thing here
-    CompletionCall cc{labels, n_clusters, guided, rows, cols, blur_type, flags == DCMT_PATH_GENERIC ? DCMT_PATH_GENERIC : DCMT_PATH_FUSED};
-    const bool fused = fused_applies(cc);
-    Arena* ar = nullptr;
-    if ((rc = arena_acquire(st, completion_ws_bytes(rows, cols, n_frames, blur_type == DCMT_BLUR_BILATERAL, fused, true, false, u16_out), &ar)))
-        return rc;
-    return enqueue_completion(cc, nullptr, labels, out_desc(dense, u16_out, go), 0, 0, n_frames, stats, nullptr, nullptr, nullptr, ar,
-                              st, nullptr, U16Input{sparse, gi.pitch, gi.fstride});
-}
-
-// copy_only: the kernels left out; uint16 output echoes the input, float32 output is zeroed (dcmt_debug_host_copy_u16*)
-int run_completion_u16_host(const uint16_t* sparse, const int32_t* labels, int n_clusters, bool guided, void* dense, bool u16_out,
-                            int rows, int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
-                            size_t out_frame_stride_bytes, int n_frames, int blur_type, int flags, int32_t* stats,
-                            const int* devices = nullptr, int n_devices = 0, bool multi = false, bool copy_only = false) {
-    Geometry gi, go;
-    int rc = validate_completion_u16(sparse, labels, guided, dense, u16_out, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
-                                     out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, &gi, &go);
-    if (rc) return rc;
-    if (n_frames == 0) return DCMT_OK;
-    HostCall call;
-    if ((rc = call.open(devices, n_devices, multi))) return rc;
-    call.split(n_frames);
-    const size_t fpix = (size_t)rows * cols;
-    const size_t in_pitch = ((size_t)cols + 7) / 8 * 8;  // device rows 16-byte aligned: vector loads in k_q8_front
-    const size_t out_elem = u16_out ? sizeof(uint16_t) : sizeof(float);
-    int longest = 0;
-    for (Lane& l : call.lanes) longest = std::max(longest, l.f_end - l.f_begin);
-    const int hc = host_chunk_frames(rows, cols, longest);
-    CompletionCall cc{labels, n_clusters, guided, rows, cols, blur_type, flags == DCMT_PATH_GENERIC ? DCMT_PATH_GENERIC : DCMT_PATH_FUSED};
-    const bool fused = fused_applies(cc);
-    const size_t bytes = carve_bytes((size_t)rows * in_pitch * hc, sizeof(uint16_t)) + carve_bytes(fpix * hc, out_elem) +
-                         (guided ? carve_bytes(fpix * hc, sizeof(int32_t)) : 0) + carve_bytes((size_t)hc * DCMT_STATS_STRIDE, sizeof(int32_t)) +
-                         completion_ws_bytes(rows, cols, hc, blur_type == DCMT_BLUR_BILATERAL, fused, true, false, u16_out);
-    for (Lane& l : call.lanes) {
-        if (l.f_end == l.f_begin) continue;
-        if ((rc = call.use(l))) return rc;
-        API_CUDA(dcmt::generic_configure(), "kernel attribute setup");
-        API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
-    }
-    for (bool more = true; more;) {
-        more = false;
-        for (Lane& l : call.lanes) {
-            if (l.next >= l.f_end) continue;
-            more = true;
-            if ((rc = call.use(l))) return rc;
-            const int f0 = l.next, nf = std::min(hc, l.f_end - f0);
-            l.next += nf;
-            cudaStream_t st = l.hs->s[l.slot];
-            l.slot = (l.slot + 1) % kHostStreams;
-            Arena* ar = nullptr;
-            if ((rc = arena_acquire(st, bytes, &ar))) return rc;
-            uint16_t* d_in = carve<uint16_t>(ar, (size_t)rows * in_pitch * hc);
-            void* d_out = u16_out ? static_cast<void*>(carve<uint16_t>(ar, fpix * hc)) : static_cast<void*>(carve<float>(ar, fpix * hc));
-            int32_t* d_lab = guided ? carve<int32_t>(ar, fpix * hc) : nullptr;
-            int32_t* d_stats = carve<int32_t>(ar, (size_t)hc * DCMT_STATS_STRIDE);
-            if ((rc = arena_ok(ar))) return rc;
-            if ((rc = copy_frames_h2d(d_in, in_pitch * sizeof(uint16_t), sparse + (size_t)f0 * gi.fstride, gi.pitch * sizeof(uint16_t),
-                                      gi.fstride * sizeof(uint16_t), (size_t)cols * sizeof(uint16_t), rows, nf, st)))
-                return rc;
-            if (guided)
-                API_CUDA(cudaMemcpyAsync(d_lab, labels + (size_t)f0 * fpix, fpix * nf * sizeof(int32_t), cudaMemcpyHostToDevice, st),
-                         "host to device copy");
-            size_t d_pitch_bytes = (size_t)cols * out_elem;
-            if (copy_only && u16_out) {
-                d_out = d_in;
-                d_pitch_bytes = in_pitch * sizeof(uint16_t);
-            } else if (copy_only) {
-                API_CUDA(cudaMemsetAsync(d_out, 0, fpix * nf * sizeof(float), st), "memset");
-            } else if ((rc = enqueue_completion(cc, nullptr, d_lab, out_desc(d_out, u16_out, Geometry{(size_t)cols, fpix, 0}), 0, 0, nf,
-                                                stats ? d_stats : nullptr, nullptr, nullptr, nullptr, ar, st, nullptr,
-                                                U16Input{d_in, in_pitch, (size_t)rows * in_pitch}))) {
-                return rc;
-            }
-            if ((rc = copy_frames_d2h(static_cast<char*>(dense) + (size_t)f0 * go.fstride * out_elem, go.pitch * out_elem,
-                                      go.fstride * out_elem, d_out, (size_t)cols * out_elem, rows, nf, st, d_pitch_bytes)))
-                return rc;
-            if (stats && !copy_only)
-                API_CUDA(cudaMemcpyAsync(stats + (size_t)f0 * DCMT_STATS_STRIDE, d_stats, (size_t)nf * DCMT_STATS_STRIDE * sizeof(int32_t),
-                                         cudaMemcpyDeviceToHost, st),
-                         "device to host copy");
-        }
-    }
-    return call.finish();
 }
 
 }  // namespace
@@ -970,7 +874,9 @@ int dcmt_release_workspaces(void) {
 
 size_t dcmt_workspace_bytes(int rows, int cols, int n_frames) {
     if (rows < 1 || cols < 1 || n_frames < 1) return 0;
-    return completion_ws_bytes(rows, cols, n_frames, true, true, true, true);  // upper bound over the paths a call may take
+    // upper bound over the paths a call may take: fused chunks, bilateral scratch, the guided front and the dictionary
+    const int chunk = chunk_frames(rows, cols, n_frames, true);
+    return generic_ws_bytes(rows, cols, chunk, true) + fused_ws_bytes(rows, cols, chunk, true, true);
 }
 
 int dcmt_profile_begin(void) {
@@ -1024,65 +930,63 @@ long long dcmt_launch_count(void) { return dcmt::g_launches.load(std::memory_ord
 int dcmt_img_completion_f32(const float* sparse, float* dense, int rows, int cols, size_t pitch_bytes,
                             size_t frame_stride_bytes, int n_frames, int blur_type, int flags, int32_t* stats,
                             void* cuda_stream) {
-    return run_completion(sparse, nullptr, 0, false, dense, rows, cols, pitch_bytes, frame_stride_bytes, n_frames, blur_type,
-                          flags, stats, nullptr, nullptr, static_cast<cudaStream_t>(cuda_stream));
+    return run_completion({nullptr, 0, false, rows, cols, blur_type, flags}, {sparse, nullptr, pitch_bytes, frame_stride_bytes},
+                          {dense, nullptr, pitch_bytes, frame_stride_bytes}, n_frames, stats, static_cast<cudaStream_t>(cuda_stream));
 }
 
 int dcmt_img_completion_f32_host(const float* sparse, float* dense, int rows, int cols, size_t pitch_bytes,
                                  size_t frame_stride_bytes, int n_frames, int blur_type, int flags, int32_t* stats) {
-    return run_completion_host(sparse, nullptr, 0, false, dense, rows, cols, pitch_bytes, frame_stride_bytes, n_frames,
-                               blur_type, flags, stats);
+    return run_completion_host({nullptr, 0, false, rows, cols, blur_type, flags}, {sparse, nullptr, pitch_bytes, frame_stride_bytes},
+                               {dense, nullptr, pitch_bytes, frame_stride_bytes}, n_frames, stats);
 }
 
 int dcmt_img_completion_u16(const uint16_t* sparse_u16, float* dense, int rows, int cols, size_t in_pitch_bytes,
                             size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames,
                             int blur_type, int flags, int32_t* stats, void* cuda_stream) {
-    return run_completion_u16(sparse_u16, nullptr, 0, false, dense, false, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
-                              out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, stats,
-                              static_cast<cudaStream_t>(cuda_stream));
+    return run_completion({nullptr, 0, false, rows, cols, blur_type, flags}, {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                          {dense, nullptr, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats, static_cast<cudaStream_t>(cuda_stream));
 }
 
 int dcmt_img_completion_u16_host(const uint16_t* sparse_u16, float* dense, int rows, int cols, size_t in_pitch_bytes,
                                  size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
                                  int n_frames, int blur_type, int flags, int32_t* stats) {
-    return run_completion_u16_host(sparse_u16, nullptr, 0, false, dense, false, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
-                                   out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, stats);
+    return run_completion_host({nullptr, 0, false, rows, cols, blur_type, flags}, {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                               {dense, nullptr, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats);
 }
 
 int dcmt_img_completion_f32_host_multi(const float* sparse, float* dense, int rows, int cols, size_t pitch_bytes,
                                        size_t frame_stride_bytes, int n_frames, int blur_type, int flags, int32_t* stats,
                                        const int* devices, int n_devices) {
-    return run_completion_host(sparse, nullptr, 0, false, dense, rows, cols, pitch_bytes, frame_stride_bytes, n_frames,
-                               blur_type, flags, stats, devices, n_devices, true);
+    return run_completion_host({nullptr, 0, false, rows, cols, blur_type, flags}, {sparse, nullptr, pitch_bytes, frame_stride_bytes},
+                               {dense, nullptr, pitch_bytes, frame_stride_bytes}, n_frames, stats, devices, n_devices, true);
 }
 
 int dcmt_img_completion_u16_host_multi(const uint16_t* sparse_u16, float* dense, int rows, int cols, size_t in_pitch_bytes,
                                        size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
                                        int n_frames, int blur_type, int flags, int32_t* stats, const int* devices, int n_devices) {
-    return run_completion_u16_host(sparse_u16, nullptr, 0, false, dense, false, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
-                                   out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, stats, devices, n_devices, true);
+    return run_completion_host({nullptr, 0, false, rows, cols, blur_type, flags}, {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                               {dense, nullptr, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats, devices, n_devices, true);
 }
 
 int dcmt_img_completion_u16_u16(const uint16_t* sparse_u16, uint16_t* dense_u16, int rows, int cols, size_t in_pitch_bytes,
                                 size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames,
                                 int blur_type, int flags, int32_t* stats, void* cuda_stream) {
-    return run_completion_u16(sparse_u16, nullptr, 0, false, dense_u16, true, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
-                              out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, stats,
-                              static_cast<cudaStream_t>(cuda_stream));
+    return run_completion({nullptr, 0, false, rows, cols, blur_type, flags}, {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                          {nullptr, dense_u16, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats, static_cast<cudaStream_t>(cuda_stream));
 }
 
 int dcmt_img_completion_u16_u16_host(const uint16_t* sparse_u16, uint16_t* dense_u16, int rows, int cols, size_t in_pitch_bytes,
                                      size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
                                      int n_frames, int blur_type, int flags, int32_t* stats) {
-    return run_completion_u16_host(sparse_u16, nullptr, 0, false, dense_u16, true, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
-                                   out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, stats);
+    return run_completion_host({nullptr, 0, false, rows, cols, blur_type, flags}, {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                               {nullptr, dense_u16, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats);
 }
 
 int dcmt_img_completion_u16_u16_host_multi(const uint16_t* sparse_u16, uint16_t* dense_u16, int rows, int cols, size_t in_pitch_bytes,
                                            size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
                                            int n_frames, int blur_type, int flags, int32_t* stats, const int* devices, int n_devices) {
-    return run_completion_u16_host(sparse_u16, nullptr, 0, false, dense_u16, true, rows, cols, in_pitch_bytes, in_frame_stride_bytes,
-                                   out_pitch_bytes, out_frame_stride_bytes, n_frames, blur_type, flags, stats, devices, n_devices, true);
+    return run_completion_host({nullptr, 0, false, rows, cols, blur_type, flags}, {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                               {nullptr, dense_u16, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats, devices, n_devices, true);
 }
 
 // (a2) on KITTI uint16 input; the blur is unconditionally Gaussian in the reference (img_completion_lc.cpp:183-192)
@@ -1090,45 +994,45 @@ int dcmt_interpolate_with_superpixels_u16(const uint16_t* sparse_u16, const int3
                                           int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
                                           size_t out_frame_stride_bytes, int n_frames, int use_superpixel, int flags, int32_t* stats,
                                           void* cuda_stream) {
-    return run_completion_u16(sparse_u16, labels, n_clusters, use_superpixel != 0, dense, false, rows, cols, in_pitch_bytes,
-                              in_frame_stride_bytes, out_pitch_bytes, out_frame_stride_bytes, n_frames, DCMT_BLUR_GAUSSIAN, flags, stats,
-                              static_cast<cudaStream_t>(cuda_stream));
+    return run_completion({labels, n_clusters, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags},
+                          {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes}, {dense, nullptr, out_pitch_bytes, out_frame_stride_bytes},
+                          n_frames, stats, static_cast<cudaStream_t>(cuda_stream));
 }
 
 int dcmt_interpolate_with_superpixels_u16_host(const uint16_t* sparse_u16, const int32_t* labels, int n_clusters, float* dense, int rows,
                                                int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
                                                size_t out_frame_stride_bytes, int n_frames, int use_superpixel, int flags,
                                                int32_t* stats) {
-    return run_completion_u16_host(sparse_u16, labels, n_clusters, use_superpixel != 0, dense, false, rows, cols, in_pitch_bytes,
-                                   in_frame_stride_bytes, out_pitch_bytes, out_frame_stride_bytes, n_frames, DCMT_BLUR_GAUSSIAN, flags,
-                                   stats);
+    return run_completion_host({labels, n_clusters, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags},
+                               {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                               {dense, nullptr, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats);
 }
 
 int dcmt_interpolate_with_superpixels_u16_host_multi(const uint16_t* sparse_u16, const int32_t* labels, int n_clusters, float* dense,
                                                      int rows, int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes,
                                                      size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames,
                                                      int use_superpixel, int flags, int32_t* stats, const int* devices, int n_devices) {
-    return run_completion_u16_host(sparse_u16, labels, n_clusters, use_superpixel != 0, dense, false, rows, cols, in_pitch_bytes,
-                                   in_frame_stride_bytes, out_pitch_bytes, out_frame_stride_bytes, n_frames, DCMT_BLUR_GAUSSIAN, flags,
-                                   stats, devices, n_devices, true);
+    return run_completion_host({labels, n_clusters, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags},
+                               {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                               {dense, nullptr, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats, devices, n_devices, true);
 }
 
 int dcmt_interpolate_with_superpixels_u16_u16(const uint16_t* sparse_u16, const int32_t* labels, int n_clusters, uint16_t* dense_u16,
                                               int rows, int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes,
                                               size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames, int use_superpixel,
                                               int flags, int32_t* stats, void* cuda_stream) {
-    return run_completion_u16(sparse_u16, labels, n_clusters, use_superpixel != 0, dense_u16, true, rows, cols, in_pitch_bytes,
-                              in_frame_stride_bytes, out_pitch_bytes, out_frame_stride_bytes, n_frames, DCMT_BLUR_GAUSSIAN, flags, stats,
-                              static_cast<cudaStream_t>(cuda_stream));
+    return run_completion({labels, n_clusters, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags},
+                          {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                          {nullptr, dense_u16, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats, static_cast<cudaStream_t>(cuda_stream));
 }
 
 int dcmt_interpolate_with_superpixels_u16_u16_host(const uint16_t* sparse_u16, const int32_t* labels, int n_clusters,
                                                    uint16_t* dense_u16, int rows, int cols, size_t in_pitch_bytes,
                                                    size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
                                                    int n_frames, int use_superpixel, int flags, int32_t* stats) {
-    return run_completion_u16_host(sparse_u16, labels, n_clusters, use_superpixel != 0, dense_u16, true, rows, cols, in_pitch_bytes,
-                                   in_frame_stride_bytes, out_pitch_bytes, out_frame_stride_bytes, n_frames, DCMT_BLUR_GAUSSIAN, flags,
-                                   stats);
+    return run_completion_host({labels, n_clusters, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags},
+                               {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                               {nullptr, dense_u16, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats);
 }
 
 int dcmt_interpolate_with_superpixels_u16_u16_host_multi(const uint16_t* sparse_u16, const int32_t* labels, int n_clusters,
@@ -1136,9 +1040,9 @@ int dcmt_interpolate_with_superpixels_u16_u16_host_multi(const uint16_t* sparse_
                                                          size_t in_frame_stride_bytes, size_t out_pitch_bytes,
                                                          size_t out_frame_stride_bytes, int n_frames, int use_superpixel, int flags,
                                                          int32_t* stats, const int* devices, int n_devices) {
-    return run_completion_u16_host(sparse_u16, labels, n_clusters, use_superpixel != 0, dense_u16, true, rows, cols, in_pitch_bytes,
-                                   in_frame_stride_bytes, out_pitch_bytes, out_frame_stride_bytes, n_frames, DCMT_BLUR_GAUSSIAN, flags,
-                                   stats, devices, n_devices, true);
+    return run_completion_host({labels, n_clusters, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags},
+                               {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                               {nullptr, dense_u16, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats, devices, n_devices, true);
 }
 
 int dcmt_depth_to_u16(const float* depth, uint16_t* out, int rows, int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes,
@@ -1160,38 +1064,41 @@ int dcmt_depth_to_u16(const float* depth, uint16_t* out, int rows, int cols, siz
 int dcmt_interpolate_with_superpixels_f32_host_multi(const float* sparse, const int32_t* labels, int n_clusters, float* dense, int rows,
                                                      int cols, size_t pitch_bytes, size_t frame_stride_bytes, int n_frames,
                                                      int use_superpixel, int flags, int32_t* stats, const int* devices, int n_devices) {
-    return run_completion_host(sparse, labels, n_clusters, use_superpixel != 0, dense, rows, cols, pitch_bytes, frame_stride_bytes,
-                               n_frames, DCMT_BLUR_GAUSSIAN, flags, stats, devices, n_devices, true);
+    return run_completion_host({labels, n_clusters, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags},
+                               {sparse, nullptr, pitch_bytes, frame_stride_bytes}, {dense, nullptr, pitch_bytes, frame_stride_bytes},
+                               n_frames, stats, devices, n_devices, true);
 }
 
 int dcmt_debug_host_copy_f32(const float* in, float* out, int rows, int cols, int n_frames, const int* devices, int n_devices) {
-    return run_completion_host(in, nullptr, 0, false, out, rows, cols, 0, 0, n_frames, DCMT_BLUR_NONE, DCMT_PATH_AUTO, nullptr, devices,
+    return run_completion_host({nullptr, 0, false, rows, cols, DCMT_BLUR_NONE, DCMT_PATH_AUTO}, {in}, {out}, n_frames, nullptr, devices,
                                n_devices, devices != nullptr || n_devices != 0, true);
 }
 
 int dcmt_debug_host_copy_u16(const uint16_t* in, float* out, int rows, int cols, int n_frames, const int* devices, int n_devices) {
-    return run_completion_u16_host(in, nullptr, 0, false, out, false, rows, cols, 0, 0, 0, 0, n_frames, DCMT_BLUR_NONE, DCMT_PATH_AUTO,
-                                   nullptr, devices, n_devices, devices != nullptr || n_devices != 0, true);
+    return run_completion_host({nullptr, 0, false, rows, cols, DCMT_BLUR_NONE, DCMT_PATH_AUTO}, {nullptr, in}, {out}, n_frames, nullptr,
+                               devices, n_devices, devices != nullptr || n_devices != 0, true);
 }
 
 int dcmt_debug_host_copy_u16_u16(const uint16_t* in, uint16_t* out, int rows, int cols, int n_frames, const int* devices, int n_devices) {
-    return run_completion_u16_host(in, nullptr, 0, false, out, true, rows, cols, 0, 0, 0, 0, n_frames, DCMT_BLUR_NONE, DCMT_PATH_AUTO,
-                                   nullptr, devices, n_devices, devices != nullptr || n_devices != 0, true);
+    return run_completion_host({nullptr, 0, false, rows, cols, DCMT_BLUR_NONE, DCMT_PATH_AUTO}, {nullptr, in}, {nullptr, out}, n_frames,
+                               nullptr, devices, n_devices, devices != nullptr || n_devices != 0, true);
 }
 
 int dcmt_interpolate_with_superpixels_ex_f32(const float* sparse, const int32_t* labels, int n_clusters, float* dense, int rows,
                                              int cols, size_t pitch_bytes, size_t frame_stride_bytes, int n_frames, int use_superpixel,
                                              int flags, int32_t* stats, void* cuda_stream) {
     // blur is unconditionally Gaussian in the reference (img_completion_lc.cpp:183-192)
-    return run_completion(sparse, labels, n_clusters, use_superpixel != 0, dense, rows, cols, pitch_bytes, frame_stride_bytes,
-                          n_frames, DCMT_BLUR_GAUSSIAN, flags, stats, nullptr, nullptr, static_cast<cudaStream_t>(cuda_stream));
+    return run_completion({labels, n_clusters, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags},
+                          {sparse, nullptr, pitch_bytes, frame_stride_bytes}, {dense, nullptr, pitch_bytes, frame_stride_bytes}, n_frames,
+                          stats, static_cast<cudaStream_t>(cuda_stream));
 }
 
 int dcmt_interpolate_with_superpixels_ex_f32_host(const float* sparse, const int32_t* labels, int n_clusters, float* dense, int rows,
                                                   int cols, size_t pitch_bytes, size_t frame_stride_bytes, int n_frames,
                                                   int use_superpixel, int flags, int32_t* stats) {
-    return run_completion_host(sparse, labels, n_clusters, use_superpixel != 0, dense, rows, cols, pitch_bytes, frame_stride_bytes,
-                               n_frames, DCMT_BLUR_GAUSSIAN, flags, stats);
+    return run_completion_host({labels, n_clusters, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags},
+                               {sparse, nullptr, pitch_bytes, frame_stride_bytes}, {dense, nullptr, pitch_bytes, frame_stride_bytes},
+                               n_frames, stats);
 }
 
 int dcmt_interpolate_with_superpixels_f32(const float* sparse, const int32_t* labels, int n_clusters, float* dense,
@@ -1212,8 +1119,8 @@ int dcmt_img_completion_stages_f32(const float* sparse, float* dense, int rows, 
                                    int n_stages, uint32_t* stage_mask_out, void* cuda_stream) {
     if (!stages || n_stages < dcmt::kOracleStages) return fail(DCMT_E_BADARG, "stages buffer must hold %d planes", dcmt::kOracleStages);
     uint32_t mask = 0;
-    int rc = run_completion(sparse, nullptr, 0, false, dense, rows, cols, 0, 0, 1, blur_type, DCMT_PATH_GENERIC, nullptr,
-                            stages, &mask, static_cast<cudaStream_t>(cuda_stream));
+    int rc = run_completion({nullptr, 0, false, rows, cols, blur_type, DCMT_PATH_GENERIC}, {sparse}, {dense}, 1, nullptr,
+                            static_cast<cudaStream_t>(cuda_stream), stages, &mask);
     if (stage_mask_out) *stage_mask_out = mask;
     return rc;
 }
@@ -1230,22 +1137,12 @@ int dcmt_debug_q8_phase_cycles(const float* sparse, float* dense, int rows, int 
     if (!fused_applies(cc)) return fail(DCMT_E_UNSUPPORTED, "shape not served by the fused kernels");
     Arena* ar = nullptr;
     const size_t fpix = (size_t)rows * cols;
-    const size_t mid_pitch = ((size_t)cols + 7) / 8 * 8;
-    const size_t bytes = 2 * carve_bytes(fpix * n_frames, 4) + carve_bytes(n_frames, sizeof(dcmt::FrameCounters)) +
-                         carve_bytes((size_t)rows * mid_pitch * n_frames, 2) + 2 * carve_bytes(mid_pitch * n_frames, 4);
-    if ((rc = arena_acquire(st, bytes, &ar))) return rc;
-    dcmt::Q8Plan p{};
-    p.rows = rows;
-    p.cols = cols;
-    dcmt::q8_choose_tile(rows, cols, &p.th, &p.tw);
-    p.mid_pitch = (int)mid_pitch;
-    p.max_frames = n_frames;
-    p.w1 = carve<float>(ar, fpix * n_frames);
-    p.w2 = carve<float>(ar, fpix * n_frames);
-    p.ctr = carve<dcmt::FrameCounters>(ar, n_frames);
-    p.mid = carve<uint16_t>(ar, (size_t)rows * mid_pitch * n_frames);
-    p.col_first = carve<uint32_t>(ar, mid_pitch * n_frames);
-    p.col_last = carve<uint32_t>(ar, mid_pitch * n_frames);
+    if ((rc = arena_acquire(st, generic_ws_bytes(rows, cols, n_frames, false) + fused_ws_bytes(rows, cols, n_frames, false, false), &ar)))
+        return rc;
+    float* w1 = carve<float>(ar, fpix * n_frames);
+    float* w2 = carve<float>(ar, fpix * n_frames);
+    dcmt::FrameCounters* ctr = carve<dcmt::FrameCounters>(ar, n_frames);
+    dcmt::Q8Plan p = carve_fused(ar, rows, cols, n_frames, false, false, w1, w2, ctr).p;
     if ((rc = arena_ok(ar))) return rc;
     p.prof_front = front_stamps;
     p.prof_tail = tail_stamps;

@@ -177,3 +177,26 @@ def test_host_multi_on_emulator(emu_lib):
         assert np.array_equal(got[f].view(np.uint32), co.img_completion(s[f], "none").view(np.uint32)), f
     plain = api.img_completion(s, False, "none", lib=emu_lib)
     assert np.array_equal(got.view(np.uint32), plain.view(np.uint32))
+    # the copy-only ceiling leg echoes the input
+    echo = np.zeros_like(s)
+    emu_lib.check(emu_lib.dcmt_debug_host_copy_f32(s.ctypes.data, echo.ctypes.data, rows, cols, len(s), None, 0))
+    assert np.array_equal(echo.view(np.uint32), s.view(np.uint32))
+
+
+def test_q8_phase_cycles_on_emulator(emu_lib):
+    """dcmt_debug_q8_phase_cycles runs the fused kernels with Gaussian blur: same bytes as DCMT_PATH_FUSED"""
+    from depth_completion_mt_b200 import synth
+
+    rows, cols = 64, 100
+    s = synth.sparse_depth(710, rows, cols, 0.05)
+    want = np.zeros_like(s)
+    emu_lib.check(emu_lib.dcmt_img_completion_f32(s.ctypes.data, want.ctypes.data, rows, cols, 0, 0, 1, _lib.BLUR["gaussian"],
+                                                  _lib.PATH["fused"], None, None))
+    got = np.zeros_like(s)
+    stamps = [np.zeros(1 << 12, np.int64) for _ in range(2)]
+    tiles = C.c_int(0)
+    rc = emu_lib.dcmt_debug_q8_phase_cycles(s.ctypes.data, got.ctypes.data, rows, cols, 1, stamps[0].ctypes.data,
+                                            stamps[1].ctypes.data, C.byref(tiles), None)
+    assert rc == _lib.DCMT_OK, emu_lib.dcmt_last_error()
+    assert np.array_equal(got.view(np.uint32), want.view(np.uint32))
+    assert tiles.value == 1  # 64 x 100 fits one tile of at most 96 x 160

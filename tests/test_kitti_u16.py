@@ -263,6 +263,9 @@ def body_host(lib, rows, cols, multi_devices):
     echo = np.zeros_like(u16)
     lib.check(lib.dcmt_debug_host_copy_u16_u16(u16.ctypes.data, echo.ctypes.data, rows, cols, n, None, 0))
     assert np.array_equal(echo, u16), "dcmt_debug_host_copy_u16_u16 must echo its input"
+    zeros = np.full(u16.shape, 7.0, np.float32)
+    lib.check(lib.dcmt_debug_host_copy_u16(u16.ctypes.data, zeros.ctypes.data, rows, cols, n, None, 0))
+    assert not zeros.any(), "dcmt_debug_host_copy_u16 must leave a float output all zeros"
 
 
 # ------------------------------------------------------------------ 5. argument errors
@@ -424,6 +427,7 @@ def test_emu_a2(emu_lib):
 
 def test_emu_host_variants(emu_lib):
     body_host(emu_lib, 48, 72, [0])
+    body_host(emu_lib, 45, 77, [0])  # width not a multiple of 8: device staging rows are padded past the host's
 
 
 def test_emu_argument_errors(emu_lib):
@@ -457,6 +461,7 @@ def test_gpu_a2(gpu_lib):
 @pytest.mark.gpu
 def test_gpu_host_variants(gpu_lib):
     body_host(gpu_lib, 352, 1216, [0])
+    body_host(gpu_lib, 45, 77, [0])
 
 
 @pytest.mark.gpu
