@@ -13,12 +13,6 @@
 #define DCMT_DYN_SMEM(type, name)                                         \
     extern __shared__ __align__(128) unsigned char dcmt_dyn_smem_raw[];   \
     type* name = reinterpret_cast<type*>(dcmt_dyn_smem_raw)
-// 16-byte asynchronous global -> shared copy (LDGSTS): no registers, many copies in flight per thread
-#define DCMT_CP_ASYNC_16(smem_ptr, gmem_ptr)                                                                        \
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((unsigned)__cvta_generic_to_shared(smem_ptr)), \
-                 "l"(gmem_ptr)                                                                                     \
-                 : "memory")
-#define DCMT_CP_ASYNC_WAIT_ALL() asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory")
 namespace dcmt { void note_launch(); }  // launch counter behind dcmt_launch_count() (api.cu)
 #define DCMT_LAUNCH(kernel, grid, block, smem, stream, ...) \
     (dcmt::note_launch(), kernel<<<(grid), (block), (smem), (stream)>>>(__VA_ARGS__))

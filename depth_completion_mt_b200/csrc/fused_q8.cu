@@ -10,7 +10,7 @@
 //                                    VIMNMX3.U16x2 / PRMT; writes a uint16 plane + per-column first/last keys
 //   k_q8_tail    (A5..A10, :103-202) column extrapolation applied on load, 31x31 fill (vertical log-doubling +
 //                                    ballot/popc-compacted horizontal pass over hole words only), median5 by
-//                                    shared sorted columns + a 54-comparator selection network, Gaussian in
+//                                    sorted rows and merges shared along runs of rows, Gaussian in
 //                                    integer q16, final inversion, float32 store
 //                                    holes that survive the first 31x31 fill (the reference's loop then runs more passes) are
 //                                    resolved in the tile by a warp scanning growing squares of the A5 image in global memory
@@ -20,7 +20,6 @@
 
 #include <cstdlib>
 
-#include "median_net.cuh"
 #include "median_rows.cuh"
 #include "rank_f32.cuh"
 
@@ -39,16 +38,12 @@ namespace {
 #ifndef DCMT_FRONT_CTAS
 #define DCMT_FRONT_CTAS 4
 #endif
-#ifndef DCMT_MEDIAN_ROWS
-#define DCMT_MEDIAN_ROWS 1  // 1: shared-work median over runs of rows (median_rows.cuh); 0: independent selection networks
-#endif
 constexpr int QT = DCMT_QT;     // threads per CTA of k_q8_front (DCMT_FRONT_CTAS CTAs per SM on tiles of half the tail's height)
 constexpr int QTT = DCMT_QTT;   // threads per CTA of k_q8_tail (2 CTAs per SM: their phases overlap)
 
 #define SPLAT16(x) ((uint32_t)(x) | ((uint32_t)(x) << 16))
 constexpr uint32_t E_VALID_MIN = 27;   // e >= 27  <=>  depth >= 0.1f  (26/256 = 0.1015625 is the smallest q8 value >= 0.1f)
 constexpr uint32_t E_HUNDRED = 25601;  // encoding of 100.0 (empty-column fill, img_completion.cpp:110)
-constexpr uint32_t kAbsMax = 0u;           // identity of max in the encoding (two lanes)
 
 __device__ __forceinline__ uint32_t pmax(uint32_t a, uint32_t b) { return __vmaxu2(a, b); }
 __device__ __forceinline__ uint32_t pmin(uint32_t a, uint32_t b) { return __vminu2(a, b); }
@@ -202,10 +197,6 @@ __device__ __forceinline__ void tile_columns(Tile& t, int gx0, int cols) {
             t.smask = make_uint4(m[0], m[1], m[2], m[3]);
         }
     }
-}
-__device__ __forceinline__ bool outside(const Tile& t, int r, int q) { return r < t.rlo || r >= t.rhi || q < t.qlo || q >= t.qhi; }
-__device__ __forceinline__ uint4 blend(uint4 v, uint4 m, uint32_t ident) {
-    return make_uint4((v.x & m.x) | (ident & ~m.x), (v.y & m.y) | (ident & ~m.y), (v.z & m.z) | (ident & ~m.z), (v.w & m.w) | (ident & ~m.w));
 }
 __device__ __forceinline__ uint4 and4(uint4 v, uint4 m) { return make_uint4(v.x & m.x, v.y & m.y, v.z & m.z, v.w & m.w); }
 
@@ -585,6 +576,49 @@ __device__ __forceinline__ void front_decode_staged(const FrontArgs& a, const ui
     }
 }
 
+// pass 7 of both fronts on one quad: horizontal half of dilate7 of the vertical maxima at v, hole fill (:92-100) of the
+// closed image at d, in place (only this thread touches the quad in this pass); returns the filled quad
+__device__ __forceinline__ uint4 dilate7_fill_quad(const uint32_t* v, uint32_t* d) {
+    const uint4 tt = h7_max_quad(v);
+    uint4 q = lds4(d);
+    q.x = fill_holes(q.x, tt.x);
+    q.y = fill_holes(q.y, tt.y);
+    q.z = fill_holes(q.z, tt.z);
+    q.w = fill_holes(q.w, tt.w);
+    sts4(d, q);
+    return q;
+}
+
+// per-column first / last valid row inside the tile's core (feeds :103-129), merged across tiles by atomics.  Two threads
+// per column: one searches from the top, one from the bottom.  core: the core's first row of the filled image in shared
+// memory, `stride` uint16 per row; hrows: core rows inside the image.
+template <int NT>
+__device__ __forceinline__ void column_keys(const FrontArgs& a, const uint16_t* core, int stride, int frame, int y0, int x0, int hrows) {
+    for (int c2 = threadIdx.x; c2 < 2 * a.tw; c2 += NT) {
+        const int col = c2 >> 1, from_bottom = c2 & 1;
+        const int gx = x0 + col;
+        if (gx >= a.cols) continue;
+        const uint16_t* p = core + col;
+        if (!from_bottom) {
+            for (int cy = 0; cy < hrows; ++cy) {
+                const uint32_t e = p[(size_t)cy * stride];
+                if (e >= E_VALID_MIN) {
+                    atomicMin(a.col_first + (size_t)frame * a.mid_pitch + gx, ((uint32_t)(y0 + cy) << 16) | e);
+                    break;
+                }
+            }
+        } else {
+            for (int cy = hrows - 1; cy >= 0; --cy) {
+                const uint32_t e = p[(size_t)cy * stride];
+                if (e >= E_VALID_MIN) {
+                    atomicMax(a.col_last + (size_t)frame * a.mid_pitch + gx, ((uint32_t)(y0 + cy) << 16) | e);
+                    break;
+                }
+            }
+        }
+    }
+}
+
 template <bool kStraddle>
 __global__ void __launch_bounds__(QT, DCMT_FRONT_CTAS) k_q8_front(FrontArgs a, const __grid_constant__ TensorMap3D tmap) {
     DCMT_DYN_SMEM(uint32_t, smem);
@@ -651,47 +685,14 @@ __global__ void __launch_bounds__(QT, DCMT_FRONT_CTAS) k_q8_front(FrontArgs a, c
             uint16_t* mp = mid + (size_t)(y0 + r0) * a.mid_pitch + gx;
             const size_t mstep = (size_t)m.nrt * a.mid_pitch;
 #pragma unroll 2
-            for (int r = r0; r < rend; r += m.nrt, off += dstep, pc += cstep, mp += mstep) {
-                const uint4 tt = h7_max_quad(A + off);
-                uint4 d = lds4(pc);
-                d.x = fill_holes(d.x, tt.x);
-                d.y = fill_holes(d.y, tt.y);
-                d.z = fill_holes(d.z, tt.z);
-                d.w = fill_holes(d.w, tt.w);
-                sts4(pc, d);  // only this thread touches this quad of C in this pass
-                *reinterpret_cast<uint4*>(mp) = d;
-            }
+            for (int r = r0; r < rend; r += m.nrt, off += dstep, pc += cstep, mp += mstep)
+                *reinterpret_cast<uint4*>(mp) = dilate7_fill_quad(A + off, pc);
         }
     }
     __syncthreads();
     DCMT_STAMP(a, 3);
-    // ---- per-column first / last valid row inside this tile (feeds :103-129), merged across tiles by atomics.
-    //      Two threads per column: one searches from the top, one from the bottom.
-    const uint16_t* Ch = reinterpret_cast<const uint16_t*>(C);
-    const int hrows = min(th, rows - y0);
-    for (int c2 = threadIdx.x; c2 < 2 * tw; c2 += QT) {
-        const int col = c2 >> 1, from_bottom = c2 & 1;
-        const int gx = x0 + col;
-        if (gx >= cols) continue;
-        const uint16_t* p = Ch + col;
-        if (!from_bottom) {
-            for (int cy = 0; cy < hrows; ++cy) {
-                const uint32_t e = p[(size_t)cy * tw];
-                if (e >= E_VALID_MIN) {
-                    atomicMin(a.col_first + (size_t)frame * a.mid_pitch + gx, ((uint32_t)(y0 + cy) << 16) | e);
-                    break;
-                }
-            }
-        } else {
-            for (int cy = hrows - 1; cy >= 0; --cy) {
-                const uint32_t e = p[(size_t)cy * tw];
-                if (e >= E_VALID_MIN) {
-                    atomicMax(a.col_last + (size_t)frame * a.mid_pitch + gx, ((uint32_t)(y0 + cy) << 16) | e);
-                    break;
-                }
-            }
-        }
-    }
+    // ---- per-column first / last valid row (C holds the core: th rows of tw uint16)
+    column_keys<QT>(a, reinterpret_cast<const uint16_t*>(C), tw, frame, y0, x0, min(th, rows - y0));
     DCMT_STAMP(a, 4);
 }
 
@@ -1086,42 +1087,12 @@ __global__ void __launch_bounds__(GT, kPerLabel ? DCMT_GUIDED_CTAS : 2) k_q8_gui
             const int gx = x0 + q * 8;
             if (gx >= cols) continue;
             const int off = ((r + FU) * t.RQ + q + FLQ) * 4;
-            const uint4 tt = h7_max_quad(A + off);
-            uint4 d = lds4(B + off);
-            d.x = fill_holes(d.x, tt.x);
-            d.y = fill_holes(d.y, tt.y);
-            d.z = fill_holes(d.z, tt.z);
-            d.w = fill_holes(d.w, tt.w);
-            sts4(B + off, d);
+            const uint4 d = dilate7_fill_quad(A + off, B + off);
             *reinterpret_cast<uint4*>(mid + (size_t)(y0 + r) * a.mid_pitch + gx) = d;
         }
     }
     __syncthreads();
-    const uint16_t* Bh = reinterpret_cast<const uint16_t*>(B);
-    const int hrows = min(th, rows - y0);
-    for (int c2 = threadIdx.x; c2 < 2 * tw; c2 += GT) {
-        const int col = c2 >> 1, from_bottom = c2 & 1;
-        const int gx = x0 + col;
-        if (gx >= cols) continue;
-        const uint16_t* p = Bh + (size_t)FU * t.pitchw * 2 + FLQ * 8 + col;
-        if (!from_bottom) {
-            for (int cy = 0; cy < hrows; ++cy) {
-                const uint32_t e = p[(size_t)cy * t.pitchw * 2];
-                if (e >= E_VALID_MIN) {
-                    atomicMin(a.col_first + (size_t)frame * a.mid_pitch + gx, ((uint32_t)(y0 + cy) << 16) | e);
-                    break;
-                }
-            }
-        } else {
-            for (int cy = hrows - 1; cy >= 0; --cy) {
-                const uint32_t e = p[(size_t)cy * t.pitchw * 2];
-                if (e >= E_VALID_MIN) {
-                    atomicMax(a.col_last + (size_t)frame * a.mid_pitch + gx, ((uint32_t)(y0 + cy) << 16) | e);
-                    break;
-                }
-            }
-        }
-    }
+    column_keys<GT>(a, reinterpret_cast<const uint16_t*>(B) + (size_t)FU * t.pitchw * 2 + FLQ * 8, t.pitchw * 2, frame, y0, x0, min(th, rows - y0));
 }
 
 // set-up of a front launch in one kernel: the per-column keys and -- unless the caller did it (ctr == nullptr) -- the per-frame counters
@@ -1130,14 +1101,6 @@ __global__ void k_q8_init_cols(uint32_t* first, uint32_t* last, size_t n, FrameC
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) { first[i] = 0xffffffffu; last[i] = 0u; }
     if (ctr && i < (size_t)n_frames) { ctr[i] = FrameCounters{}; ctr[i].path = 1; }
-}
-
-// debugging / test aid: decode a uint16 plane back to float metres in inverted space
-__global__ void k_q8_decode(const uint16_t* __restrict__ mid, size_t mid_pitch, float* __restrict__ out, int rows, int cols) {
-    const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
-    if (x >= cols || y >= rows) return;
-    const uint32_t e = mid[(size_t)y * mid_pitch + x];
-    out[(size_t)y * cols + x] = e == 0 ? -FLT_MAX : (float)(e - 1) * (1.0f / 256.0f);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1159,8 +1122,7 @@ struct TailArgs {
     size_t out_pitch, out_fstride;  // elements of the output type
     int rows, cols, th, tw, blur, vec_ok;
     int one;          // the constant 1, opaque to the compiler (see other_of_pair)
-    int use_tma;      // tile load by one TMA box copy (else 16-byte cp.async per thread)
-    ItemsDesc i_load, i_vert, i_scan, i_scanw, i_med, i_gauss;  // row lengths RQ, pitchw, SQ, 4 SQ, MI, NP
+    ItemsDesc i_vert, i_scan, i_scanw, i_gauss;  // row lengths pitchw, SQ, 4 SQ, NP
     ItemsDesc i_vert2; // row length pitchw / 2: pairs of word columns (vertical maxima)
     ItemsDesc i_medr;  // row length tw / 2 + 2: one item = one word column x med_len rows (shared-work median)
     int med_len, med_segs;
@@ -1178,19 +1140,9 @@ __device__ __forceinline__ uint32_t other_of_pair(uint32_t a, uint32_t b, uint32
     return a * one + (b * one - lo);
 }
 
-#ifndef DCMT_OTH_NUM
-#define DCMT_OTH_NUM 0  // of every DCMT_OTH_DEN compare-exchanges of the merge networks, this many take their maximum on the ALU pipe
-#endif
-#ifndef DCMT_OTH_DEN
-#define DCMT_OTH_DEN 1
-#endif
 struct PackedOps {
     uint32_t one;
     __device__ __forceinline__ uint32_t other(uint32_t a, uint32_t b, uint32_t lo) const { return other_of_pair(a, b, lo, one); }
-    template <int I>
-    __device__ __forceinline__ uint32_t oth(uint32_t a, uint32_t b, uint32_t lo) const {
-        return (I % DCMT_OTH_DEN) < DCMT_OTH_NUM ? pmax(a, b) : other_of_pair(a, b, lo, one);
-    }
     static __device__ __forceinline__ uint32_t mn(uint32_t a, uint32_t b) { return pmin(a, b); }
     static __device__ __forceinline__ uint32_t mx(uint32_t a, uint32_t b) { return pmax(a, b); }
     static __device__ __forceinline__ uint32_t mn3(uint32_t a, uint32_t b, uint32_t c) { return pmin3(a, b, c); }
@@ -1297,32 +1249,10 @@ __global__ void __launch_bounds__(QTT, DCMT_TAIL_CTAS) k_q8_tail(TailArgs a, con
     DCMT_STAMP(a, 0);
     // ---- load the A4 plane: ONE TMA box copy (200 x 126 uint16 for the KITTI tiles) issued by one thread; the hardware
     //      zero-fills everything outside the image (0 = absent, exactly what the border cells must hold) and signals
-    //      an mbarrier.  The per-column keys of the A5 step are fetched while the copy is in flight.  Fallback (no
-    //      tensor map): 16-byte cp.async copies by all threads with the border handled in software.
-    Tile t;
-    t.RH = RH;
-    t.RQ = RQ;
-    t.pitchw = pitchw;
-    t.rlo = max(0, -gy0);
-    t.rhi = min(RH, rows - gy0);
-    if (a.use_tma) {
-        if (threadIdx.x == 0) tma_bar_init(&s_bar);
-        __syncthreads();
-        if (threadIdx.x == 0) tma_load_3d(A, &tmap, gx0, gy0, slot, &s_bar, (uint32_t)(RH * pitchw * 4));
-    } else {
-        tile_columns(t, gx0, cols);
-        const uint16_t* mp = mid + ((ptrdiff_t)gy0 * (ptrdiff_t)a.mid_pitch + gx0);
-        const int mpitch = (int)a.mid_pitch;
-        if (!border) {
-            for (Items i(a.i_load); i.r < RH; i.next()) DCMT_CP_ASYNC_16(A + i.lin * 4, mp + (i.r * mpitch + i.q * 8));
-        } else {
-            for (Items i(a.i_load); i.r < RH; i.next()) {
-                if (outside(t, i.r, i.q)) sts4(A + i.lin * 4, splat4(kAbsMax));
-                else if (i.q == t.qs) sts4(A + i.lin * 4, blend(__ldg(reinterpret_cast<const uint4*>(mp + (i.r * mpitch + i.q * 8))), t.smask, kAbsMax));
-                else DCMT_CP_ASYNC_16(A + i.lin * 4, mp + (i.r * mpitch + i.q * 8));
-            }
-        }
-    }
+    //      an mbarrier.  The per-column keys of the A5 step are fetched while the copy is in flight.
+    if (threadIdx.x == 0) tma_bar_init(&s_bar);
+    __syncthreads();
+    if (threadIdx.x == 0) tma_load_3d(A, &tmap, gx0, gy0, slot, &s_bar, (uint32_t)(RH * pitchw * 4));
     // A5 (:103-129): two threads per region column, one per zone (rows <= first, rows >= last)
     const int a5_item = threadIdx.x, a5_c = a5_item >> 1, a5_bottom = a5_item & 1;
     const int a5_gx = gx0 + a5_c;
@@ -1332,8 +1262,7 @@ __global__ void __launch_bounds__(QTT, DCMT_TAIL_CTAS) k_q8_tail(TailArgs a, con
         a5_kf = __ldg(a.col_first + (size_t)slot * a.mid_pitch + a5_gx);
         a5_kl = __ldg(a.col_last + (size_t)slot * a.mid_pitch + a5_gx);
     }
-    if (a.use_tma) tma_bar_wait(&s_bar, 0);
-    else DCMT_CP_ASYNC_WAIT_ALL();
+    tma_bar_wait(&s_bar, 0);
     __syncthreads();
     DCMT_STAMP(a, 1);
     // rows >= last <- value(last), rows <= first <- value(first) (the second write wins); empty column <- 100
@@ -1565,7 +1494,6 @@ __global__ void __launch_bounds__(QTT, DCMT_TAIL_CTAS) k_q8_tail(TailArgs a, con
         __syncthreads();
     }
     DCMT_STAMP(a, 6);
-#if DCMT_MEDIAN_ROWS
     // ---- A8 median 5x5 (:170): shared-work form, see median_step
     {
         const int MH = th + 4;  // rows core +- 2, words core +- 1 (a.i_medr)
@@ -1596,56 +1524,6 @@ __global__ void __launch_bounds__(QTT, DCMT_TAIL_CTAS) k_q8_tail(TailArgs a, con
             }
         }
     }
-#else
-    // ---- A8 median 5x5 (:170): one item = four output words of one row.  The six word columns it touches are sorted
-    //      once (9 compare-exchanges each, both lanes at once), the odd-aligned pixel pairs between them come from
-    //      PRMTs of the sorted columns, and each output is the 54-comparator selection network of median_net.cuh on
-    //      its five sorted columns.
-    {
-        const int MH = th + 4;  // rows core +- 2; items of four words cover core +- 1 word (a.i_med)
-        const int mr0 = TV - 2, mw0 = TQ * 4 - 1;
-        const PackedOps ops{(uint32_t)a.one};
-        for (Items i(a.i_med); i.r < MH; i.next()) {
-            const int r = mr0 + i.r, w = mw0 + 4 * i.q;  // output words w .. w+3; columns w-1 .. w+4
-            uint32_t col[6][5];
-            const uint32_t* p = A + (r - 2) * pitchw + (w - 1);  // w - 1 is even: 8-byte aligned
-#pragma unroll
-            for (int k = 0; k < 5; ++k) {
-                const uint2 p0 = *reinterpret_cast<const uint2*>(p + k * pitchw), p1 = *reinterpret_cast<const uint2*>(p + k * pitchw + 2),
-                            p2 = *reinterpret_cast<const uint2*>(p + k * pitchw + 4);
-                col[0][k] = p0.x; col[1][k] = p0.y; col[2][k] = p1.x; col[3][k] = p1.y; col[4][k] = p2.x; col[5][k] = p2.y;
-            }
-#pragma unroll
-            for (int j = 0; j < 6; ++j) sort5(col[j], ops.one);
-            uint32_t res[4];
-            uint32_t oddl[5];  // sorted column of the odd-aligned pair left of the current output word
-#pragma unroll
-            for (int k = 0; k < 5; ++k) oddl[k] = odd_pair(col[0][k], col[1][k]);
-#pragma unroll
-            for (int o = 0; o < 4; ++o) {
-                uint32_t oddr[5];
-#pragma unroll
-                for (int k = 0; k < 5; ++k) oddr[k] = odd_pair(col[o + 1][k], col[o + 2][k]);
-                uint32_t c[25];
-#pragma unroll
-                for (int k = 0; k < 5; ++k) {
-                    c[k] = col[o][k];
-                    c[5 + k] = oddl[k];
-                    c[10 + k] = col[o + 1][k];
-                    c[15 + k] = oddr[k];
-                    c[20 + k] = col[o + 2][k];
-                }
-                res[o] = median25_sorted_columns(ops, c);
-#pragma unroll
-                for (int k = 0; k < 5; ++k) oddl[k] = oddr[k];
-            }
-            uint32_t* q = B + r * pitchw + w;  // w is odd: store as 1 + 2 + 1 words
-            q[0] = res[0];
-            *reinterpret_cast<uint2*>(q + 1) = make_uint2(res[1], res[2]);
-            q[3] = res[3];
-        }
-    }
-#endif
     __syncthreads();
     DCMT_STAMP(a, 7);
     // ---- BORDER_REFLECT_101 for the Gaussian (:179): mirror the median image into the 2 cells beyond each edge.
@@ -1910,8 +1788,8 @@ cudaError_t tma_encode_f32_3d(TensorMap3D* m, const float* base, int cols, int r
 }
 #endif
 
-// DCMT_NO_TMA=1: the front and the tail load their tiles with per-thread copies (the path for inputs a tensor map cannot
-// describe), e.g. to test that path on any input
+// DCMT_NO_TMA=1: k_q8_front loads its region with per-thread loads (the path for inputs a tensor map cannot describe), e.g.
+// to test that path on any input.  k_q8_tail reads the library's own intermediate plane, which a tensor map always describes.
 static bool tma_disabled() {
     static const bool no_tma = [] { const char* e = getenv("DCMT_NO_TMA"); return e && e[0] == '1'; }();
     return no_tma;
@@ -1931,8 +1809,7 @@ void q8_choose_tile(int rows, int cols, int* th, int* tw) {
     // Tiles of at most 96 x 160 that divide the frame evenly (KITTI 352 x 1216 -> 88 x 152, 4 x 8 tiles).  Among the
     // splits near that size, take the one with the least halo work whose shared memory lets TWO CTAs of each kernel
     // share an SM (228 KB per SM, 1 KB reserved per CTA): the phases of the two overlap.
-    static const int max_h = [] { const char* e = getenv("DCMT_TILE_MAX_H"); return e ? atoi(e) : 96; }();  // experiments
-    const int ny0 = (rows + max_h - 1) / max_h, nx0 = (cols + 159) / 160;
+    const int ny0 = (rows + 95) / 96, nx0 = (cols + 159) / 160;
     long best_cost = -1;
     for (int ny = ny0; ny <= ny0 + 3; ++ny)
         for (int nx = nx0; nx <= nx0 + 3; ++nx) {
@@ -1975,31 +1852,24 @@ cudaError_t q8_run_front(const Q8Plan& plan, const float* in, const uint16_t* in
     // A tile width of 8 (8 m - 2) pixels makes those rows 16 m half-quads long -- whole 128-byte wavefronts -- which is
     // worth 6 - 7 % at equal work (measured at 1216 x 352: 112-pixel tiles 1.387 ms against 1.480 ms for the tail's 152): such
     // widths compete with the tail's on (region quads x region rows), with that bonus.
-    // DCMT_FRONT_TILE_H / DCMT_FRONT_TILE_W override the height bound / the width (experiments).
-    static const int front_h = [] { const char* e = getenv("DCMT_FRONT_TILE_H"); const int v = e ? atoi(e) : 0; return v > 0 && v < 8 ? 8 : v; }();
-    static const int front_w = [] { const char* e = getenv("DCMT_FRONT_TILE_W"); return e ? atoi(e) / 8 * 8 : -1; }();
     Q8Plan p = plan;
     auto height_for = [&](int tw) {
-        int hmax = front_h > 0 ? front_h : plan.th;
-        if (front_h <= 0 && DCMT_FRONT_CTAS > 2)
+        int hmax = plan.th;
+        if (DCMT_FRONT_CTAS > 2)
             while (hmax > 8 && (size_t)DCMT_FRONT_CTAS * (q8_front_smem(hmax, tw) + 1024) > (size_t)228 * 1024) --hmax;
         if (hmax >= plan.th) return plan.th;
         const int ny = (p.rows + hmax - 1) / hmax;
         return (p.rows + ny - 1) / ny;
     };
     auto width_ok = [&](int tw) { return tw >= 8 && (tw / 8 + FLQ + FRQ) * 9 <= QT; };  // more than 8 rows per sweep: col_pass relies on it
-    if (front_w >= 0) {
-        if (width_ok(front_w)) p.tw = front_w;
-    } else {
-        double best = -1.0;
-        const int widths[4] = {plan.tw, 48, 112, 176};
-        for (int tw : widths) {
-            if (!width_ok(tw)) continue;
-            const int th = height_for(tw), nx = (p.cols + tw - 1) / tw, ny = (p.rows + th - 1) / th;
-            const double work = (double)nx * (tw / 8 + FLQ + FRQ) * ny * (th + FU + FD);
-            const double cost = work * ((tw / 8 + FLQ + FRQ - 1) % 8 == 0 ? 0.93 : 1.0);
-            if (best < 0 || cost < best) { best = cost; p.tw = tw; }
-        }
+    double best = -1.0;
+    const int widths[4] = {plan.tw, 48, 112, 176};
+    for (int tw : widths) {
+        if (!width_ok(tw)) continue;
+        const int th = height_for(tw), nx = (p.cols + tw - 1) / tw, ny = (p.rows + th - 1) / th;
+        const double work = (double)nx * (tw / 8 + FLQ + FRQ) * ny * (th + FU + FD);
+        const double cost = work * ((tw / 8 + FLQ + FRQ - 1) % 8 == 0 ? 0.93 : 1.0);
+        if (best < 0 || cost < best) { best = cost; p.tw = tw; }
     }
     p.th = height_for(p.tw);
     const size_t ncol = (size_t)p.mid_pitch * n_frames;
@@ -2087,7 +1957,7 @@ cudaError_t q8_run_tail(const Q8Plan& p, float* out, uint16_t* out16, size_t out
     // 4-pixel stores (16 bytes of float32 / 8 bytes of uint16) need every row start aligned to their size
     const int vec2 = out_pitch % 4 == 0 && out_fstride % 4 == 0 &&
                      (out16 ? (reinterpret_cast<uintptr_t>(out16) & 7) : (reinterpret_cast<uintptr_t>(out) & 15)) == 0;
-    const int RQ = p.tw / 8 + 2 * TQ, RH = p.th + 2 * TV, SQ = p.tw / 8 + 2, MI = (p.tw / 2 + 2 + 3) / 4, NP = p.tw / 4;
+    const int RQ = p.tw / 8 + 2 * TQ, RH = p.th + 2 * TV, SQ = p.tw / 8 + 2, NP = p.tw / 4;
     // shared-work median: word columns x runs of an even number of rows.  A run starts with four extra row sorts and a pair
     // merge, so longer runs execute fewer instructions while shorter ones keep more threads busy; measured on the B200 at the
     // KITTI tile (92 median rows x 78 word columns): runs of 16 / 20 / 28 / 32 / 36 / 40 rows -> tail 2.108 / 2.175 / 2.091 /
@@ -2100,18 +1970,20 @@ cudaError_t q8_run_tail(const Q8Plan& p, float* out, uint16_t* out16, size_t out
     if (segs < 1) segs = 1;
     int med_len = 2 * ((MH + 2 * segs - 1) / (2 * segs));
     if (med_len < 8) med_len = 8;
-    static const int env_len = [] { const char* e = getenv("DCMT_MED_LEN"); return e ? atoi(e) : 0; }();  // experiments
-    if (env_len >= 2) med_len = env_len & ~1;
     const int med_segs = (MH + med_len - 1) / med_len;
     // tile load by TMA: a 3-D map (columns, rows, slots) of the intermediate plane whose column extent is the true
-    // image width, so that the padding columns of the plane read as absent like everything else outside the image
+    // image width, so that the padding columns of the plane read as absent like everything else outside the image.  The
+    // map can always be encoded: the plane's pitch (cols padded to 8 uint16) and frame stride are multiples of 16 bytes,
+    // arena carves are 256-byte aligned, and q8_choose_tile keeps th <= 96 and tw <= 160, so the box (tw + 48 x th + 38)
+    // stays within 256 in both dimensions.
     TensorMap3D tmap{};
-    const int use_tma = !tma_disabled() && tma_encode_u16_3d(&tmap, p.mid, p.cols, p.rows, p.max_frames, (size_t)p.mid_pitch * 2,
-                                                     (size_t)p.mid_pitch * p.rows * 2, RQ * 8, RH) == cudaSuccess;
+    const cudaError_t e = tma_encode_u16_3d(&tmap, p.mid, p.cols, p.rows, p.max_frames, (size_t)p.mid_pitch * 2,
+                                            (size_t)p.mid_pitch * p.rows * 2, RQ * 8, RH);
+    if (e != cudaSuccess) return e;
     TailArgs a{p.mid, (size_t)p.mid_pitch, (size_t)p.mid_pitch * p.rows, p.col_first, p.col_last, p.ctr,
                out16 ? static_cast<void*>(out16) : static_cast<void*>(out), out_pitch,
-               out_fstride, p.rows, p.cols, p.th, p.tw, blur, vec2, 1, use_tma,
-               make_items(RQ, QTT), make_items(RQ * 4, QTT), make_items(SQ, QTT), make_items(SQ * 4, QTT), make_items(MI, QTT),
+               out_fstride, p.rows, p.cols, p.th, p.tw, blur, vec2, 1,
+               make_items(RQ * 4, QTT), make_items(SQ, QTT), make_items(SQ * 4, QTT),
                make_items(NP, QTT), make_items(RQ * 2, QTT), make_items(NW, QTT), med_len, med_segs, p.lut ? kRankHundred : E_HUNDRED, p.lut, p.prof_tail};
     const dim3 grid((p.cols + p.tw - 1) / p.tw, (p.rows + p.th - 1) / p.th, n_frames);
     if (p.lut) DCMT_LAUNCH(k_q8_tail<true>, grid, dim3(QTT), q8_tail_smem(p.th, p.tw), st, a, tmap);
@@ -2149,11 +2021,6 @@ cudaError_t depth_to_u16(const float* in, size_t in_pitch, size_t in_fstride, ui
         if (e != cudaSuccess) return e;
     }
     return cudaSuccess;
-}
-
-cudaError_t q8_decode_plane(const uint16_t* mid, size_t mid_pitch, float* out, int rows, int cols, cudaStream_t st) {
-    DCMT_LAUNCH(k_q8_decode, dim3((cols + 127) / 128, rows), dim3(128), 0, st, mid, mid_pitch, out, rows, cols);
-    return cudaGetLastError();
 }
 
 }  // namespace dcmt

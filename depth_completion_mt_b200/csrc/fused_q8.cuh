@@ -61,7 +61,5 @@ cudaError_t depth_to_u16(const float* in, size_t in_pitch, size_t in_fstride, ui
 cudaError_t q8_zero_counters(const Q8Plan& p, int n_frames, cudaStream_t st);
 // counters -> stats[4*n] (optional) and flags[n] (1 = frame must be redone by the generic pipeline)
 cudaError_t q8_write_stats(const Q8Plan& p, int32_t* stats, int32_t* flags, int n_frames, cudaStream_t st);
-// test aid: decode a uint16 plane (inverted space) into float
-cudaError_t q8_decode_plane(const uint16_t* mid, size_t mid_pitch, float* out, int rows, int cols, cudaStream_t st);
 
 }  // namespace dcmt

@@ -67,8 +67,6 @@ long launches();
 }  // namespace dcmt_emu
 
 #define DCMT_DYN_SMEM(type, name) type* name = reinterpret_cast<type*>(dcmt_emu::dyn_smem())
-#define DCMT_CP_ASYNC_16(smem_ptr, gmem_ptr) std::memcpy((smem_ptr), (gmem_ptr), 16)
-#define DCMT_CP_ASYNC_WAIT_ALL() ((void)0)
 namespace dcmt { void note_launch(); }
 #define DCMT_LAUNCH(kernel, grid, block, smem, stream, ...) \
     (dcmt::note_launch(), dcmt_emu::launch((grid), (block), (smem), [=]() { kernel(__VA_ARGS__); }))

@@ -13,7 +13,7 @@ largest at least 13, so only ranks 7..12 can be the median, which is then rank 1
 elements of the remaining row:  rank_5(A, B) = max(A0, min(A1,B4), min(A2,B3), min(A3,B2), min(A4,B1), min(A5,B0)).
 
 Per output: 9 + 13/2 + 24/2 comparators and 8 min/max for the final selection (58 min/max ops) against 9 * 1.5 + 54
-(111 ops) for the independent selection network of median_net.cuh.
+(111 ops) for an independent 54-comparator selection network per output.
 
     python tools/median_rows_scheme.py            # verify the networks (0-1 principle) and the scheme (random windows)
     python tools/median_rows_scheme.py --emit     # write depth_completion_mt_b200/csrc/median_rows.cuh
@@ -144,12 +144,8 @@ def emit_fn(name, doc, net, n_in, outs, in_expr, n_out, sig):
     no = sum(1 for o in ops if o[1] == "other")
     lines = [f"// {doc}", f"// {len(net)} comparators -> {n2} two-input + {n3} three-input min/max ops + {no} `other` ops.",
              "template <class Ops, class T>", f"__device__ __forceinline__ void {name}({sig}) {{"]
-    k_other = 0
     for nm, kind, args in ops:
         fn = kind + ("3" if len(args) == 3 and kind != "other" else "")
-        if kind == "other":  # numbered: Ops decides per index which pipe computes the maximum (oth<I>)
-            fn = f"template oth<{k_other}>"
-            k_other += 1
         lines.append(f"    const T {nm} = ops.{fn}({', '.join(args)});")
     for r in range(n_out):
         lines.append(f"    o[{r}] = {res[r]};")
@@ -161,9 +157,8 @@ def emit():
     lines = [
         "// median_rows.cuh -- GENERATED by tools/median_rows_scheme.py (networks found by tools/select_network.py); do not edit.",
         "// Building blocks of the shared-work 5x5 median (cv::medianBlur(5), img_completion.cpp:170): merge of two sorted",
-        "// fives, and ranks 7..12 of the merge of two sorted tens.  Ops: mn, mx, mn3, mx3 as in median_net.cuh, and oth<I>(a, b, lo) =",
-        "// the element of {a, b} that is not lo = mn(a, b); I numbers the compare-exchanges of a network so that Ops can split",
-        "// them between the min/max pipe (mx) and the multiply-add pipe (a + b - lo).",
+        "// fives, and ranks 7..12 of the merge of two sorted tens.  Ops: mn, mx (two-input min / max), mn3, mx3 (three-input),",
+        "// and other(a, b, lo) = the element of {a, b} that is not lo = mn(a, b).",
         "#pragma once", "", "namespace dcmt {", ""]
     lines += emit_fn("merge_5_5", "o = merge(a, b), all ascending", MERGE55, 10, MERGE55_OUT,
                      [f"a[{k}]" for k in range(5)] + [f"b[{k}]" for k in range(5)], 10,
