@@ -74,6 +74,10 @@ _SIGNATURES = {
     "dcmt_retrieve_optimized_depth_f32": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, _P]),
     "dcmt_evaluate_f32": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_float, C.c_int, _P, _P]),
     "dcmt_evaluate_f32_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_float, C.c_int, _P]),
+    "dcmt_evaluate_u16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_float, C.c_int, _P, _P]),
+    "dcmt_evaluate_u16_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_float, C.c_int, _P]),
+    "dcmt_evaluate_u16_u16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_float, C.c_int, _P, _P]),
+    "dcmt_evaluate_u16_u16_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_float, C.c_int, _P]),
     "dcmt_lidar_project_f32": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, C.c_int, _P, _P, C.c_float, C.c_float, _P, _P]),
     "dcmt_lidar_project_batch_f32": (C.c_int, [_P, _P, C.c_int, C.c_size_t, C.c_int, _P, _P, C.c_int, C.c_int, _P, _P, C.c_float, C.c_float, _P, _P]),
     "dcmt_lidar_project_f32_host": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, C.c_int, _P, _P, C.c_float, C.c_float, _P]),

@@ -398,39 +398,58 @@ EVAL_VARIANTS = {
 }
 
 
+def _eval_entry(lib, g_u16: bool, r_u16: bool, host: bool):
+    """the entry point for the plane types: float32 pair, KITTI uint16 GT with a float32 or a uint16 result"""
+    if r_u16 and not g_u16:
+        raise ValueError("a uint16 (KITTI) result is scored against uint16 (KITTI) gt only; pass float32 gt with a float32 result")
+    name = "dcmt_evaluate_" + ("u16_u16" if r_u16 else "u16" if g_u16 else "f32") + ("_host" if host else "")
+    fn = getattr(lib, name)
+    if not g_u16:
+        return lambda g, r, rows, cols, n, *rest: fn(g, r, rows, cols, 0, 0, n, *rest)
+    return lambda g, r, rows, cols, n, *rest: fn(g, r, rows, cols, 0, 0, 0, 0, n, *rest)
+
+
 def evaluate(gt, dense, variant: str = "lidar_camera", *, stream=None, lib: _lib.Library | None = None):
     """The masked error sums behind the reference's evaluation functions, one record per frame.
 
     Returns a numpy structured array with fields count, sum_err, sum_abs, sum_sq (float64) and mean_err, mae, rmse
-    (float32).  ``gt`` / ``dense`` are float32 (rows, cols) or (n, rows, cols), numpy (host entry point) or torch CUDA
-    tensors (device entry point; the records are read back, which synchronises the stream)."""
+    (float32).  ``gt`` / ``dense`` are (rows, cols) or (n, rows, cols), numpy (host entry points) or torch CUDA tensors
+    (device entry points; the records are read back, which synchronises the stream).  ``gt`` is float32 metres or KITTI
+    uint16 (metres * 256, the depth PNG as read -- it stands for the ``convertTo(CV_32F, 1.0 / 256.0)`` of main.cpp:82);
+    ``dense`` is float32, or KITTI uint16 when ``gt`` is uint16 (``dcmt_evaluate_u16`` / ``dcmt_evaluate_u16_u16``: the
+    same records as the float32 call on ``u / 256``)."""
     lib = lib or _lib.load()
     mode, tol = EVAL_VARIANTS[variant]
     dt = np.dtype([("count", "f8"), ("sum_err", "f8"), ("sum_abs", "f8"), ("sum_sq", "f8"), ("mean_err", "f4"), ("mae", "f4"),
                    ("rmse", "f4"), ("pad", "i4")])
     if _is_torch(gt):
-        g3, _ = _batch3(_prep_torch(gt, torch.float32, "gt"), "gt")
-        r3, _ = _batch3(_prep_torch(dense, torch.float32, "dense"), "dense")
+        g_u16, r_u16 = gt.dtype == torch.uint16, _is_torch(dense) and dense.dtype == torch.uint16
+        call = _eval_entry(lib, g_u16, r_u16, host=False)
+        g3, _ = _batch3(_prep_torch(gt, torch.uint16 if g_u16 else torch.float32, "gt"), "gt")
+        r3, _ = _batch3(_prep_torch(dense, torch.uint16 if r_u16 else torch.float32, "dense"), "dense")
         if g3.shape != r3.shape:
             raise ValueError("gt and dense shapes differ")
         n, rows, cols = g3.shape
         res = torch.empty((n, dt.itemsize), dtype=torch.uint8, device=g3.device)
         with torch.cuda.device(g3.device):
-            lib.check(lib.dcmt_evaluate_f32(g3.data_ptr(), r3.data_ptr(), rows, cols, 0, 0, n, float(tol), mode, res.data_ptr(),
-                                            _stream_ptr(stream)))
+            lib.check(call(g3.data_ptr(), r3.data_ptr(), rows, cols, n, float(tol), mode, res.data_ptr(), _stream_ptr(stream)))
         return res.cpu().numpy().view(dt).reshape(n)
-    g3, _ = _batch3(_prep_numpy(gt, np.float32, "gt"), "gt")
-    r3, _ = _batch3(_prep_numpy(dense, np.float32, "dense"), "dense")
+    g_u16 = isinstance(gt, np.ndarray) and gt.dtype == np.uint16
+    r_u16 = isinstance(dense, np.ndarray) and dense.dtype == np.uint16
+    call = _eval_entry(lib, g_u16, r_u16, host=True)
+    g3, _ = _batch3(_prep_numpy(gt, np.uint16 if g_u16 else np.float32, "gt"), "gt")
+    r3, _ = _batch3(_prep_numpy(dense, np.uint16 if r_u16 else np.float32, "dense"), "dense")
     if g3.shape != r3.shape:
         raise ValueError("gt and dense shapes differ")
     n, rows, cols = g3.shape
     res = np.zeros(n, dt)
-    lib.check(lib.dcmt_evaluate_f32_host(_np_ptr(g3), _np_ptr(r3), rows, cols, 0, 0, n, float(tol), mode, _np_ptr(res)))
+    lib.check(call(_np_ptr(g3), _np_ptr(r3), rows, cols, n, float(tol), mode, _np_ptr(res)))
     return res
 
 
 def evaluate_performance(GT_img, r_img, variant: str = "lidar_camera", **kw):
-    """evaluate_performance(GT_img, r_img, mse[, mae]) of the reference, for ONE frame.
+    """evaluate_performance(GT_img, r_img, mse[, mae]) of the reference, for ONE frame (GT and result types as for
+    ``evaluate``: a KITTI uint16 GT as read, with a float32 or uint16 result).
 
     variant "lidar_only"   (main.cpp:16-34)      -> mse            (= mean of gt - r over gt > 0: a signed mean, sic)
     variant "lidar_camera" (main_lc.cpp:85-116)  -> (mse, mae)     (mse = sqrt(sum d^2 / count), sic)"""
@@ -441,7 +460,8 @@ def evaluate_performance(GT_img, r_img, variant: str = "lidar_camera", **kw):
 
 
 def evaluate_performances(GT_img, r_img, **kw):
-    """evaluate_performances(GT_img, r_img, mae, rmse), main_sl.cpp:1031-1061 (tolerance 2) -> (mae, rmse)."""
+    """evaluate_performances(GT_img, r_img, mae, rmse), main_sl.cpp:1031-1061 (tolerance 2) -> (mae, rmse); types as for
+    ``evaluate``."""
     rec = evaluate(GT_img, r_img, "stereo_lidar", **kw)[0]
     return float(rec["mae"]), float(rec["rmse"])
 

@@ -829,6 +829,103 @@ int run_completion_host(CompletionCall cc, InDesc in, OutDesc out, int n_frames,
     return DCMT_OK;
 }
 
+// ---- evaluation: one device driver and one host driver behind every dcmt_evaluate_* entry point.  Each side is an InDesc:
+// float32 metres or KITTI uint16 (metres * 256), with the ABI's pitch and frame stride in bytes (0 = dense) until
+// validate_evaluation checks them against the side's element size and converts them to elements.  uint16 results come
+// with a uint16 GT only (the entry points offer no other pair).
+int validate_evaluation(InDesc* gt, InDesc* r, int rows, int cols, int n_frames, int mode, const void* results, size_t* gt_span,
+                        size_t* r_span) {
+    if (!gt->ptr() || !r->ptr() || !results) return fail(DCMT_E_BADARG, "null pointer");
+    if (mode != DCMT_EVAL_GT_VALID && mode != DCMT_EVAL_BOTH_VALID) return fail(DCMT_E_BADARG, "mode %d", mode);
+    Geometry g, q;
+    int rc = check_geometry(rows, cols, gt->pitch, gt->fstride, n_frames, &g, gt->elem());
+    if (rc) return rc;
+    if ((rc = check_geometry(rows, cols, r->pitch, r->fstride, n_frames, &q, r->elem()))) return rc;
+    gt->pitch = g.pitch;
+    gt->fstride = g.fstride;
+    r->pitch = q.pitch;
+    r->fstride = q.fstride;
+    *gt_span = g.span_bytes;
+    *r_span = q.span_bytes;
+    return DCMT_OK;
+}
+
+// partial sums in the stream's arena, then the two kernels of evaluate.cu (validated arguments, n_frames >= 1)
+int enqueue_evaluation(const InDesc& gt, const InDesc& r, int rows, int cols, int n_frames, float tolerance, int mode,
+                       dcmt_eval_result* results, cudaStream_t st) {
+    Arena* ar = nullptr;
+    int rc = arena_acquire(st, carve_bytes(dcmt::eval_partial_doubles(n_frames), sizeof(double)), &ar);
+    if (rc) return rc;
+    double* partials = carve<double>(ar, dcmt::eval_partial_doubles(n_frames));
+    if ((rc = arena_ok(ar))) return rc;
+    dcmt::EvalResult* out = reinterpret_cast<dcmt::EvalResult*>(results);
+    cudaError_t e;
+    if (!gt.u)
+        e = dcmt::eval_run(gt.f, gt.pitch, gt.fstride, r.f, r.pitch, r.fstride, rows, cols, n_frames, tolerance, mode, partials, out, st);
+    else if (!r.u)
+        e = dcmt::eval_run(gt.u, gt.pitch, gt.fstride, r.f, r.pitch, r.fstride, rows, cols, n_frames, tolerance, mode, partials, out, st);
+    else
+        e = dcmt::eval_run(gt.u, gt.pitch, gt.fstride, r.u, r.pitch, r.fstride, rows, cols, n_frames, tolerance, mode, partials, out, st);
+    API_CUDA(e, "evaluation launch");
+    return DCMT_OK;
+}
+
+int run_evaluation(InDesc gt, InDesc r, int rows, int cols, int n_frames, float tolerance, int mode, dcmt_eval_result* results,
+                   void* cuda_stream) {
+    size_t gt_span = 0, r_span = 0;
+    int rc = validate_evaluation(&gt, &r, rows, cols, n_frames, mode, results, &gt_span, &r_span);
+    if (rc) return rc;
+    if (n_frames == 0) return DCMT_OK;
+    if ((rc = check_device())) return rc;
+    return enqueue_evaluation(gt, r, rows, cols, n_frames, tolerance, mode, results, static_cast<cudaStream_t>(cuda_stream));
+}
+
+// host pointers: both planes are staged whole (each side's own span, so 2 B/px for a uint16 side), evaluated on the
+// staging copies with the caller's geometry, and the records copied back
+int run_evaluation_host(InDesc gt, InDesc r, int rows, int cols, int n_frames, float tolerance, int mode, dcmt_eval_result* results) {
+    size_t gt_span = 0, r_span = 0;
+    int rc = validate_evaluation(&gt, &r, rows, cols, n_frames, mode, results, &gt_span, &r_span);
+    if (rc) return rc;
+    if (n_frames == 0) return DCMT_OK;
+    HostCall call;
+    if ((rc = call.open(nullptr, 0, false))) return rc;
+    cudaStream_t st = call.lanes[0].hs->s[0], st2 = call.lanes[0].hs->s[1];
+    Arena* stage = nullptr;
+    if ((rc = arena_acquire(st2, carve_bytes(gt_span, 1) + carve_bytes(r_span, 1) + carve_bytes((size_t)n_frames, sizeof(dcmt_eval_result)),
+                            &stage)))
+        return rc;
+    char* d_gt = carve<char>(stage, gt_span);
+    char* d_r = carve<char>(stage, r_span);
+    dcmt_eval_result* d_res = carve<dcmt_eval_result>(stage, (size_t)n_frames);
+    if ((rc = arena_ok(stage))) return rc;
+    call.use(call.lanes[0]);
+    API_CUDA(cudaMemcpyAsync(d_gt, gt.ptr(), gt_span, cudaMemcpyHostToDevice, st), "host to device copy");
+    API_CUDA(cudaMemcpyAsync(d_r, r.ptr(), r_span, cudaMemcpyHostToDevice, st), "host to device copy");
+    InDesc dgt = gt, dr = r;
+    if (gt.u) dgt.u = reinterpret_cast<const uint16_t*>(d_gt);
+    else dgt.f = reinterpret_cast<const float*>(d_gt);
+    if (r.u) dr.u = reinterpret_cast<const uint16_t*>(d_r);
+    else dr.f = reinterpret_cast<const float*>(d_r);
+    if ((rc = enqueue_evaluation(dgt, dr, rows, cols, n_frames, tolerance, mode, d_res, st))) return rc;
+    API_CUDA(cudaMemcpyAsync(results, d_res, (size_t)n_frames * sizeof(dcmt_eval_result), cudaMemcpyDeviceToHost, st), "device to host copy");
+    return call.finish();
+}
+
+InDesc eval_f32(const float* p, size_t pitch_bytes, size_t fstride_bytes) {
+    InDesc d;
+    d.f = p;
+    d.pitch = pitch_bytes;
+    d.fstride = fstride_bytes;
+    return d;
+}
+InDesc eval_u16(const uint16_t* p, size_t pitch_bytes, size_t fstride_bytes) {
+    InDesc d;
+    d.u = p;
+    d.pitch = pitch_bytes;
+    d.fstride = fstride_bytes;
+    return d;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1326,47 +1423,44 @@ static_assert(sizeof(dcmt_eval_result) == sizeof(dcmt::EvalResult), "dcmt_eval_r
 
 int dcmt_evaluate_f32(const float* gt, const float* dense, int rows, int cols, size_t pitch_bytes, size_t frame_stride_bytes,
                       int n_frames, float tolerance, int mode, dcmt_eval_result* results, void* cuda_stream) {
-    if (!gt || !dense || !results) return fail(DCMT_E_BADARG, "null pointer");
-    if (mode != DCMT_EVAL_GT_VALID && mode != DCMT_EVAL_BOTH_VALID) return fail(DCMT_E_BADARG, "mode %d", mode);
-    Geometry g;
-    int rc = check_geometry(rows, cols, pitch_bytes, frame_stride_bytes, n_frames, &g);
-    if (rc) return rc;
-    if (n_frames == 0) return DCMT_OK;
-    if ((rc = check_device())) return rc;
-    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-    Arena* ar = nullptr;
-    if ((rc = arena_acquire(st, carve_bytes(dcmt::eval_partial_doubles(n_frames), sizeof(double)), &ar))) return rc;
-    double* partials = carve<double>(ar, dcmt::eval_partial_doubles(n_frames));
-    if ((rc = arena_ok(ar))) return rc;
-    API_CUDA(dcmt::eval_run(gt, dense, rows, cols, g.pitch, g.fstride, n_frames, tolerance, mode, partials,
-                            reinterpret_cast<dcmt::EvalResult*>(results), st),
-             "evaluation launch");
-    return DCMT_OK;
+    return run_evaluation(eval_f32(gt, pitch_bytes, frame_stride_bytes), eval_f32(dense, pitch_bytes, frame_stride_bytes), rows, cols,
+                          n_frames, tolerance, mode, results, cuda_stream);
 }
 
 int dcmt_evaluate_f32_host(const float* gt, const float* dense, int rows, int cols, size_t pitch_bytes, size_t frame_stride_bytes,
                            int n_frames, float tolerance, int mode, dcmt_eval_result* results) {
-    if (!gt || !dense || !results) return fail(DCMT_E_BADARG, "null pointer");
-    if (mode != DCMT_EVAL_GT_VALID && mode != DCMT_EVAL_BOTH_VALID) return fail(DCMT_E_BADARG, "mode %d", mode);
-    Geometry g;
-    int rc = check_geometry(rows, cols, pitch_bytes, frame_stride_bytes, n_frames, &g);
-    if (rc) return rc;
-    if (n_frames == 0) return DCMT_OK;
-    HostCall call;
-    if ((rc = call.open(nullptr, 0, false))) return rc;
-    cudaStream_t st = call.lanes[0].hs->s[0], st2 = call.lanes[0].hs->s[1];
-    Arena* stage = nullptr;
-    if ((rc = arena_acquire(st2, 2 * carve_bytes(g.span_bytes, 1) + carve_bytes((size_t)n_frames, sizeof(dcmt_eval_result)), &stage))) return rc;
-    float* d_gt = reinterpret_cast<float*>(carve<char>(stage, g.span_bytes));
-    float* d_r = reinterpret_cast<float*>(carve<char>(stage, g.span_bytes));
-    dcmt_eval_result* d_res = carve<dcmt_eval_result>(stage, (size_t)n_frames);
-    if ((rc = arena_ok(stage))) return rc;
-    call.use(call.lanes[0]);
-    API_CUDA(cudaMemcpyAsync(d_gt, gt, g.span_bytes, cudaMemcpyHostToDevice, st), "host to device copy");
-    API_CUDA(cudaMemcpyAsync(d_r, dense, g.span_bytes, cudaMemcpyHostToDevice, st), "host to device copy");
-    if ((rc = dcmt_evaluate_f32(d_gt, d_r, rows, cols, pitch_bytes, frame_stride_bytes, n_frames, tolerance, mode, d_res, st))) return rc;
-    API_CUDA(cudaMemcpyAsync(results, d_res, (size_t)n_frames * sizeof(dcmt_eval_result), cudaMemcpyDeviceToHost, st), "device to host copy");
-    return call.finish();
+    return run_evaluation_host(eval_f32(gt, pitch_bytes, frame_stride_bytes), eval_f32(dense, pitch_bytes, frame_stride_bytes), rows, cols,
+                               n_frames, tolerance, mode, results);
+}
+
+int dcmt_evaluate_u16(const uint16_t* gt_u16, const float* dense, int rows, int cols, size_t gt_pitch_bytes, size_t gt_frame_stride_bytes,
+                      size_t dense_pitch_bytes, size_t dense_frame_stride_bytes, int n_frames, float tolerance, int mode,
+                      dcmt_eval_result* results, void* cuda_stream) {
+    return run_evaluation(eval_u16(gt_u16, gt_pitch_bytes, gt_frame_stride_bytes), eval_f32(dense, dense_pitch_bytes, dense_frame_stride_bytes),
+                          rows, cols, n_frames, tolerance, mode, results, cuda_stream);
+}
+
+int dcmt_evaluate_u16_host(const uint16_t* gt_u16, const float* dense, int rows, int cols, size_t gt_pitch_bytes,
+                           size_t gt_frame_stride_bytes, size_t dense_pitch_bytes, size_t dense_frame_stride_bytes, int n_frames,
+                           float tolerance, int mode, dcmt_eval_result* results) {
+    return run_evaluation_host(eval_u16(gt_u16, gt_pitch_bytes, gt_frame_stride_bytes),
+                               eval_f32(dense, dense_pitch_bytes, dense_frame_stride_bytes), rows, cols, n_frames, tolerance, mode, results);
+}
+
+int dcmt_evaluate_u16_u16(const uint16_t* gt_u16, const uint16_t* dense_u16, int rows, int cols, size_t gt_pitch_bytes,
+                          size_t gt_frame_stride_bytes, size_t dense_pitch_bytes, size_t dense_frame_stride_bytes, int n_frames,
+                          float tolerance, int mode, dcmt_eval_result* results, void* cuda_stream) {
+    return run_evaluation(eval_u16(gt_u16, gt_pitch_bytes, gt_frame_stride_bytes),
+                          eval_u16(dense_u16, dense_pitch_bytes, dense_frame_stride_bytes), rows, cols, n_frames, tolerance, mode, results,
+                          cuda_stream);
+}
+
+int dcmt_evaluate_u16_u16_host(const uint16_t* gt_u16, const uint16_t* dense_u16, int rows, int cols, size_t gt_pitch_bytes,
+                               size_t gt_frame_stride_bytes, size_t dense_pitch_bytes, size_t dense_frame_stride_bytes, int n_frames,
+                               float tolerance, int mode, dcmt_eval_result* results) {
+    return run_evaluation_host(eval_u16(gt_u16, gt_pitch_bytes, gt_frame_stride_bytes),
+                               eval_u16(dense_u16, dense_pitch_bytes, dense_frame_stride_bytes), rows, cols, n_frames, tolerance, mode,
+                               results);
 }
 
 void dcmt_stereo_params_default(dcmt_stereo_params* p) {

@@ -385,6 +385,33 @@ DCMT_API int dcmt_evaluate_f32(const float *gt, const float *dense, int rows, in
 DCMT_API int dcmt_evaluate_f32_host(const float *gt, const float *dense, int rows, int cols, size_t pitch_bytes,
                                     size_t frame_stride_bytes, int n_frames, float tolerance, int mode,
                                     dcmt_eval_result *results /* host, n_frames */);
+/* (8f #3, KITTI on-disk format) the same reductions on KITTI ground truth as read: the uint16 payload of the depth PNG
+ * (cv::imread(..., IMREAD_ANYDEPTH); uint16 = metres * 256, 0 = no measurement) -- it replaces the GT's
+ * convertTo(CV_32F, 1.0 / 256.0) of main.cpp:82 and main_lc.cpp:159-224 in front of evaluate_performance, and serves
+ * evaluate_performances (main_sl.cpp:1031-1061) as well.  dcmt_evaluate_u16 scores a float32 result;
+ * dcmt_evaluate_u16_u16 scores a KITTI uint16 result as well (the output of the *_u16_u16 completion calls, what a caller
+ * stores as a PNG).  A uint16 value u is decoded to (float)u * (1.0f / 256.0f), which is exact; the mask test, the
+ * float32 subtraction and the double accumulation are those of dcmt_evaluate_f32.  GT and result have their own pitches
+ * and frame strides in bytes (0 = dense); a pitch or stride that is not a multiple of the element size or too small is
+ * DCMT_E_BADARG.  Results are byte-identical to dcmt_evaluate_f32 on the decoded planes (u / 256) whenever those planes
+ * have the same pitch, frame stride and base alignment counted in elements (the 4-pixel vector loads are taken under
+ * the same condition).  HBM traffic is 6 (u16 GT, float32 result) or 4 (both uint16) bytes per pixel instead of 8, and
+ * the *_host variants stage 2 + 4 or 2 + 2 bytes per pixel. */
+DCMT_API int dcmt_evaluate_u16(const uint16_t *gt_u16, const float *dense, int rows, int cols, size_t gt_pitch_bytes,
+                               size_t gt_frame_stride_bytes, size_t dense_pitch_bytes, size_t dense_frame_stride_bytes,
+                               int n_frames, float tolerance, int mode, dcmt_eval_result *results /* device, n_frames */,
+                               void *cuda_stream);
+DCMT_API int dcmt_evaluate_u16_host(const uint16_t *gt_u16, const float *dense, int rows, int cols, size_t gt_pitch_bytes,
+                                    size_t gt_frame_stride_bytes, size_t dense_pitch_bytes, size_t dense_frame_stride_bytes,
+                                    int n_frames, float tolerance, int mode, dcmt_eval_result *results /* host, n_frames */);
+DCMT_API int dcmt_evaluate_u16_u16(const uint16_t *gt_u16, const uint16_t *dense_u16, int rows, int cols, size_t gt_pitch_bytes,
+                                   size_t gt_frame_stride_bytes, size_t dense_pitch_bytes, size_t dense_frame_stride_bytes,
+                                   int n_frames, float tolerance, int mode, dcmt_eval_result *results /* device, n_frames */,
+                                   void *cuda_stream);
+DCMT_API int dcmt_evaluate_u16_u16_host(const uint16_t *gt_u16, const uint16_t *dense_u16, int rows, int cols,
+                                        size_t gt_pitch_bytes, size_t gt_frame_stride_bytes, size_t dense_pitch_bytes,
+                                        size_t dense_frame_stride_bytes, int n_frames, float tolerance, int mode,
+                                        dcmt_eval_result *results /* host, n_frames */);
 
 /* (8f #2) LiDAR projection + normalisation: replaces the loops of src/DC_stereo_lidar/main_sl.cpp:478-523 (withSuperPixels;
  * the same code in vedi_pc :340-385): Velodyne points (n_points x 4 float32: x, y, z, intensity -- the .bin payload)

@@ -103,6 +103,25 @@ inline dcmt_eval_result evaluate(const MatView& GT_img, const MatView& r_img, fl
                                  GT_img.step, 0, 1, tolerance, mode, &res));
     return res;
 }
+// The same on KITTI ground truth as read: the uint16 payload of the depth PNG (CV_16UC1 view, metres * 256), which stands for
+// the GT's convertTo(CV_32F, 1.0 / 256.0) of main.cpp:82 / main_lc.cpp:159-224 (dcmt_evaluate_u16), scored against a float32
+// result, or against a KITTI uint16 result such as img_completion_u16_u16's (dcmt_evaluate_u16_u16).  GT and result have
+// their own steps here.  The records equal evaluate() on the decoded views (u / 256) when those have the same steps in
+// elements.
+inline dcmt_eval_result evaluate_u16(const MatView& GT_u16, const MatView& r_img, float tolerance, int mode) {
+    if (GT_u16.rows != r_img.rows || GT_u16.cols != r_img.cols) throw std::invalid_argument("dcmt: evaluate_u16 needs same-shaped Mats");
+    dcmt_eval_result res;
+    check(dcmt_evaluate_u16_host(static_cast<const uint16_t*>(GT_u16.data), static_cast<const float*>(r_img.data), GT_u16.rows, GT_u16.cols,
+                                 GT_u16.step, 0, r_img.step, 0, 1, tolerance, mode, &res));
+    return res;
+}
+inline dcmt_eval_result evaluate_u16_u16(const MatView& GT_u16, const MatView& r_u16, float tolerance, int mode) {
+    if (GT_u16.rows != r_u16.rows || GT_u16.cols != r_u16.cols) throw std::invalid_argument("dcmt: evaluate_u16_u16 needs same-shaped Mats");
+    dcmt_eval_result res;
+    check(dcmt_evaluate_u16_u16_host(static_cast<const uint16_t*>(GT_u16.data), static_cast<const uint16_t*>(r_u16.data), GT_u16.rows,
+                                     GT_u16.cols, GT_u16.step, 0, r_u16.step, 0, 1, tolerance, mode, &res));
+    return res;
+}
 // src/DC_lidar_only/main.cpp:16-34: "mse" = mean of (gt - r) over gt > 0 (a signed mean, sic)
 inline void evaluate_performance(const MatView& GT_img, const MatView& r_img, float& mse) {
     mse = evaluate(GT_img, r_img, 0.0f, DCMT_EVAL_GT_VALID).mean_err;
@@ -398,18 +417,32 @@ inline void stereo_refine(const cv::Mat& dense_range_img, const cv::Mat& left_gr
     optimized_depth = out;
 }
 
-// the evaluation functions of main.cpp:16 / main_lc.cpp:85 / main_sl.cpp:1031 (CV_32FC1 Mats)
+namespace dcmt {
+// GT and result Mats as the three programs hold them: a CV_32FC1 pair, or the KITTI GT as read (CV_16UC1, no convertTo) with a
+// CV_32FC1 or CV_16UC1 result.  A float32 GT with a uint16 result, and every other combination, throws.
+inline dcmt_eval_result evaluate_mats(const cv::Mat& GT_img, const cv::Mat& r_img, float tolerance, int mode) {
+    if (GT_img.type() == CV_16UC1 && r_img.type() == CV_16UC1) return evaluate_u16_u16(view_of(GT_img), view_of(r_img), tolerance, mode);
+    if (GT_img.type() == CV_16UC1 && r_img.type() == CV_32FC1) return evaluate_u16(view_of(GT_img), view_of(r_img), tolerance, mode);
+    CV_Assert(GT_img.type() == CV_32FC1 && r_img.type() == CV_32FC1);
+    const cv::Mat g = continuous(GT_img), r = continuous(r_img);
+    return evaluate(view_of(g), view_of(r), tolerance, mode);
+}
+}  // namespace dcmt
+
+// the evaluation functions of main.cpp:16 / main_lc.cpp:85 / main_sl.cpp:1031, with the tolerances and masks of the MatView
+// forms above
 inline void evaluate_performance(const cv::Mat& GT_img, const cv::Mat& r_img, float& mse) {
-    const cv::Mat g = dcmt::continuous(GT_img), r = dcmt::continuous(r_img);
-    dcmt::evaluate_performance(dcmt::view_of(g), dcmt::view_of(r), mse);
+    mse = dcmt::evaluate_mats(GT_img, r_img, 0.0f, DCMT_EVAL_GT_VALID).mean_err;
 }
 inline void evaluate_performance(const cv::Mat& GT_img, const cv::Mat& r_img, float& mse, float& mae) {
-    const cv::Mat g = dcmt::continuous(GT_img), r = dcmt::continuous(r_img);
-    dcmt::evaluate_performance(dcmt::view_of(g), dcmt::view_of(r), mse, mae);
+    const dcmt_eval_result r = dcmt::evaluate_mats(GT_img, r_img, 0.0f, DCMT_EVAL_BOTH_VALID);
+    mse = r.rmse;
+    mae = r.mae;
 }
 inline void evaluate_performances(cv::Mat& GT_img, cv::Mat& r_img, float& mae, float& rmse) {
-    const cv::Mat g = dcmt::continuous(GT_img), r = dcmt::continuous(r_img);
-    dcmt::evaluate_performances(dcmt::view_of(g), dcmt::view_of(r), mae, rmse);
+    const dcmt_eval_result r = dcmt::evaluate_mats(GT_img, r_img, 2.0f, DCMT_EVAL_BOTH_VALID);
+    mae = r.mae;
+    rmse = r.rmse;
 }
 #endif  // DCMT_HAVE_OPENCV
 
