@@ -36,6 +36,15 @@ class EvalResult(C.Structure):
                 ("mean_err", C.c_float), ("mae", C.c_float), ("rmse", C.c_float), ("pad", C.c_int32)]
 
 
+class KittiMetrics(C.Structure):
+    """dcmt_kitti_metrics (include/dcmt.h)."""
+
+    _fields_ = [("n_gt", C.c_double), ("n_pred", C.c_double), ("n_unfilled", C.c_double), ("sum_abs", C.c_double),
+                ("sum_sq", C.c_double), ("sum_iabs", C.c_double), ("sum_isq", C.c_double), ("mae_mm", C.c_float),
+                ("rmse_mm", C.c_float), ("imae_per_km", C.c_float), ("irmse_per_km", C.c_float), ("density", C.c_float),
+                ("pad", C.c_int32)]
+
+
 class DcmtError(RuntimeError):
     def __init__(self, status: int, message: str):
         super().__init__(f"dcmt status {status}: {message}")
@@ -78,6 +87,12 @@ _SIGNATURES = {
     "dcmt_evaluate_u16_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_float, C.c_int, _P]),
     "dcmt_evaluate_u16_u16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_float, C.c_int, _P, _P]),
     "dcmt_evaluate_u16_u16_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_float, C.c_int, _P]),
+    "dcmt_evaluate_kitti_f32": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, _P, _P]),
+    "dcmt_evaluate_kitti_f32_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, _P]),
+    "dcmt_evaluate_kitti_u16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, _P, _P]),
+    "dcmt_evaluate_kitti_u16_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, _P]),
+    "dcmt_evaluate_kitti_u16_u16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, _P, _P]),
+    "dcmt_evaluate_kitti_u16_u16_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, _P]),
     "dcmt_lidar_project_f32": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, C.c_int, _P, _P, C.c_float, C.c_float, _P, _P]),
     "dcmt_lidar_project_batch_f32": (C.c_int, [_P, _P, C.c_int, C.c_size_t, C.c_int, _P, _P, C.c_int, C.c_int, _P, _P, C.c_float, C.c_float, _P, _P]),
     "dcmt_lidar_project_f32_host": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, C.c_int, _P, _P, C.c_float, C.c_float, _P]),

@@ -447,6 +447,50 @@ def evaluate(gt, dense, variant: str = "lidar_camera", *, stream=None, lib: _lib
     return res
 
 
+KITTI_METRICS = np.dtype([("n_gt", "f8"), ("n_pred", "f8"), ("n_unfilled", "f8"), ("sum_abs", "f8"), ("sum_sq", "f8"),
+                          ("sum_iabs", "f8"), ("sum_isq", "f8"), ("mae_mm", "f4"), ("rmse_mm", "f4"), ("imae_per_km", "f4"),
+                          ("irmse_per_km", "f4"), ("density", "f4"), ("pad", "i4")])
+
+
+def evaluate_kitti(gt, pred, *, stream=None, lib: _lib.Library | None = None):
+    """The KITTI depth-completion benchmark's figures, one record per frame (``dcmt_evaluate_kitti_*``; the rule is stated
+    in include/dcmt.h and restates the devkit's background interpolation and error loop).
+
+    Returns a numpy structured array (``KITTI_METRICS``): n_gt, n_pred, n_unfilled and the sums of |g - p|, its square,
+    |1/g - 1/p| and its square (float64), then mae_mm, rmse_mm, imae_per_km, irmse_per_km and density (float32, NaN for a
+    frame without GT).  The benchmark publishes the mean of each figure over the frames: ``rec["rmse_mm"].mean()``.
+    Types and backends as for ``evaluate``: float32 ``gt`` and ``pred``, or KITTI uint16 ``gt`` with a float32 or uint16
+    ``pred``; numpy arrays go through the host entry points, torch CUDA tensors through the device ones."""
+    lib = lib or _lib.load()
+    if _is_torch(gt):
+        g_u16, r_u16 = gt.dtype == torch.uint16, _is_torch(pred) and pred.dtype == torch.uint16
+    else:
+        g_u16 = isinstance(gt, np.ndarray) and gt.dtype == np.uint16
+        r_u16 = isinstance(pred, np.ndarray) and pred.dtype == np.uint16
+    if r_u16 and not g_u16:
+        raise ValueError("a uint16 (KITTI) pred is scored against uint16 (KITTI) gt only; pass float32 gt with a float32 pred")
+    name = "dcmt_evaluate_kitti_" + ("u16_u16" if r_u16 else "u16" if g_u16 else "f32")
+    dt = KITTI_METRICS
+    if _is_torch(gt):
+        g3, _ = _batch3(_prep_torch(gt, torch.uint16 if g_u16 else torch.float32, "gt"), "gt")
+        r3, _ = _batch3(_prep_torch(pred, torch.uint16 if r_u16 else torch.float32, "pred"), "pred")
+        if g3.shape != r3.shape:
+            raise ValueError("gt and pred shapes differ")
+        n, rows, cols = g3.shape
+        res = torch.empty((n, dt.itemsize), dtype=torch.uint8, device=g3.device)
+        with torch.cuda.device(g3.device):
+            lib.check(getattr(lib, name)(g3.data_ptr(), r3.data_ptr(), rows, cols, 0, 0, 0, 0, n, res.data_ptr(), _stream_ptr(stream)))
+        return res.cpu().numpy().view(dt).reshape(n)
+    g3, _ = _batch3(_prep_numpy(gt, np.uint16 if g_u16 else np.float32, "gt"), "gt")
+    r3, _ = _batch3(_prep_numpy(pred, np.uint16 if r_u16 else np.float32, "pred"), "pred")
+    if g3.shape != r3.shape:
+        raise ValueError("gt and pred shapes differ")
+    n, rows, cols = g3.shape
+    res = np.zeros(n, dt)
+    lib.check(getattr(lib, name + "_host")(_np_ptr(g3), _np_ptr(r3), rows, cols, 0, 0, 0, 0, n, _np_ptr(res)))
+    return res
+
+
 def evaluate_performance(GT_img, r_img, variant: str = "lidar_camera", **kw):
     """evaluate_performance(GT_img, r_img, mse[, mae]) of the reference, for ONE frame (GT and result types as for
     ``evaluate``: a KITTI uint16 GT as read, with a float32 or uint16 result).

@@ -850,39 +850,78 @@ int validate_evaluation(InDesc* gt, InDesc* r, int rows, int cols, int n_frames,
     return DCMT_OK;
 }
 
-// partial sums in the stream's arena, then the two kernels of evaluate.cu (validated arguments, n_frames >= 1)
-int enqueue_evaluation(const InDesc& gt, const InDesc& r, int rows, int cols, int n_frames, float tolerance, int mode,
-                       dcmt_eval_result* results, cudaStream_t st) {
-    Arena* ar = nullptr;
-    int rc = arena_acquire(st, carve_bytes(dcmt::eval_partial_doubles(n_frames), sizeof(double)), &ar);
-    if (rc) return rc;
-    double* partials = carve<double>(ar, dcmt::eval_partial_doubles(n_frames));
-    if ((rc = arena_ok(ar))) return rc;
-    dcmt::EvalResult* out = reinterpret_cast<dcmt::EvalResult*>(results);
-    cudaError_t e;
-    if (!gt.u)
-        e = dcmt::eval_run(gt.f, gt.pitch, gt.fstride, r.f, r.pitch, r.fstride, rows, cols, n_frames, tolerance, mode, partials, out, st);
-    else if (!r.u)
-        e = dcmt::eval_run(gt.u, gt.pitch, gt.fstride, r.f, r.pitch, r.fstride, rows, cols, n_frames, tolerance, mode, partials, out, st);
-    else
-        e = dcmt::eval_run(gt.u, gt.pitch, gt.fstride, r.u, r.pitch, r.fstride, rows, cols, n_frames, tolerance, mode, partials, out, st);
-    API_CUDA(e, "evaluation launch");
-    return DCMT_OK;
-}
+// One kind of evaluation: the size of its per-frame record and how its kernels are enqueued on validated arguments
+// (n_frames >= 1): the reductions of dcmt_evaluate_* (EvalReductions) or the KITTI benchmark's figures (EvalKitti).
+struct EvalKind {
+    size_t rec_bytes;
+    explicit EvalKind(size_t bytes) : rec_bytes(bytes) {}
+    virtual int enqueue(const InDesc& gt, const InDesc& r, int rows, int cols, int n_frames, void* results, cudaStream_t st) const = 0;
+};
 
-int run_evaluation(InDesc gt, InDesc r, int rows, int cols, int n_frames, float tolerance, int mode, dcmt_eval_result* results,
-                   void* cuda_stream) {
+// partial sums in the stream's arena, then the two kernels of evaluate.cu
+struct EvalReductions : EvalKind {
+    float tolerance;
+    int mode;
+    EvalReductions(float tol, int m) : EvalKind(sizeof(dcmt_eval_result)), tolerance(tol), mode(m) {}
+    int enqueue(const InDesc& gt, const InDesc& r, int rows, int cols, int n_frames, void* results, cudaStream_t st) const override {
+        Arena* ar = nullptr;
+        int rc = arena_acquire(st, carve_bytes(dcmt::eval_partial_doubles(n_frames), sizeof(double)), &ar);
+        if (rc) return rc;
+        double* partials = carve<double>(ar, dcmt::eval_partial_doubles(n_frames));
+        if ((rc = arena_ok(ar))) return rc;
+        dcmt::EvalResult* out = static_cast<dcmt::EvalResult*>(results);
+        cudaError_t e;
+        if (!gt.u)
+            e = dcmt::eval_run(gt.f, gt.pitch, gt.fstride, r.f, r.pitch, r.fstride, rows, cols, n_frames, tolerance, mode, partials, out, st);
+        else if (!r.u)
+            e = dcmt::eval_run(gt.u, gt.pitch, gt.fstride, r.f, r.pitch, r.fstride, rows, cols, n_frames, tolerance, mode, partials, out, st);
+        else
+            e = dcmt::eval_run(gt.u, gt.pitch, gt.fstride, r.u, r.pitch, r.fstride, rows, cols, n_frames, tolerance, mode, partials, out, st);
+        API_CUDA(e, "evaluation launch");
+        return DCMT_OK;
+    }
+};
+
+// partial sums, the first / last valid prediction rows and (rows of more than 262 144 columns) the blocks' validity bits
+// in the stream's arena, then the three kernels of evaluate.cu
+struct EvalKitti : EvalKind {
+    EvalKitti() : EvalKind(sizeof(dcmt_kitti_metrics)) {}
+    int enqueue(const InDesc& gt, const InDesc& r, int rows, int cols, int n_frames, void* results, cudaStream_t st) const override {
+        const size_t nd = dcmt::kitti_partial_doubles(n_frames), nw = dcmt::kitti_bits_words(rows, cols, n_frames);
+        Arena* ar = nullptr;
+        int rc = arena_acquire(st, carve_bytes(nd, sizeof(double)) + carve_bytes(2 * (size_t)n_frames, sizeof(int32_t)) +
+                                       carve_bytes(nw, sizeof(unsigned)), &ar);
+        if (rc) return rc;
+        double* partials = carve<double>(ar, nd);
+        int32_t* first_last = carve<int32_t>(ar, 2 * (size_t)n_frames);
+        unsigned* bits = nw ? carve<unsigned>(ar, nw) : nullptr;
+        if ((rc = arena_ok(ar))) return rc;
+        dcmt::KittiMetrics* out = static_cast<dcmt::KittiMetrics*>(results);
+        cudaError_t e;
+        if (!gt.u)
+            e = dcmt::kitti_run(gt.f, gt.pitch, gt.fstride, r.f, r.pitch, r.fstride, rows, cols, n_frames, partials, first_last, bits, out, st);
+        else if (!r.u)
+            e = dcmt::kitti_run(gt.u, gt.pitch, gt.fstride, r.f, r.pitch, r.fstride, rows, cols, n_frames, partials, first_last, bits, out, st);
+        else
+            e = dcmt::kitti_run(gt.u, gt.pitch, gt.fstride, r.u, r.pitch, r.fstride, rows, cols, n_frames, partials, first_last, bits, out, st);
+        API_CUDA(e, "KITTI evaluation launch");
+        return DCMT_OK;
+    }
+};
+
+// `mode` is the mask of the reductions; the KITTI figures have the fixed mask g > 0 and pass DCMT_EVAL_GT_VALID
+int run_evaluation(InDesc gt, InDesc r, int rows, int cols, int n_frames, int mode, void* results, void* cuda_stream, const EvalKind& kind) {
     size_t gt_span = 0, r_span = 0;
     int rc = validate_evaluation(&gt, &r, rows, cols, n_frames, mode, results, &gt_span, &r_span);
     if (rc) return rc;
     if (n_frames == 0) return DCMT_OK;
     if ((rc = check_device())) return rc;
-    return enqueue_evaluation(gt, r, rows, cols, n_frames, tolerance, mode, results, static_cast<cudaStream_t>(cuda_stream));
+    return kind.enqueue(gt, r, rows, cols, n_frames, results, static_cast<cudaStream_t>(cuda_stream));
 }
 
 // host pointers: both planes are staged whole (each side's own span, so 2 B/px for a uint16 side), evaluated on the
 // staging copies with the caller's geometry, and the records copied back
-int run_evaluation_host(InDesc gt, InDesc r, int rows, int cols, int n_frames, float tolerance, int mode, dcmt_eval_result* results) {
+int run_evaluation_host(InDesc gt, InDesc r, int rows, int cols, int n_frames, int mode, void* results, const EvalKind& kind) {
     size_t gt_span = 0, r_span = 0;
     int rc = validate_evaluation(&gt, &r, rows, cols, n_frames, mode, results, &gt_span, &r_span);
     if (rc) return rc;
@@ -890,13 +929,12 @@ int run_evaluation_host(InDesc gt, InDesc r, int rows, int cols, int n_frames, f
     HostCall call;
     if ((rc = call.open(nullptr, 0, false))) return rc;
     cudaStream_t st = call.lanes[0].hs->s[0], st2 = call.lanes[0].hs->s[1];
+    const size_t res_bytes = (size_t)n_frames * kind.rec_bytes;
     Arena* stage = nullptr;
-    if ((rc = arena_acquire(st2, carve_bytes(gt_span, 1) + carve_bytes(r_span, 1) + carve_bytes((size_t)n_frames, sizeof(dcmt_eval_result)),
-                            &stage)))
-        return rc;
+    if ((rc = arena_acquire(st2, carve_bytes(gt_span, 1) + carve_bytes(r_span, 1) + carve_bytes(res_bytes, 1), &stage))) return rc;
     char* d_gt = carve<char>(stage, gt_span);
     char* d_r = carve<char>(stage, r_span);
-    dcmt_eval_result* d_res = carve<dcmt_eval_result>(stage, (size_t)n_frames);
+    char* d_res = carve<char>(stage, res_bytes);
     if ((rc = arena_ok(stage))) return rc;
     call.use(call.lanes[0]);
     API_CUDA(cudaMemcpyAsync(d_gt, gt.ptr(), gt_span, cudaMemcpyHostToDevice, st), "host to device copy");
@@ -906,8 +944,8 @@ int run_evaluation_host(InDesc gt, InDesc r, int rows, int cols, int n_frames, f
     else dgt.f = reinterpret_cast<const float*>(d_gt);
     if (r.u) dr.u = reinterpret_cast<const uint16_t*>(d_r);
     else dr.f = reinterpret_cast<const float*>(d_r);
-    if ((rc = enqueue_evaluation(dgt, dr, rows, cols, n_frames, tolerance, mode, d_res, st))) return rc;
-    API_CUDA(cudaMemcpyAsync(results, d_res, (size_t)n_frames * sizeof(dcmt_eval_result), cudaMemcpyDeviceToHost, st), "device to host copy");
+    if ((rc = kind.enqueue(dgt, dr, rows, cols, n_frames, d_res, st))) return rc;
+    API_CUDA(cudaMemcpyAsync(results, d_res, res_bytes, cudaMemcpyDeviceToHost, st), "device to host copy");
     return call.finish();
 }
 
@@ -1424,43 +1462,92 @@ static_assert(sizeof(dcmt_eval_result) == sizeof(dcmt::EvalResult), "dcmt_eval_r
 int dcmt_evaluate_f32(const float* gt, const float* dense, int rows, int cols, size_t pitch_bytes, size_t frame_stride_bytes,
                       int n_frames, float tolerance, int mode, dcmt_eval_result* results, void* cuda_stream) {
     return run_evaluation(eval_f32(gt, pitch_bytes, frame_stride_bytes), eval_f32(dense, pitch_bytes, frame_stride_bytes), rows, cols,
-                          n_frames, tolerance, mode, results, cuda_stream);
+                          n_frames, mode, results, cuda_stream, EvalReductions(tolerance, mode));
 }
 
 int dcmt_evaluate_f32_host(const float* gt, const float* dense, int rows, int cols, size_t pitch_bytes, size_t frame_stride_bytes,
                            int n_frames, float tolerance, int mode, dcmt_eval_result* results) {
     return run_evaluation_host(eval_f32(gt, pitch_bytes, frame_stride_bytes), eval_f32(dense, pitch_bytes, frame_stride_bytes), rows, cols,
-                               n_frames, tolerance, mode, results);
+                               n_frames, mode, results, EvalReductions(tolerance, mode));
 }
 
 int dcmt_evaluate_u16(const uint16_t* gt_u16, const float* dense, int rows, int cols, size_t gt_pitch_bytes, size_t gt_frame_stride_bytes,
                       size_t dense_pitch_bytes, size_t dense_frame_stride_bytes, int n_frames, float tolerance, int mode,
                       dcmt_eval_result* results, void* cuda_stream) {
     return run_evaluation(eval_u16(gt_u16, gt_pitch_bytes, gt_frame_stride_bytes), eval_f32(dense, dense_pitch_bytes, dense_frame_stride_bytes),
-                          rows, cols, n_frames, tolerance, mode, results, cuda_stream);
+                          rows, cols, n_frames, mode, results, cuda_stream, EvalReductions(tolerance, mode));
 }
 
 int dcmt_evaluate_u16_host(const uint16_t* gt_u16, const float* dense, int rows, int cols, size_t gt_pitch_bytes,
                            size_t gt_frame_stride_bytes, size_t dense_pitch_bytes, size_t dense_frame_stride_bytes, int n_frames,
                            float tolerance, int mode, dcmt_eval_result* results) {
     return run_evaluation_host(eval_u16(gt_u16, gt_pitch_bytes, gt_frame_stride_bytes),
-                               eval_f32(dense, dense_pitch_bytes, dense_frame_stride_bytes), rows, cols, n_frames, tolerance, mode, results);
+                               eval_f32(dense, dense_pitch_bytes, dense_frame_stride_bytes), rows, cols, n_frames, mode, results,
+                               EvalReductions(tolerance, mode));
 }
 
 int dcmt_evaluate_u16_u16(const uint16_t* gt_u16, const uint16_t* dense_u16, int rows, int cols, size_t gt_pitch_bytes,
                           size_t gt_frame_stride_bytes, size_t dense_pitch_bytes, size_t dense_frame_stride_bytes, int n_frames,
                           float tolerance, int mode, dcmt_eval_result* results, void* cuda_stream) {
     return run_evaluation(eval_u16(gt_u16, gt_pitch_bytes, gt_frame_stride_bytes),
-                          eval_u16(dense_u16, dense_pitch_bytes, dense_frame_stride_bytes), rows, cols, n_frames, tolerance, mode, results,
-                          cuda_stream);
+                          eval_u16(dense_u16, dense_pitch_bytes, dense_frame_stride_bytes), rows, cols, n_frames, mode, results, cuda_stream,
+                          EvalReductions(tolerance, mode));
 }
 
 int dcmt_evaluate_u16_u16_host(const uint16_t* gt_u16, const uint16_t* dense_u16, int rows, int cols, size_t gt_pitch_bytes,
                                size_t gt_frame_stride_bytes, size_t dense_pitch_bytes, size_t dense_frame_stride_bytes, int n_frames,
                                float tolerance, int mode, dcmt_eval_result* results) {
     return run_evaluation_host(eval_u16(gt_u16, gt_pitch_bytes, gt_frame_stride_bytes),
-                               eval_u16(dense_u16, dense_pitch_bytes, dense_frame_stride_bytes), rows, cols, n_frames, tolerance, mode,
-                               results);
+                               eval_u16(dense_u16, dense_pitch_bytes, dense_frame_stride_bytes), rows, cols, n_frames, mode, results,
+                               EvalReductions(tolerance, mode));
+}
+
+static_assert(sizeof(dcmt_kitti_metrics) == sizeof(dcmt::KittiMetrics) && sizeof(dcmt_kitti_metrics) == 80,
+              "dcmt_kitti_metrics and dcmt::KittiMetrics must match");
+
+int dcmt_evaluate_kitti_f32(const float* gt, const float* pred, int rows, int cols, size_t gt_pitch_bytes, size_t gt_frame_stride_bytes,
+                            size_t pred_pitch_bytes, size_t pred_frame_stride_bytes, int n_frames, dcmt_kitti_metrics* results,
+                            void* cuda_stream) {
+    return run_evaluation(eval_f32(gt, gt_pitch_bytes, gt_frame_stride_bytes), eval_f32(pred, pred_pitch_bytes, pred_frame_stride_bytes),
+                          rows, cols, n_frames, DCMT_EVAL_GT_VALID, results, cuda_stream, EvalKitti());
+}
+
+int dcmt_evaluate_kitti_f32_host(const float* gt, const float* pred, int rows, int cols, size_t gt_pitch_bytes,
+                                 size_t gt_frame_stride_bytes, size_t pred_pitch_bytes, size_t pred_frame_stride_bytes, int n_frames,
+                                 dcmt_kitti_metrics* results) {
+    return run_evaluation_host(eval_f32(gt, gt_pitch_bytes, gt_frame_stride_bytes), eval_f32(pred, pred_pitch_bytes, pred_frame_stride_bytes),
+                               rows, cols, n_frames, DCMT_EVAL_GT_VALID, results, EvalKitti());
+}
+
+int dcmt_evaluate_kitti_u16(const uint16_t* gt_u16, const float* pred, int rows, int cols, size_t gt_pitch_bytes,
+                            size_t gt_frame_stride_bytes, size_t pred_pitch_bytes, size_t pred_frame_stride_bytes, int n_frames,
+                            dcmt_kitti_metrics* results, void* cuda_stream) {
+    return run_evaluation(eval_u16(gt_u16, gt_pitch_bytes, gt_frame_stride_bytes), eval_f32(pred, pred_pitch_bytes, pred_frame_stride_bytes),
+                          rows, cols, n_frames, DCMT_EVAL_GT_VALID, results, cuda_stream, EvalKitti());
+}
+
+int dcmt_evaluate_kitti_u16_host(const uint16_t* gt_u16, const float* pred, int rows, int cols, size_t gt_pitch_bytes,
+                                 size_t gt_frame_stride_bytes, size_t pred_pitch_bytes, size_t pred_frame_stride_bytes, int n_frames,
+                                 dcmt_kitti_metrics* results) {
+    return run_evaluation_host(eval_u16(gt_u16, gt_pitch_bytes, gt_frame_stride_bytes),
+                               eval_f32(pred, pred_pitch_bytes, pred_frame_stride_bytes), rows, cols, n_frames, DCMT_EVAL_GT_VALID, results,
+                               EvalKitti());
+}
+
+int dcmt_evaluate_kitti_u16_u16(const uint16_t* gt_u16, const uint16_t* pred_u16, int rows, int cols, size_t gt_pitch_bytes,
+                                size_t gt_frame_stride_bytes, size_t pred_pitch_bytes, size_t pred_frame_stride_bytes, int n_frames,
+                                dcmt_kitti_metrics* results, void* cuda_stream) {
+    return run_evaluation(eval_u16(gt_u16, gt_pitch_bytes, gt_frame_stride_bytes),
+                          eval_u16(pred_u16, pred_pitch_bytes, pred_frame_stride_bytes), rows, cols, n_frames, DCMT_EVAL_GT_VALID, results,
+                          cuda_stream, EvalKitti());
+}
+
+int dcmt_evaluate_kitti_u16_u16_host(const uint16_t* gt_u16, const uint16_t* pred_u16, int rows, int cols, size_t gt_pitch_bytes,
+                                     size_t gt_frame_stride_bytes, size_t pred_pitch_bytes, size_t pred_frame_stride_bytes, int n_frames,
+                                     dcmt_kitti_metrics* results) {
+    return run_evaluation_host(eval_u16(gt_u16, gt_pitch_bytes, gt_frame_stride_bytes),
+                               eval_u16(pred_u16, pred_pitch_bytes, pred_frame_stride_bytes), rows, cols, n_frames, DCMT_EVAL_GT_VALID,
+                               results, EvalKitti());
 }
 
 void dcmt_stereo_params_default(dcmt_stereo_params* p) {

@@ -22,4 +22,25 @@ template <class G, class R>
 cudaError_t eval_run(const G* gt, size_t gpitch, size_t gfstride, const R* r, size_t rpitch, size_t rfstride, int rows, int cols,
                      int n_frames, float tol, int mode, double* partials, EvalResult* out, cudaStream_t st);
 
+// per-frame figures of the KITTI depth-completion benchmark (mirrors dcmt_kitti_metrics in include/dcmt.h, which states
+// the rule: the devkit's background interpolation of the prediction, then the error terms at every GT-valid pixel)
+struct KittiMetrics {
+    double n_gt, n_pred, n_unfilled;                // GT-valid pixels; of those, valid in the prediction; left unfilled (p = -1)
+    double sum_abs, sum_sq, sum_iabs, sum_isq;      // sums of |g - p|, its square, |1/g - 1/p|, its square
+    float mae_mm, rmse_mm, imae_per_km, irmse_per_km, density;  // NaN when n_gt == 0
+    int32_t pad;
+};
+
+// Workspace of kitti_run: partial sums, the first / last rows holding a valid prediction (two int32 per frame), and --
+// for rows too wide for the validity bits to fit in shared memory -- one bit row per block in device memory (0 words
+// otherwise).
+size_t kitti_partial_doubles(int n_frames);
+size_t kitti_bits_words(int rows, int cols, int n_frames);
+// Same block layout, pixel order and lane / warp / block reduction as eval_run, so that on a prediction with no invalid
+// pixel n_gt, sum_abs and sum_sq are the bytes of eval_run's count, sum_abs and sum_sq in mode 0 with tolerance 0.
+// Instantiated for <float, float>, <uint16_t, float> and <uint16_t, uint16_t>.
+template <class G, class R>
+cudaError_t kitti_run(const G* gt, size_t gpitch, size_t gfstride, const R* r, size_t rpitch, size_t rfstride, int rows, int cols,
+                      int n_frames, double* partials, int32_t* first_last, unsigned* bits, KittiMetrics* out, cudaStream_t st);
+
 }  // namespace dcmt

@@ -413,6 +413,57 @@ DCMT_API int dcmt_evaluate_u16_u16_host(const uint16_t *gt_u16, const uint16_t *
                                         size_t dense_frame_stride_bytes, int n_frames, float tolerance, int mode,
                                         dcmt_eval_result *results /* host, n_frames */);
 
+/* The figures the KITTI depth-completion benchmark publishes: MAE and RMSE in mm, iMAE and iRMSE in 1/km, over every
+ * pixel with ground truth after the prediction's holes are filled by the devkit's background interpolation.  The rule
+ * below restates the devkit's interpolateBackground and per-image error loop; the tests pin the library to a numpy
+ * restatement of this text, not to the devkit itself.  Per frame, with g the GT and p the prediction in metres:
+ *  1. A uint16 value u decodes to (float)u * (1.0f / 256.0f).  g is valid iff g > 0, p iff p > 0 (so uint16 0, float32 0,
+ *     negatives and NaN are invalid).
+ *  2. Background interpolation of p.  Row pass: in each row, an invalid pixel takes min(L, R) of the values of the nearest
+ *     valid pixels to its left and right in that row, or the one that exists; a row with no valid pixel stays invalid.
+ *     Column pass: with F / B the first / last rows holding a valid p, every pixel of a row above F takes the row-pass
+ *     value of its column in row F, every pixel of a row below B that of row B.  Invalid rows strictly between F and B,
+ *     and every pixel of a frame with no valid p, stay unfilled and carry the devkit's marker p = -1.
+ *  3. At GT-valid pixels only: e = fabsf(g - p) (float32, then widened to double), ie = fabs(1.0 / g - 1.0 / p) in double.
+ *  4. Sums in double, combined in a fixed order: n_gt (GT-valid pixels), n_pred (of those, valid in p before the
+ *     interpolation), n_unfilled (left unfilled by step 2), sum_abs = sum e, sum_sq = sum e^2, sum_iabs = sum ie,
+ *     sum_isq = sum ie^2.
+ *  5. mae_mm = 1000 * sum_abs / n_gt, rmse_mm = 1000 * sqrt(sum_sq / n_gt), imae_per_km = 1000 * sum_iabs / n_gt,
+ *     irmse_per_km = 1000 * sqrt(sum_isq / n_gt), density = n_pred / n_gt; each computed in double and rounded once to
+ *     float; NaN when n_gt == 0.
+ * One record per frame; the benchmark reports the mean of the per-image figures over the set, which the caller takes.
+ * Type pairs, pitches and frame strides (bytes per side, 0 = dense) are those of dcmt_evaluate_u16[_u16] plus a float32
+ * pair; a uint16 call gives the bytes of the float32 call on the decoded planes laid out alike in elements.  The pixels of
+ * a valid prediction are visited in the order of dcmt_evaluate_*, so on a prediction with no invalid pixel n_gt, sum_abs
+ * and sum_sq are byte-equal to count, sum_abs and sum_sq of dcmt_evaluate_* in mode DCMT_EVAL_GT_VALID with tolerance 0.
+ * Bad arguments return DCMT_E_BADARG before any device work; n_frames == 0 is a no-op. */
+typedef struct dcmt_kitti_metrics {
+    double n_gt, n_pred, n_unfilled;
+    double sum_abs, sum_sq, sum_iabs, sum_isq;
+    float mae_mm, rmse_mm, imae_per_km, irmse_per_km, density;
+    int32_t pad;
+} dcmt_kitti_metrics;
+DCMT_API int dcmt_evaluate_kitti_f32(const float *gt, const float *pred, int rows, int cols, size_t gt_pitch_bytes,
+                                     size_t gt_frame_stride_bytes, size_t pred_pitch_bytes, size_t pred_frame_stride_bytes,
+                                     int n_frames, dcmt_kitti_metrics *results /* device, n_frames */, void *cuda_stream);
+DCMT_API int dcmt_evaluate_kitti_f32_host(const float *gt, const float *pred, int rows, int cols, size_t gt_pitch_bytes,
+                                          size_t gt_frame_stride_bytes, size_t pred_pitch_bytes, size_t pred_frame_stride_bytes,
+                                          int n_frames, dcmt_kitti_metrics *results /* host, n_frames */);
+DCMT_API int dcmt_evaluate_kitti_u16(const uint16_t *gt_u16, const float *pred, int rows, int cols, size_t gt_pitch_bytes,
+                                     size_t gt_frame_stride_bytes, size_t pred_pitch_bytes, size_t pred_frame_stride_bytes,
+                                     int n_frames, dcmt_kitti_metrics *results /* device, n_frames */, void *cuda_stream);
+DCMT_API int dcmt_evaluate_kitti_u16_host(const uint16_t *gt_u16, const float *pred, int rows, int cols, size_t gt_pitch_bytes,
+                                          size_t gt_frame_stride_bytes, size_t pred_pitch_bytes, size_t pred_frame_stride_bytes,
+                                          int n_frames, dcmt_kitti_metrics *results /* host, n_frames */);
+DCMT_API int dcmt_evaluate_kitti_u16_u16(const uint16_t *gt_u16, const uint16_t *pred_u16, int rows, int cols,
+                                         size_t gt_pitch_bytes, size_t gt_frame_stride_bytes, size_t pred_pitch_bytes,
+                                         size_t pred_frame_stride_bytes, int n_frames,
+                                         dcmt_kitti_metrics *results /* device, n_frames */, void *cuda_stream);
+DCMT_API int dcmt_evaluate_kitti_u16_u16_host(const uint16_t *gt_u16, const uint16_t *pred_u16, int rows, int cols,
+                                              size_t gt_pitch_bytes, size_t gt_frame_stride_bytes, size_t pred_pitch_bytes,
+                                              size_t pred_frame_stride_bytes, int n_frames,
+                                              dcmt_kitti_metrics *results /* host, n_frames */);
+
 /* (8f #2) LiDAR projection + normalisation: replaces the loops of src/DC_stereo_lidar/main_sl.cpp:478-523 (withSuperPixels;
  * the same code in vedi_pc :340-385): Velodyne points (n_points x 4 float32: x, y, z, intensity -- the .bin payload)
  * -> T (4x4, velodyne to camera; rows 0..2 used) -> keep z > 0 -> P (3x4) -> perspective division -> bounds test ->

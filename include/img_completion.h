@@ -15,6 +15,8 @@
 //     void retrieve_optimized_depth(cv::Mat& disparity, cv::Mat& depth);                                            :863
 //     void evaluate_performance / evaluate_performances                      main.cpp:16, main_lc.cpp:85, main_sl.cpp:1031
 //
+// and, beyond the reference, dcmt::evaluate_kitti: the KITTI depth-completion benchmark's figures of a result.
+//
 // The stereo functions take the reference's own containers: EntryType matrices (struct { float value;
 // Eigen::Vector2f derivative; }, main_sl.cpp:23-26) stored as cv::Mat(rows, cols, CV_32FC(sizeof(EntryType))) (:1165).
 // EntryType itself stays the caller's (main_sl.cpp defines it); this header only relies on its 12-byte layout.
@@ -120,6 +122,32 @@ inline dcmt_eval_result evaluate_u16_u16(const MatView& GT_u16, const MatView& r
     dcmt_eval_result res;
     check(dcmt_evaluate_u16_u16_host(static_cast<const uint16_t*>(GT_u16.data), static_cast<const uint16_t*>(r_u16.data), GT_u16.rows,
                                      GT_u16.cols, GT_u16.step, 0, r_u16.step, 0, 1, tolerance, mode, &res));
+    return res;
+}
+// The KITTI depth-completion benchmark's figures for one frame (dcmt_evaluate_kitti_*; include/dcmt.h states the rule,
+// a restatement of the devkit's background interpolation and error loop): MAE / RMSE in mm, iMAE / iRMSE in 1/km and
+// density, with the sums behind them.  A float32 pair (evaluate_kitti), or the KITTI GT as read (CV_16UC1 view, metres *
+// 256) with a float32 or a KITTI uint16 prediction.  Each view has its own step.
+inline dcmt_kitti_metrics evaluate_kitti(const MatView& gt, const MatView& pred) {
+    if (gt.rows != pred.rows || gt.cols != pred.cols) throw std::invalid_argument("dcmt: evaluate_kitti needs same-shaped Mats");
+    dcmt_kitti_metrics res;
+    check(dcmt_evaluate_kitti_f32_host(static_cast<const float*>(gt.data), static_cast<const float*>(pred.data), gt.rows, gt.cols, gt.step, 0,
+                                       pred.step, 0, 1, &res));
+    return res;
+}
+inline dcmt_kitti_metrics evaluate_kitti_u16(const MatView& gt_u16, const MatView& pred) {
+    if (gt_u16.rows != pred.rows || gt_u16.cols != pred.cols) throw std::invalid_argument("dcmt: evaluate_kitti_u16 needs same-shaped Mats");
+    dcmt_kitti_metrics res;
+    check(dcmt_evaluate_kitti_u16_host(static_cast<const uint16_t*>(gt_u16.data), static_cast<const float*>(pred.data), gt_u16.rows,
+                                       gt_u16.cols, gt_u16.step, 0, pred.step, 0, 1, &res));
+    return res;
+}
+inline dcmt_kitti_metrics evaluate_kitti_u16_u16(const MatView& gt_u16, const MatView& pred_u16) {
+    if (gt_u16.rows != pred_u16.rows || gt_u16.cols != pred_u16.cols)
+        throw std::invalid_argument("dcmt: evaluate_kitti_u16_u16 needs same-shaped Mats");
+    dcmt_kitti_metrics res;
+    check(dcmt_evaluate_kitti_u16_u16_host(static_cast<const uint16_t*>(gt_u16.data), static_cast<const uint16_t*>(pred_u16.data),
+                                           gt_u16.rows, gt_u16.cols, gt_u16.step, 0, pred_u16.step, 0, 1, &res));
     return res;
 }
 // src/DC_lidar_only/main.cpp:16-34: "mse" = mean of (gt - r) over gt > 0 (a signed mean, sic)
@@ -426,6 +454,14 @@ inline dcmt_eval_result evaluate_mats(const cv::Mat& GT_img, const cv::Mat& r_im
     CV_Assert(GT_img.type() == CV_32FC1 && r_img.type() == CV_32FC1);
     const cv::Mat g = continuous(GT_img), r = continuous(r_img);
     return evaluate(view_of(g), view_of(r), tolerance, mode);
+}
+// The KITTI benchmark's figures on Mats: CV_16UC1 GT with a CV_32FC1 or CV_16UC1 prediction, or a CV_32FC1 pair; any other
+// pair throws.
+inline dcmt_kitti_metrics evaluate_kitti(const cv::Mat& gt, const cv::Mat& pred) {
+    if (gt.type() == CV_16UC1 && pred.type() == CV_16UC1) return evaluate_kitti_u16_u16(view_of(gt), view_of(pred));
+    if (gt.type() == CV_16UC1 && pred.type() == CV_32FC1) return evaluate_kitti_u16(view_of(gt), view_of(pred));
+    CV_Assert(gt.type() == CV_32FC1 && pred.type() == CV_32FC1);
+    return evaluate_kitti(view_of(gt), view_of(pred));
 }
 }  // namespace dcmt
 
