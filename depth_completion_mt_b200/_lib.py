@@ -116,6 +116,12 @@ _SIGNATURES = {
     "dcmt_interpolate_with_superpixels_u16_u16": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P, _P]),
     "dcmt_interpolate_with_superpixels_u16_u16_host": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P]),
     "dcmt_interpolate_with_superpixels_u16_u16_host_multi": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int]),
+    "dcmt_interpolate_with_superpixels_bgr_u16": (C.c_int, [_P, C.c_size_t, C.c_size_t, _P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
+    "dcmt_interpolate_with_superpixels_bgr_u16_host": (C.c_int, [_P, C.c_size_t, C.c_size_t, _P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
+    "dcmt_interpolate_with_superpixels_bgr_u16_host_multi": (C.c_int, [_P, C.c_size_t, C.c_size_t, _P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int]),
+    "dcmt_interpolate_with_superpixels_bgr_u16_u16": (C.c_int, [_P, C.c_size_t, C.c_size_t, _P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
+    "dcmt_interpolate_with_superpixels_bgr_u16_u16_host": (C.c_int, [_P, C.c_size_t, C.c_size_t, _P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
+    "dcmt_interpolate_with_superpixels_bgr_u16_u16_host_multi": (C.c_int, [_P, C.c_size_t, C.c_size_t, _P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int]),
     "dcmt_depth_to_u16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, _P]),
     "dcmt_bgr2gray_u8": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, _P]),
     "dcmt_bgr2gray_u8_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int]),

@@ -254,6 +254,64 @@ def interpolate_with_superpixels(labels, sparse, blur_type="gaussian", use_super
     return (out, stats) if return_stats else out
 
 
+def interpolate_with_superpixels_bgr(bgr, sparse_u16, step, nc: int, *, use_superpixel: int = 1, iterations: int = 10,
+                                     out_dtype=np.float32, path: str = "auto", return_stats: bool = False, devices=None, stream=None,
+                                     lib: _lib.Library | None = None):
+    """main_lc.cpp:159-220 from the camera frame in one call: ``cvtColor(COLOR_BGR2Lab)``, ``generate_superpixels(lab, step, nc)``
+    and ``interpolate_with_superpixels`` of the KITTI uint16 depth (``dcmt_interpolate_with_superpixels_bgr_u16[_u16]``); the
+    Lab image and the labels stay on the device.
+
+    ``bgr`` is the uint8 colour image as read, (rows, cols, 3) or (n, rows, cols, 3); ``sparse_u16`` the uint16 depth
+    (metres * 256), (rows, cols) or (n, rows, cols).  ``step`` is truncated to int as the reference's int parameter does
+    (main_lc.cpp:197-201).  Returns what ``interpolate_with_superpixels(generate_superpixels_bgr(bgr, step, nc), sparse_u16,
+    n_clusters=K)`` returns, byte for byte: float32 metres, or KITTI uint16 with ``out_dtype`` uint16.  CUDA tensors use the
+    device entry point on ``stream``; numpy arrays the host entry point, or -- with ``devices`` ("all" or a list of
+    ordinals) -- the frames spread over those GPUs.  Float32 depth has no one-call form: run ``generate_superpixels_bgr``
+    and ``interpolate_with_superpixels``."""
+    lib = lib or _lib.load()
+    step = int(step)
+    is_t = _is_torch(sparse_u16)
+    u16_in = sparse_u16.dtype == (torch.uint16 if is_t else np.uint16)
+    if not u16_in:
+        raise ValueError("interpolate_with_superpixels_bgr takes uint16 (KITTI) depth only; for float32 depth call "
+                         "generate_superpixels_bgr and then interpolate_with_superpixels")
+    u16_out = _u16_output(out_dtype, True)
+    if is_t:
+        if devices is not None:
+            raise ValueError("devices= applies to host (numpy) input; a CUDA tensor already lives on one device")
+        x = _prep_torch(bgr, torch.uint8, "bgr")
+        s3, squeeze = _batch3(_prep_torch(sparse_u16, torch.uint16, "sparse_u16"), "sparse_u16")
+    else:
+        x = _prep_numpy(bgr, np.uint8, "bgr")
+        s3, squeeze = _batch3(_prep_numpy(sparse_u16, np.uint16, "sparse_u16"), "sparse_u16")
+    x4 = x[None] if x.ndim == 3 else x
+    if x4.ndim != 4 or tuple(x4.shape) != tuple(s3.shape) + (3,):
+        raise ValueError(f"bgr must be the (rows, cols, 3) colour image of each depth frame, got {tuple(x.shape)} for {tuple(s3.shape)}")
+    n, rows, cols = (int(v) for v in s3.shape)
+    suffix = "u16_u16" if u16_out else "u16"
+    args = (rows, cols, 0, 0, 0, 0, n, step, int(nc), int(iterations), int(use_superpixel), PATH[path])
+    if is_t:
+        out = _out_torch(None, s3, torch.uint16 if u16_out else torch.float32)
+        stats = torch.zeros((n, STATS_STRIDE), dtype=torch.int32, device=s3.device) if return_stats else None
+        with torch.cuda.device(s3.device):
+            lib.check(getattr(lib, "dcmt_interpolate_with_superpixels_bgr_" + suffix)(
+                x4.data_ptr(), 0, 0, s3.data_ptr(), out.data_ptr(), *args, stats.data_ptr() if return_stats else None, _stream_ptr(stream)))
+    else:
+        out = _out_numpy(None, s3, np.uint16 if u16_out else np.float32)
+        stats = np.zeros((n, STATS_STRIDE), np.int32) if return_stats else None
+        st_ptr = _np_ptr(stats) if return_stats else None
+        keep, dev_ptr, n_dev = _device_list(devices)
+        if devices is not None:
+            lib.check(getattr(lib, f"dcmt_interpolate_with_superpixels_bgr_{suffix}_host_multi")(
+                _np_ptr(x4), 0, 0, _np_ptr(s3), _np_ptr(out), *args, st_ptr, dev_ptr, n_dev))
+        else:
+            lib.check(getattr(lib, f"dcmt_interpolate_with_superpixels_bgr_{suffix}_host")(
+                _np_ptr(x4), 0, 0, _np_ptr(s3), _np_ptr(out), *args, st_ptr))
+        del keep
+    out = out[0] if squeeze else out
+    return (out, stats) if return_stats else out
+
+
 def depth_to_u16(depth, *, out=None, stream=None, lib: _lib.Library | None = None):
     """``depth.convertTo(png, CV_16U, 256)`` on the device (``dcmt_depth_to_u16``): float32 metres (CUDA tensor, (rows, cols)
     or (n, rows, cols)) -> KITTI uint16 = metres * 256, rounded half to even, clamped to [0, 65535], NaN -> 0."""

@@ -186,12 +186,21 @@ cudaError_t prof_mark(cudaStream_t st, int which, ProfEvents* pe) {
     return cudaEventRecord(pe->e[which], st);
 }
 
+// cv::cvtColor(COLOR_BGR2Lab) + Slic::generate_superpixels in front of a guided completion: the labels are made on the
+// device from the caller's BGR frames (dcmt_interpolate_with_superpixels_bgr_*) instead of being passed in
+struct BgrFront {
+    const uint8_t* bgr;
+    size_t pitch, fstride;  // bytes; the ABI's 0 = dense until validate_completion fills them in
+    int step, nc, iterations;
+};
+
 // one completion call as its entry point describes it (checked by validate_completion)
 struct CompletionCall {
     const int32_t* labels;
     int n_clusters;
     bool guided;
     int rows, cols, blur, flags;
+    BgrFront* front = nullptr;  // labels from BGR frames (`labels` unused; validate_completion sets n_clusters)
 };
 
 // the strict-q8 fused path serves plain img_completion with blur none/gaussian on frames of a sane size
@@ -436,11 +445,21 @@ int pinned_flags(cudaStream_t key, size_t n, int32_t** out) {
     return DCMT_OK;
 }
 
-// Checks a completion call -- pointers, labels, blur, flags, input geometry, output geometry, overlap, in this order --
-// and converts the pitches and frame strides of `in` and `out` from the ABI's bytes into elements.
-int validate_completion(const CompletionCall& cc, InDesc* in, OutDesc* out, int n_frames) {
+// SLIC's own limits (slic.cpp:72-99 and the kernels' index arithmetic), on frames already checked to be 1..2^30 pixels
+int check_slic(int rows, int cols, int step, int nc, int iterations) {
+    if (nc == 0 || iterations < 0) return fail(DCMT_E_BADARG, "nc %d, iterations %d", nc, iterations);
+    if (step < 4) return fail(DCMT_E_UNSUPPORTED, "step %d: find_local_minimum (slic.cpp:72-99) reads outside the image below 4", step);
+    if (rows >= 1 << 24 || cols >= 1 << 24) return fail(DCMT_E_UNSUPPORTED, "SLIC frames are limited to 2^24 rows / columns");
+    return DCMT_OK;
+}
+
+// Checks a completion call -- pointers, labels, blur, flags, input geometry, output geometry, overlap, in this order, then
+// for a BGR front its pointer, SLIC's arguments, its geometry and its overlap with the output -- and converts the pitches
+// and frame strides of `in` and `out` from the ABI's bytes into elements.  A BGR front gets its dense pitch / frame stride
+// filled in and `cc.n_clusters` is set to SLIC's centre count.
+int validate_completion(CompletionCall& cc, InDesc* in, OutDesc* out, int n_frames) {
     if (!in->ptr() || !out->ptr()) return fail(DCMT_E_BADARG, "null image pointer");
-    if (cc.guided && !cc.labels) return fail(DCMT_E_BADARG, "null label pointer");
+    if (cc.guided && !cc.labels && !cc.front) return fail(DCMT_E_BADARG, "null label pointer");
     if (cc.blur < DCMT_BLUR_NONE || cc.blur > DCMT_BLUR_BILATERAL) return fail(DCMT_E_BADARG, "blur_type %d", cc.blur);
     if (cc.flags < DCMT_PATH_AUTO || cc.flags > DCMT_PATH_RANK) return fail(DCMT_E_BADARG, "flags %d", cc.flags);
     Geometry gi, go;
@@ -448,6 +467,19 @@ int validate_completion(const CompletionCall& cc, InDesc* in, OutDesc* out, int 
     if (rc) return rc;
     if ((rc = check_geometry(cc.rows, cc.cols, out->pitch, out->fstride, n_frames, &go, out->elem()))) return rc;
     if (n_frames && overlaps(in->ptr(), gi.span_bytes, out->ptr(), go.span_bytes)) return fail(DCMT_E_BADARG, "input and output overlap");
+    if (BgrFront* fr = cc.front) {
+        if (!fr->bgr) return fail(DCMT_E_BADARG, "null image pointer");
+        if ((rc = check_slic(cc.rows, cc.cols, fr->step, fr->nc, fr->iterations))) return rc;
+        const size_t row = (size_t)cc.cols * 3;
+        if (fr->pitch == 0) fr->pitch = row;
+        if (fr->fstride == 0) fr->fstride = fr->pitch * cc.rows;
+        if (fr->pitch < row) return fail(DCMT_E_BADARG, "bgr_pitch_bytes %zu below %d columns of 3 bytes", fr->pitch, cc.cols);
+        const size_t frame = fr->pitch * (size_t)(cc.rows - 1) + row;
+        if (fr->fstride < frame) return fail(DCMT_E_BADARG, "bgr_frame_stride_bytes %zu invalid", fr->fstride);
+        if (n_frames && overlaps(fr->bgr, fr->fstride * (size_t)(n_frames - 1) + frame, out->ptr(), go.span_bytes))
+            return fail(DCMT_E_BADARG, "BGR input and output overlap");
+        cc.n_clusters = dcmt::slic_center_count(cc.rows, cc.cols, fr->step);
+    }
     in->pitch = gi.pitch;
     in->fstride = gi.fstride;
     out->pitch = go.pitch;
@@ -508,6 +540,79 @@ int run_completion(CompletionCall cc, InDesc in, OutDesc out, int n_frames, int3
             f = e;
         }
         if (level == DCMT_PATH_GENERIC || !any) break;
+    }
+    return DCMT_OK;
+}
+
+// ---- SLIC on a workspace carved from an arena the caller holds, so that the chained calls keep their staging buffers,
+// labels and completion workspace in the same arena.  slic_ws_bytes() sizes what enqueue_slic() carves for n frames: the
+// work arrays of SlicWork and, with from_bgr, the Lab frames.
+size_t slic_ws_bytes(int rows, int cols, int n, int step, bool from_bgr) {
+    int bx = 0, by = 0;
+    const int k = dcmt::slic_center_count(rows, cols, step);
+    const size_t nbins = dcmt::slic_bins(rows, cols, step, &bx, &by);
+    const size_t kk = (k > 0 ? (size_t)k : 1) * n, nb = nbins * n;
+    return 2 * carve_bytes(kk * 5, sizeof(double)) + carve_bytes(kk * 6, sizeof(unsigned long long)) + carve_bytes(nb + n, sizeof(int)) +
+           carve_bytes(nb, sizeof(int)) + carve_bytes(kk, sizeof(int)) + (from_bgr ? carve_bytes((size_t)rows * cols * 3 * n, 1) : 0);
+}
+
+// Slic::generate_superpixels of n frames (arguments checked, 1 <= n <= 65535) into `labels` (and `centers` when given):
+// on the Lab frames `img` (dense), or, with from_bgr, on the cvtColor(COLOR_BGR2Lab) of the BGR frames `img` (pitch and
+// frame stride in bytes), made into the arena first
+int enqueue_slic(const uint8_t* img, size_t pitch, size_t fstride, bool from_bgr, int rows, int cols, int n, int step, int nc, int iterations,
+                 int32_t* labels, double* centers, Arena* ar, cudaStream_t st) {
+    const int k = dcmt::slic_center_count(rows, cols, step);
+    dcmt::SlicWork w{};
+    const size_t nbins = dcmt::slic_bins(rows, cols, step, &w.bins_x, &w.bins_y);
+    const size_t kk = (k > 0 ? (size_t)k : 1) * n, nb = nbins * n;
+    w.centers = carve<double>(ar, kk * 5);
+    w.sums = carve<unsigned long long>(ar, kk * 6);
+    w.bin_count = carve<int>(ar, nb + n);
+    w.bin_fill = carve<int>(ar, nb);
+    w.bin_items = carve<int>(ar, kk);
+    w.sorted = carve<double>(ar, kk * 5);
+    uint8_t* lab = from_bgr ? carve<uint8_t>(ar, (size_t)rows * cols * 3 * n) : nullptr;
+    if (int rc = arena_ok(ar)) return rc;
+    if (from_bgr) {
+        const size_t lab_pitch = (size_t)cols * 3;
+        API_CUDA(dcmt::color_bgr2lab(img, pitch, fstride, lab, lab_pitch, lab_pitch * rows, rows, cols, n, st), "BGR2Lab launch");
+    }
+    API_CUDA(dcmt::slic_run(from_bgr ? lab : img, rows, cols, n, step, nc, iterations, labels, k, w, st), "SLIC launch");
+    if (centers && k > 0)
+        API_CUDA(cudaMemcpyAsync(centers, w.centers, (size_t)k * n * 5 * sizeof(double), cudaMemcpyDeviceToDevice, st), "centre copy");
+    return DCMT_OK;
+}
+
+// device-pointer driver of the dcmt_interpolate_with_superpixels_bgr_* entry points (uint16 input: never synchronises).
+// Chunks of the completion's size, each in one workspace of the caller's stream: Lab frames, labels, SLIC's work arrays
+// and the completion workspace; BGR2Lab, SLIC and the guided completion run on that stream.
+int run_completion_bgr(CompletionCall cc, InDesc in, OutDesc out, int n_frames, int32_t* stats, cudaStream_t st) {
+    int rc = validate_completion(cc, &in, &out, n_frames);
+    if (rc) return rc;
+    if (n_frames == 0) return DCMT_OK;
+    if ((rc = check_device())) return rc;
+    API_CUDA(dcmt::generic_configure(), "kernel attribute setup");
+    API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
+    cc.flags = input_path(in, cc.flags);
+    const BgrFront& fr = *cc.front;
+    const size_t fpix = (size_t)cc.rows * cc.cols;
+    const int chunk = chunk_frames(cc.rows, cc.cols, n_frames, fused_applies(cc));
+    const size_t bytes = completion_ws_bytes(cc, chunk, in.elem(), out.elem()) +
+                         (cc.guided ? carve_bytes(fpix * chunk, sizeof(int32_t)) + slic_ws_bytes(cc.rows, cc.cols, chunk, fr.step, true) : 0);
+    for (int f0 = 0; f0 < n_frames; f0 += chunk) {
+        const int nf = std::min(chunk, n_frames - f0);
+        Arena* ar = nullptr;
+        if ((rc = arena_acquire(st, bytes, &ar))) return rc;  // stream order: the previous chunk is done with it
+        int32_t* labels = nullptr;
+        if (cc.guided) {
+            labels = carve<int32_t>(ar, fpix * nf);
+            if ((rc = enqueue_slic(fr.bgr + (size_t)f0 * fr.fstride, fr.pitch, fr.fstride, true, cc.rows, cc.cols, nf, fr.step, fr.nc,
+                                   fr.iterations, labels, nullptr, ar, st)))
+                return rc;
+        }
+        if ((rc = enqueue_completion(cc, in.frames_from((size_t)f0), labels, out.frames_from((size_t)f0), nf,
+                                     stats ? stats + (size_t)f0 * DCMT_STATS_STRIDE : nullptr, nullptr, nullptr, nullptr, ar, st)))
+            return rc;
     }
     return DCMT_OK;
 }
@@ -729,8 +834,11 @@ int run_completion_host(CompletionCall cc, InDesc in, OutDesc out, int n_frames,
         API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
         if (flagged && (rc = pinned_flags(nullptr, (size_t)(l.f_end - l.f_begin), &l.h_flags))) return rc;
     }
+    // labels made from BGR frames on the device (staged packed, 3 bytes per pixel) instead of copied in
+    const BgrFront* front = cc.guided ? cc.front : nullptr;
+    const size_t bgr_row = (size_t)cols * 3;
     // one chunk [f0, f0 + nf) of lane l on its next stream: H2D, kernels, D2H; its arena is sized for chunks of hc2 frames
-    // of the pass: staging of input, output, labels, stats and flags, then the workspace
+    // of the pass: staging of input, output, labels, stats, flags and BGR frames, then the workspace (SLIC's first)
     auto do_chunk = [&](Lane& l, int f0, int nf, const CompletionCall& c2, int hc2) -> int {
         int rc2;
         cudaStream_t st = l.hs->s[l.slot];
@@ -739,6 +847,7 @@ int run_completion_host(CompletionCall cc, InDesc in, OutDesc out, int n_frames,
         const size_t bytes = carve_bytes((size_t)rows * d_pitch * hc2, in_elem) + carve_bytes(fpix * hc2, out_elem) +
                              (cc.guided ? carve_bytes(fpix * hc2, sizeof(int32_t)) : 0) +
                              carve_bytes((size_t)hc2 * DCMT_STATS_STRIDE, sizeof(int32_t)) + (flagged ? carve_bytes((size_t)hc2, sizeof(int32_t)) : 0) +
+                             (front ? carve_bytes(bgr_row * rows * hc2, 1) + slic_ws_bytes(rows, cols, hc2, front->step, true) : 0) +
                              (copy_only ? 0 : completion_ws_bytes(c2, hc2, in_elem, out_elem));
         Arena* ar = nullptr;
         if ((rc2 = arena_acquire(st, bytes, &ar))) return rc2;  // stream order protects reuse by the chunk 3 steps later
@@ -747,13 +856,22 @@ int run_completion_host(CompletionCall cc, InDesc in, OutDesc out, int n_frames,
         int32_t* d_lab = cc.guided ? carve<int32_t>(ar, fpix * hc2) : nullptr;
         int32_t* d_stats = carve<int32_t>(ar, (size_t)hc2 * DCMT_STATS_STRIDE);
         int32_t* d_flags = flagged ? carve<int32_t>(ar, (size_t)hc2) : nullptr;
+        uint8_t* d_bgr = front ? carve<uint8_t>(ar, bgr_row * rows * hc2) : nullptr;
         if ((rc2 = arena_ok(ar))) return rc2;
+        if (front && (rc2 = copy_frames_h2d(d_bgr, bgr_row, front->bgr + (size_t)f0 * front->fstride, front->pitch, front->fstride, bgr_row,
+                                            rows, nf, st)))
+            return rc2;
         const InDesc hi = in.frames_from((size_t)f0);
         if ((rc2 = copy_frames_h2d(d_in, d_pitch * in_elem, hi.ptr(), in.pitch * in_elem, in.fstride * in_elem, cols * in_elem, rows, nf, st)))
             return rc2;
-        if (cc.guided)
+        if (front) {
+            if ((rc2 = enqueue_slic(d_bgr, bgr_row, bgr_row * rows, true, rows, cols, nf, front->step, front->nc, front->iterations, d_lab,
+                                    nullptr, ar, st)))
+                return rc2;
+        } else if (cc.guided) {
             API_CUDA(cudaMemcpyAsync(d_lab, cc.labels + (size_t)f0 * fpix, fpix * nf * sizeof(int32_t), cudaMemcpyHostToDevice, st),
                      "host to device copy");
+        }
         size_t d_out_pitch = cols;  // elements
         if (copy_only && in_elem == out_elem) {
             d_out = d_in;
@@ -1180,6 +1298,76 @@ int dcmt_interpolate_with_superpixels_u16_u16_host_multi(const uint16_t* sparse_
                                {nullptr, dense_u16, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats, devices, n_devices, true);
 }
 
+// main_lc.cpp:159-220 from the BGR frame: cvtColor(COLOR_BGR2Lab), generate_superpixels and interpolate_with_superpixels of
+// KITTI uint16 depth; the Lab frames and the labels stay in the workspace
+int dcmt_interpolate_with_superpixels_bgr_u16(const uint8_t* bgr, size_t bgr_pitch_bytes, size_t bgr_frame_stride_bytes,
+                                              const uint16_t* sparse_u16, float* dense, int rows, int cols, size_t in_pitch_bytes,
+                                              size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
+                                              int n_frames, int step, int nc, int iterations, int use_superpixel, int flags, int32_t* stats,
+                                              void* cuda_stream) {
+    BgrFront fr{bgr, bgr_pitch_bytes, bgr_frame_stride_bytes, step, nc, iterations};
+    return run_completion_bgr({nullptr, 0, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags, &fr},
+                              {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                              {dense, nullptr, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats, static_cast<cudaStream_t>(cuda_stream));
+}
+
+int dcmt_interpolate_with_superpixels_bgr_u16_host(const uint8_t* bgr, size_t bgr_pitch_bytes, size_t bgr_frame_stride_bytes,
+                                                   const uint16_t* sparse_u16, float* dense, int rows, int cols, size_t in_pitch_bytes,
+                                                   size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
+                                                   int n_frames, int step, int nc, int iterations, int use_superpixel, int flags,
+                                                   int32_t* stats) {
+    BgrFront fr{bgr, bgr_pitch_bytes, bgr_frame_stride_bytes, step, nc, iterations};
+    return run_completion_host({nullptr, 0, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags, &fr},
+                               {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                               {dense, nullptr, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats);
+}
+
+int dcmt_interpolate_with_superpixels_bgr_u16_host_multi(const uint8_t* bgr, size_t bgr_pitch_bytes, size_t bgr_frame_stride_bytes,
+                                                         const uint16_t* sparse_u16, float* dense, int rows, int cols, size_t in_pitch_bytes,
+                                                         size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
+                                                         int n_frames, int step, int nc, int iterations, int use_superpixel, int flags,
+                                                         int32_t* stats, const int* devices, int n_devices) {
+    BgrFront fr{bgr, bgr_pitch_bytes, bgr_frame_stride_bytes, step, nc, iterations};
+    return run_completion_host({nullptr, 0, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags, &fr},
+                               {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                               {dense, nullptr, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats, devices, n_devices, true);
+}
+
+int dcmt_interpolate_with_superpixels_bgr_u16_u16(const uint8_t* bgr, size_t bgr_pitch_bytes, size_t bgr_frame_stride_bytes,
+                                                  const uint16_t* sparse_u16, uint16_t* dense_u16, int rows, int cols, size_t in_pitch_bytes,
+                                                  size_t in_frame_stride_bytes, size_t out_pitch_bytes, size_t out_frame_stride_bytes,
+                                                  int n_frames, int step, int nc, int iterations, int use_superpixel, int flags,
+                                                  int32_t* stats, void* cuda_stream) {
+    BgrFront fr{bgr, bgr_pitch_bytes, bgr_frame_stride_bytes, step, nc, iterations};
+    return run_completion_bgr({nullptr, 0, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags, &fr},
+                              {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                              {nullptr, dense_u16, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats,
+                              static_cast<cudaStream_t>(cuda_stream));
+}
+
+int dcmt_interpolate_with_superpixels_bgr_u16_u16_host(const uint8_t* bgr, size_t bgr_pitch_bytes, size_t bgr_frame_stride_bytes,
+                                                       const uint16_t* sparse_u16, uint16_t* dense_u16, int rows, int cols,
+                                                       size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                                       size_t out_frame_stride_bytes, int n_frames, int step, int nc, int iterations,
+                                                       int use_superpixel, int flags, int32_t* stats) {
+    BgrFront fr{bgr, bgr_pitch_bytes, bgr_frame_stride_bytes, step, nc, iterations};
+    return run_completion_host({nullptr, 0, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags, &fr},
+                               {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                               {nullptr, dense_u16, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats);
+}
+
+int dcmt_interpolate_with_superpixels_bgr_u16_u16_host_multi(const uint8_t* bgr, size_t bgr_pitch_bytes, size_t bgr_frame_stride_bytes,
+                                                             const uint16_t* sparse_u16, uint16_t* dense_u16, int rows, int cols,
+                                                             size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                                             size_t out_frame_stride_bytes, int n_frames, int step, int nc, int iterations,
+                                                             int use_superpixel, int flags, int32_t* stats, const int* devices,
+                                                             int n_devices) {
+    BgrFront fr{bgr, bgr_pitch_bytes, bgr_frame_stride_bytes, step, nc, iterations};
+    return run_completion_host({nullptr, 0, use_superpixel != 0, rows, cols, DCMT_BLUR_GAUSSIAN, flags, &fr},
+                               {nullptr, sparse_u16, in_pitch_bytes, in_frame_stride_bytes},
+                               {nullptr, dense_u16, out_pitch_bytes, out_frame_stride_bytes}, n_frames, stats, devices, n_devices, true);
+}
+
 int dcmt_depth_to_u16(const float* depth, uint16_t* out, int rows, int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes,
                       size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames, void* cuda_stream) {
     if (!depth || !out) return fail(DCMT_E_BADARG, "null image pointer");
@@ -1299,40 +1487,16 @@ static int slic_device(const uint8_t* img, bool from_bgr, int rows, int cols, in
     if (!img || !labels) return fail(DCMT_E_BADARG, "null pointer");
     int rc = check_planes(rows, cols, n_frames);
     if (rc) return rc;
-    if (nc == 0 || iterations < 0) return fail(DCMT_E_BADARG, "nc %d, iterations %d", nc, iterations);
-    if (step < 4) return fail(DCMT_E_UNSUPPORTED, "step %d: find_local_minimum (slic.cpp:72-99) reads outside the image below 4", step);
-    if (rows >= 1 << 24 || cols >= 1 << 24) return fail(DCMT_E_UNSUPPORTED, "SLIC frames are limited to 2^24 rows / columns");
+    if ((rc = check_slic(rows, cols, step, nc, iterations))) return rc;
     if ((size_t)rows * (size_t)cols > (size_t)1 << 30) return fail(DCMT_E_UNSUPPORTED, "frame larger than 2^30 pixels");
     if (n_frames > 65535) return fail(DCMT_E_UNSUPPORTED, "at most 65535 frames per call");
     if (n_frames == 0) return DCMT_OK;
     if ((rc = check_device())) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-    const int k = dcmt::slic_center_count(rows, cols, step);
-    dcmt::SlicWork w{};
-    const size_t nbins = dcmt::slic_bins(rows, cols, step, &w.bins_x, &w.bins_y);
-    const size_t kk = (k > 0 ? (size_t)k : 1) * n_frames, nb = nbins * n_frames;
     Arena* ar = nullptr;
-    if ((rc = arena_acquire(st, 2 * carve_bytes(kk * 5, sizeof(double)) + carve_bytes(kk * 6, sizeof(unsigned long long)) +
-                                    carve_bytes(nb + n_frames, sizeof(int)) + carve_bytes(nb, sizeof(int)) + carve_bytes(kk, sizeof(int)) +
-                                    (from_bgr ? carve_bytes((size_t)rows * cols * 3 * n_frames, 1) : 0),
-                            &ar)))
-        return rc;
-    w.centers = carve<double>(ar, kk * 5);
-    w.sums = carve<unsigned long long>(ar, kk * 6);
-    w.bin_count = carve<int>(ar, nb + n_frames);
-    w.bin_fill = carve<int>(ar, nb);
-    w.bin_items = carve<int>(ar, kk);
-    w.sorted = carve<double>(ar, kk * 5);
-    uint8_t* lab = from_bgr ? carve<uint8_t>(ar, (size_t)rows * cols * 3 * n_frames) : nullptr;
-    if ((rc = arena_ok(ar))) return rc;
-    if (from_bgr) {
-        const size_t pitch = (size_t)cols * 3;
-        API_CUDA(dcmt::color_bgr2lab(img, pitch, pitch * rows, lab, pitch, pitch * rows, rows, cols, n_frames, st), "BGR2Lab launch");
-    }
-    API_CUDA(dcmt::slic_run(from_bgr ? lab : img, rows, cols, n_frames, step, nc, iterations, labels, k, w, st), "SLIC launch");
-    if (centers && k > 0)
-        API_CUDA(cudaMemcpyAsync(centers, w.centers, (size_t)k * n_frames * 5 * sizeof(double), cudaMemcpyDeviceToDevice, st), "centre copy");
-    return DCMT_OK;
+    if ((rc = arena_acquire(st, slic_ws_bytes(rows, cols, n_frames, step, from_bgr), &ar))) return rc;
+    const size_t pitch = (size_t)cols * 3;
+    return enqueue_slic(img, pitch, pitch * rows, from_bgr, rows, cols, n_frames, step, nc, iterations, labels, centers, ar, st);
 }
 
 int dcmt_slic_u8c3(const uint8_t* lab, int rows, int cols, int n_frames, int step, int nc, int iterations, int32_t* labels,

@@ -265,6 +265,63 @@ DCMT_API int dcmt_interpolate_with_superpixels_u16_u16_host_multi(const uint16_t
                                                                   int flags, int32_t *stats_or_null, const int *devices_or_null,
                                                                   int n_devices);
 
+/* (a2 from the camera frame) main_lc.cpp:159-220 in one call: the CV_8UC3 BGR frame as read and the uint16 payload of the
+ * KITTI depth PNG in, completed depth out -- cv::cvtColor(COLOR_BGR2Lab), Slic::generate_superpixels(lab, step, nc) and
+ * interpolate_with_superpixels, with nothing in between leaving the device.
+ *   - Meaning: the result (and stats) is byte-equal to dcmt_slic_bgr_u8c3(bgr, rows, cols, n_frames, step, nc, iterations,
+ *     labels, NULL) followed by dcmt_interpolate_with_superpixels_u16[_u16](sparse_u16, labels, dcmt_slic_center_count(rows,
+ *     cols, step), ..., use_superpixel, flags, stats), on every entry point, for any batch size and any device list.
+ *   - The Lab frames and the label map live only in the workspace and are never returned.  A host caller moves 3 + 2 bytes
+ *     per pixel in and 2 (uint16 output) or 4 (float32 output) out, where the two calls move the label map out and back
+ *     in as well (8 more bytes per pixel).
+ *   - Layout: `bgr` has its own pitch and frame stride in bytes (0 = dense), so a cv::Mat ROI (e.g. the 1216 x 352 crop
+ *     of a raw frame) is passed as it is; pitches / frame strides of the depth planes as for dcmt_img_completion_u16.
+ *   - Arguments are checked before any device work: those of dcmt_slic_bgr_u8c3 (step >= 4 else DCMT_E_UNSUPPORTED,
+ *     nc != 0, iterations >= 0, frames below 2^24 rows / columns) and of dcmt_interpolate_with_superpixels_u16, and the
+ *     output must not overlap either input.  There is no limit on n_frames: the batch runs in chunks.
+ *   - Only uint16 (strict q8) sparse input is offered, so DCMT_PATH_AUTO / _FUSED / _RANK all mean the fused kernels
+ *     (the generic pipeline for shapes they do not serve, or DCMT_PATH_GENERIC) and the call never synchronises; the
+ *     device entry point can be captured in a CUDA graph.  Float32 sparse input keeps the two calls.
+ *   - use_superpixel == 0: plain completion (as the guided call does); the BGR frames are checked but not read.
+ * The _u16_u16 variants store the result as KITTI uint16 by the rule of dcmt_depth_to_u16.  _host: host pointers, chunks
+ * of frames flow H2D -> Lab -> SLIC -> completion -> D2H on three streams (page-locked buffers let the copies overlap the
+ * kernels); _host_multi: the same over several devices as for dcmt_img_completion_f32_host_multi. */
+DCMT_API int dcmt_interpolate_with_superpixels_bgr_u16(const uint8_t *bgr, size_t bgr_pitch_bytes, size_t bgr_frame_stride_bytes,
+                                                       const uint16_t *sparse_u16, float *dense, int rows, int cols,
+                                                       size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                                       size_t out_frame_stride_bytes, int n_frames, int step, int nc, int iterations,
+                                                       int use_superpixel, int flags, int32_t *stats_or_null, void *cuda_stream);
+DCMT_API int dcmt_interpolate_with_superpixels_bgr_u16_host(const uint8_t *bgr, size_t bgr_pitch_bytes, size_t bgr_frame_stride_bytes,
+                                                            const uint16_t *sparse_u16, float *dense, int rows, int cols,
+                                                            size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                                            size_t out_frame_stride_bytes, int n_frames, int step, int nc,
+                                                            int iterations, int use_superpixel, int flags, int32_t *stats_or_null);
+DCMT_API int dcmt_interpolate_with_superpixels_bgr_u16_host_multi(const uint8_t *bgr, size_t bgr_pitch_bytes,
+                                                                  size_t bgr_frame_stride_bytes, const uint16_t *sparse_u16, float *dense,
+                                                                  int rows, int cols, size_t in_pitch_bytes, size_t in_frame_stride_bytes,
+                                                                  size_t out_pitch_bytes, size_t out_frame_stride_bytes, int n_frames,
+                                                                  int step, int nc, int iterations, int use_superpixel, int flags,
+                                                                  int32_t *stats_or_null, const int *devices_or_null, int n_devices);
+DCMT_API int dcmt_interpolate_with_superpixels_bgr_u16_u16(const uint8_t *bgr, size_t bgr_pitch_bytes, size_t bgr_frame_stride_bytes,
+                                                           const uint16_t *sparse_u16, uint16_t *dense_u16, int rows, int cols,
+                                                           size_t in_pitch_bytes, size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                                           size_t out_frame_stride_bytes, int n_frames, int step, int nc, int iterations,
+                                                           int use_superpixel, int flags, int32_t *stats_or_null, void *cuda_stream);
+DCMT_API int dcmt_interpolate_with_superpixels_bgr_u16_u16_host(const uint8_t *bgr, size_t bgr_pitch_bytes,
+                                                                size_t bgr_frame_stride_bytes, const uint16_t *sparse_u16,
+                                                                uint16_t *dense_u16, int rows, int cols, size_t in_pitch_bytes,
+                                                                size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                                                size_t out_frame_stride_bytes, int n_frames, int step, int nc,
+                                                                int iterations, int use_superpixel, int flags, int32_t *stats_or_null);
+DCMT_API int dcmt_interpolate_with_superpixels_bgr_u16_u16_host_multi(const uint8_t *bgr, size_t bgr_pitch_bytes,
+                                                                      size_t bgr_frame_stride_bytes, const uint16_t *sparse_u16,
+                                                                      uint16_t *dense_u16, int rows, int cols, size_t in_pitch_bytes,
+                                                                      size_t in_frame_stride_bytes, size_t out_pitch_bytes,
+                                                                      size_t out_frame_stride_bytes, int n_frames, int step, int nc,
+                                                                      int iterations, int use_superpixel, int flags,
+                                                                      int32_t *stats_or_null, const int *devices_or_null,
+                                                                      int n_devices);
+
 /* parameters of the stereo refinement; dcmt_stereo_params_default() fills the values hard-coded in
  * main_sl.cpp, dcmt_stereo_params_official() those of main_sl_OFFICIAL.cpp:832-918. */
 typedef struct dcmt_stereo_params {

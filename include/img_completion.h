@@ -15,7 +15,9 @@
 //     void retrieve_optimized_depth(cv::Mat& disparity, cv::Mat& depth);                                            :863
 //     void evaluate_performance / evaluate_performances                      main.cpp:16, main_lc.cpp:85, main_sl.cpp:1031
 //
-// and, beyond the reference, dcmt::evaluate_kitti: the KITTI depth-completion benchmark's figures of a result.
+// and, beyond the reference, dcmt::evaluate_kitti: the KITTI depth-completion benchmark's figures of a result, and
+// dcmt::interpolate_with_superpixels_bgr[_to_u16]: main_lc.cpp's cvtColor + generate_superpixels + interpolate_with_superpixels
+// in one call from the BGR frame.
 //
 // The stereo functions take the reference's own containers: EntryType matrices (struct { float value;
 // Eigen::Vector2f derivative; }, main_sl.cpp:23-26) stored as cv::Mat(rows, cols, CV_32FC(sizeof(EntryType))) (:1165).
@@ -229,6 +231,33 @@ inline void interpolate_with_superpixels_u16_u16(const std::vector<std::vector<i
                                                          sparse_u16.step, 0, dense_u16.step, 0, 1, use_superpixel, path, nullptr));
 }
 
+// main_lc.cpp:182-220 in one call: the BGR frame as read (CV_8UC3 view) and the uint16 payload of the KITTI depth PNG
+// (CV_16UC1 view) -> dense float32 metres (interpolate_with_superpixels_bgr) or KITTI uint16 (..._bgr_to_u16): the
+// cvtColor(COLOR_BGR2Lab), Slic::generate_superpixels(lab, step, nc) and interpolate_with_superpixels of the reference
+// with the Lab image and the labels kept on the device (dcmt_interpolate_with_superpixels_bgr_u16[_u16]_host).  `step` is
+// the reference's int parameter (main_lc.cpp:197-201 passes a double, truncated).  Every view has its own step.
+inline void interpolate_with_superpixels_bgr(const MatView& bgr, const MatView& sparse_u16, MatView& dense, int step, int nc,
+                                             int use_superpixel = 1, int path = DCMT_PATH_AUTO) {
+    if (bgr.rows != sparse_u16.rows || bgr.cols != sparse_u16.cols || dense.rows != sparse_u16.rows || dense.cols != sparse_u16.cols || !dense.data)
+        throw std::invalid_argument("dcmt: interpolate_with_superpixels_bgr needs same-shaped, allocated views");
+    check(dcmt_interpolate_with_superpixels_bgr_u16_host(static_cast<const uint8_t*>(bgr.data), bgr.step, 0,
+                                                         static_cast<const uint16_t*>(sparse_u16.data), static_cast<float*>(dense.data),
+                                                         sparse_u16.rows, sparse_u16.cols, sparse_u16.step, 0, dense.step, 0, 1, step, nc,
+                                                         10, use_superpixel, path, nullptr));
+}
+
+inline void interpolate_with_superpixels_bgr_to_u16(const MatView& bgr, const MatView& sparse_u16, MatView& dense_u16, int step, int nc,
+                                                    int use_superpixel = 1, int path = DCMT_PATH_AUTO) {
+    if (bgr.rows != sparse_u16.rows || bgr.cols != sparse_u16.cols || dense_u16.rows != sparse_u16.rows || dense_u16.cols != sparse_u16.cols ||
+        !dense_u16.data)
+        throw std::invalid_argument("dcmt: interpolate_with_superpixels_bgr_to_u16 needs same-shaped, allocated views");
+    check(dcmt_interpolate_with_superpixels_bgr_u16_u16_host(static_cast<const uint8_t*>(bgr.data), bgr.step, 0,
+                                                             static_cast<const uint16_t*>(sparse_u16.data),
+                                                             static_cast<uint16_t*>(dense_u16.data), sparse_u16.rows, sparse_u16.cols,
+                                                             sparse_u16.step, 0, dense_u16.step, 0, 1, step, nc, 10, use_superpixel, path,
+                                                             nullptr));
+}
+
 // ---- the stereo functions on EntryType matrices (views whose rows hold `cols` entries of kEntryBytes at the start) ----
 // main_sl.cpp:715-745
 inline void calculateMeasuementDerivatives(MatView& entries) {
@@ -379,6 +408,26 @@ inline void interpolate_with_superpixels_to_u16(SlicT& slic, const cv::Mat& spar
     cv::Mat out(sparse_u16.rows, sparse_u16.cols, CV_16UC1);
     MatView d = view_of(out);
     interpolate_with_superpixels_u16_u16(slic.clusters, slic.centers.size(), view_of(sparse_u16), d, use_superpixel);
+    dense_u16 = out;
+}
+
+// main_lc.cpp:182-220 in one call on the Mats as read: a CV_8UC3 BGR image (an ROI too) and a CV_16UC1 depth PNG payload;
+// the result is a fresh continuous CV_32FC1 (metres) or CV_16UC1 (KITTI uint16) matrix.  Any other type throws.
+inline void interpolate_with_superpixels_bgr(const cv::Mat& bgr, const cv::Mat& sparse_u16, cv::Mat& dense, int step, int nc,
+                                             int use_superpixel = 1) {
+    CV_Assert(bgr.type() == CV_8UC3 && sparse_u16.type() == CV_16UC1);
+    cv::Mat out(sparse_u16.rows, sparse_u16.cols, CV_32FC1);
+    MatView d = view_of(out);
+    interpolate_with_superpixels_bgr(view_of(bgr), view_of(sparse_u16), d, step, nc, use_superpixel);
+    dense = out;
+}
+
+inline void interpolate_with_superpixels_bgr_to_u16(const cv::Mat& bgr, const cv::Mat& sparse_u16, cv::Mat& dense_u16, int step, int nc,
+                                                    int use_superpixel = 1) {
+    CV_Assert(bgr.type() == CV_8UC3 && sparse_u16.type() == CV_16UC1);
+    cv::Mat out(sparse_u16.rows, sparse_u16.cols, CV_16UC1);
+    MatView d = view_of(out);
+    interpolate_with_superpixels_bgr_to_u16(view_of(bgr), view_of(sparse_u16), d, step, nc, use_superpixel);
     dense_u16 = out;
 }
 }  // namespace dcmt
