@@ -44,6 +44,9 @@ int cuda_fail(cudaError_t e, const char* what) {
     return fail(DCMT_E_CUDA, "%s: %s", what, cudaGetErrorString(e));
 }
 
+// DCMT_OK, or the error of a launch or copy that returned `e`
+int cuda_rc(cudaError_t e, const char* what) { return e == cudaSuccess ? DCMT_OK : cuda_fail(e, what); }
+
 #define API_CUDA(x, what)                                  \
     do {                                                   \
         cudaError_t e__ = (x);                             \
@@ -145,10 +148,15 @@ struct Geometry {
     size_t span_bytes;      // bytes touched by the whole batch
 };
 
-int check_geometry(int rows, int cols, size_t pitch_bytes, size_t frame_stride_bytes, int n_frames, Geometry* g,
-                   size_t elem = sizeof(float)) {
+int check_planes(int rows, int cols, int n_frames) {
     if (rows < 1 || cols < 1) return fail(DCMT_E_BADARG, "rows and cols must be >= 1 (got %d x %d)", rows, cols);
     if (n_frames < 0) return fail(DCMT_E_BADARG, "n_frames must be >= 0 (got %d)", n_frames);
+    return DCMT_OK;
+}
+
+int check_geometry(int rows, int cols, size_t pitch_bytes, size_t frame_stride_bytes, int n_frames, Geometry* g,
+                   size_t elem = sizeof(float)) {
+    if (int rc = check_planes(rows, cols, n_frames)) return rc;
     if ((size_t)rows * (size_t)cols > (size_t)1 << 30) return fail(DCMT_E_UNSUPPORTED, "frame larger than 2^30 pixels");
     if (pitch_bytes == 0) pitch_bytes = (size_t)cols * elem;
     if (pitch_bytes % elem != 0 || pitch_bytes < (size_t)cols * elem)
@@ -804,6 +812,44 @@ int copy_frames_d2h(void* h, size_t h_pitch_bytes, size_t h_fstride_bytes, const
     return DCMT_OK;
 }
 
+// One caller buffer of a single-shot host call: `rows` rows of `row_bytes`, `pitch` bytes apart on the host, packed on the
+// device.
+struct Staged {
+    const void* from;     // copied to the device before the work (nullptr: not read)
+    void* to;             // copied back after the work (nullptr: not written back)
+    size_t pitch, row_bytes, rows;
+    void* dev = nullptr;  // set by run_staged
+};
+
+// Driver of the single-shot host entry points, called on validated arguments: a HostCall on the current device, the staging
+// of `bufs` carved from the arena of the lane's second stream, then H2D, work(stream) and D2H on the first stream, whose
+// arena is left to the work's own workspace; HostCall::finish waits for all of it.
+template <class Work>
+int run_staged(std::initializer_list<Staged*> bufs, Work&& work) {
+    HostCall call;
+    int rc = call.open(nullptr, 0, false);
+    if (rc) return rc;
+    Lane& l = call.lanes[0];
+    const cudaStream_t st = l.hs->s[0];
+    size_t bytes = 0;
+    for (const Staged* b : bufs) bytes += carve_bytes(b->rows * b->row_bytes, 1);
+    Arena* stage = nullptr;
+    if ((rc = arena_acquire(l.hs->s[1], bytes, &stage))) return rc;
+    for (Staged* b : bufs) b->dev = carve<char>(stage, b->rows * b->row_bytes);
+    if ((rc = arena_ok(stage)) || (rc = call.use(l))) return rc;
+    // one copy when the host rows are packed, a 2-D copy otherwise
+    auto copy = [st](void* dst, size_t dst_pitch, const void* src, size_t src_pitch, const Staged* b, cudaMemcpyKind kind) {
+        return dst_pitch == src_pitch ? cudaMemcpyAsync(dst, src, b->rows * b->row_bytes, kind, st)
+                                      : cudaMemcpy2DAsync(dst, dst_pitch, src, src_pitch, b->row_bytes, b->rows, kind, st);
+    };
+    for (const Staged* b : bufs)
+        if (b->from) API_CUDA(copy(b->dev, b->row_bytes, b->from, b->pitch, b, cudaMemcpyHostToDevice), "host to device copy");
+    if ((rc = work(st))) return rc;
+    for (const Staged* b : bufs)
+        if (b->to) API_CUDA(copy(b->to, b->pitch, b->dev, b->row_bytes, b, cudaMemcpyDeviceToHost), "device to host copy");
+    return call.finish();
+}
+
 // Host-pointer driver of every completion entry point.  Device staging rows are packed for float32 input and padded to
 // 16 bytes for uint16 input (vector loads in k_q8_front).
 // copy_only: the same buffers, chunking and streams with the kernels left out -- the ceiling the host <-> device links put
@@ -1044,27 +1090,16 @@ int run_evaluation_host(InDesc gt, InDesc r, int rows, int cols, int n_frames, i
     int rc = validate_evaluation(&gt, &r, rows, cols, n_frames, mode, results, &gt_span, &r_span);
     if (rc) return rc;
     if (n_frames == 0) return DCMT_OK;
-    HostCall call;
-    if ((rc = call.open(nullptr, 0, false))) return rc;
-    cudaStream_t st = call.lanes[0].hs->s[0], st2 = call.lanes[0].hs->s[1];
     const size_t res_bytes = (size_t)n_frames * kind.rec_bytes;
-    Arena* stage = nullptr;
-    if ((rc = arena_acquire(st2, carve_bytes(gt_span, 1) + carve_bytes(r_span, 1) + carve_bytes(res_bytes, 1), &stage))) return rc;
-    char* d_gt = carve<char>(stage, gt_span);
-    char* d_r = carve<char>(stage, r_span);
-    char* d_res = carve<char>(stage, res_bytes);
-    if ((rc = arena_ok(stage))) return rc;
-    call.use(call.lanes[0]);
-    API_CUDA(cudaMemcpyAsync(d_gt, gt.ptr(), gt_span, cudaMemcpyHostToDevice, st), "host to device copy");
-    API_CUDA(cudaMemcpyAsync(d_r, r.ptr(), r_span, cudaMemcpyHostToDevice, st), "host to device copy");
-    InDesc dgt = gt, dr = r;
-    if (gt.u) dgt.u = reinterpret_cast<const uint16_t*>(d_gt);
-    else dgt.f = reinterpret_cast<const float*>(d_gt);
-    if (r.u) dr.u = reinterpret_cast<const uint16_t*>(d_r);
-    else dr.f = reinterpret_cast<const float*>(d_r);
-    if ((rc = kind.enqueue(dgt, dr, rows, cols, n_frames, d_res, st))) return rc;
-    API_CUDA(cudaMemcpyAsync(results, d_res, res_bytes, cudaMemcpyDeviceToHost, st), "device to host copy");
-    return call.finish();
+    Staged sg{gt.ptr(), nullptr, gt_span, gt_span, 1}, sr{r.ptr(), nullptr, r_span, r_span, 1}, sres{nullptr, results, res_bytes, res_bytes, 1};
+    return run_staged({&sg, &sr, &sres}, [&](cudaStream_t st) {
+        InDesc dgt = gt, dr = r;
+        if (gt.u) dgt.u = static_cast<const uint16_t*>(sg.dev);
+        else dgt.f = static_cast<const float*>(sg.dev);
+        if (r.u) dr.u = static_cast<const uint16_t*>(sr.dev);
+        else dr.f = static_cast<const float*>(sr.dev);
+        return kind.enqueue(dgt, dr, rows, cols, n_frames, sres.dev, st);
+    });
 }
 
 InDesc eval_f32(const float* p, size_t pitch_bytes, size_t fstride_bytes) {
@@ -1085,8 +1120,6 @@ InDesc eval_u16(const uint16_t* p, size_t pitch_bytes, size_t fstride_bytes) {
 }  // namespace
 
 extern "C" {
-
-static int check_planes(int rows, int cols, int n_frames);
 
 int dcmt_version(void) { return DCMT_VERSION; }
 const char* dcmt_build_info(void) {
@@ -1480,16 +1513,22 @@ int dcmt_slic_center_count(int rows, int cols, int step) {
     return dcmt::slic_center_count(rows, cols, step);
 }
 
-// Slic::generate_superpixels on the Lab image `img`, or, with from_bgr, on the cvtColor(COLOR_BGR2Lab) of the BGR image
-// `img`: the Lab frames then live in the SLIC workspace of (device, stream) and never leave the device
-static int slic_device(const uint8_t* img, bool from_bgr, int rows, int cols, int n_frames, int step, int nc, int iterations,
-                       int32_t* labels, double* centers, void* cuda_stream) {
+static int check_slic_call(const uint8_t* img, const int32_t* labels, int rows, int cols, int n_frames, int step, int nc, int iterations) {
     if (!img || !labels) return fail(DCMT_E_BADARG, "null pointer");
     int rc = check_planes(rows, cols, n_frames);
     if (rc) return rc;
     if ((rc = check_slic(rows, cols, step, nc, iterations))) return rc;
     if ((size_t)rows * (size_t)cols > (size_t)1 << 30) return fail(DCMT_E_UNSUPPORTED, "frame larger than 2^30 pixels");
     if (n_frames > 65535) return fail(DCMT_E_UNSUPPORTED, "at most 65535 frames per call");
+    return DCMT_OK;
+}
+
+// Slic::generate_superpixels on the Lab image `img`, or, with from_bgr, on the cvtColor(COLOR_BGR2Lab) of the BGR image
+// `img`: the Lab frames then live in the SLIC workspace of (device, stream) and never leave the device
+static int slic_device(const uint8_t* img, bool from_bgr, int rows, int cols, int n_frames, int step, int nc, int iterations,
+                       int32_t* labels, double* centers, void* cuda_stream) {
+    int rc = check_slic_call(img, labels, rows, cols, n_frames, step, nc, iterations);
+    if (rc) return rc;
     if (n_frames == 0) return DCMT_OK;
     if ((rc = check_device())) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
@@ -1511,32 +1550,19 @@ int dcmt_slic_bgr_u8c3(const uint8_t* bgr, int rows, int cols, int n_frames, int
 
 static int slic_host(const uint8_t* img, bool from_bgr, int rows, int cols, int n_frames, int step, int nc, int iterations,
                      int32_t* labels, double* centers) {
-    if (!img || !labels) return fail(DCMT_E_BADARG, "null pointer");
-    int rc = check_planes(rows, cols, n_frames);
+    int rc = check_slic_call(img, labels, rows, cols, n_frames, step, nc, iterations);
     if (rc) return rc;
     if (n_frames == 0) return DCMT_OK;
-    HostCall call;
-    if ((rc = call.open(nullptr, 0, false))) return rc;
-    // staging buffers come from the arena of an internal stream (no cudaMalloc per call), copies are asynchronous on it
-    cudaStream_t st = call.lanes[0].hs->s[0];
     const size_t n = (size_t)rows * cols * n_frames;
-    const size_t k = (size_t)(step >= 1 ? dcmt::slic_center_count(rows, cols, step) : 0) * n_frames;
-    Arena* stage = nullptr;
-    {
-        // a second arena key on the same device: the SLIC work arena is keyed by `st`, the staging one by the next stream
-        cudaStream_t st2 = call.lanes[0].hs->s[1];
-        if ((rc = arena_acquire(st2, carve_bytes(n * 3, 1) + carve_bytes(n, 4) + carve_bytes((k > 0 ? k : 1) * 5, sizeof(double)), &stage))) return rc;
-    }
-    uint8_t* d_img = carve<uint8_t>(stage, n * 3);
-    int32_t* d_labels = carve<int32_t>(stage, n);
-    double* d_centers = carve<double>(stage, (k > 0 ? k : 1) * 5);
-    if ((rc = arena_ok(stage))) return rc;
-    call.use(call.lanes[0]);
-    API_CUDA(cudaMemcpyAsync(d_img, img, n * 3, cudaMemcpyHostToDevice, st), "host to device copy");
-    if ((rc = slic_device(d_img, from_bgr, rows, cols, n_frames, step, nc, iterations, d_labels, centers ? d_centers : nullptr, st))) return rc;
-    API_CUDA(cudaMemcpyAsync(labels, d_labels, n * 4, cudaMemcpyDeviceToHost, st), "device to host copy");
-    if (centers && k > 0) API_CUDA(cudaMemcpyAsync(centers, d_centers, k * 5 * sizeof(double), cudaMemcpyDeviceToHost, st), "device to host copy");
-    return call.finish();
+    const size_t kb = (size_t)dcmt::slic_center_count(rows, cols, step) * n_frames * 5 * sizeof(double);
+    Staged si{img, nullptr, n * 3, n * 3, 1}, sl{nullptr, labels, n * 4, n * 4, 1}, sc{nullptr, kb ? centers : nullptr, kb, kb, 1};
+    return run_staged({&si, &sl, &sc}, [&](cudaStream_t st) {
+        Arena* ar = nullptr;
+        if (int rc2 = arena_acquire(st, slic_ws_bytes(rows, cols, n_frames, step, from_bgr), &ar)) return rc2;
+        const size_t pitch = (size_t)cols * 3;
+        return enqueue_slic(static_cast<const uint8_t*>(si.dev), pitch, pitch * rows, from_bgr, rows, cols, n_frames, step, nc, iterations,
+                            static_cast<int32_t*>(sl.dev), centers ? static_cast<double*>(sc.dev) : nullptr, ar, st);
+    });
 }
 
 int dcmt_slic_u8c3_host(const uint8_t* lab, int rows, int cols, int n_frames, int step, int nc, int iterations, int32_t* labels,
@@ -1549,24 +1575,36 @@ int dcmt_slic_bgr_u8c3_host(const uint8_t* bgr, int rows, int cols, int n_frames
     return slic_host(bgr, true, rows, cols, n_frames, step, nc, iterations, labels, centers);
 }
 
-int dcmt_lidar_project_f32(const float* points, int n_points, const float* T_host, const float* P_host, int rows, int cols,
-                           float* projected, float* normalized, float norm_a, float norm_b, int32_t* n_projected, void* cuda_stream) {
+static int check_project(const float* points, int n_points, const float* T_host, const float* P_host, int rows, int cols) {
     if ((!points && n_points > 0) || !T_host || !P_host) return fail(DCMT_E_BADARG, "null pointer");
     if (n_points < 0) return fail(DCMT_E_BADARG, "n_points must be >= 0 (got %d)", n_points);
     int rc = check_planes(rows, cols, 1);
     if (rc) return rc;
     if ((size_t)rows * (size_t)cols > (size_t)1 << 30) return fail(DCMT_E_UNSUPPORTED, "frame larger than 2^30 pixels");
-    if (points && (reinterpret_cast<uintptr_t>(points) & 15)) return fail(DCMT_E_BADARG, "points must be 16-byte aligned");
-    if ((rc = check_device())) return rc;
-    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    return DCMT_OK;
+}
+
+// the projection on validated arguments, 16-byte aligned points: its keys and counters in the stream's arena
+static int enqueue_project(const float* points, int n_points, const float* T_host, const float* P_host, int rows, int cols,
+                           float* projected, float* normalized, float norm_a, float norm_b, int32_t* n_projected, cudaStream_t st) {
     Arena* ar = nullptr;
     const size_t nk = dcmt::project_key_count(rows, cols);
-    if ((rc = arena_acquire(st, carve_bytes(nk, sizeof(unsigned long long)) + carve_bytes(8, sizeof(unsigned)), &ar))) return rc;
+    int rc = arena_acquire(st, carve_bytes(nk, sizeof(unsigned long long)) + carve_bytes(8, sizeof(unsigned)), &ar);
+    if (rc) return rc;
     dcmt::ProjectWork w{carve<unsigned long long>(ar, nk), carve<unsigned>(ar, 8)};
     if ((rc = arena_ok(ar))) return rc;
-    API_CUDA(dcmt::project_run(points, n_points, T_host, P_host, rows, cols, projected, normalized, norm_a, norm_b, n_projected, w, st),
-             "projection launch");
-    return DCMT_OK;
+    return cuda_rc(dcmt::project_run(points, n_points, T_host, P_host, rows, cols, projected, normalized, norm_a, norm_b, n_projected, w, st),
+                   "projection launch");
+}
+
+int dcmt_lidar_project_f32(const float* points, int n_points, const float* T_host, const float* P_host, int rows, int cols,
+                           float* projected, float* normalized, float norm_a, float norm_b, int32_t* n_projected, void* cuda_stream) {
+    int rc = check_project(points, n_points, T_host, P_host, rows, cols);
+    if (rc) return rc;
+    if (points && (reinterpret_cast<uintptr_t>(points) & 15)) return fail(DCMT_E_BADARG, "points must be 16-byte aligned");
+    if ((rc = check_device())) return rc;
+    return enqueue_project(points, n_points, T_host, P_host, rows, cols, projected, normalized, norm_a, norm_b, n_projected,
+                           static_cast<cudaStream_t>(cuda_stream));
 }
 
 int dcmt_lidar_project_batch_f32(const float* points, const int32_t* n_points_dev_or_null, int max_points, size_t cloud_stride_points,
@@ -1596,29 +1634,16 @@ int dcmt_lidar_project_batch_f32(const float* points, const int32_t* n_points_de
 
 int dcmt_lidar_project_f32_host(const float* points, int n_points, const float* T_host, const float* P_host, int rows, int cols,
                                 float* projected, float* normalized, float norm_a, float norm_b, int32_t* n_projected) {
-    if ((!points && n_points > 0) || !T_host || !P_host) return fail(DCMT_E_BADARG, "null pointer");
-    if (n_points < 0) return fail(DCMT_E_BADARG, "n_points must be >= 0 (got %d)", n_points);
-    int rc = check_planes(rows, cols, 1);
+    int rc = check_project(points, n_points, T_host, P_host, rows, cols);
     if (rc) return rc;
-    HostCall call;
-    if ((rc = call.open(nullptr, 0, false))) return rc;
-    cudaStream_t st = call.lanes[0].hs->s[0], st2 = call.lanes[0].hs->s[1];
-    const size_t n = (size_t)rows * cols;
-    Arena* stage = nullptr;
-    if ((rc = arena_acquire(st2, carve_bytes((size_t)(n_points > 0 ? n_points : 1) * 4, 4) + 2 * carve_bytes(n, 4) + carve_bytes(1, 4), &stage)))
-        return rc;
-    float* d_pts = carve<float>(stage, (size_t)(n_points > 0 ? n_points : 1) * 4);
-    float* d_proj = carve<float>(stage, n);
-    float* d_norm = carve<float>(stage, n);
-    int32_t* d_cnt = carve<int32_t>(stage, 1);
-    if ((rc = arena_ok(stage))) return rc;
-    call.use(call.lanes[0]);
-    if (n_points > 0) API_CUDA(cudaMemcpyAsync(d_pts, points, (size_t)n_points * 16, cudaMemcpyHostToDevice, st), "host to device copy");
-    if ((rc = dcmt_lidar_project_f32(d_pts, n_points, T_host, P_host, rows, cols, d_proj, d_norm, norm_a, norm_b, d_cnt, st))) return rc;
-    if (projected) API_CUDA(cudaMemcpyAsync(projected, d_proj, n * 4, cudaMemcpyDeviceToHost, st), "device to host copy");
-    if (normalized) API_CUDA(cudaMemcpyAsync(normalized, d_norm, n * 4, cudaMemcpyDeviceToHost, st), "device to host copy");
-    if (n_projected) API_CUDA(cudaMemcpyAsync(n_projected, d_cnt, 4, cudaMemcpyDeviceToHost, st), "device to host copy");
-    return call.finish();
+    // the points are staged whole into an aligned buffer; the kernel writes every plane, copied back where the caller wants it
+    const size_t pb = (size_t)n_points * 16, n = (size_t)rows * cols * 4;
+    Staged sp{n_points > 0 ? points : nullptr, nullptr, pb, pb, 1}, sj{nullptr, projected, n, n, 1}, sn{nullptr, normalized, n, n, 1},
+        sc{nullptr, n_projected, 4, 4, 1};
+    return run_staged({&sp, &sj, &sn, &sc}, [&](cudaStream_t st) {
+        return enqueue_project(static_cast<const float*>(sp.dev), n_points, T_host, P_host, rows, cols, static_cast<float*>(sj.dev),
+                               static_cast<float*>(sn.dev), norm_a, norm_b, static_cast<int32_t*>(sc.dev), st);
+    });
 }
 
 static_assert(sizeof(dcmt_eval_result) == sizeof(dcmt::EvalResult), "dcmt_eval_result and dcmt::EvalResult must match");
@@ -1735,20 +1760,21 @@ void dcmt_stereo_params_official(dcmt_stereo_params* p, int num_iterations) {
     p->final_gauss = 0;
 }
 
-static int check_planes(int rows, int cols, int n_frames) {
-    if (rows < 1 || cols < 1) return fail(DCMT_E_BADARG, "rows and cols must be >= 1 (got %d x %d)", rows, cols);
-    if (n_frames < 0) return fail(DCMT_E_BADARG, "n_frames must be >= 0 (got %d)", n_frames);
+static int check_stereo_refine(const float* depth_ig, const uint8_t* left_gray, const uint8_t* right_gray, const float* depth_out,
+                               int rows, int cols, int n_frames, const dcmt_stereo_params* prm) {
+    if (!depth_ig || !left_gray || !right_gray || !depth_out || !prm) return fail(DCMT_E_BADARG, "null pointer");
+    int rc = check_planes(rows, cols, n_frames);
+    if (rc) return rc;
+    if (prm->num_iterations < 0) return fail(DCMT_E_BADARG, "num_iterations %d", prm->num_iterations);
+    if ((size_t)rows * (size_t)cols > (size_t)1 << 30) return fail(DCMT_E_UNSUPPORTED, "frame larger than 2^30 pixels");
     return DCMT_OK;
 }
 
 int dcmt_stereo_refine_f32(const float* depth_ig, const uint8_t* left_gray, const uint8_t* right_gray, float* depth_out,
                            float* disp_out, int rows, int cols, int n_frames, const dcmt_stereo_params* prm,
                            void* cuda_stream) {
-    if (!depth_ig || !left_gray || !right_gray || !depth_out || !prm) return fail(DCMT_E_BADARG, "null pointer");
-    int rc = check_planes(rows, cols, n_frames);
+    int rc = check_stereo_refine(depth_ig, left_gray, right_gray, depth_out, rows, cols, n_frames, prm);
     if (rc) return rc;
-    if (prm->num_iterations < 0) return fail(DCMT_E_BADARG, "num_iterations %d", prm->num_iterations);
-    if ((size_t)rows * (size_t)cols > (size_t)1 << 30) return fail(DCMT_E_UNSUPPORTED, "frame larger than 2^30 pixels");
     if (n_frames == 0) return DCMT_OK;
     const size_t bytes = (size_t)rows * cols * n_frames * sizeof(float);
     if (overlaps(depth_ig, bytes, depth_out, bytes)) return fail(DCMT_E_BADARG, "input and output overlap");
@@ -1763,17 +1789,14 @@ int dcmt_stereo_refine_f32(const float* depth_ig, const uint8_t* left_gray, cons
 int dcmt_stereo_refine_f32_host(const float* depth_ig, const uint8_t* left_gray, const uint8_t* right_gray,
                                 float* depth_out, float* disp_out, int rows, int cols, int n_frames,
                                 const dcmt_stereo_params* prm) {
-    if (!depth_ig || !left_gray || !right_gray || !depth_out || !prm) return fail(DCMT_E_BADARG, "null pointer");
-    int rc = check_planes(rows, cols, n_frames);
+    int rc = check_stereo_refine(depth_ig, left_gray, right_gray, depth_out, rows, cols, n_frames, prm);
     if (rc) return rc;
-    if (prm->num_iterations < 0) return fail(DCMT_E_BADARG, "num_iterations %d", prm->num_iterations);
-    if ((size_t)rows * (size_t)cols > (size_t)1 << 30) return fail(DCMT_E_UNSUPPORTED, "frame larger than 2^30 pixels");
     if (n_frames == 0) return DCMT_OK;
     // chunks of frames flow H2D -> kernel -> D2H round-robin over the three host streams (asynchronous for page-locked buffers)
     HostCall call;
     if ((rc = call.open(nullptr, 0, false))) return rc;
     HostStreams* hs = call.lanes[0].hs;
-    call.use(call.lanes[0]);
+    if ((rc = call.use(call.lanes[0]))) return rc;
     const size_t fpix = (size_t)rows * cols;
     const int hc = host_chunk_frames(rows, cols, n_frames);
     const size_t bytes = 2 * carve_bytes(fpix * hc, sizeof(float)) + (disp_out ? carve_bytes(fpix * hc, sizeof(float)) : 0) +
@@ -1794,7 +1817,9 @@ int dcmt_stereo_refine_f32_host(const float* depth_ig, const uint8_t* left_gray,
         API_CUDA(cudaMemcpyAsync(d_ig, depth_ig + off, n * 4, cudaMemcpyHostToDevice, st), "host to device copy");
         API_CUDA(cudaMemcpyAsync(d_l, left_gray + off, n, cudaMemcpyHostToDevice, st), "host to device copy");
         API_CUDA(cudaMemcpyAsync(d_r, right_gray + off, n, cudaMemcpyHostToDevice, st), "host to device copy");
-        if ((rc = dcmt_stereo_refine_f32(d_ig, d_l, d_r, d_out, d_disp, rows, cols, nf, prm, st))) return rc;
+        API_CUDA(dcmt::stereo_refine(d_ig, d_l, d_r, d_out, d_disp, rows, cols, nf, prm->baseline, prm->focal, prm->damp_factor,
+                                     prm->err_clip, prm->depth_clip, prm->num_iterations, prm->final_gauss, st),
+                 "stereo refine launch");
         API_CUDA(cudaMemcpyAsync(depth_out + off, d_out, n * 4, cudaMemcpyDeviceToHost, st), "device to host copy");
         if (disp_out) API_CUDA(cudaMemcpyAsync(disp_out + off, d_disp, n * 4, cudaMemcpyDeviceToHost, st), "device to host copy");
     }
@@ -1875,20 +1900,12 @@ int dcmt_bgr2gray_u8_host(const uint8_t* bgr, uint8_t* gray, int rows, int cols,
     int rc = check_gray(bgr, gray, rows, cols, &bgr_pitch_bytes, &gray_pitch_bytes, n_frames);
     if (rc) return rc;
     if (n_frames == 0) return DCMT_OK;
-    HostCall call;
-    if ((rc = call.open(nullptr, 0, false))) return rc;
-    cudaStream_t st = call.lanes[0].hs->s[0];
     const size_t in_row = (size_t)cols * 3, frames_rows = (size_t)rows * n_frames;
-    Arena* ar = nullptr;
-    if ((rc = arena_acquire(st, carve_bytes(in_row * frames_rows, 1) + carve_bytes((size_t)cols * frames_rows, 1), &ar))) return rc;
-    uint8_t* d_in = carve<uint8_t>(ar, in_row * frames_rows);
-    uint8_t* d_out = carve<uint8_t>(ar, (size_t)cols * frames_rows);
-    if ((rc = arena_ok(ar))) return rc;
-    call.use(call.lanes[0]);
-    API_CUDA(cudaMemcpy2DAsync(d_in, in_row, bgr, bgr_pitch_bytes, in_row, frames_rows, cudaMemcpyHostToDevice, st), "host to device copy");
-    if ((rc = dcmt_bgr2gray_u8(d_in, d_out, rows, cols, 0, 0, n_frames, st))) return rc;
-    API_CUDA(cudaMemcpy2DAsync(gray, gray_pitch_bytes, d_out, cols, cols, frames_rows, cudaMemcpyDeviceToHost, st), "device to host copy");
-    return call.finish();
+    Staged si{bgr, nullptr, bgr_pitch_bytes, in_row, frames_rows}, so{nullptr, gray, gray_pitch_bytes, (size_t)cols, frames_rows};
+    return run_staged({&si, &so}, [&](cudaStream_t st) {
+        return cuda_rc(dcmt::stereo_bgr2gray(static_cast<const uint8_t*>(si.dev), in_row, in_row * rows, static_cast<uint8_t*>(so.dev), cols,
+                                             (size_t)cols * rows, rows, cols, n_frames, st), "BGR2GRAY launch");
+    });
 }
 
 // ---- cv::cvtColor(COLOR_BGR2Lab) in front of Slic::generate_superpixels (main_lc.cpp:182-184, main_sl.cpp:438) ----
@@ -1926,20 +1943,12 @@ int dcmt_bgr2lab_u8_host(const uint8_t* bgr, uint8_t* lab, int rows, int cols, s
     int rc = check_lab(bgr, lab, rows, cols, &bgr_pitch_bytes, &lab_pitch_bytes, n_frames);
     if (rc) return rc;
     if (n_frames == 0) return DCMT_OK;
-    HostCall call;
-    if ((rc = call.open(nullptr, 0, false))) return rc;
-    cudaStream_t st = call.lanes[0].hs->s[0];
     const size_t row = (size_t)cols * 3, frames_rows = (size_t)rows * n_frames;
-    Arena* ar = nullptr;
-    if ((rc = arena_acquire(st, 2 * carve_bytes(row * frames_rows, 1), &ar))) return rc;
-    uint8_t* d_in = carve<uint8_t>(ar, row * frames_rows);
-    uint8_t* d_out = carve<uint8_t>(ar, row * frames_rows);
-    if ((rc = arena_ok(ar))) return rc;
-    call.use(call.lanes[0]);
-    API_CUDA(cudaMemcpy2DAsync(d_in, row, bgr, bgr_pitch_bytes, row, frames_rows, cudaMemcpyHostToDevice, st), "host to device copy");
-    if ((rc = dcmt_bgr2lab_u8(d_in, d_out, rows, cols, 0, 0, n_frames, st))) return rc;
-    API_CUDA(cudaMemcpy2DAsync(lab, lab_pitch_bytes, d_out, row, row, frames_rows, cudaMemcpyDeviceToHost, st), "device to host copy");
-    return call.finish();
+    Staged si{bgr, nullptr, bgr_pitch_bytes, row, frames_rows}, so{nullptr, lab, lab_pitch_bytes, row, frames_rows};
+    return run_staged({&si, &so}, [&](cudaStream_t st) {
+        return cuda_rc(dcmt::color_bgr2lab(static_cast<const uint8_t*>(si.dev), row, row * rows, static_cast<uint8_t*>(so.dev), row, row * rows,
+                                           rows, cols, n_frames, st), "BGR2Lab launch");
+    });
 }
 
 // ---- (a3) the reference's own containers: EntryType matrices and pitched CV_32FC1 matrices with in-place semantics ----
@@ -1969,14 +1978,23 @@ int dcmt_entries_measurement_derivatives(void* entries, int rows, int cols, size
     return DCMT_OK;
 }
 
-int dcmt_entries_optimize_ig(const void* entries_left, size_t left_row_step_bytes, const void* entries_right, size_t right_row_step_bytes,
-                             size_t elem_stride_bytes, float* disp, size_t disp_pitch_bytes, int rows, int cols, int num_iterations,
-                             float damp_factor, float err_clip, void* cuda_stream) {
+static int check_entries_optimize_ig(const void* entries_left, size_t left_row_step_bytes, const void* entries_right,
+                                     size_t right_row_step_bytes, size_t elem_stride_bytes, const float* disp, size_t* disp_pitch_bytes,
+                                     int rows, int cols, int num_iterations) {
     int rc = check_entries(entries_left, rows, cols, left_row_step_bytes, elem_stride_bytes);
     if (rc) return rc;
     if ((rc = check_entries(entries_right, rows, cols, right_row_step_bytes, elem_stride_bytes))) return rc;
-    if ((rc = check_mat_f32(disp, rows, cols, &disp_pitch_bytes))) return rc;
+    if ((rc = check_mat_f32(disp, rows, cols, disp_pitch_bytes))) return rc;
     if (num_iterations < 0) return fail(DCMT_E_BADARG, "num_iterations %d", num_iterations);
+    return DCMT_OK;
+}
+
+int dcmt_entries_optimize_ig(const void* entries_left, size_t left_row_step_bytes, const void* entries_right, size_t right_row_step_bytes,
+                             size_t elem_stride_bytes, float* disp, size_t disp_pitch_bytes, int rows, int cols, int num_iterations,
+                             float damp_factor, float err_clip, void* cuda_stream) {
+    int rc = check_entries_optimize_ig(entries_left, left_row_step_bytes, entries_right, right_row_step_bytes, elem_stride_bytes, disp,
+                                       &disp_pitch_bytes, rows, cols, num_iterations);
+    if (rc) return rc;
     if ((rc = check_device())) return rc;
     API_CUDA(dcmt::stereo_entries_optimize_ig(entries_left, left_row_step_bytes, entries_right, right_row_step_bytes, elem_stride_bytes, disp,
                                               disp_pitch_bytes / sizeof(float), rows, cols, num_iterations, damp_factor, err_clip,
@@ -1985,12 +2003,19 @@ int dcmt_entries_optimize_ig(const void* entries_left, size_t left_row_step_byte
     return DCMT_OK;
 }
 
-int dcmt_get_initial_disparity_mat_f32(const float* depth, size_t depth_pitch_bytes, float* disp, size_t disp_pitch_bytes, int rows, int cols,
-                                       float baseline, float focal, void* cuda_stream) {
+// the two CV_32FC1 Mat operations, input then output
+static int check_mat_pair(const float* in, size_t* in_pitch_bytes, const float* out, size_t* out_pitch_bytes, int rows, int cols) {
     int rc = check_planes(rows, cols, 1);
     if (rc) return rc;
     if (rows > 65535) return fail(DCMT_E_UNSUPPORTED, "at most 65535 rows");
-    if ((rc = check_mat_f32(depth, rows, cols, &depth_pitch_bytes)) || (rc = check_mat_f32(disp, rows, cols, &disp_pitch_bytes))) return rc;
+    if ((rc = check_mat_f32(in, rows, cols, in_pitch_bytes)) || (rc = check_mat_f32(out, rows, cols, out_pitch_bytes))) return rc;
+    return DCMT_OK;
+}
+
+int dcmt_get_initial_disparity_mat_f32(const float* depth, size_t depth_pitch_bytes, float* disp, size_t disp_pitch_bytes, int rows, int cols,
+                                       float baseline, float focal, void* cuda_stream) {
+    int rc = check_mat_pair(depth, &depth_pitch_bytes, disp, &disp_pitch_bytes, rows, cols);
+    if (rc) return rc;
     if ((rc = check_device())) return rc;
     API_CUDA(dcmt::stereo_initial_disparity_mat(depth, depth_pitch_bytes / sizeof(float), disp, disp_pitch_bytes / sizeof(float), rows, cols,
                                                 baseline, focal, static_cast<cudaStream_t>(cuda_stream)),
@@ -2000,10 +2025,8 @@ int dcmt_get_initial_disparity_mat_f32(const float* depth, size_t depth_pitch_by
 
 int dcmt_retrieve_optimized_depth_mat_f32(const float* disp, size_t disp_pitch_bytes, float* depth, size_t depth_pitch_bytes, int rows, int cols,
                                           float baseline, float focal, float depth_clip, void* cuda_stream) {
-    int rc = check_planes(rows, cols, 1);
+    int rc = check_mat_pair(disp, &disp_pitch_bytes, depth, &depth_pitch_bytes, rows, cols);
     if (rc) return rc;
-    if (rows > 65535) return fail(DCMT_E_UNSUPPORTED, "at most 65535 rows");
-    if ((rc = check_mat_f32(disp, rows, cols, &disp_pitch_bytes)) || (rc = check_mat_f32(depth, rows, cols, &depth_pitch_bytes))) return rc;
     if ((rc = check_device())) return rc;
     API_CUDA(dcmt::stereo_retrieve_depth_mat(disp, disp_pitch_bytes / sizeof(float), depth, depth_pitch_bytes / sizeof(float), rows, cols,
                                              baseline, focal, depth_clip, static_cast<cudaStream_t>(cuda_stream)),
@@ -2016,80 +2039,51 @@ int dcmt_retrieve_optimized_depth_mat_f32(const float* disp, size_t disp_pitch_b
 int dcmt_entries_measurement_derivatives_host(void* entries, int rows, int cols, size_t row_step_bytes, size_t elem_stride_bytes) {
     int rc = check_entries(entries, rows, cols, row_step_bytes, elem_stride_bytes);
     if (rc) return rc;
-    HostCall call;
-    if ((rc = call.open(nullptr, 0, false))) return rc;
-    cudaStream_t st = call.lanes[0].hs->s[0];
     const size_t used = (size_t)cols * elem_stride_bytes;
-    Arena* ar = nullptr;
-    if ((rc = arena_acquire(st, carve_bytes(used * rows, 1), &ar))) return rc;
-    char* d = carve<char>(ar, used * rows);
-    if ((rc = arena_ok(ar))) return rc;
-    call.use(call.lanes[0]);
-    API_CUDA(cudaMemcpy2DAsync(d, used, entries, row_step_bytes, used, rows, cudaMemcpyHostToDevice, st), "host to device copy");
-    if ((rc = dcmt_entries_measurement_derivatives(d, rows, cols, used, elem_stride_bytes, st))) return rc;
-    API_CUDA(cudaMemcpy2DAsync(entries, row_step_bytes, d, used, used, rows, cudaMemcpyDeviceToHost, st), "device to host copy");
-    return call.finish();
+    Staged se{entries, entries, row_step_bytes, used, (size_t)rows};
+    return run_staged({&se}, [&](cudaStream_t st) {
+        return cuda_rc(dcmt::stereo_entries_derivatives(se.dev, used, elem_stride_bytes, rows, cols, st), "measurement derivatives launch");
+    });
 }
 
 int dcmt_entries_optimize_ig_host(const void* entries_left, size_t left_row_step_bytes, const void* entries_right,
                                   size_t right_row_step_bytes, size_t elem_stride_bytes, float* disp, size_t disp_pitch_bytes, int rows,
                                   int cols, int num_iterations, float damp_factor, float err_clip) {
-    int rc = check_entries(entries_left, rows, cols, left_row_step_bytes, elem_stride_bytes);
+    int rc = check_entries_optimize_ig(entries_left, left_row_step_bytes, entries_right, right_row_step_bytes, elem_stride_bytes, disp,
+                                       &disp_pitch_bytes, rows, cols, num_iterations);
     if (rc) return rc;
-    if ((rc = check_entries(entries_right, rows, cols, right_row_step_bytes, elem_stride_bytes))) return rc;
-    if ((rc = check_mat_f32(disp, rows, cols, &disp_pitch_bytes))) return rc;
-    HostCall call;
-    if ((rc = call.open(nullptr, 0, false))) return rc;
-    cudaStream_t st = call.lanes[0].hs->s[0];
-    const size_t used = (size_t)cols * elem_stride_bytes, drow = (size_t)cols * sizeof(float);
-    Arena* ar = nullptr;
-    if ((rc = arena_acquire(st, 2 * carve_bytes(used * rows, 1) + carve_bytes(drow * rows, 1), &ar))) return rc;
-    char* dl = carve<char>(ar, used * rows);
-    char* dr = carve<char>(ar, used * rows);
-    float* dd = reinterpret_cast<float*>(carve<char>(ar, drow * rows));
-    if ((rc = arena_ok(ar))) return rc;
-    call.use(call.lanes[0]);
-    API_CUDA(cudaMemcpy2DAsync(dl, used, entries_left, left_row_step_bytes, used, rows, cudaMemcpyHostToDevice, st), "host to device copy");
-    API_CUDA(cudaMemcpy2DAsync(dr, used, entries_right, right_row_step_bytes, used, rows, cudaMemcpyHostToDevice, st), "host to device copy");
-    API_CUDA(cudaMemcpy2DAsync(dd, drow, disp, disp_pitch_bytes, drow, rows, cudaMemcpyHostToDevice, st), "host to device copy");
-    if ((rc = dcmt_entries_optimize_ig(dl, used, dr, used, elem_stride_bytes, dd, drow, rows, cols, num_iterations, damp_factor, err_clip, st)))
-        return rc;
-    API_CUDA(cudaMemcpy2DAsync(disp, disp_pitch_bytes, dd, drow, drow, rows, cudaMemcpyDeviceToHost, st), "device to host copy");
-    return call.finish();
+    const size_t used = (size_t)cols * elem_stride_bytes;
+    Staged sl{entries_left, nullptr, left_row_step_bytes, used, (size_t)rows}, sr{entries_right, nullptr, right_row_step_bytes, used, (size_t)rows},
+        sd{disp, disp, disp_pitch_bytes, (size_t)cols * sizeof(float), (size_t)rows};
+    return run_staged({&sl, &sr, &sd}, [&](cudaStream_t st) {
+        return cuda_rc(dcmt::stereo_entries_optimize_ig(sl.dev, used, sr.dev, used, elem_stride_bytes, static_cast<float*>(sd.dev), cols, rows, cols,
+                                                        num_iterations, damp_factor, err_clip, st), "optimize_IG launch");
+    });
 }
 
-static int mat_pair_host(const float* in, size_t in_pitch, float* out, size_t out_pitch, int rows, int cols, int which, float baseline,
-                         float focal, float clip) {
-    int rc = check_planes(rows, cols, 1);
-    if (rc) return rc;
-    if ((rc = check_mat_f32(in, rows, cols, &in_pitch)) || (rc = check_mat_f32(out, rows, cols, &out_pitch))) return rc;
-    HostCall call;
-    if ((rc = call.open(nullptr, 0, false))) return rc;
-    cudaStream_t st = call.lanes[0].hs->s[0];
-    const size_t drow = (size_t)cols * sizeof(float);
-    Arena* ar = nullptr;
-    if ((rc = arena_acquire(st, 2 * carve_bytes(drow * rows, 1), &ar))) return rc;
-    float* di = reinterpret_cast<float*>(carve<char>(ar, drow * rows));
-    float* dout = reinterpret_cast<float*>(carve<char>(ar, drow * rows));
-    if ((rc = arena_ok(ar))) return rc;
-    call.use(call.lanes[0]);
-    API_CUDA(cudaMemcpy2DAsync(di, drow, in, in_pitch, drow, rows, cudaMemcpyHostToDevice, st), "host to device copy");
-    API_CUDA(cudaMemcpy2DAsync(dout, drow, out, out_pitch, drow, rows, cudaMemcpyHostToDevice, st), "host to device copy");  // untouched pixels keep their value
-    rc = which == 0 ? dcmt_get_initial_disparity_mat_f32(di, drow, dout, drow, rows, cols, baseline, focal, st)
-                    : dcmt_retrieve_optimized_depth_mat_f32(di, drow, dout, drow, rows, cols, baseline, focal, clip, st);
-    if (rc) return rc;
-    API_CUDA(cudaMemcpy2DAsync(out, out_pitch, dout, drow, drow, rows, cudaMemcpyDeviceToHost, st), "device to host copy");
-    return call.finish();
-}
-
+// the output is copied in as well: pixels the kernel skips keep the caller's value
 int dcmt_get_initial_disparity_mat_f32_host(const float* depth, size_t depth_pitch_bytes, float* disp, size_t disp_pitch_bytes, int rows,
                                             int cols, float baseline, float focal) {
-    return mat_pair_host(depth, depth_pitch_bytes, disp, disp_pitch_bytes, rows, cols, 0, baseline, focal, 0.0f);
+    int rc = check_mat_pair(depth, &depth_pitch_bytes, disp, &disp_pitch_bytes, rows, cols);
+    if (rc) return rc;
+    const size_t row = (size_t)cols * sizeof(float);
+    Staged si{depth, nullptr, depth_pitch_bytes, row, (size_t)rows}, so{disp, disp, disp_pitch_bytes, row, (size_t)rows};
+    return run_staged({&si, &so}, [&](cudaStream_t st) {
+        return cuda_rc(dcmt::stereo_initial_disparity_mat(static_cast<const float*>(si.dev), cols, static_cast<float*>(so.dev), cols, rows, cols,
+                                                          baseline, focal, st), "initial disparity launch");
+    });
 }
 
 int dcmt_retrieve_optimized_depth_mat_f32_host(const float* disp, size_t disp_pitch_bytes, float* depth, size_t depth_pitch_bytes, int rows,
                                                int cols, float baseline, float focal, float depth_clip) {
-    return mat_pair_host(disp, disp_pitch_bytes, depth, depth_pitch_bytes, rows, cols, 1, baseline, focal, depth_clip);
+    int rc = check_mat_pair(disp, &disp_pitch_bytes, depth, &depth_pitch_bytes, rows, cols);
+    if (rc) return rc;
+    const size_t row = (size_t)cols * sizeof(float);
+    Staged si{disp, nullptr, disp_pitch_bytes, row, (size_t)rows}, so{depth, depth, depth_pitch_bytes, row, (size_t)rows};
+    return run_staged({&si, &so}, [&](cudaStream_t st) {
+        return cuda_rc(dcmt::stereo_retrieve_depth_mat(static_cast<const float*>(si.dev), cols, static_cast<float*>(so.dev), cols, rows, cols,
+                                                       baseline, focal, depth_clip, st), "retrieve depth launch");
+    });
 }
 
 }  // extern "C"
