@@ -52,6 +52,9 @@ class DcmtError(RuntimeError):
 
 
 _P = C.c_void_p
+# dcmt_stereo_chain_f32_host's arguments; the device form adds the stream, _host_multi the device list
+_CHAIN = [_P, _P, C.c_int, C.c_size_t, _P, _P, C.c_float, C.c_float, _P, _P, C.c_size_t, C.c_size_t, _P, _P, C.c_int, C.c_int, C.c_int,
+          C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(StereoParams), _P]
 _SIGNATURES = {
     "dcmt_version": (C.c_int, []),
     "dcmt_build_info": (C.c_char_p, []),
@@ -77,6 +80,9 @@ _SIGNATURES = {
     "dcmt_stereo_params_official": (None, [C.POINTER(StereoParams), C.c_int]),
     "dcmt_stereo_refine_f32": (C.c_int, [_P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.POINTER(StereoParams), _P]),
     "dcmt_stereo_refine_f32_host": (C.c_int, [_P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.POINTER(StereoParams)]),
+    "dcmt_stereo_chain_f32": (C.c_int, _CHAIN + [_P]),
+    "dcmt_stereo_chain_f32_host": (C.c_int, _CHAIN),
+    "dcmt_stereo_chain_f32_host_multi": (C.c_int, _CHAIN + [_P, C.c_int]),
     "dcmt_measurement_derivatives_f32": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, _P]),
     "dcmt_get_initial_disparity_f32": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, _P]),
     "dcmt_optimize_ig_f32": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, _P]),

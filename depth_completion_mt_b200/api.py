@@ -380,6 +380,84 @@ def stereo_refine(depth_ig, left_gray, right_gray, params: StereoParams | None =
     return (out, disp) if return_disparity else out
 
 
+def stereo_chain(points, counts, T, P, left_bgr, right_bgr, step, nc: int = 40, *, norm=(0.0, 80.0), use_superpixel: int = 1,
+                 iterations: int = 10, params: StereoParams | None = None, path: str = "auto", return_disparity: bool = False,
+                 return_stats: bool = False, devices=None, stream=None, lib: _lib.Library | None = None):
+    """The stereo program's per-frame chain in one call (``dcmt_stereo_chain_f32``; main_sl.cpp:435-563 withSuperPixels and
+    :1162-1253): LiDAR projection + ``cv::normalize(norm)``, ``generate_superpixels_bgr(left_bgr, step, nc)``,
+    ``interpolate_with_superpixels`` of the normalised floats, ``cvtColor(COLOR_BGR2GRAY)`` of both frames and
+    ``stereo_refine``, with every intermediate on the device.
+
+    ``points`` is (n, max_points, 4) float32, or (m, 4) for one frame; ``counts`` the points of each cloud ((n,) int32) or
+    None for max_points each.  ``left_bgr`` / ``right_bgr`` are the uint8 colour images as read, (rows, cols, 3) or
+    (n, rows, cols, 3).  ``T`` (4x4) and ``P`` (3x4) are one calibration for the batch.  ``step`` is truncated to int as
+    the reference's int parameter.  Returns the refined depth, then the disparity with ``return_disparity`` and the
+    completion's stats with ``return_stats``.  CUDA tensors use the device entry point on ``stream``; numpy arrays the host
+    entry point, or -- with ``devices`` ("all" or a list of ordinals) -- the frames spread over those GPUs."""
+    lib = lib or _lib.load()
+    step = int(step)
+    if path not in ("auto", "generic", "rank"):
+        raise ValueError("path must be 'auto', 'generic' or 'rank' (the normalised projection is not strict q8)")
+    Tm = np.ascontiguousarray(np.asarray(T, np.float32).reshape(4, 4))
+    Pm = np.ascontiguousarray(np.asarray(P, np.float32).reshape(3, 4))
+    prm = params or stereo_params(lib=lib)
+    is_t = _is_torch(points)
+    if is_t:
+        if devices is not None:
+            raise ValueError("devices= applies to host (numpy) input; a CUDA tensor already lives on one device")
+        pts, lft, rgt = (_prep_torch(x, d, w) for x, d, w in ((points, torch.float32, "points"), (left_bgr, torch.uint8, "left_bgr"),
+                                                               (right_bgr, torch.uint8, "right_bgr")))
+        cnt = _prep_torch(counts, torch.int32, "counts") if counts is not None else None
+    else:
+        pts, lft, rgt = (_prep_numpy(x, d, w) for x, d, w in ((points, np.float32, "points"), (left_bgr, np.uint8, "left_bgr"),
+                                                               (right_bgr, np.uint8, "right_bgr")))
+        cnt = _prep_numpy(np.asarray(counts, np.int32), np.int32, "counts") if counts is not None else None
+    squeeze = pts.ndim == 2
+    p3 = pts[None] if squeeze else pts
+    l4, r4 = (x[None] if x.ndim == 3 else x for x in (lft, rgt))
+    if p3.ndim != 3 or p3.shape[2] != 4:
+        raise ValueError(f"points must be (n, max_points, 4) or (m, 4), got {tuple(pts.shape)}")
+    n, mp = int(p3.shape[0]), int(p3.shape[1])
+    if l4.ndim != 4 or l4.shape[0] != n or l4.shape[3] != 3 or tuple(r4.shape) != tuple(l4.shape):
+        raise ValueError(f"left_bgr and right_bgr must be the (rows, cols, 3) colour images of each cloud, got {tuple(lft.shape)} and "
+                         f"{tuple(rgt.shape)} for {n} clouds")
+    if cnt is not None and tuple(cnt.shape) != (n,):
+        raise ValueError(f"counts must hold one int32 per cloud, got shape {tuple(cnt.shape)} for {n} clouds")
+    rows, cols = int(l4.shape[1]), int(l4.shape[2])
+    args = (float(norm[0]), float(norm[1]))
+    tail = (rows, cols, n, step, int(nc), int(iterations), int(use_superpixel), PATH[path], C.byref(prm))
+    if is_t:
+        depth = torch.empty((n, rows, cols), dtype=torch.float32, device=p3.device)
+        disp = torch.empty_like(depth) if return_disparity else None
+        stats = torch.zeros((n, STATS_STRIDE), dtype=torch.int32, device=p3.device) if return_stats else None
+        with torch.cuda.device(p3.device):
+            lib.check(lib.dcmt_stereo_chain_f32(p3.data_ptr() if p3.numel() else None, cnt.data_ptr() if cnt is not None else None, mp, mp,
+                                                _np_ptr(Tm), _np_ptr(Pm), *args, l4.data_ptr(), r4.data_ptr(), 0, 0, depth.data_ptr(),
+                                                disp.data_ptr() if return_disparity else None, *tail,
+                                                stats.data_ptr() if return_stats else None, _stream_ptr(stream)))
+    else:
+        depth = np.empty((n, rows, cols), np.float32)
+        disp = np.empty_like(depth) if return_disparity else None
+        stats = np.zeros((n, STATS_STRIDE), np.int32) if return_stats else None
+        head = (_np_ptr(p3) if p3.size else None, _np_ptr(cnt) if cnt is not None else None, mp, mp, _np_ptr(Tm), _np_ptr(Pm), *args,
+                _np_ptr(l4), _np_ptr(r4), 0, 0, _np_ptr(depth), _np_ptr(disp) if return_disparity else None, *tail,
+                _np_ptr(stats) if return_stats else None)
+        keep, dev_ptr, n_dev = _device_list(devices)
+        if devices is not None:
+            lib.check(lib.dcmt_stereo_chain_f32_host_multi(*head, dev_ptr, n_dev))
+        else:
+            lib.check(lib.dcmt_stereo_chain_f32_host(*head))
+        del keep
+    out = [depth]
+    if return_disparity:
+        out.append(disp)
+    if return_stats:
+        out.append(stats)
+    if squeeze:
+        out = [o[0] for o in out]
+    return tuple(out) if len(out) > 1 else out[0]
+
+
 def _device_planes(lib, fn_name, arrays, n_out, extra, stream, out_like=None):
     """Helper for the per-function stereo entry points (device pointers only in the ABI): numpy inputs are
     staged through torch."""

@@ -461,6 +461,19 @@ int check_slic(int rows, int cols, int step, int nc, int iterations) {
     return DCMT_OK;
 }
 
+// The pitch and frame stride in bytes of n_frames BGR frames of rows x cols (0 = dense: filled in); *span receives the bytes
+// the frames cover
+int check_bgr_geometry(int rows, int cols, size_t* pitch, size_t* fstride, int n_frames, size_t* span) {
+    const size_t row = (size_t)cols * 3;
+    if (*pitch == 0) *pitch = row;
+    if (*fstride == 0) *fstride = *pitch * rows;
+    if (*pitch < row) return fail(DCMT_E_BADARG, "bgr_pitch_bytes %zu below %d columns of 3 bytes", *pitch, cols);
+    const size_t frame = *pitch * (size_t)(rows - 1) + row;
+    if (*fstride < frame) return fail(DCMT_E_BADARG, "bgr_frame_stride_bytes %zu invalid", *fstride);
+    *span = n_frames ? *fstride * (size_t)(n_frames - 1) + frame : 0;
+    return DCMT_OK;
+}
+
 // Checks a completion call -- pointers, labels, blur, flags, input geometry, output geometry, overlap, in this order, then
 // for a BGR front its pointer, SLIC's arguments, its geometry and its overlap with the output -- and converts the pitches
 // and frame strides of `in` and `out` from the ABI's bytes into elements.  A BGR front gets its dense pitch / frame stride
@@ -478,14 +491,9 @@ int validate_completion(CompletionCall& cc, InDesc* in, OutDesc* out, int n_fram
     if (BgrFront* fr = cc.front) {
         if (!fr->bgr) return fail(DCMT_E_BADARG, "null image pointer");
         if ((rc = check_slic(cc.rows, cc.cols, fr->step, fr->nc, fr->iterations))) return rc;
-        const size_t row = (size_t)cc.cols * 3;
-        if (fr->pitch == 0) fr->pitch = row;
-        if (fr->fstride == 0) fr->fstride = fr->pitch * cc.rows;
-        if (fr->pitch < row) return fail(DCMT_E_BADARG, "bgr_pitch_bytes %zu below %d columns of 3 bytes", fr->pitch, cc.cols);
-        const size_t frame = fr->pitch * (size_t)(cc.rows - 1) + row;
-        if (fr->fstride < frame) return fail(DCMT_E_BADARG, "bgr_frame_stride_bytes %zu invalid", fr->fstride);
-        if (n_frames && overlaps(fr->bgr, fr->fstride * (size_t)(n_frames - 1) + frame, out->ptr(), go.span_bytes))
-            return fail(DCMT_E_BADARG, "BGR input and output overlap");
+        size_t span = 0;
+        if ((rc = check_bgr_geometry(cc.rows, cc.cols, &fr->pitch, &fr->fstride, n_frames, &span))) return rc;
+        if (n_frames && overlaps(fr->bgr, span, out->ptr(), go.span_bytes)) return fail(DCMT_E_BADARG, "BGR input and output overlap");
         cc.n_clusters = dcmt::slic_center_count(cc.rows, cc.cols, fr->step);
     }
     in->pitch = gi.pitch;
@@ -493,6 +501,24 @@ int validate_completion(CompletionCall& cc, InDesc* in, OutDesc* out, int n_fram
     out->pitch = go.pitch;
     out->fstride = go.fstride;
     return DCMT_OK;
+}
+
+// frames [f, e) of a call
+struct Run {
+    int f, e;
+};
+
+// the runs of consecutive frames whose flag is set, in frame order: the frames a pass did not serve
+std::vector<Run> flagged_runs(const int32_t* flags, int n) {
+    std::vector<Run> runs;
+    for (int f = 0; f < n;) {
+        if (!flags[f]) { ++f; continue; }
+        int e = f;
+        while (e < n && flags[e]) ++e;
+        runs.push_back(Run{f, e});
+        f = e;
+    }
+    return runs;
 }
 
 // uint16 input needs no validation: AUTO, RANK and FUSED are the same thing there
@@ -525,11 +551,9 @@ int run_completion(CompletionCall cc, InDesc in, OutDesc out, int n_frames, int3
     for (int level = cc.flags == DCMT_PATH_AUTO ? DCMT_PATH_RANK : DCMT_PATH_GENERIC;; level = DCMT_PATH_GENERIC) {
         cc.flags = level;
         const bool want_flags = level == DCMT_PATH_RANK;
-        bool any = false;
-        for (int f = 0; f < n_frames;) {
-            if (!h_flags[f]) { ++f; continue; }
-            int e = f;
-            while (e < n_frames && h_flags[e]) ++e;
+        const std::vector<Run> runs = flagged_runs(h_flags, n_frames);
+        for (const Run& r : runs) {
+            const int f = r.f, e = r.e;
             // the previous pass has completed (stream synchronised): the arena is free again, but it was sized for that
             // pass -- this one may need more (the generic pipeline: two float planes per frame of its chunk)
             const size_t fb = want_flags ? carve_bytes((size_t)(e - f), sizeof(int32_t)) : 0;
@@ -544,10 +568,8 @@ int run_completion(CompletionCall cc, InDesc in, OutDesc out, int n_frames, int3
                 API_CUDA(cudaMemcpyAsync(h_flags + f, run_flags, (size_t)(e - f) * sizeof(int32_t), cudaMemcpyDeviceToHost, st), "flag readback");
                 API_CUDA(cudaStreamSynchronize(st), "kernel execution");
             }
-            any = true;
-            f = e;
         }
-        if (level == DCMT_PATH_GENERIC || !any) break;
+        if (level == DCMT_PATH_GENERIC || runs.empty()) break;
     }
     return DCMT_OK;
 }
@@ -589,6 +611,37 @@ int enqueue_slic(const uint8_t* img, size_t pitch, size_t fstride, bool from_bgr
     if (centers && k > 0)
         API_CUDA(cudaMemcpyAsync(centers, w.centers, (size_t)k * n * 5 * sizeof(double), cudaMemcpyDeviceToDevice, st), "centre copy");
     return DCMT_OK;
+}
+
+// ---- the batched LiDAR projection, checked and enqueued on an arena its caller holds (dcmt_lidar_project_batch_f32 and the
+// stereo chain).  max_clouds: 65535 for one launch; the chain runs in chunks and has no limit.
+int check_project_batch(const float* points, int max_points, size_t cloud_stride_points, int n_clouds, int max_clouds, const float* T_host,
+                        const float* P_host, int rows, int cols) {
+    if ((!points && max_points > 0) || !T_host || !P_host) return fail(DCMT_E_BADARG, "null pointer");
+    if (max_points < 0 || n_clouds < 0) return fail(DCMT_E_BADARG, "max_points %d, n_clouds %d", max_points, n_clouds);
+    if (n_clouds > max_clouds) return fail(DCMT_E_UNSUPPORTED, "at most %d clouds per call", max_clouds);
+    if (n_clouds > 1 && cloud_stride_points < (size_t)max_points) return fail(DCMT_E_BADARG, "cloud_stride_points %zu < max_points %d", cloud_stride_points, max_points);
+    int rc = check_planes(rows, cols, 1);
+    if (rc) return rc;
+    if ((size_t)rows * (size_t)cols > (size_t)1 << 30) return fail(DCMT_E_UNSUPPORTED, "frame larger than 2^30 pixels");
+    return DCMT_OK;
+}
+
+// the keys and min / max words of n clouds
+size_t project_ws_bytes(int rows, int cols, int n) {
+    return carve_bytes(dcmt::project_key_count(rows, cols) * n, sizeof(unsigned long long)) + carve_bytes(8 * (size_t)n, sizeof(unsigned));
+}
+
+// the projection of n (1..65535) clouds on checked arguments and 16-byte aligned points, its work arrays carved from `ar`
+int enqueue_project_batch(const float* points, const int32_t* counts_dev, int max_points, size_t cloud_stride_points, int n, const float* T_host,
+                          const float* P_host, int rows, int cols, float* projected, float* normalized, float norm_a, float norm_b,
+                          int32_t* n_projected, Arena* ar, cudaStream_t st) {
+    const size_t nk = dcmt::project_key_count(rows, cols) * n;
+    dcmt::ProjectWork w{carve<unsigned long long>(ar, nk), carve<unsigned>(ar, 8 * (size_t)n)};
+    if (int rc = arena_ok(ar)) return rc;
+    return cuda_rc(dcmt::project_run_batch(points, max_points, counts_dev, cloud_stride_points, n, T_host, P_host, rows, cols, projected,
+                                           normalized, norm_a, norm_b, n_projected, w, st),
+                   "projection launch");
 }
 
 // device-pointer driver of the dcmt_interpolate_with_superpixels_bgr_* entry points (uint16 input: never synchronises).
@@ -850,6 +903,28 @@ int run_staged(std::initializer_list<Staged*> bufs, Work&& work) {
     return call.finish();
 }
 
+// Enqueues again, on the device that served them, the frames of a host-pointer call whose flag (Lane::h_flags, read back by
+// the previous pass) is set: runs of consecutive frames, cut into host chunks, redo(lane, f0, nf, chunk frames) per chunk.
+// The runs are fixed before anything is enqueued (a pass may write the flags it reads).  *any: whether a frame was flagged.
+template <class Redo>
+int redo_flagged(HostCall& call, int rows, int cols, bool* any, Redo&& redo) {
+    struct LaneRun {
+        Lane* l;
+        Run r;
+    };
+    std::vector<LaneRun> runs;
+    for (Lane& l : call.lanes)
+        for (const Run& r : flagged_runs(l.h_flags, l.f_end - l.f_begin)) runs.push_back(LaneRun{&l, Run{l.f_begin + r.f, l.f_begin + r.e}});
+    *any = !runs.empty();
+    for (const LaneRun& lr : runs) {
+        if (int rc = call.use(*lr.l)) return rc;
+        const int hc = host_chunk_frames(rows, cols, lr.r.e - lr.r.f);
+        for (int f = lr.r.f; f < lr.r.e; f += hc)
+            if (int rc = redo(*lr.l, f, std::min(hc, lr.r.e - f), hc)) return rc;
+    }
+    return DCMT_OK;
+}
+
 // Host-pointer driver of every completion entry point.  Device staging rows are packed for float32 input and padded to
 // 16 bytes for uint16 input (vector loads in k_q8_front).
 // copy_only: the same buffers, chunking and streams with the kernels left out -- the ceiling the host <-> device links put
@@ -966,31 +1041,263 @@ int run_completion_host(CompletionCall cc, InDesc in, OutDesc out, int n_frames,
             CompletionCall cg = cc;
             cg.flags = level;
             bool any = false;
-            // the runs are fixed before anything is enqueued: the rank pass overwrites the flags it reads
-            struct Run { Lane* l; int f, e; };
-            std::vector<Run> runs;
-            for (Lane& l : call.lanes) {
-                const int n_lane = l.f_end - l.f_begin;
-                for (int i = 0; i < n_lane;) {
-                    if (!l.h_flags[i]) { ++i; continue; }
-                    int e = i;
-                    while (e < n_lane && l.h_flags[e]) ++e;
-                    runs.push_back(Run{&l, l.f_begin + i, l.f_begin + e});
-                    i = e;
-                }
-            }
-            for (const Run& r : runs) {
-                if ((rc = call.use(*r.l))) return rc;
-                const int hc2 = host_chunk_frames(rows, cols, r.e - r.f);
-                for (int f = r.f; f < r.e; f += hc2)
-                    if ((rc = do_chunk(*r.l, f, std::min(hc2, r.e - f), cg, hc2))) return rc;
-                any = true;
-            }
+            if ((rc = redo_flagged(call, rows, cols, &any, [&](Lane& l, int f0, int nf, int hc2) { return do_chunk(l, f0, nf, cg, hc2); })))
+                return rc;
             if (any && (rc = call.finish())) return rc;
             if (level == DCMT_PATH_GENERIC || !any) break;
         }
     }
     return DCMT_OK;
+}
+
+// ---- the stereo program's per-frame chain (dcmt_stereo_chain_f32*, main_sl.cpp:435-563 + :1162-1253): batched projection
+// + cv::normalize, SLIC of the left frame from BGR, the guided completion of the normalised floats, BGR2GRAY of both frames
+// and the stereo refinement, with every intermediate in the workspace.
+struct StereoChain {
+    const float* points;
+    const int32_t* counts;  // n_points per cloud (device array on the device form, host array on the host forms) or null
+    int max_points;
+    size_t cloud_stride;  // points
+    const float *T, *P;
+    float norm_a, norm_b;
+    const uint8_t *left, *right;
+    size_t bgr_pitch, bgr_fstride;  // bytes; the ABI's 0 = dense until validate_stereo_chain fills them in
+    float *depth, *disp;
+    int rows, cols, n_frames, step, nc, iterations, use_superpixel, flags;
+    const dcmt_stereo_params* prm;
+    int32_t* stats;
+};
+
+// Checks a chain call: the projection's arguments, the other pointers, flags, the refinement's parameters, SLIC's limits,
+// BGR2GRAY's rows, the BGR geometry and overlap of the outputs, in this order; on the host forms (host_counts) the cloud
+// sizes last, the only caller data a check reads.
+int validate_stereo_chain(StereoChain& c, bool host_counts) {
+    int rc = check_project_batch(c.points, c.max_points, c.cloud_stride, c.n_frames, INT32_MAX, c.T, c.P, c.rows, c.cols);
+    if (rc) return rc;
+    if (!c.left || !c.right || !c.depth || !c.prm) return fail(DCMT_E_BADARG, "null pointer");
+    if (c.flags < DCMT_PATH_AUTO || c.flags > DCMT_PATH_RANK) return fail(DCMT_E_BADARG, "flags %d", c.flags);
+    if (c.flags == DCMT_PATH_FUSED) return fail(DCMT_E_BADARG, "DCMT_PATH_FUSED: the normalised projection is not strict q8");
+    if (c.prm->num_iterations < 0) return fail(DCMT_E_BADARG, "num_iterations %d", c.prm->num_iterations);
+    if ((rc = check_slic(c.rows, c.cols, c.step, c.nc, c.iterations))) return rc;
+    if (c.rows > 65535) return fail(DCMT_E_UNSUPPORTED, "at most 65535 rows");
+    size_t bgr_span = 0;
+    if ((rc = check_bgr_geometry(c.rows, c.cols, &c.bgr_pitch, &c.bgr_fstride, c.n_frames, &bgr_span))) return rc;
+    if (c.n_frames) {
+        const size_t plane = (size_t)c.rows * c.cols * c.n_frames * sizeof(float);
+        const size_t cloud_span = c.points ? ((size_t)(c.n_frames - 1) * c.cloud_stride + c.max_points) * 16 : 0;
+        const size_t count_span = c.counts ? (size_t)c.n_frames * sizeof(int32_t) : 0;
+        for (const float* o : {c.depth, c.disp}) {
+            if (!o) continue;
+            if (overlaps(o, plane, c.points, cloud_span) || overlaps(o, plane, c.counts, count_span) || overlaps(o, plane, c.left, bgr_span) ||
+                overlaps(o, plane, c.right, bgr_span))
+                return fail(DCMT_E_BADARG, "an output overlaps an input");
+        }
+        if (c.disp && overlaps(c.depth, plane, c.disp, plane)) return fail(DCMT_E_BADARG, "depth_out and disp_out overlap");
+    }
+    if (host_counts && c.counts)
+        for (int f = 0; f < c.n_frames; ++f)
+            if (c.counts[f] < 0 || c.counts[f] > c.max_points)
+                return fail(DCMT_E_BADARG, "n_points[%d] = %d outside [0, max_points %d]", f, c.counts[f], c.max_points);
+    return DCMT_OK;
+}
+
+// The completion of the chain: the guided call on the normalised floats, AUTO going straight to the dictionary level (the
+// strict-q8 pass would fail on every frame with points; every level gives the same bits)
+CompletionCall chain_completion(const StereoChain& c) {
+    return CompletionCall{nullptr, dcmt::slic_center_count(c.rows, c.cols, c.step), c.use_superpixel != 0, c.rows, c.cols, DCMT_BLUR_GAUSSIAN,
+                          c.flags == DCMT_PATH_GENERIC ? DCMT_PATH_GENERIC : DCMT_PATH_RANK};
+}
+
+// Frames per chunk of the device form: the generic pipeline's 2^27 pixels (DCMT_GENERIC_CHUNK to override).  The chain
+// holds about 37 bytes per pixel (chain_ws_bytes), 4.8 GB at 313 KITTI frames.
+int chain_chunk_frames(int rows, int cols, int n_frames) { return chunk_frames(rows, cols, n_frames, false); }
+
+// the workspace of chunks of `chunk` frames: normalised plane, completed depth, the two gray planes, the projection's keys
+// and min / max words, labels, Lab frames and SLIC's work arrays (guided only), and the completion's workspace
+size_t chain_ws_bytes(const CompletionCall& cc, int chunk, int step) {
+    const size_t px = (size_t)cc.rows * cc.cols * chunk;
+    return 2 * carve_bytes(px, sizeof(float)) + 2 * carve_bytes(px, 1) + project_ws_bytes(cc.rows, cc.cols, chunk) +
+           (cc.guided ? carve_bytes(px, sizeof(int32_t)) + slic_ws_bytes(cc.rows, cc.cols, chunk, step, true) : 0) +
+           completion_ws_bytes(cc, chunk, sizeof(float), sizeof(float));
+}
+
+// Device pointers of nf frames of the chain: 16-byte aligned clouds `cloud_stride` points apart (counts: device array or
+// null), the BGR pairs, and dense outputs (disp, stats and the completion's "not served" flags optional)
+struct ChainFrames {
+    const float* points;
+    const int32_t* counts;
+    size_t cloud_stride;
+    const uint8_t *left, *right;
+    size_t bgr_pitch, bgr_fstride;
+    float *depth, *disp;
+    int32_t *stats, *flags;
+};
+
+// one chunk (1 <= nf <= 65535 frames) of the chain on one stream, its intermediates carved from `ar` (chain_ws_bytes)
+int enqueue_chain(const StereoChain& c, const CompletionCall& cc, const ChainFrames& io, int nf, Arena* ar, cudaStream_t st) {
+    const int rows = c.rows, cols = c.cols;
+    const size_t fpix = (size_t)rows * cols, px = fpix * nf;
+    float* nrm = carve<float>(ar, px);
+    float* dense = carve<float>(ar, px);
+    uint8_t* gray_l = carve<uint8_t>(ar, px);
+    uint8_t* gray_r = carve<uint8_t>(ar, px);
+    int32_t* labels = cc.guided ? carve<int32_t>(ar, px) : nullptr;
+    int rc = enqueue_project_batch(io.points, io.counts, c.max_points, io.cloud_stride, nf, c.T, c.P, rows, cols, nullptr, nrm, c.norm_a, c.norm_b,
+                                   nullptr, ar, st);
+    if (rc) return rc;
+    if (cc.guided &&
+        (rc = enqueue_slic(io.left, io.bgr_pitch, io.bgr_fstride, true, rows, cols, nf, c.step, c.nc, c.iterations, labels, nullptr, ar, st)))
+        return rc;
+    if ((rc = enqueue_completion(cc, InDesc{nrm, nullptr, (size_t)cols, fpix}, labels, OutDesc{dense, nullptr, (size_t)cols, fpix}, nf, io.stats,
+                                 io.flags, nullptr, nullptr, ar, st)))
+        return rc;
+    API_CUDA(dcmt::stereo_bgr2gray(io.left, io.bgr_pitch, io.bgr_fstride, gray_l, cols, fpix, rows, cols, nf, st), "BGR2GRAY launch");
+    API_CUDA(dcmt::stereo_bgr2gray(io.right, io.bgr_pitch, io.bgr_fstride, gray_r, cols, fpix, rows, cols, nf, st), "BGR2GRAY launch");
+    const dcmt_stereo_params& p = *c.prm;
+    API_CUDA(dcmt::stereo_refine(dense, gray_l, gray_r, io.depth, io.disp, rows, cols, nf, p.baseline, p.focal, p.damp_factor, p.err_clip,
+                                 p.depth_clip, p.num_iterations, p.final_gauss, st),
+             "stereo refine launch");
+    return DCMT_OK;
+}
+
+// Device-pointer driver of dcmt_stereo_chain_f32: chunks of chain_chunk_frames on the caller's stream.  On the dictionary
+// path the "not served" flags of the whole call sit at the start of every chunk's arena (the same bytes each time) and are
+// read back once; those frames are redone through the chain with the completion on the generic pipeline.
+int run_stereo_chain(StereoChain c, cudaStream_t st) {
+    int rc = validate_stereo_chain(c, false);
+    if (rc) return rc;
+    if (c.points && (reinterpret_cast<uintptr_t>(c.points) & 15)) return fail(DCMT_E_BADARG, "points must be 16-byte aligned");
+    if (c.n_frames == 0) return DCMT_OK;
+    if ((rc = check_device())) return rc;
+    API_CUDA(dcmt::generic_configure(), "kernel attribute setup");
+    API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
+    CompletionCall cc = chain_completion(c);
+    const int n = c.n_frames, chunk = chain_chunk_frames(c.rows, c.cols, n);
+    const bool flagged = cc.flags == DCMT_PATH_RANK && fused_applies(cc);
+    const size_t fpix = (size_t)c.rows * c.cols;
+    auto frames = [&](int f0, int32_t* flags) {
+        return ChainFrames{c.points ? c.points + (size_t)f0 * c.cloud_stride * 4 : nullptr, c.counts ? c.counts + f0 : nullptr, c.cloud_stride,
+                           c.left + (size_t)f0 * c.bgr_fstride, c.right + (size_t)f0 * c.bgr_fstride, c.bgr_pitch, c.bgr_fstride,
+                           c.depth + (size_t)f0 * fpix, c.disp ? c.disp + (size_t)f0 * fpix : nullptr,
+                           c.stats ? c.stats + (size_t)f0 * DCMT_STATS_STRIDE : nullptr, flags};
+    };
+    const size_t flag_bytes = flagged ? carve_bytes((size_t)n, sizeof(int32_t)) : 0;
+    int32_t* d_flags = nullptr;
+    for (int f0 = 0; f0 < n; f0 += chunk) {
+        const int nf = std::min(chunk, n - f0);
+        Arena* ar = nullptr;
+        if ((rc = arena_acquire(st, flag_bytes + chain_ws_bytes(cc, chunk, c.step), &ar))) return rc;  // stream order: the previous chunk is done with it
+        if (flagged) d_flags = carve<int32_t>(ar, (size_t)n);
+        if ((rc = enqueue_chain(c, cc, frames(f0, d_flags ? d_flags + f0 : nullptr), nf, ar, st))) return rc;
+    }
+    if (!flagged) return DCMT_OK;
+    int32_t* h_flags = nullptr;
+    if ((rc = pinned_flags(st, (size_t)n, &h_flags))) return rc;
+    API_CUDA(cudaMemcpyAsync(h_flags, d_flags, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st), "flag readback");
+    API_CUDA(cudaStreamSynchronize(st), "kernel execution");
+    cc.flags = DCMT_PATH_GENERIC;
+    for (const Run& r : flagged_runs(h_flags, n)) {
+        for (int f0 = r.f; f0 < r.e; f0 += chunk) {
+            Arena* ar = nullptr;
+            if ((rc = arena_acquire(st, chain_ws_bytes(cc, chunk, c.step), &ar))) return rc;
+            if ((rc = enqueue_chain(c, cc, frames(f0, nullptr), std::min(chunk, r.e - f0), ar, st))) return rc;
+        }
+    }
+    return DCMT_OK;
+}
+
+// Host-pointer driver of dcmt_stereo_chain_f32_host[_multi]: host chunks on the three streams of each device, as the completion's
+// host driver.  A chunk stages n_points[c] * 16 bytes of each cloud (max_points apart), the cloud sizes and both BGR frames
+// (packed), runs the chain into its arena and copies depth, disparity, stats and the dictionary's flags back.  Flagged frames
+// are redone, on the device that served them, with the completion on the generic pipeline.
+int run_stereo_chain_host(StereoChain c, const int* devices = nullptr, int n_devices = 0, bool multi = false) {
+    int rc = validate_stereo_chain(c, true);
+    if (rc) return rc;
+    if (c.n_frames == 0) return DCMT_OK;
+    if (c.n_frames == 1) c.cloud_stride = c.max_points;  // one cloud: the ABI lets its stride be anything; staged clouds are max_points apart
+    HostCall call;
+    if ((rc = call.open(devices, n_devices, multi))) return rc;
+    call.split(c.n_frames);
+    const int rows = c.rows, cols = c.cols;
+    const size_t fpix = (size_t)rows * cols, bgr_row = (size_t)cols * 3, cloud_bytes = (size_t)c.max_points * 16;
+    const CompletionCall cc = chain_completion(c);
+    const bool flagged = cc.flags == DCMT_PATH_RANK && fused_applies(cc);
+    int longest = 0;
+    for (Lane& l : call.lanes) longest = std::max(longest, l.f_end - l.f_begin);
+    const int hc = host_chunk_frames(rows, cols, longest);
+    for (Lane& l : call.lanes) {
+        if (l.f_end == l.f_begin) continue;
+        if ((rc = call.use(l))) return rc;
+        API_CUDA(dcmt::generic_configure(), "kernel attribute setup");
+        API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
+        if (flagged && (rc = pinned_flags(nullptr, (size_t)(l.f_end - l.f_begin), &l.h_flags))) return rc;
+    }
+    auto do_chunk = [&](Lane& l, int f0, int nf, const CompletionCall& c2, int hc2) -> int {
+        int rc2;
+        cudaStream_t st = l.hs->s[l.slot];
+        l.slot = (l.slot + 1) % kHostStreams;
+        const bool flags2 = flagged && c2.flags == DCMT_PATH_RANK;
+        const size_t px = fpix * hc2;
+        const size_t bytes = carve_bytes(cloud_bytes * hc2, 1) + carve_bytes((size_t)hc2, sizeof(int32_t)) + 2 * carve_bytes(bgr_row * rows * hc2, 1) +
+                             (c.disp ? 2 : 1) * carve_bytes(px, sizeof(float)) + carve_bytes((size_t)hc2 * DCMT_STATS_STRIDE, sizeof(int32_t)) +
+                             (flags2 ? carve_bytes((size_t)hc2, sizeof(int32_t)) : 0) + chain_ws_bytes(c2, hc2, c.step);
+        Arena* ar = nullptr;
+        if ((rc2 = arena_acquire(st, bytes, &ar))) return rc2;  // stream order protects reuse by the chunk 3 steps later
+        float* d_pts = carve<float>(ar, (size_t)c.max_points * 4 * hc2);
+        int32_t* d_counts = c.counts ? carve<int32_t>(ar, (size_t)hc2) : nullptr;
+        uint8_t* d_left = carve<uint8_t>(ar, bgr_row * rows * hc2);
+        uint8_t* d_right = carve<uint8_t>(ar, bgr_row * rows * hc2);
+        float* d_depth = carve<float>(ar, px);
+        float* d_disp = c.disp ? carve<float>(ar, px) : nullptr;
+        int32_t* d_stats = carve<int32_t>(ar, (size_t)hc2 * DCMT_STATS_STRIDE);
+        int32_t* d_flags = flags2 ? carve<int32_t>(ar, (size_t)hc2) : nullptr;
+        if ((rc2 = arena_ok(ar))) return rc2;
+        const float* h_pts = c.points ? c.points + (size_t)f0 * c.cloud_stride * 4 : nullptr;
+        if (c.counts) {
+            API_CUDA(cudaMemcpyAsync(d_counts, c.counts + f0, (size_t)nf * sizeof(int32_t), cudaMemcpyHostToDevice, st), "host to device copy");
+            for (int i = 0; i < nf; ++i)
+                if (c.counts[f0 + i] > 0)
+                    API_CUDA(cudaMemcpyAsync(d_pts + (size_t)i * c.max_points * 4, h_pts + (size_t)i * c.cloud_stride * 4, (size_t)c.counts[f0 + i] * 16,
+                                             cudaMemcpyHostToDevice, st),
+                             "host to device copy");
+        } else if (cloud_bytes > 0 &&
+                   (rc2 = copy_frames_h2d(d_pts, cloud_bytes, h_pts, c.cloud_stride * 16, c.cloud_stride * 16, cloud_bytes, 1, nf, st))) {
+            return rc2;
+        }
+        if ((rc2 = copy_frames_h2d(d_left, bgr_row, c.left + (size_t)f0 * c.bgr_fstride, c.bgr_pitch, c.bgr_fstride, bgr_row, rows, nf, st)) ||
+            (rc2 = copy_frames_h2d(d_right, bgr_row, c.right + (size_t)f0 * c.bgr_fstride, c.bgr_pitch, c.bgr_fstride, bgr_row, rows, nf, st)))
+            return rc2;
+        const ChainFrames io{d_pts, d_counts, (size_t)c.max_points, d_left, d_right, bgr_row, bgr_row * rows, d_depth, d_disp,
+                             c.stats ? d_stats : nullptr, d_flags};
+        if ((rc2 = enqueue_chain(c, c2, io, nf, ar, st))) return rc2;
+        if (flags2)
+            API_CUDA(cudaMemcpyAsync(l.h_flags + (f0 - l.f_begin), d_flags, (size_t)nf * sizeof(int32_t), cudaMemcpyDeviceToHost, st), "flag readback");
+        API_CUDA(cudaMemcpyAsync(c.depth + (size_t)f0 * fpix, d_depth, fpix * nf * sizeof(float), cudaMemcpyDeviceToHost, st), "device to host copy");
+        if (c.disp)
+            API_CUDA(cudaMemcpyAsync(c.disp + (size_t)f0 * fpix, d_disp, fpix * nf * sizeof(float), cudaMemcpyDeviceToHost, st), "device to host copy");
+        if (c.stats)
+            API_CUDA(cudaMemcpyAsync(c.stats + (size_t)f0 * DCMT_STATS_STRIDE, d_stats, (size_t)nf * DCMT_STATS_STRIDE * sizeof(int32_t),
+                                     cudaMemcpyDeviceToHost, st),
+                     "device to host copy");
+        return DCMT_OK;
+    };
+    for (bool more = true; more;) {
+        more = false;
+        for (Lane& l : call.lanes) {
+            if (l.next >= l.f_end) continue;
+            more = true;
+            if ((rc = call.use(l))) return rc;
+            const int f0 = l.next, nf = std::min(hc, l.f_end - f0);
+            l.next += nf;
+            if ((rc = do_chunk(l, f0, nf, cc, hc))) return rc;
+        }
+    }
+    if ((rc = call.finish()) || !flagged) return rc;
+    CompletionCall cg = cc;
+    cg.flags = DCMT_PATH_GENERIC;
+    bool any = false;
+    if ((rc = redo_flagged(call, rows, cols, &any, [&](Lane& l, int f0, int nf, int hc2) { return do_chunk(l, f0, nf, cg, hc2); }))) return rc;
+    return any ? call.finish() : DCMT_OK;
 }
 
 // ---- evaluation: one device driver and one host driver behind every dcmt_evaluate_* entry point.  Each side is an InDesc:
@@ -1588,13 +1895,10 @@ static int check_project(const float* points, int n_points, const float* T_host,
 static int enqueue_project(const float* points, int n_points, const float* T_host, const float* P_host, int rows, int cols,
                            float* projected, float* normalized, float norm_a, float norm_b, int32_t* n_projected, cudaStream_t st) {
     Arena* ar = nullptr;
-    const size_t nk = dcmt::project_key_count(rows, cols);
-    int rc = arena_acquire(st, carve_bytes(nk, sizeof(unsigned long long)) + carve_bytes(8, sizeof(unsigned)), &ar);
+    int rc = arena_acquire(st, project_ws_bytes(rows, cols, 1), &ar);
     if (rc) return rc;
-    dcmt::ProjectWork w{carve<unsigned long long>(ar, nk), carve<unsigned>(ar, 8)};
-    if ((rc = arena_ok(ar))) return rc;
-    return cuda_rc(dcmt::project_run(points, n_points, T_host, P_host, rows, cols, projected, normalized, norm_a, norm_b, n_projected, w, st),
-                   "projection launch");
+    return enqueue_project_batch(points, nullptr, n_points, 0, 1, T_host, P_host, rows, cols, projected, normalized, norm_a, norm_b, n_projected,
+                                 ar, st);
 }
 
 int dcmt_lidar_project_f32(const float* points, int n_points, const float* T_host, const float* P_host, int rows, int cols,
@@ -1610,26 +1914,16 @@ int dcmt_lidar_project_f32(const float* points, int n_points, const float* T_hos
 int dcmt_lidar_project_batch_f32(const float* points, const int32_t* n_points_dev_or_null, int max_points, size_t cloud_stride_points,
                                  int n_clouds, const float* T_host, const float* P_host, int rows, int cols, float* projected,
                                  float* normalized, float norm_a, float norm_b, int32_t* n_projected, void* cuda_stream) {
-    if ((!points && max_points > 0) || !T_host || !P_host) return fail(DCMT_E_BADARG, "null pointer");
-    if (max_points < 0 || n_clouds < 0) return fail(DCMT_E_BADARG, "max_points %d, n_clouds %d", max_points, n_clouds);
-    if (n_clouds > 65535) return fail(DCMT_E_UNSUPPORTED, "at most 65535 clouds per call");
-    if (n_clouds > 1 && cloud_stride_points < (size_t)max_points) return fail(DCMT_E_BADARG, "cloud_stride_points %zu < max_points %d", cloud_stride_points, max_points);
-    int rc = check_planes(rows, cols, 1);
+    int rc = check_project_batch(points, max_points, cloud_stride_points, n_clouds, 65535, T_host, P_host, rows, cols);
     if (rc) return rc;
-    if ((size_t)rows * (size_t)cols > (size_t)1 << 30) return fail(DCMT_E_UNSUPPORTED, "frame larger than 2^30 pixels");
     if (points && (reinterpret_cast<uintptr_t>(points) & 15)) return fail(DCMT_E_BADARG, "points must be 16-byte aligned");
     if (n_clouds == 0) return DCMT_OK;
     if ((rc = check_device())) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
     Arena* ar = nullptr;
-    const size_t nk = dcmt::project_key_count(rows, cols) * n_clouds;
-    if ((rc = arena_acquire(st, carve_bytes(nk, sizeof(unsigned long long)) + carve_bytes(8 * (size_t)n_clouds, sizeof(unsigned)), &ar))) return rc;
-    dcmt::ProjectWork w{carve<unsigned long long>(ar, nk), carve<unsigned>(ar, 8 * (size_t)n_clouds)};
-    if ((rc = arena_ok(ar))) return rc;
-    API_CUDA(dcmt::project_run_batch(points, max_points, n_points_dev_or_null, cloud_stride_points, n_clouds, T_host, P_host, rows, cols,
-                                     projected, normalized, norm_a, norm_b, n_projected, w, st),
-             "projection launch");
-    return DCMT_OK;
+    if ((rc = arena_acquire(st, project_ws_bytes(rows, cols, n_clouds), &ar))) return rc;
+    return enqueue_project_batch(points, n_points_dev_or_null, max_points, cloud_stride_points, n_clouds, T_host, P_host, rows, cols, projected,
+                                 normalized, norm_a, norm_b, n_projected, ar, st);
 }
 
 int dcmt_lidar_project_f32_host(const float* points, int n_points, const float* T_host, const float* P_host, int rows, int cols,
@@ -1824,6 +2118,39 @@ int dcmt_stereo_refine_f32_host(const float* depth_ig, const uint8_t* left_gray,
         if (disp_out) API_CUDA(cudaMemcpyAsync(disp_out + off, d_disp, n * 4, cudaMemcpyDeviceToHost, st), "device to host copy");
     }
     return call.finish();
+}
+
+int dcmt_stereo_chain_f32(const float* points, const int32_t* n_points_or_null, int max_points, size_t cloud_stride_points, const float* T_host,
+                          const float* P_host, float norm_a, float norm_b, const uint8_t* left_bgr, const uint8_t* right_bgr, size_t bgr_pitch_bytes,
+                          size_t bgr_frame_stride_bytes, float* depth_out, float* disp_out_or_null, int rows, int cols, int n_frames, int step,
+                          int nc, int iterations, int use_superpixel, int flags, const dcmt_stereo_params* params, int32_t* stats_or_null,
+                          void* cuda_stream) {
+    return run_stereo_chain({points, n_points_or_null, max_points, cloud_stride_points, T_host, P_host, norm_a, norm_b, left_bgr, right_bgr,
+                             bgr_pitch_bytes, bgr_frame_stride_bytes, depth_out, disp_out_or_null, rows, cols, n_frames, step, nc, iterations,
+                             use_superpixel, flags, params, stats_or_null},
+                            static_cast<cudaStream_t>(cuda_stream));
+}
+
+int dcmt_stereo_chain_f32_host(const float* points, const int32_t* n_points_or_null, int max_points, size_t cloud_stride_points,
+                               const float* T_host, const float* P_host, float norm_a, float norm_b, const uint8_t* left_bgr,
+                               const uint8_t* right_bgr, size_t bgr_pitch_bytes, size_t bgr_frame_stride_bytes, float* depth_out,
+                               float* disp_out_or_null, int rows, int cols, int n_frames, int step, int nc, int iterations, int use_superpixel,
+                               int flags, const dcmt_stereo_params* params, int32_t* stats_or_null) {
+    return run_stereo_chain_host({points, n_points_or_null, max_points, cloud_stride_points, T_host, P_host, norm_a, norm_b, left_bgr, right_bgr,
+                                  bgr_pitch_bytes, bgr_frame_stride_bytes, depth_out, disp_out_or_null, rows, cols, n_frames, step, nc,
+                                  iterations, use_superpixel, flags, params, stats_or_null});
+}
+
+int dcmt_stereo_chain_f32_host_multi(const float* points, const int32_t* n_points_or_null, int max_points, size_t cloud_stride_points,
+                                     const float* T_host, const float* P_host, float norm_a, float norm_b, const uint8_t* left_bgr,
+                                     const uint8_t* right_bgr, size_t bgr_pitch_bytes, size_t bgr_frame_stride_bytes, float* depth_out,
+                                     float* disp_out_or_null, int rows, int cols, int n_frames, int step, int nc, int iterations,
+                                     int use_superpixel, int flags, const dcmt_stereo_params* params, int32_t* stats_or_null,
+                                     const int* devices_or_null, int n_devices) {
+    return run_stereo_chain_host({points, n_points_or_null, max_points, cloud_stride_points, T_host, P_host, norm_a, norm_b, left_bgr, right_bgr,
+                                  bgr_pitch_bytes, bgr_frame_stride_bytes, depth_out, disp_out_or_null, rows, cols, n_frames, step, nc,
+                                  iterations, use_superpixel, flags, params, stats_or_null},
+                                 devices_or_null, n_devices, true);
 }
 
 int dcmt_measurement_derivatives_f32(const float* value, float* dx, float* dy, int rows, int cols, int n_frames,

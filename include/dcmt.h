@@ -348,6 +348,56 @@ DCMT_API int dcmt_stereo_refine_f32_host(const float *depth_ig, const uint8_t *l
                                          float *depth_out, float *disp_out_or_null, int rows, int cols, int n_frames,
                                          const dcmt_stereo_params *params);
 
+/* (g1) the stereo program's per-frame chain in one call -- withSuperPixels (main_sl.cpp:435-563) and :1162-1253: the
+ * Velodyne clouds and the BGR stereo pairs as read in, refined float32 depth (and the disparity) out.
+ *   - Meaning: depth, disparity and stats are byte-equal, on every form, chunking and device list, to
+ *       1. dcmt_lidar_project_batch_f32(points, n_points, max_points, cloud_stride_points, n_frames, T, P, rows, cols, NULL,
+ *          normalized, norm_a, norm_b, NULL) -- the reference normalises to (0, 80);
+ *       2. dcmt_slic_bgr_u8c3(left_bgr, rows, cols, n_frames, step, nc, iterations, labels, NULL);
+ *       3. dcmt_interpolate_with_superpixels_ex_f32(normalized, labels, dcmt_slic_center_count(rows, cols, step), dense, rows,
+ *          cols, 0, 0, n_frames, use_superpixel, flags', stats) with flags' = DCMT_PATH_GENERIC for DCMT_PATH_GENERIC and
+ *          DCMT_PATH_RANK for DCMT_PATH_AUTO / DCMT_PATH_RANK;
+ *       4. dcmt_bgr2gray_u8 of the left and of the right frames;
+ *       5. dcmt_stereo_refine_f32(dense, left_gray, right_gray, depth_out, disp_out_or_null, rows, cols, n_frames, params).
+ *     Nothing in between leaves the device.  A host caller moves the clouds (16 bytes a point) and 6 bytes per pixel in and
+ *     4 (8 with the disparity) out, where the five host calls move 45.5 bytes per pixel at 352 x 1216 with 120 000 points.
+ *   - Clouds: cloud c holds n_points[c] points (x, y, z, intensity float32) at points + c * cloud_stride_points * 4 floats;
+ *     n_points NULL means max_points each.  The device form takes a DEVICE n_points array bounded by max_points, as
+ *     dcmt_lidar_project_batch_f32, and 16-byte aligned points; the host forms take a HOST array, each count in
+ *     [0, max_points], and points at any address.  T (4x4) and P (3x4) are host, row-major, one pair for the call.
+ *   - Frames: left and right BGR (CV_8UC3) share one pitch and one frame stride in bytes (0 = dense), so a cv::Mat ROI is
+ *     passed as it is.  depth_out, disp_out_or_null: dense n_frames x rows x cols float32.  stats: DCMT_STATS_STRIDE int32 per
+ *     frame from the completion (stats[3]: 2 on the dictionary path, 0 on the generic pipeline).
+ *   - Arguments are checked before any device work and before any read of the caller's buffers other than `params`; the
+ *     host forms then read n_points to check it: the projection's checks (max_points >= 0, cloud_stride_points >= max_points for more
+ *     than one frame, frames of at most 2^30 pixels), the pointers, flags (DCMT_PATH_FUSED is DCMT_E_BADARG: the normalised
+ *     projection is not strict q8), params->num_iterations >= 0, SLIC's limits, at most 65535 rows, the BGR geometry, and no
+ *     overlap of either output with the other or with any input.  There is no limit on n_frames: the batch runs in chunks.
+ *   - Paths: DCMT_PATH_AUTO / _RANK run the completion on the dictionary path; frames it cannot serve (more than 32 768
+ *     valid pixels, or a NaN) are found by one read-back of per-frame flags (one synchronisation) and redone through the
+ *     chain with the completion on the generic pipeline.  DCMT_PATH_GENERIC never synchronises.
+ *   - use_superpixel == 0: unguided completion, SLIC is skipped (the left frame is still read for gray).
+ * _host: host pointers, chunks of frames flow H2D -> chain -> D2H on three streams; _host_multi: the same over several
+ * devices as for dcmt_img_completion_f32_host_multi. */
+DCMT_API int dcmt_stereo_chain_f32(const float *points, const int32_t *n_points_or_null, int max_points, size_t cloud_stride_points,
+                                   const float *T_host, const float *P_host, float norm_a, float norm_b, const uint8_t *left_bgr,
+                                   const uint8_t *right_bgr, size_t bgr_pitch_bytes, size_t bgr_frame_stride_bytes, float *depth_out,
+                                   float *disp_out_or_null, int rows, int cols, int n_frames, int step, int nc, int iterations,
+                                   int use_superpixel, int flags, const dcmt_stereo_params *params, int32_t *stats_or_null,
+                                   void *cuda_stream);
+DCMT_API int dcmt_stereo_chain_f32_host(const float *points, const int32_t *n_points_or_null, int max_points, size_t cloud_stride_points,
+                                        const float *T_host, const float *P_host, float norm_a, float norm_b, const uint8_t *left_bgr,
+                                        const uint8_t *right_bgr, size_t bgr_pitch_bytes, size_t bgr_frame_stride_bytes, float *depth_out,
+                                        float *disp_out_or_null, int rows, int cols, int n_frames, int step, int nc, int iterations,
+                                        int use_superpixel, int flags, const dcmt_stereo_params *params, int32_t *stats_or_null);
+DCMT_API int dcmt_stereo_chain_f32_host_multi(const float *points, const int32_t *n_points_or_null, int max_points,
+                                              size_t cloud_stride_points, const float *T_host, const float *P_host, float norm_a,
+                                              float norm_b, const uint8_t *left_bgr, const uint8_t *right_bgr, size_t bgr_pitch_bytes,
+                                              size_t bgr_frame_stride_bytes, float *depth_out, float *disp_out_or_null, int rows,
+                                              int cols, int n_frames, int step, int nc, int iterations, int use_superpixel, int flags,
+                                              const dcmt_stereo_params *params, int32_t *stats_or_null, const int *devices_or_null,
+                                              int n_devices);
+
 /* the individual stereo functions, for callers that use them one by one (device pointers) */
 /* (a4) calculateMeasuementDerivatives, main_sl.cpp:715-745: value plane -> dx, dy planes */
 DCMT_API int dcmt_measurement_derivatives_f32(const float *value, float *dx, float *dy, int rows, int cols,

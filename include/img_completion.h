@@ -344,6 +344,31 @@ inline void stereo_refine(const MatView& depth_ig, const MatView& left_gray, con
                                       cols, 1, &p));
 }
 
+// withSuperPixels (main_sl.cpp:435-563) and :1162-1253 in one call (dcmt_stereo_chain_f32_host): one Velodyne cloud (the .bin
+// payload, n_points x 4 floats) and the BGR stereo pair as read (CV_8UC3 views with one step) -> the refined depth and,
+// optionally, the disparity (continuous CV_32FC1 views).  cv::normalize(0, 80), SLIC with `step` (the reference's int) and
+// `nc`, interpolate_with_superpixels, cvtColor(BGR2GRAY) of both images and the refinement run on the device.  T (4x4) and
+// P (3x4) are row-major, as for project_lidar: from Eigen pass `Eigen::Matrix<float, 4, 4, Eigen::RowMajor>(T).data()`.
+// `params` defaults to the main_sl.cpp literals (dcmt_stereo_params_default).
+inline void stereo_chain(const float* points, int n_points, const float* T_row_major, const float* P_row_major, const MatView& left_bgr,
+                         const MatView& right_bgr, MatView& depth, int step, int nc = 40, MatView* disparity = nullptr,
+                         const dcmt_stereo_params* params = nullptr, int use_superpixel = 1, int path = DCMT_PATH_AUTO) {
+    const int rows = left_bgr.rows, cols = left_bgr.cols;
+    if (right_bgr.rows != rows || right_bgr.cols != cols || depth.rows != rows || depth.cols != cols || !depth.data ||
+        (disparity && (disparity->rows != rows || disparity->cols != cols || !disparity->data)))
+        throw std::invalid_argument("dcmt: stereo_chain needs same-shaped, allocated views");
+    if (left_bgr.step != right_bgr.step) throw std::invalid_argument("dcmt: stereo_chain needs left and right images with one step");
+    if (depth.step != (size_t)cols * 4 || (disparity && disparity->step != (size_t)cols * 4))
+        throw std::invalid_argument("dcmt: stereo_chain needs continuous depth and disparity views");
+    dcmt_stereo_params p;
+    if (params) p = *params;
+    else dcmt_stereo_params_default(&p);
+    check(dcmt_stereo_chain_f32_host(points, nullptr, n_points, (size_t)n_points, T_row_major, P_row_major, 0.0f, 80.0f,
+                                     static_cast<const uint8_t*>(left_bgr.data), static_cast<const uint8_t*>(right_bgr.data), left_bgr.step, 0,
+                                     static_cast<float*>(depth.data), disparity ? static_cast<float*>(disparity->data) : nullptr, rows, cols, 1,
+                                     step, nc, 10, use_superpixel, path, &p, nullptr));
+}
+
 }  // namespace dcmt
 
 #ifdef DCMT_HAVE_OPENCV
@@ -429,6 +454,21 @@ inline void interpolate_with_superpixels_bgr_to_u16(const cv::Mat& bgr, const cv
     MatView d = view_of(out);
     interpolate_with_superpixels_bgr_to_u16(view_of(bgr), view_of(sparse_u16), d, step, nc, use_superpixel);
     dense_u16 = out;
+}
+
+// withSuperPixels + main_sl.cpp:1162-1253 on the Mats as read: CV_8UC3 left and right images (ROIs too) with equal steps; the
+// depth and the disparity (when asked for) come back as fresh continuous CV_32FC1 matrices.  Other types or steps throw.
+inline void stereo_chain(const float* points, int n_points, const float* T_row_major, const float* P_row_major, const cv::Mat& left_bgr,
+                         const cv::Mat& right_bgr, cv::Mat& depth, int step, int nc = 40, cv::Mat* disparity = nullptr,
+                         const dcmt_stereo_params* params = nullptr, int use_superpixel = 1) {
+    CV_Assert(left_bgr.type() == CV_8UC3 && right_bgr.type() == CV_8UC3 && view_of(left_bgr).step == view_of(right_bgr).step);
+    cv::Mat out(left_bgr.rows, left_bgr.cols, CV_32FC1), disp;
+    if (disparity) disp.create(left_bgr.rows, left_bgr.cols, CV_32FC1);
+    MatView d = view_of(out), v = view_of(disp);
+    stereo_chain(points, n_points, T_row_major, P_row_major, view_of(left_bgr), view_of(right_bgr), d, step, nc, disparity ? &v : nullptr,
+                 params, use_superpixel);
+    depth = out;
+    if (disparity) *disparity = disp;
 }
 }  // namespace dcmt
 
