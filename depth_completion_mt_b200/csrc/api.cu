@@ -58,6 +58,7 @@ struct Arena {
     char* base = nullptr;
     size_t cap = 0, used = 0;
     bool overflow = false;  // a carve() went past cap since the last acquire: the caller must not launch anything
+    bool counting = false;  // sizes a workspace: carve() adds up what it takes and hands out no memory (acquire_carved)
 };
 std::mutex g_mu;
 std::map<std::pair<int, cudaStream_t>, Arena> g_arenas;
@@ -88,10 +89,14 @@ int arena_acquire(cudaStream_t st, size_t bytes, Arena** out) {
 }
 
 // Bounds-checked: a request past the end of the arena sets `overflow` and returns the arena base (valid memory that
-// must not be used); every caller checks arena_ok() before launching.
+// must not be used); acquire_carved checks it before anything is launched.
 template <class T>
 T* carve(Arena* a, size_t count) {
     const size_t bytes = (count * sizeof(T) + 255) & ~size_t(255);
+    if (a->counting) {
+        a->used += bytes;
+        return nullptr;
+    }
     if (a->used + bytes > a->cap) {
         a->overflow = true;
         return reinterpret_cast<T*>(a->base);
@@ -100,10 +105,18 @@ T* carve(Arena* a, size_t count) {
     a->used += bytes;
     return p;
 }
-int arena_ok(const Arena* a) {
-    return a->overflow ? fail(DCMT_E_NOMEM, "internal: workspace arena of %zu bytes is too small for this call", a->cap) : DCMT_OK;
+
+// The workspace of one step of a call, in the arena of `st`: carve_ws(Arena*) runs once on a counting arena to size it, then
+// on the stream's arena for real.  The size comes from the code that lays the workspace out, so the two cannot disagree.
+template <class Carve>
+int acquire_carved(cudaStream_t st, Carve&& carve_ws) {
+    Arena count, *ar = nullptr;
+    count.counting = true;
+    carve_ws(&count);
+    if (int rc = arena_acquire(st, count.used, &ar)) return rc;
+    carve_ws(ar);
+    return ar->overflow ? fail(DCMT_E_NOMEM, "internal: workspace arena of %zu bytes is too small for this call", ar->cap) : DCMT_OK;
 }
-size_t carve_bytes(size_t count, size_t elem) { return (count * elem + 255) & ~size_t(255); }
 
 long env_long(const char* name) {
     const char* s = getenv(name);
@@ -128,13 +141,6 @@ int chunk_frames(int rows, int cols, int n_frames, bool fused) {
     long c = nchunks > 0 ? (n_frames + nchunks - 1) / nchunks : 1;
     if (c < 1) c = 1;
     return (int)c;
-}
-
-size_t generic_ws_bytes(int rows, int cols, int chunk, bool bilateral) {
-    const size_t fpix = (size_t)rows * cols;
-    size_t b = 2 * carve_bytes(fpix * chunk, sizeof(float)) + carve_bytes(chunk, sizeof(dcmt::FrameCounters));
-    if (bilateral) b += carve_bytes(2 * (size_t)chunk, sizeof(unsigned)) + carve_bytes(dcmt::generic_lut_floats() * chunk, sizeof(float));
-    return b;
 }
 
 bool overlaps(const void* a, size_t an, const void* b, size_t bn) {
@@ -253,10 +259,23 @@ struct OutDesc {
     }
 };
 
-// The fused path's buffers for chunks of `chunk` frames, next to the generic pipeline's scratch (fix-up planes and
-// counters, shared): the uint16 intermediate plane and its column keys, the tile flags of the guided front and -- on
-// DCMT_PATH_RANK -- the per-frame dictionary, its sizes and the code plane (rank_f32.cu).  fused_ws_bytes() sizes what
-// carve_fused() takes, the tile flags for 8 x 8 tiles: a bound for every tile choice.
+// The generic pipeline's scratch for launches of up to `chunk` frames, in the workspace fields of a GenericChunk: two float
+// planes, the per-frame counters and, for the bilateral blur, its min / max words and range LUTs.  The fused path shares
+// the planes and counters (fix-ups).
+dcmt::GenericChunk carve_generic(Arena* ar, int rows, int cols, int chunk, bool bilateral) {
+    const size_t px = (size_t)rows * cols * chunk;
+    dcmt::GenericChunk g{};
+    g.w1 = carve<float>(ar, px);
+    g.w2 = carve<float>(ar, px);
+    g.ctr = carve<dcmt::FrameCounters>(ar, chunk);
+    g.minmax = bilateral ? carve<unsigned>(ar, 2 * (size_t)chunk) : nullptr;
+    g.lut = bilateral ? carve<float>(ar, dcmt::generic_lut_floats() * chunk) : nullptr;
+    return g;
+}
+
+// The fused path's buffers for launches of up to `chunk` frames, next to the generic scratch `g`: the uint16 intermediate
+// plane and its column keys, the tile flags of the guided front and -- on DCMT_PATH_RANK -- the per-frame dictionary, its
+// sizes and the code plane (rank_f32.cu).
 struct FusedWork {
     dcmt::Q8Plan p{};
     int* tile_flags = nullptr;
@@ -267,17 +286,7 @@ struct FusedWork {
 
 size_t pad8(int cols) { return ((size_t)cols + 7) / 8 * 8; }
 
-size_t fused_ws_bytes(int rows, int cols, int chunk, bool guided, bool rank) {
-    const size_t mp = pad8(cols);
-    size_t b = carve_bytes((size_t)rows * mp * chunk, sizeof(uint16_t)) + 2 * carve_bytes(mp * chunk, sizeof(uint32_t));
-    if (guided) b += carve_bytes(((size_t)rows / 8 + 1) * ((size_t)cols / 8 + 1) * chunk, sizeof(int));
-    if (rank)
-        b += carve_bytes((size_t)dcmt::kRankMaxValid * chunk, sizeof(float)) + carve_bytes((size_t)chunk, sizeof(int)) +
-             carve_bytes((size_t)rows * mp * chunk, sizeof(uint16_t));
-    return b;
-}
-
-FusedWork carve_fused(Arena* ar, int rows, int cols, int chunk, bool guided, bool rank, float* w1, float* w2, dcmt::FrameCounters* ctr) {
+FusedWork carve_fused(Arena* ar, int rows, int cols, int chunk, bool guided, bool rank, const dcmt::GenericChunk& g) {
     FusedWork w;
     dcmt::Q8Plan& p = w.p;
     p.rows = rows;
@@ -288,9 +297,9 @@ FusedWork carve_fused(Arena* ar, int rows, int cols, int chunk, bool guided, boo
     p.mid = carve<uint16_t>(ar, (size_t)rows * p.mid_pitch * chunk);
     p.col_first = carve<uint32_t>(ar, (size_t)p.mid_pitch * chunk);
     p.col_last = carve<uint32_t>(ar, (size_t)p.mid_pitch * chunk);
-    p.ctr = ctr;
-    p.w1 = w1;
-    p.w2 = w2;
+    p.ctr = g.ctr;
+    p.w1 = g.w1;
+    p.w2 = g.w2;
     if (guided) w.tile_flags = carve<int>(ar, dcmt::q8_guided_tile_flags(rows, cols, p.th, p.tw, chunk));
     if (rank) {
         w.lut = carve<float>(ar, (size_t)dcmt::kRankMaxValid * chunk);
@@ -303,44 +312,59 @@ FusedWork carve_fused(Arena* ar, int rows, int cols, int chunk, bool guided, boo
     return w;
 }
 
-// device workspace of a completion call of n_frames frames (element sizes of its input and output)
-size_t completion_ws_bytes(const CompletionCall& cc, int n_frames, size_t in_elem, size_t out_elem) {
-    const bool fused = fused_applies(cc);
-    const int chunk = chunk_frames(cc.rows, cc.cols, n_frames, fused);
-    const size_t b = generic_ws_bytes(cc.rows, cc.cols, chunk, cc.blur == DCMT_BLUR_BILATERAL);
-    if (fused) return b + fused_ws_bytes(cc.rows, cc.cols, chunk, cc.guided, cc.flags == DCMT_PATH_RANK);
-    // the generic pipeline reads and writes float32: a plane in front of it for uint16 input, one behind it for uint16 output
-    const size_t plane = carve_bytes((size_t)cc.rows * cc.cols * chunk, sizeof(float));
-    return b + (in_elem == sizeof(uint16_t) ? plane : 0) + (out_elem == sizeof(uint16_t) ? plane : 0);
+// The workspace of a completion pass over up to `frames` frames, in launches of up to `chunk` frames: the generic scratch,
+// then the fused path's buffers or -- the generic pipeline reads and writes float32 -- a plane in front of it for uint16
+// input and one behind it for uint16 output.
+struct CompletionWork {
+    bool fused;
+    int chunk;
+    dcmt::GenericChunk g;
+    FusedWork f;
+    float *conv, *staged;
+};
+
+CompletionWork carve_completion(Arena* ar, const CompletionCall& cc, int frames, bool u16_in, bool u16_out) {
+    CompletionWork w{};
+    w.fused = fused_applies(cc);
+    w.chunk = chunk_frames(cc.rows, cc.cols, frames, w.fused);
+    w.g = carve_generic(ar, cc.rows, cc.cols, w.chunk, cc.blur == DCMT_BLUR_BILATERAL);
+    const size_t px = (size_t)cc.rows * cc.cols * w.chunk;
+    if (w.fused) w.f = carve_fused(ar, cc.rows, cc.cols, w.chunk, cc.guided, cc.flags == DCMT_PATH_RANK, w.g);
+    w.conv = !w.fused && u16_in ? carve<float>(ar, px) : nullptr;
+    w.staged = !w.fused && u16_out ? carve<float>(ar, px) : nullptr;
+    return w;
 }
 
-// Enqueue n_frames through the pipeline; every pointer is a device pointer, the workspace is carved from `ar`.
-// Never synchronises.  On the fused path `redo_flags` (device, one int32 per frame, optional) receives 1 for
-// frames that turned out not to be strict q8: their output is NOT valid and the caller must redo them with
-// DCMT_PATH_GENERIC.
+// Whether a completion pass reports the frames it did not serve ("not served" flags): float32 input on the fused kernels,
+// except in the debugging calls (copy only, per-stage planes)
+bool writes_flags(const CompletionCall& cc, bool f32_in, bool debug) { return fused_applies(cc) && f32_in && !debug; }
+
+// The level that redoes the frames a pass at `level` did not serve: strict-q8 kernels -> dictionary (rank_f32.cu) ->
+// generic pipeline; -1 below DCMT_PATH_GENERIC and DCMT_PATH_FUSED
+int path_below(int level) {
+    return level == DCMT_PATH_AUTO ? DCMT_PATH_RANK : level == DCMT_PATH_RANK ? DCMT_PATH_GENERIC : -1;
+}
+
+// Enqueue n_frames through the pipeline on the workspace `w` (carve_completion for at least n_frames frames); every pointer
+// is a device pointer.  Never synchronises.  On the fused path `redo_flags` (device, one int32 per frame, optional) receives
+// 1 for frames that turned out not to be strict q8: their output is NOT valid and the caller must redo them one level down.
+// `stages` (the per-stage planes of DCMT_PATH_GENERIC calls) and `stage_mask` are passed to the generic pipeline.
 //
 // uint16 input is strict q8 by construction (the drivers map every path but DCMT_PATH_GENERIC to DCMT_PATH_FUSED): the
 // fused kernels read it directly and nothing is validated or redone; shapes the fused kernels do not serve get a
 // convertTo(CV_32F, 1/256) (main.cpp:79) into a workspace plane in front of the generic pipeline.  uint16 output: the
 // fused tail stores it directly; the generic pipeline writes a float workspace plane that depth_to_u16 converts.
-int enqueue_completion(const CompletionCall& cc, const InDesc& in, const int32_t* labels, const OutDesc& out, int n_frames,
-                       int32_t* stats, int32_t* redo_flags, float* stages, uint32_t* stage_mask, Arena* ar, cudaStream_t st) {
+int enqueue_completion(const CompletionCall& cc, const CompletionWork& w, const InDesc& in, const int32_t* labels, const OutDesc& out,
+                       int n_frames, int32_t* stats, int32_t* redo_flags, float* stages, uint32_t* stage_mask, cudaStream_t st) {
     const int rows = cc.rows, cols = cc.cols;
-    const bool bilateral = cc.blur == DCMT_BLUR_BILATERAL;
-    const bool fused = fused_applies(cc) && !stages;
-    const int chunk = chunk_frames(rows, cols, n_frames, fused);
+    // launches never take more frames than the workspace holds, whatever chunk sizes the environment sets
+    const int chunk = std::min(chunk_frames(rows, cols, n_frames, w.fused), w.chunk);
     const size_t fpix = (size_t)rows * cols;
-    float* w1 = carve<float>(ar, fpix * chunk);
-    float* w2 = carve<float>(ar, fpix * chunk);
-    dcmt::FrameCounters* ctr = carve<dcmt::FrameCounters>(ar, chunk);
-    unsigned* mm = bilateral ? carve<unsigned>(ar, 2 * (size_t)chunk) : nullptr;
-    float* lut = bilateral ? carve<float>(ar, dcmt::generic_lut_floats() * chunk) : nullptr;
-    if (fused) {
+    if (w.fused) {
         // DCMT_PATH_RANK: float32 frames through the per-frame dictionary (rank_f32.cu) in front of the same kernels
         const bool rank = cc.flags == DCMT_PATH_RANK;
-        const FusedWork w = carve_fused(ar, rows, cols, chunk, cc.guided, rank, w1, w2, ctr);
-        const dcmt::Q8Plan& p = w.p;
-        if (int rc = arena_ok(ar)) return rc;
+        const FusedWork& fw = w.f;
+        const dcmt::Q8Plan& p = fw.p;
         if (rank) API_CUDA(dcmt::rank_configure(), "kernel attribute setup");
         for (int f0 = 0; f0 < n_frames; f0 += chunk) {
             const int nf = n_frames - f0 < chunk ? n_frames - f0 : chunk;
@@ -350,15 +374,15 @@ int enqueue_completion(const CompletionCall& cc, const InDesc& in, const int32_t
             InDesc fin = in.frames_from((size_t)f0);
             if (rank) {
                 API_CUDA(dcmt::q8_zero_counters(p, nf, st), "counter setup launch");
-                API_CUDA(dcmt::rank_build(fin.f, fin.pitch, fin.fstride, rows, cols, nf, w.lut, w.lut_count, w.codes, (size_t)p.mid_pitch,
-                                          ctr, st),
+                API_CUDA(dcmt::rank_build(fin.f, fin.pitch, fin.fstride, rows, cols, nf, fw.lut, fw.lut_count, fw.codes, (size_t)p.mid_pitch,
+                                          p.ctr, st),
                          "dictionary launch");
-                fin = InDesc{nullptr, w.codes, (size_t)p.mid_pitch, (size_t)p.mid_pitch * rows};
+                fin = InDesc{nullptr, fw.codes, (size_t)p.mid_pitch, (size_t)p.mid_pitch * rows};
             }
             const int validate = fin.f && cc.flags != DCMT_PATH_FUSED;
             if (cc.guided)
                 API_CUDA(dcmt::q8_run_guided_front(p, fin.f, fin.u, fin.pitch, fin.fstride, labels + (size_t)f0 * fpix, cc.n_clusters, nf,
-                                                   validate, w.tile_flags, st),
+                                                   validate, fw.tile_flags, st),
                          "fused guided front launch");
             else
                 API_CUDA(dcmt::q8_run_front(p, fin.f, fin.u, fin.pitch, fin.fstride, nf, validate, st), "fused front launch");
@@ -377,16 +401,13 @@ int enqueue_completion(const CompletionCall& cc, const InDesc& in, const int32_t
         }
         return DCMT_OK;
     }
-    float* conv = in.u ? carve<float>(ar, fpix * chunk) : nullptr;
-    float* staged = out.u ? carve<float>(ar, fpix * chunk) : nullptr;
-    if (int rc = arena_ok(ar)) return rc;
     for (int f0 = 0; f0 < n_frames; f0 += chunk) {
         const int nf = n_frames - f0 < chunk ? n_frames - f0 : chunk;
         const InDesc i = in.frames_from((size_t)f0);
-        dcmt::GenericChunk c{};
-        if (conv) {
-            API_CUDA(dcmt::q8_convert_u16(i.u, i.pitch, i.fstride, conv, rows, cols, nf, st), "uint16 conversion launch");
-            c.in = conv;
+        dcmt::GenericChunk c = w.g;
+        if (w.conv) {
+            API_CUDA(dcmt::q8_convert_u16(i.u, i.pitch, i.fstride, w.conv, rows, cols, nf, st), "uint16 conversion launch");
+            c.in = w.conv;
             c.in_pitch = (size_t)cols;
             c.in_fstride = fpix;
         } else {
@@ -398,25 +419,19 @@ int enqueue_completion(const CompletionCall& cc, const InDesc& in, const int32_t
         c.n_clusters = cc.n_clusters;
         c.guided = cc.guided;
         const OutDesc o = out.frames_from((size_t)f0);
-        c.out = staged ? staged : o.f;
-        c.out_pitch = staged ? (size_t)cols : o.pitch;
-        c.out_fstride = staged ? fpix : o.fstride;
+        c.out = w.staged ? w.staged : o.f;
+        c.out_pitch = w.staged ? (size_t)cols : o.pitch;
+        c.out_fstride = w.staged ? fpix : o.fstride;
         c.rows = rows;
         c.cols = cols;
         c.n_frames = nf;
         c.blur = cc.blur;
-        c.w1 = w1;
-        c.w2 = w2;
-        c.ctr = ctr;
-        c.minmax = mm;
-        c.lut = lut;
         c.stats = stats ? stats + (size_t)f0 * DCMT_STATS_STRIDE : nullptr;
         c.stages = stages;
         c.stage_mask = stage_mask;
-        c.skip_front = false;
         API_CUDA(dcmt::generic_run_chunk(c, st), "generic pipeline launch");
-        if (staged)
-            API_CUDA(dcmt::depth_to_u16(staged, (size_t)cols, fpix, o.u, o.pitch, o.fstride, rows, cols, nf, st), "uint16 conversion launch");
+        if (w.staged)
+            API_CUDA(dcmt::depth_to_u16(w.staged, (size_t)cols, fpix, o.u, o.pitch, o.fstride, rows, cols, nf, st), "uint16 conversion launch");
     }
     return DCMT_OK;
 }
@@ -534,82 +549,86 @@ int run_completion(CompletionCall cc, InDesc in, OutDesc out, int n_frames, int3
     API_CUDA(dcmt::generic_configure(), "kernel attribute setup");
     API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
     cc.flags = input_path(in, cc.flags);
-    const bool fused = fused_applies(cc) && !stages;
-    const bool flagged = fused && in.f;  // float32 input on the fused path: frames the pass did not serve are flagged
-    Arena* ar = nullptr;
-    const size_t flag_bytes = flagged ? carve_bytes((size_t)n_frames, sizeof(int32_t)) : 0;
-    if ((rc = arena_acquire(st, completion_ws_bytes(cc, n_frames, in.elem(), out.elem()) + flag_bytes, &ar))) return rc;
-    int32_t* d_flags = flagged ? carve<int32_t>(ar, (size_t)n_frames) : nullptr;
-    if ((rc = enqueue_completion(cc, in, cc.labels, out, n_frames, stats, d_flags, stages, stage_mask, ar, st))) return rc;
-    if (!fused || cc.flags == DCMT_PATH_FUSED || cc.flags == DCMT_PATH_GENERIC) return DCMT_OK;  // DCMT_PATH_FUSED: fully asynchronous, stats[3] = -1 marks bad frames
+    const bool flagged = writes_flags(cc, in.f, stages);
+    int32_t* d_flags = nullptr;
+    CompletionWork w;
+    if ((rc = acquire_carved(st, [&](Arena* a) {
+             d_flags = flagged ? carve<int32_t>(a, (size_t)n_frames) : nullptr;
+             w = carve_completion(a, cc, n_frames, in.u, out.u);
+         })))
+        return rc;
+    if ((rc = enqueue_completion(cc, w, in, cc.labels, out, n_frames, stats, d_flags, stages, stage_mask, st))) return rc;
+    if (!flagged || path_below(cc.flags) < 0) return DCMT_OK;  // DCMT_PATH_FUSED: fully asynchronous, stats[3] = -1 marks bad frames
     // DCMT_PATH_AUTO / DCMT_PATH_RANK: read the per-frame "not served" flags back (one synchronisation per pass) and redo
-    // those frames one level down: strict-q8 kernels -> dictionary (rank_f32.cu) -> generic pipeline
+    // those frames one level down
     int32_t* h_flags = nullptr;
     if ((rc = pinned_flags(st, (size_t)n_frames, &h_flags))) return rc;
     API_CUDA(cudaMemcpyAsync(h_flags, d_flags, (size_t)n_frames * sizeof(int32_t), cudaMemcpyDeviceToHost, st), "flag readback");
     API_CUDA(cudaStreamSynchronize(st), "kernel execution");
-    for (int level = cc.flags == DCMT_PATH_AUTO ? DCMT_PATH_RANK : DCMT_PATH_GENERIC;; level = DCMT_PATH_GENERIC) {
-        cc.flags = level;
-        const bool want_flags = level == DCMT_PATH_RANK;
+    for (cc.flags = path_below(cc.flags); cc.flags >= 0; cc.flags = path_below(cc.flags)) {
+        const bool want_flags = writes_flags(cc, in.f, false);
         const std::vector<Run> runs = flagged_runs(h_flags, n_frames);
+        if (runs.empty()) break;
         for (const Run& r : runs) {
-            const int f = r.f, e = r.e;
-            // the previous pass has completed (stream synchronised): the arena is free again, but it was sized for that
-            // pass -- this one may need more (the generic pipeline: two float planes per frame of its chunk)
-            const size_t fb = want_flags ? carve_bytes((size_t)(e - f), sizeof(int32_t)) : 0;
-            if ((rc = arena_acquire(st, completion_ws_bytes(cc, e - f, in.elem(), out.elem()) + fb, &ar))) return rc;
-            int32_t* run_flags = want_flags ? carve<int32_t>(ar, (size_t)(e - f)) : nullptr;
-            if ((rc = enqueue_completion(cc, in.frames_from((size_t)f), cc.guided ? cc.labels + (size_t)f * cc.rows * cc.cols : nullptr,
-                                         out.frames_from((size_t)f), e - f, stats ? stats + (size_t)f * DCMT_STATS_STRIDE : nullptr,
-                                         run_flags, nullptr, nullptr, ar, st)))
+            const int f = r.f, n = r.e - r.f;
+            // the previous pass has completed (stream synchronised): the arena is free again, but this pass may need more (the
+            // generic pipeline: two float planes per frame of its chunk)
+            int32_t* run_flags = nullptr;
+            if ((rc = acquire_carved(st, [&](Arena* a) {
+                     run_flags = want_flags ? carve<int32_t>(a, (size_t)n) : nullptr;
+                     w = carve_completion(a, cc, n, in.u, out.u);
+                 })))
+                return rc;
+            if ((rc = enqueue_completion(cc, w, in.frames_from((size_t)f), cc.guided ? cc.labels + (size_t)f * cc.rows * cc.cols : nullptr,
+                                         out.frames_from((size_t)f), n, stats ? stats + (size_t)f * DCMT_STATS_STRIDE : nullptr, run_flags,
+                                         nullptr, nullptr, st)))
                 return rc;
             if (want_flags) {
                 // arenas are reused by the next run of this pass in stream order; the flags leave through the pinned buffer first
-                API_CUDA(cudaMemcpyAsync(h_flags + f, run_flags, (size_t)(e - f) * sizeof(int32_t), cudaMemcpyDeviceToHost, st), "flag readback");
+                API_CUDA(cudaMemcpyAsync(h_flags + f, run_flags, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st), "flag readback");
                 API_CUDA(cudaStreamSynchronize(st), "kernel execution");
             }
         }
-        if (level == DCMT_PATH_GENERIC || runs.empty()) break;
     }
     return DCMT_OK;
 }
 
 // ---- SLIC on a workspace carved from an arena the caller holds, so that the chained calls keep their staging buffers,
-// labels and completion workspace in the same arena.  slic_ws_bytes() sizes what enqueue_slic() carves for n frames: the
-// work arrays of SlicWork and, with from_bgr, the Lab frames.
-size_t slic_ws_bytes(int rows, int cols, int n, int step, bool from_bgr) {
-    int bx = 0, by = 0;
+// labels and completion workspace in the same arena: the work arrays of SlicWork for up to n frames and, with from_bgr,
+// the Lab frames
+struct SlicBuffers {
+    dcmt::SlicWork w{};
+    uint8_t* lab = nullptr;
+};
+
+SlicBuffers carve_slic(Arena* ar, int rows, int cols, int n, int step, bool from_bgr) {
+    SlicBuffers s;
     const int k = dcmt::slic_center_count(rows, cols, step);
-    const size_t nbins = dcmt::slic_bins(rows, cols, step, &bx, &by);
+    const size_t nbins = dcmt::slic_bins(rows, cols, step, &s.w.bins_x, &s.w.bins_y);
     const size_t kk = (k > 0 ? (size_t)k : 1) * n, nb = nbins * n;
-    return 2 * carve_bytes(kk * 5, sizeof(double)) + carve_bytes(kk * 6, sizeof(unsigned long long)) + carve_bytes(nb + n, sizeof(int)) +
-           carve_bytes(nb, sizeof(int)) + carve_bytes(kk, sizeof(int)) + (from_bgr ? carve_bytes((size_t)rows * cols * 3 * n, 1) : 0);
+    s.w.centers = carve<double>(ar, kk * 5);
+    s.w.sums = carve<unsigned long long>(ar, kk * 6);
+    s.w.bin_count = carve<int>(ar, nb + n);
+    s.w.bin_fill = carve<int>(ar, nb);
+    s.w.bin_items = carve<int>(ar, kk);
+    s.w.sorted = carve<double>(ar, kk * 5);
+    if (from_bgr) s.lab = carve<uint8_t>(ar, (size_t)rows * cols * 3 * n);
+    return s;
 }
 
-// Slic::generate_superpixels of n frames (arguments checked, 1 <= n <= 65535) into `labels` (and `centers` when given):
-// on the Lab frames `img` (dense), or, with from_bgr, on the cvtColor(COLOR_BGR2Lab) of the BGR frames `img` (pitch and
-// frame stride in bytes), made into the arena first
-int enqueue_slic(const uint8_t* img, size_t pitch, size_t fstride, bool from_bgr, int rows, int cols, int n, int step, int nc, int iterations,
-                 int32_t* labels, double* centers, Arena* ar, cudaStream_t st) {
+// Slic::generate_superpixels of n frames (arguments checked, 1 <= n <= 65535, at most the frames `s` was carved for) into
+// `labels` (and `centers` when given): on the Lab frames `img` (dense), or, with from_bgr, on the cvtColor(COLOR_BGR2Lab)
+// of the BGR frames `img` (pitch and frame stride in bytes), made into `s.lab` first
+int enqueue_slic(const SlicBuffers& s, const uint8_t* img, size_t pitch, size_t fstride, bool from_bgr, int rows, int cols, int n, int step,
+                 int nc, int iterations, int32_t* labels, double* centers, cudaStream_t st) {
     const int k = dcmt::slic_center_count(rows, cols, step);
-    dcmt::SlicWork w{};
-    const size_t nbins = dcmt::slic_bins(rows, cols, step, &w.bins_x, &w.bins_y);
-    const size_t kk = (k > 0 ? (size_t)k : 1) * n, nb = nbins * n;
-    w.centers = carve<double>(ar, kk * 5);
-    w.sums = carve<unsigned long long>(ar, kk * 6);
-    w.bin_count = carve<int>(ar, nb + n);
-    w.bin_fill = carve<int>(ar, nb);
-    w.bin_items = carve<int>(ar, kk);
-    w.sorted = carve<double>(ar, kk * 5);
-    uint8_t* lab = from_bgr ? carve<uint8_t>(ar, (size_t)rows * cols * 3 * n) : nullptr;
-    if (int rc = arena_ok(ar)) return rc;
     if (from_bgr) {
         const size_t lab_pitch = (size_t)cols * 3;
-        API_CUDA(dcmt::color_bgr2lab(img, pitch, fstride, lab, lab_pitch, lab_pitch * rows, rows, cols, n, st), "BGR2Lab launch");
+        API_CUDA(dcmt::color_bgr2lab(img, pitch, fstride, s.lab, lab_pitch, lab_pitch * rows, rows, cols, n, st), "BGR2Lab launch");
     }
-    API_CUDA(dcmt::slic_run(from_bgr ? lab : img, rows, cols, n, step, nc, iterations, labels, k, w, st), "SLIC launch");
+    API_CUDA(dcmt::slic_run(from_bgr ? s.lab : img, rows, cols, n, step, nc, iterations, labels, k, s.w, st), "SLIC launch");
     if (centers && k > 0)
-        API_CUDA(cudaMemcpyAsync(centers, w.centers, (size_t)k * n * 5 * sizeof(double), cudaMemcpyDeviceToDevice, st), "centre copy");
+        API_CUDA(cudaMemcpyAsync(centers, s.w.centers, (size_t)k * n * 5 * sizeof(double), cudaMemcpyDeviceToDevice, st), "centre copy");
     return DCMT_OK;
 }
 
@@ -627,18 +646,15 @@ int check_project_batch(const float* points, int max_points, size_t cloud_stride
     return DCMT_OK;
 }
 
-// the keys and min / max words of n clouds
-size_t project_ws_bytes(int rows, int cols, int n) {
-    return carve_bytes(dcmt::project_key_count(rows, cols) * n, sizeof(unsigned long long)) + carve_bytes(8 * (size_t)n, sizeof(unsigned));
+// the keys and min / max words of up to n clouds
+dcmt::ProjectWork carve_project(Arena* ar, int rows, int cols, int n) {
+    return dcmt::ProjectWork{carve<unsigned long long>(ar, dcmt::project_key_count(rows, cols) * n), carve<unsigned>(ar, 8 * (size_t)n)};
 }
 
-// the projection of n (1..65535) clouds on checked arguments and 16-byte aligned points, its work arrays carved from `ar`
-int enqueue_project_batch(const float* points, const int32_t* counts_dev, int max_points, size_t cloud_stride_points, int n, const float* T_host,
-                          const float* P_host, int rows, int cols, float* projected, float* normalized, float norm_a, float norm_b,
-                          int32_t* n_projected, Arena* ar, cudaStream_t st) {
-    const size_t nk = dcmt::project_key_count(rows, cols) * n;
-    dcmt::ProjectWork w{carve<unsigned long long>(ar, nk), carve<unsigned>(ar, 8 * (size_t)n)};
-    if (int rc = arena_ok(ar)) return rc;
+// the projection of n (1..65535, at most what `w` was carved for) clouds on checked arguments and 16-byte aligned points
+int enqueue_project_batch(const dcmt::ProjectWork& w, const float* points, const int32_t* counts_dev, int max_points, size_t cloud_stride_points,
+                          int n, const float* T_host, const float* P_host, int rows, int cols, float* projected, float* normalized, float norm_a,
+                          float norm_b, int32_t* n_projected, cudaStream_t st) {
     return cuda_rc(dcmt::project_run_batch(points, max_points, counts_dev, cloud_stride_points, n, T_host, P_host, rows, cols, projected,
                                            normalized, norm_a, norm_b, n_projected, w, st),
                    "projection launch");
@@ -658,21 +674,24 @@ int run_completion_bgr(CompletionCall cc, InDesc in, OutDesc out, int n_frames, 
     const BgrFront& fr = *cc.front;
     const size_t fpix = (size_t)cc.rows * cc.cols;
     const int chunk = chunk_frames(cc.rows, cc.cols, n_frames, fused_applies(cc));
-    const size_t bytes = completion_ws_bytes(cc, chunk, in.elem(), out.elem()) +
-                         (cc.guided ? carve_bytes(fpix * chunk, sizeof(int32_t)) + slic_ws_bytes(cc.rows, cc.cols, chunk, fr.step, true) : 0);
     for (int f0 = 0; f0 < n_frames; f0 += chunk) {
         const int nf = std::min(chunk, n_frames - f0);
-        Arena* ar = nullptr;
-        if ((rc = arena_acquire(st, bytes, &ar))) return rc;  // stream order: the previous chunk is done with it
         int32_t* labels = nullptr;
-        if (cc.guided) {
-            labels = carve<int32_t>(ar, fpix * nf);
-            if ((rc = enqueue_slic(fr.bgr + (size_t)f0 * fr.fstride, fr.pitch, fr.fstride, true, cc.rows, cc.cols, nf, fr.step, fr.nc,
-                                   fr.iterations, labels, nullptr, ar, st)))
-                return rc;
-        }
-        if ((rc = enqueue_completion(cc, in.frames_from((size_t)f0), labels, out.frames_from((size_t)f0), nf,
-                                     stats ? stats + (size_t)f0 * DCMT_STATS_STRIDE : nullptr, nullptr, nullptr, nullptr, ar, st)))
+        SlicBuffers s;
+        CompletionWork w;
+        if ((rc = acquire_carved(st, [&](Arena* a) {  // stream order: the previous chunk is done with the arena
+                 if (cc.guided) {
+                     labels = carve<int32_t>(a, fpix * chunk);
+                     s = carve_slic(a, cc.rows, cc.cols, chunk, fr.step, true);
+                 }
+                 w = carve_completion(a, cc, chunk, in.u, out.u);
+             })))
+            return rc;
+        if (cc.guided && (rc = enqueue_slic(s, fr.bgr + (size_t)f0 * fr.fstride, fr.pitch, fr.fstride, true, cc.rows, cc.cols, nf, fr.step,
+                                            fr.nc, fr.iterations, labels, nullptr, st)))
+            return rc;
+        if ((rc = enqueue_completion(cc, w, in.frames_from((size_t)f0), labels, out.frames_from((size_t)f0), nf,
+                                     stats ? stats + (size_t)f0 * DCMT_STATS_STRIDE : nullptr, nullptr, nullptr, nullptr, st)))
             return rc;
     }
     return DCMT_OK;
@@ -884,12 +903,11 @@ int run_staged(std::initializer_list<Staged*> bufs, Work&& work) {
     if (rc) return rc;
     Lane& l = call.lanes[0];
     const cudaStream_t st = l.hs->s[0];
-    size_t bytes = 0;
-    for (const Staged* b : bufs) bytes += carve_bytes(b->rows * b->row_bytes, 1);
-    Arena* stage = nullptr;
-    if ((rc = arena_acquire(l.hs->s[1], bytes, &stage))) return rc;
-    for (Staged* b : bufs) b->dev = carve<char>(stage, b->rows * b->row_bytes);
-    if ((rc = arena_ok(stage)) || (rc = call.use(l))) return rc;
+    if ((rc = acquire_carved(l.hs->s[1], [&](Arena* a) {
+             for (Staged* b : bufs) b->dev = carve<char>(a, b->rows * b->row_bytes);
+         })) ||
+        (rc = call.use(l)))
+        return rc;
     // one copy when the host rows are packed, a 2-D copy otherwise
     auto copy = [st](void* dst, size_t dst_pitch, const void* src, size_t src_pitch, const Staged* b, cudaMemcpyKind kind) {
         return dst_pitch == src_pitch ? cudaMemcpyAsync(dst, src, b->rows * b->row_bytes, kind, st)
@@ -903,24 +921,63 @@ int run_staged(std::initializer_list<Staged*> bufs, Work&& work) {
     return call.finish();
 }
 
-// Enqueues again, on the device that served them, the frames of a host-pointer call whose flag (Lane::h_flags, read back by
-// the previous pass) is set: runs of consecutive frames, cut into host chunks, redo(lane, f0, nf, chunk frames) per chunk.
-// The runs are fixed before anything is enqueued (a pass may write the flags it reads).  *any: whether a frame was flagged.
-template <class Redo>
-int redo_flagged(HostCall& call, int rows, int cols, bool* any, Redo&& redo) {
-    struct LaneRun {
-        Lane* l;
-        Run r;
+// The host chunk pipeline of a host-pointer call of n_frames frames: opens the call (devices, n_devices and multi as
+// HostCall::open takes them), gives every device a contiguous block of the frames and enqueues host chunks
+// (host_chunk_frames of the longest block) round-robin over the devices, each device's chunks on its three streams in
+// turn.  chunk(lane, stream, f0, nf, frames, level) enqueues frames [f0, f0 + nf) at path `level` in a workspace sized for
+// `frames` frames.  configure: the completion kernels' attributes are set on every device first.  flagged: every lane
+// gets a pinned flag buffer (Lane::h_flags) that the chunks of a pass fill with the frames they did not serve; after the
+// pass those frames are redone one level down (path_below), in runs of consecutive frames cut into host chunks, on the
+// device that served them, until a level leaves none.
+template <class Chunk>
+int run_host_chunks(int n_frames, int rows, int cols, const int* devices, int n_devices, bool multi, bool configure, bool flagged, int level,
+                    Chunk&& chunk) {
+    HostCall call;
+    int rc = call.open(devices, n_devices, multi);
+    if (rc) return rc;
+    call.split(n_frames);
+    int longest = 0;
+    for (Lane& l : call.lanes) longest = std::max(longest, l.f_end - l.f_begin);
+    const int hc = host_chunk_frames(rows, cols, longest);
+    for (Lane& l : call.lanes) {
+        if (l.f_end == l.f_begin) continue;
+        if ((rc = call.use(l))) return rc;
+        if (configure) {
+            API_CUDA(dcmt::generic_configure(), "kernel attribute setup");
+            API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
+        }
+        if (flagged && (rc = pinned_flags(nullptr, (size_t)(l.f_end - l.f_begin), &l.h_flags))) return rc;
+    }
+    // on the lane's next stream: stream order protects the reuse of its arena by the chunk three steps later
+    auto enqueue = [&](Lane& l, int f0, int nf, int frames, int lv) {
+        if (int rc2 = call.use(l)) return rc2;
+        const cudaStream_t st = l.hs->s[l.slot];
+        l.slot = (l.slot + 1) % kHostStreams;
+        return chunk(l, st, f0, nf, frames, lv);
     };
-    std::vector<LaneRun> runs;
-    for (Lane& l : call.lanes)
-        for (const Run& r : flagged_runs(l.h_flags, l.f_end - l.f_begin)) runs.push_back(LaneRun{&l, Run{l.f_begin + r.f, l.f_begin + r.e}});
-    *any = !runs.empty();
-    for (const LaneRun& lr : runs) {
-        if (int rc = call.use(*lr.l)) return rc;
-        const int hc = host_chunk_frames(rows, cols, lr.r.e - lr.r.f);
-        for (int f = lr.r.f; f < lr.r.e; f += hc)
-            if (int rc = redo(*lr.l, f, std::min(hc, lr.r.e - f), hc)) return rc;
+    for (bool more = true; more;) {
+        more = false;
+        for (Lane& l : call.lanes) {
+            if (l.next >= l.f_end) continue;
+            more = true;
+            const int f0 = l.next, nf = std::min(hc, l.f_end - f0);
+            l.next += nf;
+            if ((rc = enqueue(l, f0, nf, hc, level))) return rc;
+        }
+    }
+    if ((rc = call.finish())) return rc;
+    for (int lv = path_below(level); flagged && lv >= 0; lv = path_below(lv)) {
+        // the runs are fixed before anything is enqueued: a pass may write the flags it reads
+        std::vector<std::pair<Lane*, Run>> runs;
+        for (Lane& l : call.lanes)
+            for (const Run& r : flagged_runs(l.h_flags, l.f_end - l.f_begin)) runs.push_back({&l, Run{l.f_begin + r.f, l.f_begin + r.e}});
+        if (runs.empty()) break;
+        for (const auto& [l, r] : runs) {
+            const int rhc = host_chunk_frames(rows, cols, r.e - r.f);
+            for (int f = r.f; f < r.e; f += rhc)
+                if ((rc = enqueue(*l, f, std::min(rhc, r.e - f), rhc, lv))) return rc;
+        }
+        if ((rc = call.finish())) return rc;
     }
     return DCMT_OK;
 }
@@ -935,50 +992,36 @@ int run_completion_host(CompletionCall cc, InDesc in, OutDesc out, int n_frames,
     int rc = validate_completion(cc, &in, &out, n_frames);
     if (rc) return rc;
     if (n_frames == 0) return DCMT_OK;
-    HostCall call;
-    if ((rc = call.open(devices, n_devices, multi))) return rc;
-    call.split(n_frames);
     const int rows = cc.rows, cols = cc.cols;
     const size_t fpix = (size_t)rows * cols;
     const size_t in_elem = in.elem(), out_elem = out.elem();
     const size_t d_pitch = in.u ? pad8(cols) : (size_t)cols;  // elements of a device staging row of the input
     cc.flags = input_path(in, cc.flags);
-    const bool fused = fused_applies(cc) && !copy_only;
-    const bool flagged = fused && in.f;  // float32 input on the fused path: per-frame flags, read back for the redo passes
-    int longest = 0;
-    for (Lane& l : call.lanes) longest = std::max(longest, l.f_end - l.f_begin);
-    const int hc = host_chunk_frames(rows, cols, longest);
-    for (Lane& l : call.lanes) {
-        if (l.f_end == l.f_begin) continue;
-        if ((rc = call.use(l))) return rc;
-        API_CUDA(dcmt::generic_configure(), "kernel attribute setup");
-        API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
-        if (flagged && (rc = pinned_flags(nullptr, (size_t)(l.f_end - l.f_begin), &l.h_flags))) return rc;
-    }
+    const bool flagged = writes_flags(cc, in.f, copy_only);
     // labels made from BGR frames on the device (staged packed, 3 bytes per pixel) instead of copied in
     const BgrFront* front = cc.guided ? cc.front : nullptr;
     const size_t bgr_row = (size_t)cols * 3;
-    // one chunk [f0, f0 + nf) of lane l on its next stream: H2D, kernels, D2H; its arena is sized for chunks of hc2 frames
-    // of the pass: staging of input, output, labels, stats, flags and BGR frames, then the workspace (SLIC's first)
-    auto do_chunk = [&](Lane& l, int f0, int nf, const CompletionCall& c2, int hc2) -> int {
-        int rc2;
-        cudaStream_t st = l.hs->s[l.slot];
-        l.slot = (l.slot + 1) % kHostStreams;
-        const bool flags2 = flagged && fused_applies(c2);  // the generic redo pass reports no flags
-        const size_t bytes = carve_bytes((size_t)rows * d_pitch * hc2, in_elem) + carve_bytes(fpix * hc2, out_elem) +
-                             (cc.guided ? carve_bytes(fpix * hc2, sizeof(int32_t)) : 0) +
-                             carve_bytes((size_t)hc2 * DCMT_STATS_STRIDE, sizeof(int32_t)) + (flagged ? carve_bytes((size_t)hc2, sizeof(int32_t)) : 0) +
-                             (front ? carve_bytes(bgr_row * rows * hc2, 1) + slic_ws_bytes(rows, cols, hc2, front->step, true) : 0) +
-                             (copy_only ? 0 : completion_ws_bytes(c2, hc2, in_elem, out_elem));
-        Arena* ar = nullptr;
-        if ((rc2 = arena_acquire(st, bytes, &ar))) return rc2;  // stream order protects reuse by the chunk 3 steps later
-        char* d_in = carve<char>(ar, (size_t)rows * d_pitch * hc2 * in_elem);
-        char* d_out = carve<char>(ar, fpix * hc2 * out_elem);
-        int32_t* d_lab = cc.guided ? carve<int32_t>(ar, fpix * hc2) : nullptr;
-        int32_t* d_stats = carve<int32_t>(ar, (size_t)hc2 * DCMT_STATS_STRIDE);
-        int32_t* d_flags = flagged ? carve<int32_t>(ar, (size_t)hc2) : nullptr;
-        uint8_t* d_bgr = front ? carve<uint8_t>(ar, bgr_row * rows * hc2) : nullptr;
-        if ((rc2 = arena_ok(ar))) return rc2;
+    // H2D, kernels, D2H; the arena holds the staging of input, output, labels, stats, flags and BGR frames, then the workspace
+    auto chunk = [&](Lane& l, cudaStream_t st, int f0, int nf, int hc, int level) -> int {
+        CompletionCall c2 = cc;
+        c2.flags = level;
+        const bool flags2 = writes_flags(c2, in.f, copy_only);  // the generic redo pass reports no flags
+        char *d_in, *d_out;
+        int32_t *d_lab, *d_stats, *d_flags;
+        uint8_t* d_bgr;
+        SlicBuffers s{};
+        CompletionWork w{};
+        int rc2 = acquire_carved(st, [&](Arena* a) {
+            d_in = carve<char>(a, (size_t)rows * d_pitch * hc * in_elem);
+            d_out = carve<char>(a, fpix * hc * out_elem);
+            d_lab = cc.guided ? carve<int32_t>(a, fpix * hc) : nullptr;
+            d_stats = carve<int32_t>(a, (size_t)hc * DCMT_STATS_STRIDE);
+            d_flags = flagged ? carve<int32_t>(a, (size_t)hc) : nullptr;
+            d_bgr = front ? carve<uint8_t>(a, bgr_row * rows * hc) : nullptr;
+            if (front) s = carve_slic(a, rows, cols, hc, front->step, true);
+            if (!copy_only) w = carve_completion(a, c2, hc, in.u, out.u);
+        });
+        if (rc2) return rc2;
         if (front && (rc2 = copy_frames_h2d(d_bgr, bgr_row, front->bgr + (size_t)f0 * front->fstride, front->pitch, front->fstride, bgr_row,
                                             rows, nf, st)))
             return rc2;
@@ -986,8 +1029,8 @@ int run_completion_host(CompletionCall cc, InDesc in, OutDesc out, int n_frames,
         if ((rc2 = copy_frames_h2d(d_in, d_pitch * in_elem, hi.ptr(), in.pitch * in_elem, in.fstride * in_elem, cols * in_elem, rows, nf, st)))
             return rc2;
         if (front) {
-            if ((rc2 = enqueue_slic(d_bgr, bgr_row, bgr_row * rows, true, rows, cols, nf, front->step, front->nc, front->iterations, d_lab,
-                                    nullptr, ar, st)))
+            if ((rc2 = enqueue_slic(s, d_bgr, bgr_row, bgr_row * rows, true, rows, cols, nf, front->step, front->nc, front->iterations, d_lab,
+                                    nullptr, st)))
                 return rc2;
         } else if (cc.guided) {
             API_CUDA(cudaMemcpyAsync(d_lab, cc.labels + (size_t)f0 * fpix, fpix * nf * sizeof(int32_t), cudaMemcpyHostToDevice, st),
@@ -1004,8 +1047,7 @@ int run_completion_host(CompletionCall cc, InDesc in, OutDesc out, int n_frames,
                                    : InDesc{reinterpret_cast<float*>(d_in), nullptr, d_pitch, rows * d_pitch};
             const OutDesc dout = out.u ? OutDesc{nullptr, reinterpret_cast<uint16_t*>(d_out), (size_t)cols, fpix}
                                        : OutDesc{reinterpret_cast<float*>(d_out), nullptr, (size_t)cols, fpix};
-            if ((rc2 = enqueue_completion(c2, di, d_lab, dout, nf, stats ? d_stats : nullptr, flags2 ? d_flags : nullptr, nullptr, nullptr,
-                                          ar, st)))
+            if ((rc2 = enqueue_completion(c2, w, di, d_lab, dout, nf, stats ? d_stats : nullptr, flags2 ? d_flags : nullptr, nullptr, nullptr, st)))
                 return rc2;
         }
         if (flags2)
@@ -1021,33 +1063,7 @@ int run_completion_host(CompletionCall cc, InDesc in, OutDesc out, int n_frames,
                      "device to host copy");
         return DCMT_OK;
     };
-    for (bool more = true; more;) {
-        more = false;
-        for (Lane& l : call.lanes) {
-            if (l.next >= l.f_end) continue;
-            more = true;
-            if ((rc = call.use(l))) return rc;
-            const int f0 = l.next, nf = std::min(hc, l.f_end - f0);
-            l.next += nf;
-            if ((rc = do_chunk(l, f0, nf, cc, hc))) return rc;
-        }
-    }
-    if ((rc = call.finish())) return rc;
-    if (flagged && (cc.flags == DCMT_PATH_AUTO || cc.flags == DCMT_PATH_RANK)) {
-        // frames the pass did not serve (not strict q8; dictionary too small) are redone one level down -- strict-q8
-        // kernels -> dictionary (rank_f32.cu) -> generic pipeline -- in runs of consecutive frames, on the device that
-        // served them, through the same chunk pipeline
-        for (int level = cc.flags == DCMT_PATH_AUTO ? DCMT_PATH_RANK : DCMT_PATH_GENERIC;; level = DCMT_PATH_GENERIC) {
-            CompletionCall cg = cc;
-            cg.flags = level;
-            bool any = false;
-            if ((rc = redo_flagged(call, rows, cols, &any, [&](Lane& l, int f0, int nf, int hc2) { return do_chunk(l, f0, nf, cg, hc2); })))
-                return rc;
-            if (any && (rc = call.finish())) return rc;
-            if (level == DCMT_PATH_GENERIC || !any) break;
-        }
-    }
-    return DCMT_OK;
+    return run_host_chunks(n_frames, rows, cols, devices, n_devices, multi, true, flagged, cc.flags, chunk);
 }
 
 // ---- the stereo program's per-frame chain (dcmt_stereo_chain_f32*, main_sl.cpp:435-563 + :1162-1253): batched projection
@@ -1108,19 +1124,6 @@ CompletionCall chain_completion(const StereoChain& c) {
                           c.flags == DCMT_PATH_GENERIC ? DCMT_PATH_GENERIC : DCMT_PATH_RANK};
 }
 
-// Frames per chunk of the device form: the generic pipeline's 2^27 pixels (DCMT_GENERIC_CHUNK to override).  The chain
-// holds about 37 bytes per pixel (chain_ws_bytes), 4.8 GB at 313 KITTI frames.
-int chain_chunk_frames(int rows, int cols, int n_frames) { return chunk_frames(rows, cols, n_frames, false); }
-
-// the workspace of chunks of `chunk` frames: normalised plane, completed depth, the two gray planes, the projection's keys
-// and min / max words, labels, Lab frames and SLIC's work arrays (guided only), and the completion's workspace
-size_t chain_ws_bytes(const CompletionCall& cc, int chunk, int step) {
-    const size_t px = (size_t)cc.rows * cc.cols * chunk;
-    return 2 * carve_bytes(px, sizeof(float)) + 2 * carve_bytes(px, 1) + project_ws_bytes(cc.rows, cc.cols, chunk) +
-           (cc.guided ? carve_bytes(px, sizeof(int32_t)) + slic_ws_bytes(cc.rows, cc.cols, chunk, step, true) : 0) +
-           completion_ws_bytes(cc, chunk, sizeof(float), sizeof(float));
-}
-
 // Device pointers of nf frames of the chain: 16-byte aligned clouds `cloud_stride` points apart (counts: device array or
 // null), the BGR pairs, and dense outputs (disp, stats and the completion's "not served" flags optional)
 struct ChainFrames {
@@ -1133,36 +1136,51 @@ struct ChainFrames {
     int32_t *stats, *flags;
 };
 
-// one chunk (1 <= nf <= 65535 frames) of the chain on one stream, its intermediates carved from `ar` (chain_ws_bytes)
-int enqueue_chain(const StereoChain& c, const CompletionCall& cc, const ChainFrames& io, int nf, Arena* ar, cudaStream_t st) {
+// The intermediates of chunks of up to `chunk` frames: normalised plane, completed depth, the two gray planes, the
+// projection's keys and min / max words, labels, Lab frames and SLIC's work arrays (guided only), and the completion's
+// workspace.  About 37 bytes per pixel, 4.8 GB at 313 KITTI frames.
+struct ChainWork {
+    float *nrm, *dense;
+    uint8_t *gray_l, *gray_r;
+    dcmt::ProjectWork proj;
+    int32_t* labels;
+    SlicBuffers slic;
+    CompletionWork completion;
+};
+
+ChainWork carve_chain(Arena* ar, const StereoChain& c, const CompletionCall& cc, int chunk) {
+    const size_t px = (size_t)c.rows * c.cols * chunk;
+    return ChainWork{carve<float>(ar, px), carve<float>(ar, px), carve<uint8_t>(ar, px), carve<uint8_t>(ar, px), carve_project(ar, c.rows, c.cols, chunk),
+                     cc.guided ? carve<int32_t>(ar, px) : nullptr, cc.guided ? carve_slic(ar, c.rows, c.cols, chunk, c.step, true) : SlicBuffers{},
+                     carve_completion(ar, cc, chunk, false, false)};
+}
+
+// one chunk (1 <= nf <= 65535 frames, at most what `w` was carved for) of the chain on one stream
+int enqueue_chain(const StereoChain& c, const CompletionCall& cc, const ChainWork& w, const ChainFrames& io, int nf, cudaStream_t st) {
     const int rows = c.rows, cols = c.cols;
-    const size_t fpix = (size_t)rows * cols, px = fpix * nf;
-    float* nrm = carve<float>(ar, px);
-    float* dense = carve<float>(ar, px);
-    uint8_t* gray_l = carve<uint8_t>(ar, px);
-    uint8_t* gray_r = carve<uint8_t>(ar, px);
-    int32_t* labels = cc.guided ? carve<int32_t>(ar, px) : nullptr;
-    int rc = enqueue_project_batch(io.points, io.counts, c.max_points, io.cloud_stride, nf, c.T, c.P, rows, cols, nullptr, nrm, c.norm_a, c.norm_b,
-                                   nullptr, ar, st);
+    const size_t fpix = (size_t)rows * cols;
+    int rc = enqueue_project_batch(w.proj, io.points, io.counts, c.max_points, io.cloud_stride, nf, c.T, c.P, rows, cols, nullptr, w.nrm, c.norm_a,
+                                   c.norm_b, nullptr, st);
     if (rc) return rc;
     if (cc.guided &&
-        (rc = enqueue_slic(io.left, io.bgr_pitch, io.bgr_fstride, true, rows, cols, nf, c.step, c.nc, c.iterations, labels, nullptr, ar, st)))
+        (rc = enqueue_slic(w.slic, io.left, io.bgr_pitch, io.bgr_fstride, true, rows, cols, nf, c.step, c.nc, c.iterations, w.labels, nullptr, st)))
         return rc;
-    if ((rc = enqueue_completion(cc, InDesc{nrm, nullptr, (size_t)cols, fpix}, labels, OutDesc{dense, nullptr, (size_t)cols, fpix}, nf, io.stats,
-                                 io.flags, nullptr, nullptr, ar, st)))
+    if ((rc = enqueue_completion(cc, w.completion, InDesc{w.nrm, nullptr, (size_t)cols, fpix}, w.labels, OutDesc{w.dense, nullptr, (size_t)cols, fpix},
+                                 nf, io.stats, io.flags, nullptr, nullptr, st)))
         return rc;
-    API_CUDA(dcmt::stereo_bgr2gray(io.left, io.bgr_pitch, io.bgr_fstride, gray_l, cols, fpix, rows, cols, nf, st), "BGR2GRAY launch");
-    API_CUDA(dcmt::stereo_bgr2gray(io.right, io.bgr_pitch, io.bgr_fstride, gray_r, cols, fpix, rows, cols, nf, st), "BGR2GRAY launch");
+    API_CUDA(dcmt::stereo_bgr2gray(io.left, io.bgr_pitch, io.bgr_fstride, w.gray_l, cols, fpix, rows, cols, nf, st), "BGR2GRAY launch");
+    API_CUDA(dcmt::stereo_bgr2gray(io.right, io.bgr_pitch, io.bgr_fstride, w.gray_r, cols, fpix, rows, cols, nf, st), "BGR2GRAY launch");
     const dcmt_stereo_params& p = *c.prm;
-    API_CUDA(dcmt::stereo_refine(dense, gray_l, gray_r, io.depth, io.disp, rows, cols, nf, p.baseline, p.focal, p.damp_factor, p.err_clip,
+    API_CUDA(dcmt::stereo_refine(w.dense, w.gray_l, w.gray_r, io.depth, io.disp, rows, cols, nf, p.baseline, p.focal, p.damp_factor, p.err_clip,
                                  p.depth_clip, p.num_iterations, p.final_gauss, st),
              "stereo refine launch");
     return DCMT_OK;
 }
 
-// Device-pointer driver of dcmt_stereo_chain_f32: chunks of chain_chunk_frames on the caller's stream.  On the dictionary
-// path the "not served" flags of the whole call sit at the start of every chunk's arena (the same bytes each time) and are
-// read back once; those frames are redone through the chain with the completion on the generic pipeline.
+// Device-pointer driver of dcmt_stereo_chain_f32: chunks of the generic pipeline's size (chunk_frames) on the caller's
+// stream.  On the dictionary path the "not served" flags of the whole call sit at the start of every chunk's arena (the
+// same bytes each time: every chunk carves the same workspace) and are read back once; those frames are redone through
+// the chain one level down, on the generic pipeline, which reports no flags.
 int run_stereo_chain(StereoChain c, cudaStream_t st) {
     int rc = validate_stereo_chain(c, false);
     if (rc) return rc;
@@ -1172,8 +1190,8 @@ int run_stereo_chain(StereoChain c, cudaStream_t st) {
     API_CUDA(dcmt::generic_configure(), "kernel attribute setup");
     API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
     CompletionCall cc = chain_completion(c);
-    const int n = c.n_frames, chunk = chain_chunk_frames(c.rows, c.cols, n);
-    const bool flagged = cc.flags == DCMT_PATH_RANK && fused_applies(cc);
+    const int n = c.n_frames, chunk = chunk_frames(c.rows, c.cols, n, false);
+    const bool flagged = writes_flags(cc, true, false);
     const size_t fpix = (size_t)c.rows * c.cols;
     auto frames = [&](int f0, int32_t* flags) {
         return ChainFrames{c.points ? c.points + (size_t)f0 * c.cloud_stride * 4 : nullptr, c.counts ? c.counts + f0 : nullptr, c.cloud_stride,
@@ -1181,77 +1199,63 @@ int run_stereo_chain(StereoChain c, cudaStream_t st) {
                            c.depth + (size_t)f0 * fpix, c.disp ? c.disp + (size_t)f0 * fpix : nullptr,
                            c.stats ? c.stats + (size_t)f0 * DCMT_STATS_STRIDE : nullptr, flags};
     };
-    const size_t flag_bytes = flagged ? carve_bytes((size_t)n, sizeof(int32_t)) : 0;
     int32_t* d_flags = nullptr;
+    ChainWork w;
     for (int f0 = 0; f0 < n; f0 += chunk) {
-        const int nf = std::min(chunk, n - f0);
-        Arena* ar = nullptr;
-        if ((rc = arena_acquire(st, flag_bytes + chain_ws_bytes(cc, chunk, c.step), &ar))) return rc;  // stream order: the previous chunk is done with it
-        if (flagged) d_flags = carve<int32_t>(ar, (size_t)n);
-        if ((rc = enqueue_chain(c, cc, frames(f0, d_flags ? d_flags + f0 : nullptr), nf, ar, st))) return rc;
+        if ((rc = acquire_carved(st, [&](Arena* a) {  // stream order: the previous chunk is done with the arena
+                 d_flags = flagged ? carve<int32_t>(a, (size_t)n) : nullptr;
+                 w = carve_chain(a, c, cc, chunk);
+             })))
+            return rc;
+        if ((rc = enqueue_chain(c, cc, w, frames(f0, d_flags ? d_flags + f0 : nullptr), std::min(chunk, n - f0), st))) return rc;
     }
     if (!flagged) return DCMT_OK;
     int32_t* h_flags = nullptr;
     if ((rc = pinned_flags(st, (size_t)n, &h_flags))) return rc;
     API_CUDA(cudaMemcpyAsync(h_flags, d_flags, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st), "flag readback");
     API_CUDA(cudaStreamSynchronize(st), "kernel execution");
-    cc.flags = DCMT_PATH_GENERIC;
+    cc.flags = path_below(cc.flags);
     for (const Run& r : flagged_runs(h_flags, n)) {
         for (int f0 = r.f; f0 < r.e; f0 += chunk) {
-            Arena* ar = nullptr;
-            if ((rc = arena_acquire(st, chain_ws_bytes(cc, chunk, c.step), &ar))) return rc;
-            if ((rc = enqueue_chain(c, cc, frames(f0, nullptr), std::min(chunk, r.e - f0), ar, st))) return rc;
+            if ((rc = acquire_carved(st, [&](Arena* a) { w = carve_chain(a, c, cc, chunk); }))) return rc;
+            if ((rc = enqueue_chain(c, cc, w, frames(f0, nullptr), std::min(chunk, r.e - f0), st))) return rc;
         }
     }
     return DCMT_OK;
 }
 
-// Host-pointer driver of dcmt_stereo_chain_f32_host[_multi]: host chunks on the three streams of each device, as the completion's
-// host driver.  A chunk stages n_points[c] * 16 bytes of each cloud (max_points apart), the cloud sizes and both BGR frames
-// (packed), runs the chain into its arena and copies depth, disparity, stats and the dictionary's flags back.  Flagged frames
-// are redone, on the device that served them, with the completion on the generic pipeline.
+// Host-pointer driver of dcmt_stereo_chain_f32_host[_multi] on the host chunk pipeline.  A chunk stages n_points[c] * 16
+// bytes of each cloud (max_points apart), the cloud sizes and both BGR frames (packed), runs the chain into its arena and
+// copies depth, disparity, stats and the dictionary's flags back.
 int run_stereo_chain_host(StereoChain c, const int* devices = nullptr, int n_devices = 0, bool multi = false) {
     int rc = validate_stereo_chain(c, true);
     if (rc) return rc;
     if (c.n_frames == 0) return DCMT_OK;
     if (c.n_frames == 1) c.cloud_stride = c.max_points;  // one cloud: the ABI lets its stride be anything; staged clouds are max_points apart
-    HostCall call;
-    if ((rc = call.open(devices, n_devices, multi))) return rc;
-    call.split(c.n_frames);
     const int rows = c.rows, cols = c.cols;
     const size_t fpix = (size_t)rows * cols, bgr_row = (size_t)cols * 3, cloud_bytes = (size_t)c.max_points * 16;
     const CompletionCall cc = chain_completion(c);
-    const bool flagged = cc.flags == DCMT_PATH_RANK && fused_applies(cc);
-    int longest = 0;
-    for (Lane& l : call.lanes) longest = std::max(longest, l.f_end - l.f_begin);
-    const int hc = host_chunk_frames(rows, cols, longest);
-    for (Lane& l : call.lanes) {
-        if (l.f_end == l.f_begin) continue;
-        if ((rc = call.use(l))) return rc;
-        API_CUDA(dcmt::generic_configure(), "kernel attribute setup");
-        API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
-        if (flagged && (rc = pinned_flags(nullptr, (size_t)(l.f_end - l.f_begin), &l.h_flags))) return rc;
-    }
-    auto do_chunk = [&](Lane& l, int f0, int nf, const CompletionCall& c2, int hc2) -> int {
-        int rc2;
-        cudaStream_t st = l.hs->s[l.slot];
-        l.slot = (l.slot + 1) % kHostStreams;
-        const bool flags2 = flagged && c2.flags == DCMT_PATH_RANK;
-        const size_t px = fpix * hc2;
-        const size_t bytes = carve_bytes(cloud_bytes * hc2, 1) + carve_bytes((size_t)hc2, sizeof(int32_t)) + 2 * carve_bytes(bgr_row * rows * hc2, 1) +
-                             (c.disp ? 2 : 1) * carve_bytes(px, sizeof(float)) + carve_bytes((size_t)hc2 * DCMT_STATS_STRIDE, sizeof(int32_t)) +
-                             (flags2 ? carve_bytes((size_t)hc2, sizeof(int32_t)) : 0) + chain_ws_bytes(c2, hc2, c.step);
-        Arena* ar = nullptr;
-        if ((rc2 = arena_acquire(st, bytes, &ar))) return rc2;  // stream order protects reuse by the chunk 3 steps later
-        float* d_pts = carve<float>(ar, (size_t)c.max_points * 4 * hc2);
-        int32_t* d_counts = c.counts ? carve<int32_t>(ar, (size_t)hc2) : nullptr;
-        uint8_t* d_left = carve<uint8_t>(ar, bgr_row * rows * hc2);
-        uint8_t* d_right = carve<uint8_t>(ar, bgr_row * rows * hc2);
-        float* d_depth = carve<float>(ar, px);
-        float* d_disp = c.disp ? carve<float>(ar, px) : nullptr;
-        int32_t* d_stats = carve<int32_t>(ar, (size_t)hc2 * DCMT_STATS_STRIDE);
-        int32_t* d_flags = flags2 ? carve<int32_t>(ar, (size_t)hc2) : nullptr;
-        if ((rc2 = arena_ok(ar))) return rc2;
+    auto chunk = [&](Lane& l, cudaStream_t st, int f0, int nf, int hc, int level) -> int {
+        CompletionCall c2 = cc;
+        c2.flags = level;
+        const bool flags2 = writes_flags(c2, true, false);
+        const size_t px = fpix * hc;
+        float *d_pts, *d_depth, *d_disp;
+        int32_t *d_counts, *d_stats, *d_flags;
+        uint8_t *d_left, *d_right;
+        ChainWork w;
+        int rc2 = acquire_carved(st, [&](Arena* a) {
+            d_pts = carve<float>(a, (size_t)c.max_points * 4 * hc);
+            d_counts = c.counts ? carve<int32_t>(a, (size_t)hc) : nullptr;
+            d_left = carve<uint8_t>(a, bgr_row * rows * hc);
+            d_right = carve<uint8_t>(a, bgr_row * rows * hc);
+            d_depth = carve<float>(a, px);
+            d_disp = c.disp ? carve<float>(a, px) : nullptr;
+            d_stats = carve<int32_t>(a, (size_t)hc * DCMT_STATS_STRIDE);
+            d_flags = flags2 ? carve<int32_t>(a, (size_t)hc) : nullptr;
+            w = carve_chain(a, c, c2, hc);
+        });
+        if (rc2) return rc2;
         const float* h_pts = c.points ? c.points + (size_t)f0 * c.cloud_stride * 4 : nullptr;
         if (c.counts) {
             API_CUDA(cudaMemcpyAsync(d_counts, c.counts + f0, (size_t)nf * sizeof(int32_t), cudaMemcpyHostToDevice, st), "host to device copy");
@@ -1269,7 +1273,7 @@ int run_stereo_chain_host(StereoChain c, const int* devices = nullptr, int n_dev
             return rc2;
         const ChainFrames io{d_pts, d_counts, (size_t)c.max_points, d_left, d_right, bgr_row, bgr_row * rows, d_depth, d_disp,
                              c.stats ? d_stats : nullptr, d_flags};
-        if ((rc2 = enqueue_chain(c, c2, io, nf, ar, st))) return rc2;
+        if ((rc2 = enqueue_chain(c, c2, w, io, nf, st))) return rc2;
         if (flags2)
             API_CUDA(cudaMemcpyAsync(l.h_flags + (f0 - l.f_begin), d_flags, (size_t)nf * sizeof(int32_t), cudaMemcpyDeviceToHost, st), "flag readback");
         API_CUDA(cudaMemcpyAsync(c.depth + (size_t)f0 * fpix, d_depth, fpix * nf * sizeof(float), cudaMemcpyDeviceToHost, st), "device to host copy");
@@ -1281,23 +1285,7 @@ int run_stereo_chain_host(StereoChain c, const int* devices = nullptr, int n_dev
                      "device to host copy");
         return DCMT_OK;
     };
-    for (bool more = true; more;) {
-        more = false;
-        for (Lane& l : call.lanes) {
-            if (l.next >= l.f_end) continue;
-            more = true;
-            if ((rc = call.use(l))) return rc;
-            const int f0 = l.next, nf = std::min(hc, l.f_end - f0);
-            l.next += nf;
-            if ((rc = do_chunk(l, f0, nf, cc, hc))) return rc;
-        }
-    }
-    if ((rc = call.finish()) || !flagged) return rc;
-    CompletionCall cg = cc;
-    cg.flags = DCMT_PATH_GENERIC;
-    bool any = false;
-    if ((rc = redo_flagged(call, rows, cols, &any, [&](Lane& l, int f0, int nf, int hc2) { return do_chunk(l, f0, nf, cg, hc2); }))) return rc;
-    return any ? call.finish() : DCMT_OK;
+    return run_host_chunks(c.n_frames, rows, cols, devices, n_devices, multi, true, writes_flags(cc, true, false), cc.flags, chunk);
 }
 
 // ---- evaluation: one device driver and one host driver behind every dcmt_evaluate_* entry point.  Each side is an InDesc:
@@ -1335,11 +1323,8 @@ struct EvalReductions : EvalKind {
     int mode;
     EvalReductions(float tol, int m) : EvalKind(sizeof(dcmt_eval_result)), tolerance(tol), mode(m) {}
     int enqueue(const InDesc& gt, const InDesc& r, int rows, int cols, int n_frames, void* results, cudaStream_t st) const override {
-        Arena* ar = nullptr;
-        int rc = arena_acquire(st, carve_bytes(dcmt::eval_partial_doubles(n_frames), sizeof(double)), &ar);
-        if (rc) return rc;
-        double* partials = carve<double>(ar, dcmt::eval_partial_doubles(n_frames));
-        if ((rc = arena_ok(ar))) return rc;
+        double* partials = nullptr;
+        if (int rc = acquire_carved(st, [&](Arena* a) { partials = carve<double>(a, dcmt::eval_partial_doubles(n_frames)); })) return rc;
         dcmt::EvalResult* out = static_cast<dcmt::EvalResult*>(results);
         cudaError_t e;
         if (!gt.u)
@@ -1359,14 +1344,15 @@ struct EvalKitti : EvalKind {
     EvalKitti() : EvalKind(sizeof(dcmt_kitti_metrics)) {}
     int enqueue(const InDesc& gt, const InDesc& r, int rows, int cols, int n_frames, void* results, cudaStream_t st) const override {
         const size_t nd = dcmt::kitti_partial_doubles(n_frames), nw = dcmt::kitti_bits_words(rows, cols, n_frames);
-        Arena* ar = nullptr;
-        int rc = arena_acquire(st, carve_bytes(nd, sizeof(double)) + carve_bytes(2 * (size_t)n_frames, sizeof(int32_t)) +
-                                       carve_bytes(nw, sizeof(unsigned)), &ar);
-        if (rc) return rc;
-        double* partials = carve<double>(ar, nd);
-        int32_t* first_last = carve<int32_t>(ar, 2 * (size_t)n_frames);
-        unsigned* bits = nw ? carve<unsigned>(ar, nw) : nullptr;
-        if ((rc = arena_ok(ar))) return rc;
+        double* partials = nullptr;
+        int32_t* first_last = nullptr;
+        unsigned* bits = nullptr;
+        if (int rc = acquire_carved(st, [&](Arena* a) {
+                partials = carve<double>(a, nd);
+                first_last = carve<int32_t>(a, 2 * (size_t)n_frames);
+                bits = nw ? carve<unsigned>(a, nw) : nullptr;
+            }))
+            return rc;
         dcmt::KittiMetrics* out = static_cast<dcmt::KittiMetrics*>(results);
         cudaError_t e;
         if (!gt.u)
@@ -1469,7 +1455,10 @@ size_t dcmt_workspace_bytes(int rows, int cols, int n_frames) {
     if (rows < 1 || cols < 1 || n_frames < 1) return 0;
     // upper bound over the paths a call may take: fused chunks, bilateral scratch, the guided front and the dictionary
     const int chunk = chunk_frames(rows, cols, n_frames, true);
-    return generic_ws_bytes(rows, cols, chunk, true) + fused_ws_bytes(rows, cols, chunk, true, true);
+    Arena count;
+    count.counting = true;
+    carve_fused(&count, rows, cols, chunk, true, true, carve_generic(&count, rows, cols, chunk, true));
+    return count.used;
 }
 
 int dcmt_profile_begin(void) {
@@ -1798,15 +1787,10 @@ int dcmt_debug_q8_phase_cycles(const float* sparse, float* dense, int rows, int 
     API_CUDA(dcmt::q8_configure(), "kernel attribute setup");
     CompletionCall cc{nullptr, 0, false, rows, cols, DCMT_BLUR_GAUSSIAN, DCMT_PATH_AUTO};
     if (!fused_applies(cc)) return fail(DCMT_E_UNSUPPORTED, "shape not served by the fused kernels");
-    Arena* ar = nullptr;
     const size_t fpix = (size_t)rows * cols;
-    if ((rc = arena_acquire(st, generic_ws_bytes(rows, cols, n_frames, false) + fused_ws_bytes(rows, cols, n_frames, false, false), &ar)))
+    dcmt::Q8Plan p{};
+    if ((rc = acquire_carved(st, [&](Arena* a) { p = carve_fused(a, rows, cols, n_frames, false, false, carve_generic(a, rows, cols, n_frames, false)).p; })))
         return rc;
-    float* w1 = carve<float>(ar, fpix * n_frames);
-    float* w2 = carve<float>(ar, fpix * n_frames);
-    dcmt::FrameCounters* ctr = carve<dcmt::FrameCounters>(ar, n_frames);
-    dcmt::Q8Plan p = carve_fused(ar, rows, cols, n_frames, false, false, w1, w2, ctr).p;
-    if ((rc = arena_ok(ar))) return rc;
     p.prof_front = front_stamps;
     p.prof_tail = tail_stamps;
     if (tiles_per_frame) *tiles_per_frame = ((cols + p.tw - 1) / p.tw) * ((rows + p.th - 1) / p.th);
@@ -1839,10 +1823,10 @@ static int slic_device(const uint8_t* img, bool from_bgr, int rows, int cols, in
     if (n_frames == 0) return DCMT_OK;
     if ((rc = check_device())) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-    Arena* ar = nullptr;
-    if ((rc = arena_acquire(st, slic_ws_bytes(rows, cols, n_frames, step, from_bgr), &ar))) return rc;
+    SlicBuffers s;
+    if ((rc = acquire_carved(st, [&](Arena* a) { s = carve_slic(a, rows, cols, n_frames, step, from_bgr); }))) return rc;
     const size_t pitch = (size_t)cols * 3;
-    return enqueue_slic(img, pitch, pitch * rows, from_bgr, rows, cols, n_frames, step, nc, iterations, labels, centers, ar, st);
+    return enqueue_slic(s, img, pitch, pitch * rows, from_bgr, rows, cols, n_frames, step, nc, iterations, labels, centers, st);
 }
 
 int dcmt_slic_u8c3(const uint8_t* lab, int rows, int cols, int n_frames, int step, int nc, int iterations, int32_t* labels,
@@ -1864,11 +1848,11 @@ static int slic_host(const uint8_t* img, bool from_bgr, int rows, int cols, int 
     const size_t kb = (size_t)dcmt::slic_center_count(rows, cols, step) * n_frames * 5 * sizeof(double);
     Staged si{img, nullptr, n * 3, n * 3, 1}, sl{nullptr, labels, n * 4, n * 4, 1}, sc{nullptr, kb ? centers : nullptr, kb, kb, 1};
     return run_staged({&si, &sl, &sc}, [&](cudaStream_t st) {
-        Arena* ar = nullptr;
-        if (int rc2 = arena_acquire(st, slic_ws_bytes(rows, cols, n_frames, step, from_bgr), &ar)) return rc2;
+        SlicBuffers s;
+        if (int rc2 = acquire_carved(st, [&](Arena* a) { s = carve_slic(a, rows, cols, n_frames, step, from_bgr); })) return rc2;
         const size_t pitch = (size_t)cols * 3;
-        return enqueue_slic(static_cast<const uint8_t*>(si.dev), pitch, pitch * rows, from_bgr, rows, cols, n_frames, step, nc, iterations,
-                            static_cast<int32_t*>(sl.dev), centers ? static_cast<double*>(sc.dev) : nullptr, ar, st);
+        return enqueue_slic(s, static_cast<const uint8_t*>(si.dev), pitch, pitch * rows, from_bgr, rows, cols, n_frames, step, nc, iterations,
+                            static_cast<int32_t*>(sl.dev), centers ? static_cast<double*>(sc.dev) : nullptr, st);
     });
 }
 
@@ -1894,11 +1878,10 @@ static int check_project(const float* points, int n_points, const float* T_host,
 // the projection on validated arguments, 16-byte aligned points: its keys and counters in the stream's arena
 static int enqueue_project(const float* points, int n_points, const float* T_host, const float* P_host, int rows, int cols,
                            float* projected, float* normalized, float norm_a, float norm_b, int32_t* n_projected, cudaStream_t st) {
-    Arena* ar = nullptr;
-    int rc = arena_acquire(st, project_ws_bytes(rows, cols, 1), &ar);
-    if (rc) return rc;
-    return enqueue_project_batch(points, nullptr, n_points, 0, 1, T_host, P_host, rows, cols, projected, normalized, norm_a, norm_b, n_projected,
-                                 ar, st);
+    dcmt::ProjectWork w{};
+    if (int rc = acquire_carved(st, [&](Arena* a) { w = carve_project(a, rows, cols, 1); })) return rc;
+    return enqueue_project_batch(w, points, nullptr, n_points, 0, 1, T_host, P_host, rows, cols, projected, normalized, norm_a, norm_b, n_projected,
+                                 st);
 }
 
 int dcmt_lidar_project_f32(const float* points, int n_points, const float* T_host, const float* P_host, int rows, int cols,
@@ -1920,10 +1903,10 @@ int dcmt_lidar_project_batch_f32(const float* points, const int32_t* n_points_de
     if (n_clouds == 0) return DCMT_OK;
     if ((rc = check_device())) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-    Arena* ar = nullptr;
-    if ((rc = arena_acquire(st, project_ws_bytes(rows, cols, n_clouds), &ar))) return rc;
-    return enqueue_project_batch(points, n_points_dev_or_null, max_points, cloud_stride_points, n_clouds, T_host, P_host, rows, cols, projected,
-                                 normalized, norm_a, norm_b, n_projected, ar, st);
+    dcmt::ProjectWork w{};
+    if ((rc = acquire_carved(st, [&](Arena* a) { w = carve_project(a, rows, cols, n_clouds); }))) return rc;
+    return enqueue_project_batch(w, points, n_points_dev_or_null, max_points, cloud_stride_points, n_clouds, T_host, P_host, rows, cols, projected,
+                                 normalized, norm_a, norm_b, n_projected, st);
 }
 
 int dcmt_lidar_project_f32_host(const float* points, int n_points, const float* T_host, const float* P_host, int rows, int cols,
@@ -2086,27 +2069,19 @@ int dcmt_stereo_refine_f32_host(const float* depth_ig, const uint8_t* left_gray,
     int rc = check_stereo_refine(depth_ig, left_gray, right_gray, depth_out, rows, cols, n_frames, prm);
     if (rc) return rc;
     if (n_frames == 0) return DCMT_OK;
-    // chunks of frames flow H2D -> kernel -> D2H round-robin over the three host streams (asynchronous for page-locked buffers)
-    HostCall call;
-    if ((rc = call.open(nullptr, 0, false))) return rc;
-    HostStreams* hs = call.lanes[0].hs;
-    if ((rc = call.use(call.lanes[0]))) return rc;
+    // one device of the host chunk pipeline: H2D -> kernel -> D2H (asynchronous for page-locked buffers)
     const size_t fpix = (size_t)rows * cols;
-    const int hc = host_chunk_frames(rows, cols, n_frames);
-    const size_t bytes = 2 * carve_bytes(fpix * hc, sizeof(float)) + (disp_out ? carve_bytes(fpix * hc, sizeof(float)) : 0) +
-                         2 * carve_bytes(fpix * hc, sizeof(uint8_t));
-    int slot = 0;
-    for (int f0 = 0; f0 < n_frames; f0 += hc, slot = (slot + 1) % kHostStreams) {
-        const int nf = n_frames - f0 < hc ? n_frames - f0 : hc;
-        cudaStream_t st = hs->s[slot];
-        Arena* ar = nullptr;
-        if ((rc = arena_acquire(st, bytes, &ar))) return rc;
-        float* d_ig = carve<float>(ar, fpix * hc);
-        float* d_out = carve<float>(ar, fpix * hc);
-        float* d_disp = disp_out ? carve<float>(ar, fpix * hc) : nullptr;
-        uint8_t* d_l = carve<uint8_t>(ar, fpix * hc);
-        uint8_t* d_r = carve<uint8_t>(ar, fpix * hc);
-        if ((rc = arena_ok(ar))) return rc;
+    auto chunk = [&](Lane&, cudaStream_t st, int f0, int nf, int hc, int) -> int {
+        float *d_ig, *d_out, *d_disp;
+        uint8_t *d_l, *d_r;
+        int rc2 = acquire_carved(st, [&](Arena* a) {
+            d_ig = carve<float>(a, fpix * hc);
+            d_out = carve<float>(a, fpix * hc);
+            d_disp = disp_out ? carve<float>(a, fpix * hc) : nullptr;
+            d_l = carve<uint8_t>(a, fpix * hc);
+            d_r = carve<uint8_t>(a, fpix * hc);
+        });
+        if (rc2) return rc2;
         const size_t off = (size_t)f0 * fpix, n = fpix * nf;
         API_CUDA(cudaMemcpyAsync(d_ig, depth_ig + off, n * 4, cudaMemcpyHostToDevice, st), "host to device copy");
         API_CUDA(cudaMemcpyAsync(d_l, left_gray + off, n, cudaMemcpyHostToDevice, st), "host to device copy");
@@ -2116,8 +2091,9 @@ int dcmt_stereo_refine_f32_host(const float* depth_ig, const uint8_t* left_gray,
                  "stereo refine launch");
         API_CUDA(cudaMemcpyAsync(depth_out + off, d_out, n * 4, cudaMemcpyDeviceToHost, st), "device to host copy");
         if (disp_out) API_CUDA(cudaMemcpyAsync(disp_out + off, d_disp, n * 4, cudaMemcpyDeviceToHost, st), "device to host copy");
-    }
-    return call.finish();
+        return DCMT_OK;
+    };
+    return run_host_chunks(n_frames, rows, cols, nullptr, 0, false, false, false, DCMT_PATH_GENERIC, chunk);
 }
 
 int dcmt_stereo_chain_f32(const float* points, const int32_t* n_points_or_null, int max_points, size_t cloud_stride_points, const float* T_host,

@@ -258,6 +258,43 @@ def test_emu_device_entry_in_chunks(emu_lib):
     assert r.returncode == 0 and "CHUNKED_OK" in r.stdout, r.stdout + r.stderr
 
 
+_HOST_CHUNKED = r"""
+import sys; sys.path.insert(0, %(root)r)
+import numpy as np
+import torch
+from depth_completion_mt_b200 import _lib, api, synth
+from tests.conftest import assert_bit_equal
+from tests.test_stereo_chain_call import Scene, back_project, chain, gray, params, same, _Gpu
+lib = _lib.load()
+rows, cols = synth.KITTI_ROWS, synth.KITTI_COLS
+rng = np.random.default_rng(17)
+# 8 frames: host chunks of 3 + 3 + 2.  Frames 2-5 land on every pixel, beyond the dictionary: their redo on the generic
+# pipeline crosses the boundary of the first two chunks and runs in host chunks of 3 + 1.
+sc = Scene([back_project(rng, rows, cols, None if 2 <= f <= 5 else 3000) for f in range(8)], rows, cols, 17)
+ref = chain(lib, sc, "", step=65, be=_Gpu())
+assert [int(v) for v in ref[2][:, 3]] == [2, 2, 0, 0, 0, 0, 2, 2], ref[2][:, 3]
+for form in ("_host", "_host_multi"):
+    same(chain(lib, sc, form, step=65), ref, form)
+dig = rng.uniform(2.0, 60.0, (sc.n, rows, cols)).astype(np.float32)
+lg, rg = gray(sc.left), gray(sc.right)
+want = [t.cpu().numpy() for t in api.stereo_refine(*(torch.from_numpy(a).cuda() for a in (dig, lg, rg)), params(lib), return_disparity=True,
+                                                  lib=lib)]
+got = api.stereo_refine(dig, lg, rg, params(lib), return_disparity=True, lib=lib)
+assert_bit_equal(got[0], want[0], "stereo refinement host form: depth")
+assert_bit_equal(got[1], want[1], "stereo refinement host form: disparity")
+print("HOST_CHUNKED_OK")
+"""
+
+
+@pytest.mark.gpu
+def test_gpu_host_forms_in_chunks():
+    """the chain's host forms and the stereo refinement's in host chunks of 3 frames at 352 x 1216 (1 Mpx, read once per
+    process), with a run of dense frames redone on the generic pipeline across a chunk boundary: byte-equal to the device forms"""
+    env = dict(os.environ, DCMT_HOST_CHUNK_MPX="1")
+    r = subprocess.run([sys.executable, "-c", _HOST_CHUNKED % {"root": ROOT}], capture_output=True, text=True, timeout=1800, env=env, cwd=ROOT)
+    assert r.returncode == 0 and "HOST_CHUNKED_OK" in r.stdout, r.stdout + r.stderr
+
+
 # ---- argument errors ------------------------------------------------------------------------------------------------------
 # One argument of a valid call (2 frames of 8 x 8, 16 points a cloud) replaced at a time; "B" stands for a PROT_NONE mapping,
 # ["B", k] for k bytes into it, "PRM" for valid parameters, "PRM-1" for parameters with num_iterations -1.
